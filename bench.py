@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — guided-sampling frames/sec of the Climate2Weather hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 Workloads (config.workload), all on the ScoreUNet of configs/sda_unet.yml (random init), 4 x 128 x 128 frames, Markov
@@ -22,6 +22,8 @@ full 256-step sampling run, state resident in HBM, timed with CUDA events over e
 `e2e` = the same metric through the public API (SDAPipeline.sample) with pinned HOST noise in, HOST result out and
 the per-step NaN-flag read the reference does (src/thor/pipelines.py:90), all inside the timed region.
 `--impl reference` times the reference's CPU path (the oracle port, all host threads) on the same config.
+`--dump-outputs DIR` saves what the last timed step computed (see `dump_outputs`): the inputs are seeded, so two builds
+run with the same arguments can be compared array for array.
 """
 from __future__ import annotations
 
@@ -49,6 +51,7 @@ GAMMA = 0.0007196856730011522
 F_WIN_CONV = 115.134e9  # Conv2d FLOPs per window forward (SURVEY.md §8(d), BASELINE.md §2)
 F_WIN = 116.0e9
 FRAME_BYTES = C * H * W * 4
+DUMP_BYTES = 64_000_000  # --dump-outputs: all .npy files together, headers included
 ARCH = dict(channels=52, embedding_dim=512, hidden_channels=[128, 128, 256, 384, 512], hidden_blocks=[3, 3, 3, 3, 3],
             attention_levels=[4])
 
@@ -278,6 +281,29 @@ def hbm_kernel_rates(lib, rt, dev, peak_gbs):
     return out
 
 
+def dump_outputs(out_dir: str, st: Stepper, rank: int) -> None:
+    """Writes the state the last step left as float32 [frames, C, H, W] arrays: `x.npy`, the trajectory a caller of
+    SDAPipeline.sample receives, and `eps.npy`, the window score that step computed.  A time-sharded run gathers the
+    frames on rank 0, which writes them; in the ensemble, rank 0 writes its own member.  When the whole trajectory
+    would exceed DUMP_BYTES, both arrays hold every s-th frame (0, s, 2s, ...) for the smallest s that fits."""
+    import numpy as np
+
+    from climate2weather_b200.sharding import gather_frames
+
+    rt = st.rt
+    group = st.sf.shard[2] if st.sf.shard else None
+    arrays = {name: gather_frames(rt.owned(buf), rt.plan, group) for name, buf in (("x", rt.x), ("eps", rt.eps))}
+    if rank != 0:
+        return
+    n = arrays["x"].shape[0]
+    # 4 KB per file for the .npy header (128 B for these arrays)
+    fit = max(1, (DUMP_BYTES - 4096 * len(arrays)) // (len(arrays) * FRAME_BYTES))
+    stride = -(-n // min(n, fit))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a[::stride].cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -336,6 +362,8 @@ def run_ours(args):
         ms_total = st.timed(args.steps, args.warmup, barrier, clocks)
         launches = lib.c2w_launch_count() - launches0
     launches = launches * args.steps // (args.steps + args.warmup)  # the counter also saw the warm-up steps
+    if args.dump_outputs:  # before the roofline and e2e legs below step the same state further
+        dump_outputs(args.dump_outputs, st, rank)
     ms_step = allmax(ms_total) / args.steps
     frames_total = L * (MEMBERS if ensemble else 1)
     # ensemble: each GPU runs its members one after the other -> a GPU-step of the job costs members_per_gpu steps
@@ -709,19 +737,19 @@ def run_reference_train(args):
 
     for _ in range(args.warmup_train_ref):
         step()
-    steps = max(1, min(args.steps, args.ref_train_steps))
-    per = [step() for _ in range(steps)]
-    sec = sum(per) / steps
+    per = [step() for _ in range(args.steps)]
+    sec = sum(per) / args.steps
     value = b / sec
     line = {"impl": "reference", "metric": "DSM training samples/sec", "value": round(value, 4), "unit": "samples/s",
-            "n_gpus": args.gpus, "steps": steps, "warmup": args.warmup_train_ref, "ms_per_step": round(1e3 * sec, 1),
+            "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup_train_ref,
+            "ms_per_step": round(1e3 * sec, 1),
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": f"config5: DSM training step of the sda_unet.yml ScoreUNet on the host cores (oracle port, "
                                    f"torch autograd + torch.optim.AdamW), {b} samples of 52x128x128 per step",
                        "name": "config5", "batch_per_step": b},
             "cpu_baseline": {"value": round(value, 4), "unit": "samples/s", "cores": cores, "kind": "port",
-                             "sample": f"{steps} timed steps of {b} samples each (the configured batch is 128 per GPU; cost is "
-                                       "linear in the batch)"},
+                             "sample": f"{args.steps} timed steps of {b} samples each (the configured batch is 128 "
+                                       "per GPU; cost is linear in the batch)"},
             "e2e": {"value": round(value, 4), "unit": "samples/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "wall_s": round(time.perf_counter() - t_start, 1)}
     print(json.dumps(line), flush=True)
@@ -755,11 +783,16 @@ def main():
                     help="train: BASELINE config 5, the DSM training step (forward + backward + AdamW + EMA)")
     ap.add_argument("--batch", type=int, default=128, help="--mode train: samples per GPU (run_training.sh: 128)")
     ap.add_argument("--cpu-train-samples", type=int, default=2, help="--impl reference --mode train: samples per CPU step")
-    ap.add_argument("--ref-train-steps", type=int, default=3)
     ap.add_argument("--warmup-train-ref", type=int, default=1)
     ap.add_argument("--ddp", default="flat", choices=["flat", "torch"],
                     help="--mode train, N > 1: gradient averaging by one all-reduce of the flat buffer (default) or torch DDP")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, save the trajectory x and the score eps of the last step as "
+                         "DIR/x.npy, DIR/eps.npy (float32, at most 64 MB together: every s-th frame of a longer "
+                         "trajectory)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl, args.mode) != ("ours", "sample"):
+        ap.error("--dump-outputs saves the sampling state of --impl ours --mode sample")
     if args.e2e_steps is None:
         args.e2e_steps = 8 if args.config == 4 else SAMPLER_STEPS
     if args.impl == "reference" and args.mode == "train":

@@ -1055,3 +1055,39 @@ def test_sampler_proc_x0_hook(dev, golden_dir):
     want = same + float(pipe.mu(torch.tensor(0.0))) * (x0_last.clamp(-0.5, 0.5) - x0_last)
     assert not torch.equal(clamped, same)
     assert rel_l2(clamped, want) < 1e-5
+
+
+def test_bench_dump_outputs_hold_the_state_after_exactly_steps_steps(tmp_path):
+    """bench.py --steps K --dump-outputs DIR on a short trajectory: x.npy and eps.npy are the state after exactly K
+    timed steps and the window score of the K-th.  K = 1 is replayed from the seeded noise by the oracle predictor with
+    closed-form guidance on the dumped eps (fp32 elementwise, 1e-5); K = 2 replays its second step from K = 1's x,
+    whose window score came from another process (bf16 tolerance, 1e-3: a missing or extra step moves x by ~10 % of
+    its scale)."""
+    import json
+    import subprocess
+    import sys
+
+    import bench
+
+    L = 20
+    _, noise, y, _ = bench.make_problem(L, with_net=False)
+    std = torch.tensor(bench.STD).reshape(1, 4, 1, 1)
+    times = torch.linspace(1, 0, bench.SAMPLER_STEPS + 1)
+    pipe = pipeline_ref.RefPipeline()
+    x = noise
+    for k in (1, 2):
+        out = tmp_path / f"steps{k}"
+        r = subprocess.run([sys.executable, str(bench.ROOT / "bench.py"), "--frames", str(L), "--steps", str(k),
+                            "--warmup", "0", "--no-cpu", "--no-e2e", "--dump-outputs", str(out)],
+                           capture_output=True, text=True, timeout=900, cwd=str(bench.ROOT))
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == k
+        got, eps = (torch.from_numpy(np.load(out / f"{n}.npy")) for n in ("x", "eps"))
+        assert got.shape == eps.shape == (L, 4, 128, 128)
+
+        def guided(xx, tt, eps=eps):
+            return score_ref.guided_score_closed_form(eps, xx, tt, y, std, bench.GAMMA, bench.T_STEP, bench.S_STEP)
+
+        want = pipe.predictor(guided, x, times[k - 1], 1 / bench.SAMPLER_STEPS)
+        assert relerr(got, want) < (1e-5 if k == 1 else 1e-3), (k, relerr(got, want))
+        x = got

@@ -321,6 +321,29 @@ def test_bench_workload_selection():
     assert bench.pick_workload(A, 4) == ("config2-weak", 12 + 4 * 156, "weak", 0)
 
 
+def test_bench_dump_outputs_keep_every_frame_or_a_fixed_stride_within_64_mb(tmp_path):
+    """bench.py --dump-outputs: x and eps of every frame when both files fit 64 MB together, headers included (122
+    frames do, 123 do not), otherwise the same every-s-th frames of both for the smallest s that fits; only rank 0
+    writes."""
+    import types
+
+    sys.path.insert(0, str(ROOT))
+    import bench
+
+    for L, stride in ((20, 1), (122, 1), (123, 2), (200, 2)):
+        x = torch.arange(L * bench.FRAME_BYTES // 4, dtype=torch.float32).reshape(L, bench.C, bench.H, bench.W)
+        rt = types.SimpleNamespace(x=x, eps=-x, plan=sharding.make_plan(L, bench.K_ORDER, 0, 1), owned=lambda buf: buf)
+        st = types.SimpleNamespace(rt=rt, sf=types.SimpleNamespace(shard=None))
+        bench.dump_outputs(str(tmp_path / "rank1"), st, rank=1)
+        assert not (tmp_path / "rank1").exists()
+        out = tmp_path / str(L)
+        bench.dump_outputs(str(out), st, rank=0)
+        got = {n: np.load(out / f"{n}.npy") for n in ("x", "eps")}
+        assert sum((out / f"{n}.npy").stat().st_size for n in got) <= bench.DUMP_BYTES
+        assert got["x"].dtype == np.float32 and np.array_equal(got["x"], x[::stride].numpy()), L
+        assert np.array_equal(got["eps"], -got["x"])
+
+
 def test_bench_reference_arm_prints_the_contract_line():
     """`bench.py --impl reference` (the CPU arm the driver runs beside ours): one JSON line with the same metric, unit,
     direction and workload part of `config` as our arm, `impl: reference`, a `cpu_baseline` describing the run, an `e2e`
@@ -344,6 +367,19 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert cb["kind"] == "port" and cb["cores"] >= 1 and cb["value"] == line["value"] and "13 of the 156 windows" in cb["sample"]
     assert line["e2e"] == {"value": line["value"], "unit": "frames/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert line["value"] > 0 and line["ms_per_step"] > 0
+
+
+def test_bench_reference_training_arm_times_exactly_the_steps_asked_for():
+    """`bench.py --impl reference --mode train --steps K` times K steps, not fewer (one sample per step here)."""
+    import json
+    import subprocess
+
+    r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--mode", "train",
+                        "--steps", "4", "--cpu-train-samples", "1", "--warmup-train-ref", "0"],
+                       capture_output=True, text=True, timeout=600, cwd=str(ROOT))
+    assert r.returncode == 0, r.stderr[-2000:]
+    line = json.loads(r.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 4 and line["cpu_baseline"]["sample"].startswith("4 timed steps of 1 samples")
 
 
 @pytest.mark.parametrize("L,k,t_step", [(13, 6, 6), (14, 6, 6), (25, 6, 6), (168, 6, 6), (40, 2, 3), (31, 3, 4), (720, 6, 6),

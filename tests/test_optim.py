@@ -1,12 +1,13 @@
 """N2, optimiser half (SURVEY.md §8(f)): `optimizer.step()` + `ema.update()` of training_loop.py:381-390 as one fused
 pass (`c2w_adamw_ema_step`, climate2weather_b200/optim.py).
 
-CPU: the oracle (oracle/optim_ref.py) is pinned against torch.optim.AdamW itself and, where the reference checkout is
-present, against the reference's own thor/ema.py.  GPU (`-m gpu`): the fused kernel against the oracle over several
-steps with a changing learning rate, gradients set directly and through autograd, and its HBM rate at the reference
-model's 72.1 M parameters.
+CPU: the oracle (oracle/optim_ref.py) is pinned against torch.optim.AdamW itself and, where C2W_REFERENCE names a
+checkout of the reference, against the reference's own thor/ema.py.  GPU (`-m gpu`): the fused kernel against the
+oracle over several steps with a changing learning rate, gradients set directly and through autograd, and its HBM rate
+at the reference model's 72.1 M parameters.
 """
 import importlib.util
+import os
 import pathlib
 
 import pytest
@@ -14,7 +15,8 @@ import torch
 
 from oracle import optim_ref
 
-REF_EMA = pathlib.Path("/root/reference/src/thor/ema.py")
+REF = os.environ.get("C2W_REFERENCE")  # a checkout of schmidtjonathan/Climate2Weather
+REF_EMA = pathlib.Path(REF, "src/thor/ema.py") if REF else None
 HP = dict(lr=3e-4, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-3)  # train.py:176-181
 
 
@@ -49,7 +51,30 @@ def test_oracle_matches_torch_adamw():
             assert torch.allclose(p.detach(), q, rtol=1e-12, atol=1e-14)
 
 
-@pytest.mark.skipif(not REF_EMA.exists(), reason="reference checkout not present")
+def test_oracle_ema_matches_torch_ema():
+    """The oracle's EMA over 5 compounding AdamW steps, element for element, against torch's own EMA
+    (torch.optim.swa_utils.get_ema_multi_avg_fn): W_0 = the initial weights, W_t+1 = rate W_t + (1 - rate) p_t+1, the
+    rule the oracle restates from the reference's StandardEMA (ema.py:14,24-27)."""
+    from torch.optim.swa_utils import get_ema_multi_avg_fn
+
+    net = _tiny_net().double()
+    params = list(net.parameters())
+    ema = [p.detach().clone() for p in params]
+    ema_update = get_ema_multi_avg_fn(0.99)
+    ref = optim_ref.AdamWEMARef(params, ema_rate=0.99, **HP)
+    opt = torch.optim.AdamW(params, **HP)
+    for step in range(5):
+        grads = _grads(params, step)
+        for p, g in zip(params, grads):
+            p.grad = g.clone()
+        opt.step()
+        ema_update(ema, [p.detach() for p in params], step)
+        ref.step(grads)
+    for p, q in zip(ema, ref.ema):
+        assert torch.allclose(p, q, rtol=1e-12, atol=1e-14)
+
+
+@pytest.mark.skipif(REF_EMA is None or not REF_EMA.exists(), reason="C2W_REFERENCE does not name a reference checkout")
 def test_oracle_ema_matches_reference_ema():
     spec = importlib.util.spec_from_file_location("_ref_ema", REF_EMA)
     mod = importlib.util.module_from_spec(spec)

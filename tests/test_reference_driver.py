@@ -13,10 +13,12 @@ with its keywords, conditions it on its own `select_spatiotemporal` closure with
 `SDAPipeline.sample` — is intercepted here and its arguments checked (operator recognition included); the same flow
 with the real CUDA sampler is `tests/test_gpu_parity.py::test_driver_flow_snapshot_to_guided_sampling`.
 
-Skipped where the reference checkout is absent (the GPU box).
+Runs where the environment variable C2W_REFERENCE names a checkout of schmidtjonathan/Climate2Weather; skipped
+elsewhere.
 """
 import contextlib
 import importlib.util
+import os
 import pathlib
 import sys
 import types
@@ -26,9 +28,11 @@ import pytest
 import torch
 
 ROOT = pathlib.Path(__file__).resolve().parents[1]
-REF_DRIVER = pathlib.Path("/root/reference/exp/downscaling.py")
+REF = os.environ.get("C2W_REFERENCE")
+REF_DRIVER = pathlib.Path(REF, "exp/downscaling.py") if REF else None
 
-pytestmark = pytest.mark.skipif(not REF_DRIVER.exists(), reason="reference checkout not present")
+pytestmark = pytest.mark.skipif(REF_DRIVER is None or not REF_DRIVER.exists(),
+                                reason="C2W_REFERENCE does not name a reference checkout")
 
 
 class FakeDS:
