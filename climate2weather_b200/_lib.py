@@ -68,6 +68,12 @@ class Guide(C.Structure):
     ]
 
 
+class PointObs(C.Structure):
+    """include/c2w_b200.h: c2w_point_obs"""
+    _fields_ = [("frame_slot", C.c_void_p), ("strip_off", C.c_void_p), ("pix", C.c_void_p), ("ysum", C.c_void_p),
+                ("wsum", C.c_void_p), ("n_slots", C.c_int32), ("strip_rows", C.c_int32)]
+
+
 class ConvDesc(C.Structure):
     _fields_ = [
         ("x", C.c_void_p),
@@ -123,6 +129,7 @@ SIGNATURES = {
     "c2w_normalize_pack": (_i, [_vp, _vp, _i64, C.c_int32, C.c_int32, C.c_int32, _vp, _vp, C.c_int32, _vp]),
     "c2w_unpack_unnormalize": (_i, [_vp, _vp, _i64, C.c_int32, C.c_int32, C.c_int32, _vp, _vp, C.c_int32, _vp]),
     "c2w_guided_step": (_i, [C.POINTER(Guide), _vp]),
+    "c2w_guided_step_points": (_i, [C.POINTER(Guide), C.POINTER(PointObs), _vp]),
     "c2w_reduce_partials": (_i, [_vp, C.c_int32, _vp, _vp]),
     "c2w_corrector_update": (_i, [_vp, _vp, _vp, _vp, _d, _f, _f, _i64, _i64, C.c_uint64, C.c_uint32, _vp, _vp]),
     "c2w_corrector_update_c": (_i, [_vp, _vp, _vp, _vp, _d, _f, _f, _i64, _i64, C.c_int32, C.c_uint64, C.c_uint32, _vp,

@@ -63,7 +63,8 @@ def install(force: bool = False) -> None:
     thor = mod("thor")
     thor.score = mod("thor.score", AbstractScoreFunction=_score.AbstractScoreFunction,
                      DefaultScoreFunction=_score.DefaultScoreFunction,
-                     BatchedScoreFunction=_score.BatchedScoreFunction, CoarseGrain=_score.CoarseGrain)
+                     BatchedScoreFunction=_score.BatchedScoreFunction, CoarseGrain=_score.CoarseGrain,
+                     PointObservation=_score.PointObservation)
     thor.pipelines = mod("thor.pipelines", SDAPipeline=_pipelines.SDAPipeline)
     m = mod("model")
     m.score = mod("model.score", ScoreUNet=_model.ScoreUNet)

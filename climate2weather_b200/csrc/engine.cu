@@ -1058,7 +1058,7 @@ int run_plan(c2w_handle* h, int nn, const FinalSpec& fs, cudaStream_t st) { retu
 
 extern "C" {
 
-int c2w_abi_version(void) { return 2; }
+int c2w_abi_version(void) { return 3; }
 
 int c2w_struct_size(int which) {
   switch (which) {
@@ -1066,6 +1066,7 @@ int c2w_struct_size(int which) {
     case 1: return static_cast<int>(sizeof(c2w_guide));
     case 2: return static_cast<int>(sizeof(c2w_adamw));
     case 3: return static_cast<int>(sizeof(c2w_conv_desc));
+    case 4: return static_cast<int>(sizeof(c2w_point_obs));
     default: return -1;
   }
 }
@@ -1881,17 +1882,14 @@ int c2w_adamw_ema_step(float* p, const float* g, float* m, float* v, float* ema,
   return C2W_OK;
 }
 
-int c2w_guided_step(const c2w_guide* g, void* stream) {
-  C2W_REQUIRE(g && g->x && g->eps && g->nan_flag, "c2w_guided_step: bad argument");
-  C2W_REQUIRE(g->s_step >= 1 && g->H % g->s_step == 0 && g->W % g->s_step == 0 && g->W / g->s_step <= 32,
-              "s_step=%d must divide %dx%d with at most 32 tiles per row", g->s_step, g->H, g->W);
+// GuideParams from a c2w_guide: the checks and fields both guidance entry points share (`what` names the caller).
+static int guide_params(const c2w_guide* g, const char* what, GuideParams& p) {
+  C2W_REQUIRE(g && g->x && g->eps && g->nan_flag, "%s: bad argument", what);
   C2W_REQUIRE(g->mode != 1 || (g->eps_out && g->partials), "mode 1 needs eps_out and partials");
-  C2W_REQUIRE(g->mode != 2 || (g->cot_out && g->y), "mode 2 needs cot_out and an observation");
-  C2W_REQUIRE(g->own_n >= 1 && g->t_step >= 1, "own_n and t_step must be positive");
+  C2W_REQUIRE(g->own_n >= 1, "own_n must be positive");
   const int C = g->channels == 0 ? 4 : g->channels;
-  C2W_REQUIRE(C >= 1 && C <= C2W_MAX_VARS, "c2w_guided_step: 1 to %d variables per frame (got %d)", C2W_MAX_VARS, C);
-  C2W_REQUIRE(C == 4 || g->halo == nullptr, "c2w_guided_step: the fused halo push handles 4 variables per frame");
-  GuideParams p;
+  C2W_REQUIRE(C >= 1 && C <= C2W_MAX_VARS, "%s: 1 to %d variables per frame (got %d)", what, C2W_MAX_VARS, C);
+  C2W_REQUIRE(C == 4 || g->halo == nullptr, "%s: the fused halo push handles 4 variables per frame", what);
   p.x = g->x;
   p.eps = g->eps;
   p.eps_out = g->eps_out;
@@ -1922,7 +1920,7 @@ int c2w_guided_step(const c2w_guide* g, void* stream) {
   p.halo_k = g->halo_k;
   p.own_n = g->own_n;
   if (g->halo != nullptr && g->mode == 0) {  // fused halo push (csrc/halo.cu)
-    C2W_REQUIRE(g->halo_k >= 1 && g->own_n >= g->halo_k, "c2w_guided_step: fused halo push needs 1 <= halo_k <= own_n");
+    C2W_REQUIRE(g->halo_k >= 1 && g->own_n >= g->halo_k, "%s: fused halo push needs 1 <= halo_k <= own_n", what);
     void *sl, *sr, *fl, *fr, *dn;
     uint32_t pub;
     int rc = c2w_halo_push_targets(static_cast<c2w_halo*>(g->halo), &sl, &sr, &fl, &fr, &dn, &pub);
@@ -1934,9 +1932,46 @@ int c2w_guided_step(const c2w_guide* g, void* stream) {
     p.push_done = (sl || sr) ? static_cast<unsigned int*>(dn) : nullptr;
     p.publish = pub;
   }
+  return C2W_OK;
+}
+
+int c2w_guided_step(const c2w_guide* g, void* stream) {
+  C2W_REQUIRE(g, "c2w_guided_step: bad argument");
+  C2W_REQUIRE(g->s_step >= 1 && g->H % g->s_step == 0 && g->W % g->s_step == 0 && g->W / g->s_step <= 32,
+              "s_step=%d must divide %dx%d with at most 32 tiles per row", g->s_step, g->H, g->W);
+  C2W_REQUIRE(g->mode != 2 || (g->cot_out && g->y), "mode 2 needs cot_out and an observation");
+  C2W_REQUIRE(g->t_step >= 1, "own_n and t_step must be positive");
+  GuideParams p;
+  int rc = guide_params(g, "c2w_guided_step", p);
+  if (rc) return rc;
   dim3 grid(g->H / g->s_step, g->own_n);
-  if (C == 4) guided_step_kernel<<<grid, 32 * (g->W / g->s_step), 0, static_cast<cudaStream_t>(stream)>>>(p);
+  if (p.C == 4) guided_step_kernel<<<grid, 32 * (g->W / g->s_step), 0, static_cast<cudaStream_t>(stream)>>>(p);
   else guided_step_generic_kernel<<<grid, 32 * (g->W / g->s_step), 0, static_cast<cudaStream_t>(stream)>>>(p);
+  ++g_launches;
+  C2W_CUDA(cudaGetLastError());
+  return C2W_OK;
+}
+
+int c2w_guided_step_points(const c2w_guide* g, const c2w_point_obs* obs, void* stream) {
+  C2W_REQUIRE(g && obs && obs->frame_slot && obs->strip_off, "c2w_guided_step_points: bad argument");
+  C2W_REQUIRE(obs->n_slots == 0 || (obs->pix && obs->ysum && obs->wsum), "c2w_guided_step_points: entries missing");
+  C2W_REQUIRE(g->H >= 1 && g->W >= 1 && obs->strip_rows >= 1 && obs->strip_rows * g->W <= C2W_POINT_STRIP_PIX,
+              "c2w_guided_step_points: strip of %d rows of %d pixels exceeds %d pixels", obs->strip_rows, g->W,
+              C2W_POINT_STRIP_PIX);
+  C2W_REQUIRE(g->mode != 2 || g->cot_out, "mode 2 needs cot_out");
+  GuideParams p;
+  int rc = guide_params(g, "c2w_guided_step_points", p);
+  if (rc) return rc;
+  PointParams q;
+  q.frame_slot = obs->frame_slot;
+  q.strip_off = obs->strip_off;
+  q.pix = obs->pix;
+  q.ysum = obs->ysum;
+  q.wsum = obs->wsum;
+  q.strip_rows = obs->strip_rows;
+  dim3 grid((g->H + obs->strip_rows - 1) / obs->strip_rows, g->own_n);
+  if (p.C == 4) guided_points_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(p, q);
+  else guided_points_generic_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(p, q);
   ++g_launches;
   C2W_CUDA(cudaGetLastError());
   return C2W_OK;

@@ -1584,6 +1584,146 @@ struct GuideParams {
   int halo_k, own_n;
 };
 
+// mode 1: the CTA's sum of eps_guided^2 -> partials[blockIdx.y * gridDim.x + blockIdx.x] (fixed order, no atomics)
+__device__ __forceinline__ void block_partial(const GuideParams& p, float sq) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  __shared__ float wsum[32];
+  sq = warp_sum(sq);
+  if (lane == 0) wsum[warp] = sq;
+  __syncthreads();
+  if (warp == 0) {
+    float v = (lane < (blockDim.x >> 5)) ? wsum[lane] : 0.f;
+    v = warp_sum(v);
+    if (lane == 0) p.partials[blockIdx.y * gridDim.x + blockIdx.x] = v;
+  }
+}
+
+// The dense tail of the guidance pass, shared by K6 (coarse-grained observations) and K6p (point observations).  Per
+// pixel: grad_x log p = (g - sigma J_eps^T g) / mu  (src/thor/score.py:48-60; the second term only with exact_grad);
+// eps_guided = eps - sigma * grad  =>  per-pixel correction sigma (g - sigma vjp) / mu.  Mode 0 then updates x in place
+// (and stores the boundary frames into the neighbours' halo mailboxes), mode 1 writes eps_guided and the CTA's partial
+// sum of its squares.  The observation policy `Obs` walks this thread's pixels (first / end / step, pixel(i) = index
+// within the frame) and gives the likelihood cotangent g of pixel i: g4 for float4 pixels, entry + g for scalar lanes.
+template <class Obs>
+__device__ __forceinline__ void guide_tail4(const GuideParams& p, const Obs& obs, long long fbase) {
+  const int lane = threadIdx.x & 31;
+  const float inv_mu = 1.0f / p.mu;
+  const float sg_mu = p.sigma * inv_mu;
+  float sq = 0.f;
+  bool bad = false;
+  for (int i = obs.first(); i < obs.end(); i += obs.step()) {
+    const long long pix_in_frame = obs.pixel(i);
+    const long long o = (fbase + pix_in_frame) * 4;
+    float4 ev = *reinterpret_cast<const float4*>(p.eps + o);
+    float4 gv = obs.g4(p, i, o, ev);
+    if (p.vjp != nullptr) {
+      const float4 jv = *reinterpret_cast<const float4*>(p.vjp + o);
+      gv.x -= p.sigma * jv.x;
+      gv.y -= p.sigma * jv.y;
+      gv.z -= p.sigma * jv.z;
+      gv.w -= p.sigma * jv.w;
+    }
+    ev.x -= sg_mu * gv.x;
+    ev.y -= sg_mu * gv.y;
+    ev.z -= sg_mu * gv.z;
+    ev.w -= sg_mu * gv.w;
+    if (p.mode == 0) {
+      float4 xv = *reinterpret_cast<const float4*>(p.x + o);
+      // x0 = (x - sigma eps)/mu ; x <- mu' x0 + sigma' eps     (src/thor/pipelines.py:41-46)
+      xv.x = p.mu_next * ((xv.x - p.sigma * ev.x) * inv_mu) + p.sigma_next * ev.x;
+      xv.y = p.mu_next * ((xv.y - p.sigma * ev.y) * inv_mu) + p.sigma_next * ev.y;
+      xv.z = p.mu_next * ((xv.z - p.sigma * ev.z) * inv_mu) + p.sigma_next * ev.z;
+      xv.w = p.mu_next * ((xv.w - p.sigma * ev.w) * inv_mu) + p.sigma_next * ev.w;
+      bad |= !(isfinite(xv.x) && isfinite(xv.y) && isfinite(xv.z) && isfinite(xv.w));
+      *reinterpret_cast<float4*>(p.x + o) = xv;
+      // boundary frames also go straight into the neighbours' halo mailboxes (peer stores through NVLink)
+      const long long hw = static_cast<long long>(p.H) * p.W;
+      const int own_idx = static_cast<int>(blockIdx.y);
+      if (p.push_l != nullptr && own_idx < p.halo_k) p.push_l[own_idx * hw + pix_in_frame] = xv;
+      if (p.push_r != nullptr && own_idx >= p.own_n - p.halo_k)
+        p.push_r[(own_idx - (p.own_n - p.halo_k)) * hw + pix_in_frame] = xv;
+    } else {
+      sq += ev.x * ev.x + ev.y * ev.y + ev.z * ev.z + ev.w * ev.w;
+      *reinterpret_cast<float4*>(p.eps_out + o) = ev;
+    }
+  }
+  if (p.mode == 0) {
+    if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(p.nan_flag, 1);
+    if (p.push_done != nullptr) {  // fused halo push: fence this CTA's peer stores, the last CTA publishes the step
+      __threadfence_system();
+      __syncthreads();
+      if (threadIdx.x == 0) {
+        const unsigned int total = gridDim.x * gridDim.y;
+        if (atomicAdd(p.push_done, 1u) == total - 1) {
+          *p.push_done = 0;
+          __threadfence_system();
+          if (p.flag_l) asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p.flag_l), "r"(p.publish) : "memory");
+          if (p.flag_r) asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p.flag_r), "r"(p.publish) : "memory");
+        }
+      }
+    }
+  } else {
+    block_partial(p, sq);
+  }
+}
+
+template <class Obs>
+__device__ __forceinline__ void guide_tail_generic(const GuideParams& p, const Obs& obs, long long fbase) {
+  constexpr int MC = 8;
+  const int C = p.C;
+  const int lane = threadIdx.x & 31;
+  const float inv_mu = 1.0f / p.mu;
+  const float sg_mu = p.sigma * inv_mu;
+  float sq = 0.f;
+  bool bad = false;
+  for (int i = obs.first(); i < obs.end(); i += obs.step()) {
+    const long long o = (fbase + obs.pixel(i)) * C;
+    const int e = obs.entry(i);
+#pragma unroll
+    for (int c = 0; c < MC; ++c) {
+      if (c < C) {
+        float gv = obs.g(p, e, o, c);
+        if (p.vjp != nullptr) gv -= p.sigma * p.vjp[o + c];
+        const float ev = p.eps[o + c] - sg_mu * gv;
+        if (p.mode == 0) {
+          const float xv = p.mu_next * ((p.x[o + c] - p.sigma * ev) * inv_mu) + p.sigma_next * ev;
+          bad |= !isfinite(xv);
+          p.x[o + c] = xv;
+        } else {
+          sq += ev * ev;
+          p.eps_out[o + c] = ev;
+        }
+      }
+    }
+  }
+  if (p.mode == 0) {
+    if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(p.nan_flag, 1);
+  } else {
+    block_partial(p, sq);
+  }
+}
+
+// K6's observation policy: the warp's s x s tile, whose pixels all get the same cotangent (the tile's residual / s^2).
+struct TileObs4 {
+  int s, h0, w0, W;
+  float4 corr;
+  __device__ int first() const { return threadIdx.x & 31; }
+  __device__ int end() const { return s * s; }
+  __device__ int step() const { return 32; }
+  __device__ long long pixel(int i) const { return static_cast<long long>(h0 + i / s) * W + (w0 + i % s); }
+  __device__ float4 g4(const GuideParams&, int, long long, float4) const { return corr; }
+};
+struct TileObsC {
+  int s, h0, w0, W;
+  float corr[8];
+  __device__ int first() const { return threadIdx.x & 31; }
+  __device__ int end() const { return s * s; }
+  __device__ int step() const { return 32; }
+  __device__ long long pixel(int i) const { return static_cast<long long>(h0 + i / s) * W + (w0 + i % s); }
+  __device__ int entry(int) const { return 0; }
+  __device__ float g(const GuideParams&, int, long long, int c) const { return corr[c]; }
+};
+
 // CTA = one s-row strip of one frame; one warp per s x s observation tile (warp-shuffle tile mean, deterministic).
 __global__ void guided_step_kernel(const GuideParams p) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -1630,73 +1770,7 @@ __global__ void guided_step_kernel(const GuideParams p) {
     }
     return;
   }
-  // grad_x log p = (g - sigma J_eps^T g) / mu  (src/thor/score.py:48-60; the second term only with exact_grad);
-  // eps_guided = eps - sigma * grad  =>  per-pixel correction sigma (g - sigma vjp) / mu
-  const float sg_mu = p.sigma * inv_mu;
-  float sq = 0.f;
-  bool bad = false;
-  for (int i = lane; i < s * s; i += 32) {
-    const long long o = (fbase + static_cast<long long>(h0 + i / s) * p.W + (w0 + i % s)) * 4;
-    float4 ev = *reinterpret_cast<const float4*>(p.eps + o);
-    float4 gv = corr;
-    if (p.vjp != nullptr) {
-      const float4 jv = *reinterpret_cast<const float4*>(p.vjp + o);
-      gv.x -= p.sigma * jv.x;
-      gv.y -= p.sigma * jv.y;
-      gv.z -= p.sigma * jv.z;
-      gv.w -= p.sigma * jv.w;
-    }
-    ev.x -= sg_mu * gv.x;
-    ev.y -= sg_mu * gv.y;
-    ev.z -= sg_mu * gv.z;
-    ev.w -= sg_mu * gv.w;
-    if (p.mode == 0) {
-      float4 xv = *reinterpret_cast<const float4*>(p.x + o);
-      // x0 = (x - sigma eps)/mu ; x <- mu' x0 + sigma' eps     (src/thor/pipelines.py:41-46)
-      xv.x = p.mu_next * ((xv.x - p.sigma * ev.x) * inv_mu) + p.sigma_next * ev.x;
-      xv.y = p.mu_next * ((xv.y - p.sigma * ev.y) * inv_mu) + p.sigma_next * ev.y;
-      xv.z = p.mu_next * ((xv.z - p.sigma * ev.z) * inv_mu) + p.sigma_next * ev.z;
-      xv.w = p.mu_next * ((xv.w - p.sigma * ev.w) * inv_mu) + p.sigma_next * ev.w;
-      bad |= !(isfinite(xv.x) && isfinite(xv.y) && isfinite(xv.z) && isfinite(xv.w));
-      *reinterpret_cast<float4*>(p.x + o) = xv;
-      // boundary frames also go straight into the neighbours' halo mailboxes (peer stores through NVLink)
-      const long long pix_in_frame = static_cast<long long>(h0 + i / s) * p.W + (w0 + i % s);
-      const long long hw = static_cast<long long>(p.H) * p.W;
-      const int own_idx = static_cast<int>(blockIdx.y);
-      if (p.push_l != nullptr && own_idx < p.halo_k) p.push_l[own_idx * hw + pix_in_frame] = xv;
-      if (p.push_r != nullptr && own_idx >= p.own_n - p.halo_k)
-        p.push_r[(own_idx - (p.own_n - p.halo_k)) * hw + pix_in_frame] = xv;
-    } else {
-      sq += ev.x * ev.x + ev.y * ev.y + ev.z * ev.z + ev.w * ev.w;
-      *reinterpret_cast<float4*>(p.eps_out + o) = ev;
-    }
-  }
-  if (p.mode == 0) {
-    if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(p.nan_flag, 1);
-    if (p.push_done != nullptr) {  // fused halo push: fence this CTA's peer stores, the last CTA publishes the step
-      __threadfence_system();
-      __syncthreads();
-      if (threadIdx.x == 0) {
-        const unsigned int total = gridDim.x * gridDim.y;
-        if (atomicAdd(p.push_done, 1u) == total - 1) {
-          *p.push_done = 0;
-          __threadfence_system();
-          if (p.flag_l) asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p.flag_l), "r"(p.publish) : "memory");
-          if (p.flag_r) asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p.flag_r), "r"(p.publish) : "memory");
-        }
-      }
-    }
-  } else {
-    __shared__ float wsum[32];
-    sq = warp_sum(sq);
-    if (lane == 0) wsum[warp] = sq;
-    __syncthreads();
-    if (warp == 0) {
-      float v = (lane < (blockDim.x >> 5)) ? wsum[lane] : 0.f;
-      v = warp_sum(v);
-      if (lane == 0) p.partials[blockIdx.y * gridDim.x + blockIdx.x] = v;
-    }
-  }
+  guide_tail4(p, TileObs4{s, h0, w0, p.W, corr}, fbase);
 }
 
 // ---- any number of variables per frame (1 <= C <= 8, C != 4): the same arithmetic on [frames, H, W, C] with scalar
@@ -1713,9 +1787,9 @@ __global__ void guided_step_generic_kernel(const GuideParams p) {
   const long long fbase = (static_cast<long long>(fl) * p.H) * p.W;
   const bool observed = (p.y != nullptr) && (fg % p.t_step == 0);
   const float inv_mu = 1.0f / p.mu;
-  float corr[MC];
+  TileObsC obs{s, h0, w0, p.W, {}};
 #pragma unroll
-  for (int c = 0; c < MC; ++c) corr[c] = 0.f;
+  for (int c = 0; c < MC; ++c) obs.corr[c] = 0.f;
   if (observed) {
     float acc[MC];
 #pragma unroll
@@ -1735,7 +1809,7 @@ __global__ void guided_step_generic_kernel(const GuideParams p) {
       if (c < C) {  // C is uniform over the warp: every lane takes part in the shuffle
         const float mean = warp_sum(acc[c]) * inv_area;
         const float yv = __ldg(p.y + ((static_cast<long long>(m) * C + c) * Hs + blockIdx.x) * Ws + warp);
-        corr[c] = ((yv - mean) / (p.std2[c] + p.gamma[c] * r2)) * inv_area;
+        obs.corr[c] = ((yv - mean) / (p.std2[c] + p.gamma[c] * r2)) * inv_area;
       }
     }
   }
@@ -1744,45 +1818,113 @@ __global__ void guided_step_generic_kernel(const GuideParams p) {
       const long long o = (fbase + static_cast<long long>(h0 + i / s) * p.W + (w0 + i % s)) * C;
 #pragma unroll
       for (int c = 0; c < MC; ++c)
-        if (c < C) p.cot_out[o + c] = corr[c];
+        if (c < C) p.cot_out[o + c] = obs.corr[c];
     }
     return;
   }
-  const float sg_mu = p.sigma * inv_mu;
-  float sq = 0.f;
-  bool bad = false;
-  for (int i = lane; i < s * s; i += 32) {
-    const long long o = (fbase + static_cast<long long>(h0 + i / s) * p.W + (w0 + i % s)) * C;
-#pragma unroll
-    for (int c = 0; c < MC; ++c) {
-      if (c < C) {
-        float gv = corr[c];
-        if (p.vjp != nullptr) gv -= p.sigma * p.vjp[o + c];
-        const float ev = p.eps[o + c] - sg_mu * gv;
-        if (p.mode == 0) {
-          const float xv = p.mu_next * ((p.x[o + c] - p.sigma * ev) * inv_mu) + p.sigma_next * ev;
-          bad |= !isfinite(xv);
-          p.x[o + c] = xv;
-        } else {
-          sq += ev * ev;
-          p.eps_out[o + c] = ev;
-        }
-      }
-    }
+  guide_tail_generic(p, obs, fbase);
+}
+
+// ---- K6p: point observations (PointObservation: variables observed at single grid points of chosen frames).  The
+// host merges every (frame, pixel) into one entry holding ysum = sum(mask * y) and wsum = sum(mask) per variable, so
+// A^T((y - A x0)/var) at that pixel is (ysum - wsum * x0)/var — exact, and zero at every other pixel.  CTA = a strip of
+// `strip_rows` full rows of one owned frame; an observed frame first scatters the strip's entries (CSR by frame slot
+// and strip) into a shared-memory map pixel -> entry, then runs the dense tail above with g computed from the x and
+// eps it loads anyway.  Entries are unique per pixel: no atomics, bit-identical from run to run and under sharding.
+struct PointParams {
+  const int* frame_slot;  // [own_n] observed slot of owned frame own_lo + i, or -1
+  const int* strip_off;   // [n_slots * n_strips + 1] CSR offsets into the entries
+  const int* pix;         // [n_entries] pixel index within the frame
+  const float* ysum;      // [n_entries, C]
+  const float* wsum;      // [n_entries, C]
+  int strip_rows;
+};
+
+__device__ __forceinline__ float point_g(const GuideParams& p, float ys, float ws, float x, float e, int c) {
+  const float inv_mu = 1.0f / p.mu;
+  const float r2 = (p.sigma * inv_mu) * (p.sigma * inv_mu);
+  const float x0 = (x - p.sigma * e) * inv_mu;
+  return (ys - ws * x0) / (p.std2[c] + p.gamma[c] * r2);
+}
+
+// The CTA's pixels: `npix` pixels from `pix0` on; slot == nullptr on a frame without observations.
+struct StripObs {
+  const int* slot;
+  const float* ysum;
+  const float* wsum;
+  long long pix0;
+  int npix, C;
+  __device__ int first() const { return threadIdx.x; }
+  __device__ int end() const { return npix; }
+  __device__ int step() const { return blockDim.x; }
+  __device__ long long pixel(int i) const { return pix0 + i; }
+  __device__ float4 g4(const GuideParams& p, int i, long long o, float4 ev) const {
+    const int e = slot ? slot[i] : -1;
+    if (e < 0) return make_float4(0.f, 0.f, 0.f, 0.f);
+    const float4 xv = *reinterpret_cast<const float4*>(p.x + o);
+    const float4 ys = *reinterpret_cast<const float4*>(ysum + 4ll * e);
+    const float4 ws = *reinterpret_cast<const float4*>(wsum + 4ll * e);
+    return make_float4(point_g(p, ys.x, ws.x, xv.x, ev.x, 0), point_g(p, ys.y, ws.y, xv.y, ev.y, 1),
+                       point_g(p, ys.z, ws.z, xv.z, ev.z, 2), point_g(p, ys.w, ws.w, xv.w, ev.w, 3));
   }
-  if (p.mode == 0) {
-    if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(p.nan_flag, 1);
-  } else {
-    __shared__ float wsum[32];
-    sq = warp_sum(sq);
-    if (lane == 0) wsum[warp] = sq;
+  __device__ int entry(int i) const { return slot ? slot[i] : -1; }
+  __device__ float g(const GuideParams& p, int e, long long o, int c) const {
+    if (e < 0) return 0.f;
+    const long long k = static_cast<long long>(e) * C + c;
+    return point_g(p, ysum[k], wsum[k], p.x[o + c], p.eps[o + c], c);
+  }
+};
+
+// Shared by both point kernels: this CTA's strip and, on an observed frame, its pixel -> entry map in `slot`.
+__device__ __forceinline__ StripObs point_strip(const GuideParams& p, const PointParams& q, int* slot) {
+  const int h0 = blockIdx.x * q.strip_rows;
+  StripObs obs{nullptr, q.ysum, q.wsum, static_cast<long long>(h0) * p.W, min(q.strip_rows, p.H - h0) * p.W, p.C};
+  const int os = q.frame_slot[blockIdx.y];
+  if (os >= 0) {  // uniform over the CTA
+    for (int i = threadIdx.x; i < obs.npix; i += blockDim.x) slot[i] = -1;
     __syncthreads();
-    if (warp == 0) {
-      float v = (lane < (blockDim.x >> 5)) ? wsum[lane] : 0.f;
-      v = warp_sum(v);
-      if (lane == 0) p.partials[blockIdx.y * gridDim.x + blockIdx.x] = v;
-    }
+    const int* off = q.strip_off + static_cast<long long>(os) * gridDim.x + blockIdx.x;
+    const int e0 = off[0], e1 = off[1];
+    for (int e = e0 + static_cast<int>(threadIdx.x); e < e1; e += blockDim.x)
+      slot[q.pix[e] - static_cast<int>(obs.pix0)] = e;
+    __syncthreads();
+    obs.slot = slot;
   }
+  return obs;
+}
+
+__global__ void __launch_bounds__(256) guided_points_kernel(const GuideParams p, const PointParams q) {
+  __shared__ int slot[C2W_POINT_STRIP_PIX];
+  const long long fbase = (static_cast<long long>(p.own_lo + blockIdx.y) * p.H) * p.W;
+  const StripObs obs = point_strip(p, q, slot);
+  if (p.mode == 2) {  // g on the observed pixels, zero elsewhere
+    for (int i = obs.first(); i < obs.end(); i += obs.step()) {
+      const long long o = (fbase + obs.pixel(i)) * 4;
+      float4 gv = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (obs.entry(i) >= 0) gv = obs.g4(p, i, o, *reinterpret_cast<const float4*>(p.eps + o));
+      *reinterpret_cast<float4*>(p.cot_out + o) = gv;
+    }
+    return;
+  }
+  guide_tail4(p, obs, fbase);
+}
+
+__global__ void __launch_bounds__(256) guided_points_generic_kernel(const GuideParams p, const PointParams q) {
+  __shared__ int slot[C2W_POINT_STRIP_PIX];
+  const int C = p.C;
+  const long long fbase = (static_cast<long long>(p.own_lo + blockIdx.y) * p.H) * p.W;
+  const StripObs obs = point_strip(p, q, slot);
+  if (p.mode == 2) {
+    for (int i = obs.first(); i < obs.end(); i += obs.step()) {
+      const long long o = (fbase + obs.pixel(i)) * C;
+      const int e = obs.entry(i);
+#pragma unroll
+      for (int c = 0; c < 8; ++c)
+        if (c < C) p.cot_out[o + c] = obs.g(p, e, o, c);
+    }
+    return;
+  }
+  guide_tail_generic(p, obs, fbase);
 }
 
 // Fold of the window outputs (fp32 [n, hw, cpad], EPI_F32 of the last conv) into the composed score [frames, hw, C]:

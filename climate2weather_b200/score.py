@@ -10,6 +10,7 @@ from __future__ import annotations
 import ctypes
 from typing import Callable, Optional, Sequence, Union
 
+import numpy as np
 import torch
 import torch.distributed as dist
 import torch.nn.functional as F
@@ -32,6 +33,140 @@ class CoarseGrain:
 
     def __repr__(self):
         return f"CoarseGrain(t_step={self.t_step}, s_step={self.s_step})"
+
+
+class PointObservation:
+    """Variables observed at single grid points of chosen frames (weather stations, in-situ records with gaps, a
+    variable measured at some sites only, fully observed frames):
+
+        A(x)[m, c, p] = mask[m, c, p] * x[frames[m], c, rows[p], cols[p]]
+
+    `frames`: F distinct global frame indices in any order; `rows`, `cols`: P pixel positions shared by every observed
+    frame (several may name the same pixel; their contributions add); `mask`: bool [F, C, P], default all true — False
+    marks a missing value or a variable not measured at that site, and the matching entries of y are ignored (they may
+    be NaN).  Calling the object is the plain torch operator, so the same instance can condition the reference."""
+
+    def __init__(self, frames, rows, cols, mask=None):
+        self.frames = torch.as_tensor(frames, dtype=torch.long).reshape(-1).cpu()
+        self.rows = torch.as_tensor(rows, dtype=torch.long).reshape(-1).cpu()
+        self.cols = torch.as_tensor(cols, dtype=torch.long).reshape(-1).cpu()
+        if self.rows.numel() != self.cols.numel():
+            raise ValueError(f"PointObservation: {self.rows.numel()} rows but {self.cols.numel()} cols")
+        if self.frames.numel() == 0 or self.rows.numel() == 0:
+            raise ValueError("PointObservation: needs at least one frame and one point")
+        if torch.unique(self.frames).numel() != self.frames.numel():
+            raise ValueError(f"PointObservation: repeated frame in {self.frames.tolist()}")
+        if bool((self.frames < 0).any()):
+            raise ValueError(f"PointObservation: negative frame index in {self.frames.tolist()}")
+        self.mask = None
+        if mask is not None:
+            self.mask = torch.as_tensor(mask).cpu()
+            if self.mask.dtype != torch.bool:
+                raise ValueError(f"PointObservation: mask must be a bool tensor, got {self.mask.dtype}")
+            if self.mask.dim() != 3 or self.mask.shape[0] != self.n_frames or self.mask.shape[2] != self.n_points:
+                raise ValueError(f"PointObservation: mask of shape {tuple(self.mask.shape)} is not "
+                                 f"[{self.n_frames}, C, {self.n_points}]")
+
+    @property
+    def n_frames(self) -> int:
+        return self.frames.numel()
+
+    @property
+    def n_points(self) -> int:
+        return self.rows.numel()
+
+    def mask_for(self, C: int) -> Tensor:
+        """The mask as bool [F, C, P] (all true when none was given)."""
+        if self.mask is None:
+            return torch.ones(self.n_frames, C, self.n_points, dtype=torch.bool)
+        if self.mask.shape[1] != C:
+            raise ValueError(f"PointObservation: mask of shape {tuple(self.mask.shape)} does not match "
+                             f"[{self.n_frames}, {C}, {self.n_points}]")
+        return self.mask
+
+    def __call__(self, x: Tensor) -> Tensor:
+        dev = x.device
+        out = x[self.frames.to(dev)][:, :, self.rows.to(dev), self.cols.to(dev)]
+        if self.mask is not None:
+            out = out * self.mask.to(device=dev, dtype=out.dtype)
+        return out
+
+    def check_observation(self, y: Tensor) -> None:
+        """y must be [F, C, P], finite wherever the mask is set (conditioning time)."""
+        if y.dim() != 3 or y.shape[0] != self.n_frames or y.shape[2] != self.n_points:
+            raise ValueError(f"PointObservation: y of shape {tuple(y.shape)} is not [{self.n_frames}, C, {self.n_points}]")
+        m = self.mask_for(y.shape[1])
+        if not bool(torch.isfinite(y.cpu()[m]).all()):
+            raise ValueError("PointObservation: y is not finite at an unmasked observation")
+
+    def check_geometry(self, L: int, C: int, H: int, W: int) -> None:
+        """Frames in [0, L), points inside the H x W grid, C variables (runtime build)."""
+        if int(self.frames.max()) >= L:
+            raise ValueError(f"PointObservation: frame {int(self.frames.max())} outside a trajectory of {L} frames")
+        if int(self.rows.min()) < 0 or int(self.rows.max()) >= H or int(self.cols.min()) < 0 or int(self.cols.max()) >= W:
+            raise ValueError(f"PointObservation: a point lies outside the {H}x{W} grid")
+        self.mask_for(C)
+
+    def observed_frames(self, C: int) -> list:
+        """Global frames with at least one unmasked observation, ascending."""
+        keep = self.mask_for(C).flatten(1).any(1)
+        return sorted(int(f) for f in self.frames[keep])
+
+    def __repr__(self):
+        return f"PointObservation(frames={self.n_frames}, points={self.n_points}, masked={self.mask is not None})"
+
+
+def point_strip_rows(H: int, W: int) -> int:
+    """Rows per CTA of the point-guidance kernel: the strip's pixel -> entry map fits C2W_POINT_STRIP_PIX ints of static
+    shared memory (c2w_b200.h) — 16 rows, 8 KB at 128 x 128."""
+    return max(1, min(H, POINT_STRIP_PIX // W))
+
+
+POINT_STRIP_PIX = 2048  # C2W_POINT_STRIP_PIX
+
+
+def point_plan(op: PointObservation, y, L: int, C: int, H: int, W: int, frame_lo: int, frame_hi: int, strip: int) -> dict:
+    """The device form of a point observation for the owned global frames [frame_lo, frame_hi) (c2w_point_obs).
+
+    Observations of one (frame, pixel) merge into one entry: per variable ysum = sum(mask * y), wsum = sum(mask), summed
+    in fp64 in point order and rounded to fp32 once — exact, since sum_p mask_p (y_p - x0) / var = (ysum - wsum x0) / var.
+    Entries with wsum = 0 for every variable are dropped.  Entries are sorted by (frame, strip, pixel); frame_slot maps
+    owned frame i (global frame_lo + i) to its observed slot or -1, strip_off is the CSR over (slot, strip).  Frames
+    outside [frame_lo, frame_hi) are not kept."""
+    y = torch.as_tensor(y)
+    op.check_observation(y)
+    op.check_geometry(L, C, H, W)
+    if y.shape[1] != C:
+        raise ValueError(f"PointObservation: y has {y.shape[1]} variables, the trajectory {C}")
+    if strip < 1 or strip * W > POINT_STRIP_PIX:
+        raise ValueError(f"strip of {strip} rows of {W} pixels exceeds {POINT_STRIP_PIX} pixels")
+    n_own = frame_hi - frame_lo
+    frames = op.frames.numpy()
+    pix = (op.rows * W + op.cols).numpy()
+    mask = op.mask_for(C).numpy()
+    sel = np.nonzero((frames >= frame_lo) & (frames < frame_hi))[0]
+    sel = sel[np.argsort(frames[sel], kind="stable")]
+    yv = np.where(mask[sel], y.detach().cpu().double().numpy()[sel], 0.0)      # [n_sel, C, P]; NaN under the mask -> 0
+    wv = mask[sel].astype(np.float64)
+    key = ((frames[sel] - frame_lo)[:, None] * (H * W) + pix[None, :]).reshape(-1)  # (local frame, pixel)
+    uk, inv = np.unique(key, return_inverse=True)                                  # sorted: frame, then pixel
+    ysum = np.zeros((uk.size, C))
+    wsum = np.zeros((uk.size, C))
+    np.add.at(ysum, inv, yv.transpose(0, 2, 1).reshape(-1, C))
+    np.add.at(wsum, inv, wv.transpose(0, 2, 1).reshape(-1, C))
+    keep = (wsum > 0).any(1)
+    uk, ysum, wsum = uk[keep], ysum[keep], wsum[keep]
+    fr, px = uk // (H * W), uk % (H * W)
+    n_strips = -(-H // strip)
+    obs_frames = np.unique(fr)
+    frame_slot = np.full(n_own, -1, dtype=np.int32)
+    frame_slot[obs_frames] = np.arange(obs_frames.size, dtype=np.int32)
+    cell = frame_slot[fr].astype(np.int64) * n_strips + (px // W) // strip  # non-decreasing: the keys are sorted
+    counts = np.bincount(cell, minlength=obs_frames.size * n_strips)
+    strip_off = np.concatenate([[0], np.cumsum(counts)]).astype(np.int32)
+    return dict(frame_slot=frame_slot, strip_off=strip_off, pix=px.astype(np.int32), ysum=ysum.astype(np.float32),
+                wsum=wsum.astype(np.float32), n_slots=int(obs_frames.size), strip_rows=int(strip), n_strips=n_strips,
+                frames=[int(frame_lo + f) for f in obs_frames])
 
 
 def _per_channel(v, C: int, name: str):
@@ -68,19 +203,25 @@ def _recognise_operator(A: Callable, L: int, C: int, H: int, W: int, y_shape) ->
                               "guidance kernel supports only that family (pass climate2weather_b200.CoarseGrain)")
 
 
-def observed_windows(win_lo: int, win_hi: int, n_win_global: int, L: int, k: int, t_step: int) -> list:
+def observed_windows(win_lo: int, win_hi: int, n_win_global: int, L: int, k: int, t_step) -> list:
     """Windows j in [win_lo, win_hi) whose part of the composed score meets an OBSERVED frame.  The likelihood's cotangent
     g = A^T((y - A x0)/var) (src/thor/score.py:53-56) is non-zero on observed frames only — frame f with f % t_step == 0
-    (exp/downscaling.py:131) — and window j contributes frame j + k to the composed score (plus frames 0..k-1 if it is
-    the first window, L-k..L-1 if it is the last, src/thor/score.py:76-88): every other window has an identically zero
-    output cotangent, so its vector-Jacobian product vanishes and its backward pass is skipped."""
+    (exp/downscaling.py:131), or f in the given set of frames (PointObservation: the frames with an unmasked value) —
+    and window j contributes frame j + k to the composed score (plus frames 0..k-1 if it is the first window, L-k..L-1
+    if it is the last, src/thor/score.py:76-88): every other window has an identically zero output cotangent, so its
+    vector-Jacobian product vanishes and its backward pass is skipped."""
+    if isinstance(t_step, int):
+        observed = lambda f: f % t_step == 0
+    else:
+        frames = set(int(f) for f in t_step)
+        observed = frames.__contains__
     out = []
     for j in range(win_lo, win_hi):
-        need = (j + k) % t_step == 0
+        need = observed(j + k)
         if j == 0:
-            need = need or any(f % t_step == 0 for f in range(0, k))
+            need = need or any(observed(f) for f in range(0, k))
         if j == n_win_global - 1:
-            need = need or any(f % t_step == 0 for f in range(L - k, L))
+            need = need or any(observed(f) for f in range(L - k, L))
         if need:
             out.append(j)
     return out
@@ -98,6 +239,7 @@ class _Runtime:
         k = sf.markov_order
         self.exact = bool(exact)  # exact_grad=True: guidance through the UNet VJP (src/thor/score.py:28-33,51-52)
         self.cond = None
+        self.points = None        # PointObservation: this rank's device plan (c2w_point_obs), see set_condition
         self._engine_args = (C, 2 * k + 1, H, W, device)
         self._engine_windows = min(max_windows, plan.win_hi - plan.win_lo)
         self._engine = None
@@ -150,7 +292,9 @@ class _Runtime:
     def _selected_list(self):
         """Global indices of this rank's windows whose OUTPUT carries a non-zero cotangent (see `observed_windows`)."""
         p = self.plan
-        return observed_windows(p.win_lo, p.win_hi, p.n_win_global, self.L, self.sf.markov_order, self.cond["op"].t_step)
+        op = self.cond["op"]
+        obs = op.observed_frames(self.C) if isinstance(op, PointObservation) else op.t_step
+        return observed_windows(p.win_lo, p.win_hi, p.n_win_global, self.L, self.sf.markov_order, obs)
 
     def _selection(self):
         """(chunks of (win_list_dev, pos_dev), n_selected) for the current conditioning, cached."""
@@ -244,9 +388,24 @@ class _Runtime:
     def set_condition(self, cond) -> None:
         self.cond = cond
         self._sel = None
+        self.points = None
+        if cond is not None and isinstance(cond["op"], PointObservation):
+            # this rank's owned frames only, built once per conditioning and trajectory geometry
+            p = self.plan
+            pl = point_plan(cond["op"], cond["y"], self.L, self.C, self.H, self.W, p.own_lo, p.own_lo + p.own_n,
+                            point_strip_rows(self.H, self.W))
+            dev = {n: torch.as_tensor(pl[n]).to(self.device) for n in ("frame_slot", "strip_off", "pix", "ysum", "wsum")}
+            for n in ("pix", "ysum", "wsum"):  # no entries on this rank: still a valid pointer
+                if dev[n].numel() == 0:
+                    dev[n] = torch.zeros(max(1, self.C), dtype=dev[n].dtype, device=self.device)
+            ob = _lib.PointObs()
+            ob.frame_slot, ob.strip_off, ob.pix = (dev[n].data_ptr() for n in ("frame_slot", "strip_off", "pix"))
+            ob.ysum, ob.wsum = dev["ysum"].data_ptr(), dev["wsum"].data_ptr()
+            ob.n_slots, ob.strip_rows = pl["n_slots"], pl["strip_rows"]
+            self.points = dict(obs=ob, tensors=dev, n_strips=pl["n_strips"])
         if cond is not None and self.exact:
             self.refresh_engine()  # the stashing workspace is sized by the selection
-        if cond is not None:
+        if cond is not None and self.points is None:
             self.y_dev = cond["y"].to(device=self.device, dtype=torch.float32).contiguous()
 
     def _guide(self, mode: int, mu: float, sigma: float, mu_next: float, sigma_next: float, frames=None) -> None:
@@ -254,7 +413,13 @@ class _Runtime:
         g = _lib.Guide()
         g.x, g.eps = self.x.data_ptr(), self.eps.data_ptr()
         s = self.s_tile
-        if self.cond is not None:
+        pts = self.points if self.cond is not None else None
+        if pts is not None:  # point observations: y, t_step and s_step are not read
+            g.y, g.t_step = None, 1
+            for i in range(self.C):
+                g.std2[i] = self.cond["std"][i] ** 2
+                g.gamma[i] = self.cond["gamma"][i]
+        elif self.cond is not None:
             cg: CoarseGrain = self.cond["op"]
             s = cg.s_step
             g.y = self.y_dev.data_ptr()
@@ -282,7 +447,7 @@ class _Runtime:
                 g.halo = ph.handle
                 self._halo_pushed = True
         if mode == 1:
-            n_part = p.own_n * (self.H // s)
+            n_part = p.own_n * (pts["n_strips"] if pts is not None else self.H // s)
             if self.partials is None or self.partials.numel() < n_part:
                 self.partials = torch.zeros(n_part, dtype=torch.float32, device=self.device)
             if self.eps_g is None:
@@ -290,7 +455,11 @@ class _Runtime:
             g.eps_out, g.partials = self.eps_g.data_ptr(), self.partials.data_ptr()
             self._n_part = n_part
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.c2w_guided_step(ctypes.byref(g), self.stream), "c2w_guided_step")
+            if pts is not None:
+                _lib.check(self.lib.c2w_guided_step_points(ctypes.byref(g), ctypes.byref(pts["obs"]), self.stream),
+                           "c2w_guided_step_points")
+            else:
+                _lib.check(self.lib.c2w_guided_step(ctypes.byref(g), self.stream), "c2w_guided_step")
 
     def predictor(self, mu: float, sigma: float, mu_next: float, sigma_next: float) -> None:
         """x <- mu' (x - sigma eps_g)/mu + sigma' eps_g on the owned frames (src/thor/pipelines.py:41-46)."""
@@ -428,6 +597,8 @@ class AbstractScoreFunction:
         """src/thor/score.py:44-60.  `exact_grad=False` (every shipped config) is the closed-form guidance
         J = A^T((y - A x0)/var)/mu; `exact_grad=True` adds the term through the network,
         J = (g - sigma J_eps^T g)/mu with g = A^T((y - A x0)/var), computed by the UNet input-gradient kernels."""
+        if isinstance(A, PointObservation):
+            A.check_observation(torch.as_tensor(y))
         if self.likelihood is not None:
             print("Warning: Overwriting old conditioning")
         self.likelihood = dict(A=A, y=torch.as_tensor(y), std=std, gamma=gamma, op=None, exact=bool(exact_grad))
@@ -505,7 +676,10 @@ class AbstractScoreFunction:
             if self.likelihood is not None:
                 lk = self.likelihood
                 if lk["op"] is None:
-                    lk["op"] = _recognise_operator(lk["A"], L, C, H, W, lk["y"].shape)
+                    if isinstance(lk["A"], PointObservation):  # geometry checks run in point_plan (set_condition)
+                        lk["op"] = lk["A"]
+                    else:
+                        lk["op"] = _recognise_operator(lk["A"], L, C, H, W, lk["y"].shape)
                     lk["std_c"] = _per_channel(lk["std"], C, "std")
                     lk["gamma_c"] = _per_channel(lk["gamma"], C, "gamma")
                 rt.set_condition(dict(op=lk["op"], y=lk["y"], std=lk["std_c"], gamma=lk["gamma_c"]))

@@ -80,7 +80,7 @@ void c2w_destroy(c2w_handle* h);
 const char* c2w_last_error(void);
 int c2w_abi_version(void);
 /* sizeof() of the structs of this header as the library was compiled, for bindings to check their own layout against:
- * which = 0 c2w_config, 1 c2w_guide, 2 c2w_adamw, 3 c2w_conv_desc; -1 for an unknown index */
+ * which = 0 c2w_config, 1 c2w_guide, 2 c2w_adamw, 3 c2w_conv_desc, 4 c2w_point_obs; -1 for an unknown index */
 int c2w_struct_size(int which);
 
 /* ---- weights: reference state_dict entries by name (SURVEY.md §8(b)), fp32 host memory -------------------- */
@@ -180,6 +180,25 @@ int c2w_adamw_ema_step(float* p, const float* g, float* m, float* v, float* ema,
 
 /* ---- guided predictor / corrector (see c2w_guide) --------------------------------------------------------- */
 int c2w_guided_step(const c2w_guide* g, void* stream);
+
+/* Point observations (PointObservation in climate2weather_b200/score.py): variables observed at single grid points of
+ * chosen frames, A(x)[m, c, p] = mask[m, c, p] * x[frames[m], c, rows[p], cols[p]].  The host merges the observations
+ * of each (frame, pixel) into one entry, ysum = sum(mask * y) and wsum = sum(mask) per variable, so the likelihood
+ * cotangent at that pixel is (ysum - wsum * x0) / var and zero elsewhere.  Entries are grouped by observed frame (slot)
+ * and by strip of strip_rows full pixel rows (strip_rows * W <= C2W_POINT_STRIP_PIX), sorted by pixel within a strip. */
+#define C2W_POINT_STRIP_PIX 2048
+typedef struct c2w_point_obs {
+  const int32_t* frame_slot; /* [own_n] observed slot of the updated frame own_lo + i, or -1                      */
+  const int32_t* strip_off;  /* [n_slots * ceil(H / strip_rows) + 1] CSR offsets into the entries                */
+  const int32_t* pix;        /* [n_entries] pixel index within the frame (h * W + w), unique per (slot, strip)    */
+  const float* ysum;         /* [n_entries, C] sum of mask * y                                                    */
+  const float* wsum;         /* [n_entries, C] number of unmasked observations                                    */
+  int32_t n_slots, strip_rows;
+} c2w_point_obs;
+/* c2w_guided_step with the point operator: y, t_step and s_step of g are ignored, every other field keeps its meaning
+ * (modes 0/1/2, vjp, cot_out, nan_flag, halo for C = 4, channels).  Mode 1 writes own_n * ceil(H / strip_rows)
+ * partials. */
+int c2w_guided_step_points(const c2w_guide* g, const c2w_point_obs* obs, void* stream);
 int c2w_reduce_partials(const float* partials, int32_t n, double* sumsq, void* stream);
 /* x <- x - (delta eps + sqrt(2 delta) z) sigma_next, delta = tau / (sumsq / count)  (src/thor/pipelines.py:84-87).
  * z == NULL: on-chip Philox4x32-10 keyed by (seed, step_id, global pixel index). */
