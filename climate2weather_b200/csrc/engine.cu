@@ -5,6 +5,7 @@
 #include <algorithm>
 #include <map>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "c2w_b200.h"
@@ -411,20 +412,22 @@ int launch_attention(const bf16* qkv, bf16* out, int n, int T, int C, cudaStream
 
 int grid_for(long long items, int threads, int sms);
 
-// K0: window batch [n, hw, cin_pad] bf16 from the resident trajectory (tiled form for 4-variable frames)
-int launch_gather(const float* traj, bf16* out, int n, int hw, int C, int w, int cin_pad, int f0, int sms, cudaStream_t st) {
+// K0: window batch [n, hw, cin_pad] bf16 from the resident trajectory (tiled form for 4-variable frames); f0 and
+// win_list as gather_windows_kernel takes them.
+int launch_gather(const float* traj, bf16* out, int n, int hw, int C, int w, int cin_pad, int f0, int sms, cudaStream_t st,
+                  const int* win_list = nullptr) {
   static int tiled = -1;
   if (tiled < 0) {
     const char* e = getenv("C2W_GATHER_TILED");
     tiled = (e && e[0] == '0') ? 0 : 1;
   }
-  if (tiled && C == 4 && hw % kGatherPix == 0 && w <= 64) {
+  if (!win_list && tiled && C == 4 && hw % kGatherPix == 0 && w <= 64) {
     const size_t smem = static_cast<size_t>(kGatherWin + w - 1) * kGatherPix * sizeof(uint2);
     gather_windows_tiled_kernel<<<dim3(hw / kGatherPix, (n + kGatherWin - 1) / kGatherWin), 256, smem, st>>>(traj, out, n, hw, w,
                                                                                                        cin_pad, f0);
   } else {
     const long long items = static_cast<long long>(n) * hw * (cin_pad / 8);
-    gather_windows_kernel<<<grid_for(items, 256, sms), 256, 0, st>>>(traj, out, n, hw, C, w * C, cin_pad, f0);
+    gather_windows_kernel<<<grid_for(items, 256, sms), 256, 0, st>>>(traj, out, n, hw, C, w * C, cin_pad, f0, win_list);
   }
   C2W_CUDA(cudaGetLastError());
   return C2W_OK;
@@ -1054,6 +1057,103 @@ int run_ops(c2w_handle* h, std::vector<Op>& ops, int nn, const FinalSpec& fs, cu
 
 int run_plan(c2w_handle* h, int nn, const FinalSpec& fs, cudaStream_t st) { return run_ops(h, h->plan.ops, nn, fs, st); }
 
+// Launches a frame kernel of kernels.cuh (guidance, corrector, window adjoints) instantiated for a runtime count of
+// variables per frame: launch(std::integral_constant<int, C>{}) for 1 <= C <= C2W_MAX_VARS.
+template <class F>
+int launch_for_vars(int C, F&& launch) {
+  static_assert(C2W_MAX_VARS == 8, "one case per variable count");
+  switch (C) {
+    case 1: launch(std::integral_constant<int, 1>{}); break;
+    case 2: launch(std::integral_constant<int, 2>{}); break;
+    case 3: launch(std::integral_constant<int, 3>{}); break;
+    case 4: launch(std::integral_constant<int, 4>{}); break;
+    case 5: launch(std::integral_constant<int, 5>{}); break;
+    case 6: launch(std::integral_constant<int, 6>{}); break;
+    case 7: launch(std::integral_constant<int, 7>{}); break;
+    case 8: launch(std::integral_constant<int, 8>{}); break;
+    default: return fail(C2W_ERR_INVALID, "1 to %d variables per frame (got %d)", C2W_MAX_VARS, C);
+  }
+  ++g_launches;
+  C2W_CUDA(cudaGetLastError());
+  return C2W_OK;
+}
+
+// The windows of a window-score call: the contiguous global windows [first, first + n) when list is null, else the
+// global windows list[0..n) (device array).  pos (device, n_win_global entries, backward of a list only): the place of
+// global window j in the list, or -1.
+struct WindowSet {
+  int first, n;
+  const int* list;
+  const int* pos;
+};
+
+// Gather -> UNet -> fold into eps, in chunks of the bound workspace.  eps == null: no fold, the window outputs stay
+// stashed in a VJP workspace for the backward that follows.
+int window_score_fwd(c2w_handle* h, const float* traj, int frame_global0, const WindowSet& ws, int n_win_global, float t,
+                     float* eps, cudaStream_t st) {
+  Plan& P = h->plan;
+  const int w = h->cfg.window, k = w / 2, C = h->cfg.frame_channels;
+  const int hw = h->cfg.height * h->cfg.width;
+  int rc = run_modulation(h, t, nullptr, 1, P.h0, P.emb, P.mods, st);
+  if (rc) return rc;
+  for (int c0 = 0; c0 < ws.n; c0 += P.n_max) {
+    const int nn = std::min(P.n_max, ws.n - c0);
+    const int j0 = ws.first + c0;  // first window of the chunk (contiguous windows)
+    const int* list = ws.list ? ws.list + c0 : nullptr;
+    if ((rc = launch_gather(traj, P.xin, nn, hw, C, w, h->cin_pad, list ? frame_global0 : j0 - frame_global0, h->sms, st,
+                            list)))
+      return rc;
+    ++g_launches;
+    FinalSpec fs;
+    fs.mode = EPI_F32;
+    if (eps && C == 4) {  // the fold is the last conv's epilogue
+      fs.mode = EPI_COMPOSE;
+      fs.eps = eps;
+      fs.order_k = k;
+      fs.win_first = j0;
+      fs.win_last_global = n_win_global - 1;
+      fs.frame_base = frame_global0;
+      fs.win_list = list;
+    }
+    if ((rc = run_plan(h, nn, fs, st))) return rc;
+    if (eps && C != 4) {  // any other variable count: the fold as its own pass over the fp32 window outputs
+      const long long items = static_cast<long long>(nn) * hw * C;
+      compose_generic_kernel<<<grid_for(items, 256, h->sms), 256, 0, st>>>(P.out32, eps, nn, hw, h->levels[0].tail.cout_pad,
+                                                                           C, k, j0, n_win_global - 1, frame_global0, list);
+      ++g_launches;
+      C2W_CUDA(cudaGetLastError());
+    }
+  }
+  return C2W_OK;
+}
+
+// Compose adjoint -> input-gradient pass -> unfold adjoint of the windows whose stashing forward has just run (one
+// chunk).  vjp (fp32 [n_frames_local, H, W, C]) is accumulated on the frames the windows touch.
+int window_score_bwd(c2w_handle* h, const float* cot, int n_frames_local, int frame_global0, const WindowSet& ws,
+                     int n_win_global, float* vjp, cudaStream_t st) {
+  Plan& P = h->plan;
+  const int w = h->cfg.window, k = w / 2;
+  const int hw = h->cfg.height * h->cfg.width;
+  const int cpad = h->levels[0].tail.cout_pad;
+  const long long items = static_cast<long long>(ws.n) * hw * (cpad / 8);
+  int rc = launch_for_vars(h->cfg.frame_channels, [&](auto vars) {
+    compose_adjoint_kernel<decltype(vars)::value><<<grid_for(items, 256, h->sms), 256, 0, st>>>(
+        cot, P.cot, ws.n, hw, cpad, k, ws.first, n_win_global - 1, frame_global0, ws.list);
+  });
+  if (rc) return rc;
+  FinalSpec fs;
+  fs.mode = EPI_F32;
+  if ((rc = run_ops(h, P.bwd, ws.n, fs, st))) return rc;
+  // the local frames the windows can touch: the n + w - 1 of a contiguous range, every one for a list
+  const int f_lo = ws.list ? 0 : ws.first - frame_global0;
+  const int nf = ws.list ? n_frames_local : ws.n + w - 1;
+  const long long items2 = static_cast<long long>(nf) * hw;
+  return launch_for_vars(h->cfg.frame_channels, [&](auto vars) {
+    unfold_adjoint_kernel<decltype(vars)::value><<<grid_for(items2, 256, h->sms), 256, 0, st>>>(
+        P.out32, vjp, ws.n, f_lo, nf, hw, h->cin_pad, w, ws.first, frame_global0, n_win_global, ws.pos);
+  });
+}
+
 }  // namespace
 
 extern "C" {
@@ -1376,43 +1476,15 @@ int c2w_window_score(c2w_handle* h, const float* traj, int32_t n_frames_local, i
   C2W_REQUIRE(h && traj && eps, "c2w_window_score: bad argument");
   if (h->plan.n_max < 1) return fail(C2W_ERR_STATE, "bind a workspace first");
   if (h->plan.per_t) return fail(C2W_ERR_STATE, "window scores use one diffusion time: bind a plain workspace");
-  const int w = h->cfg.window, k = w / 2, C = h->cfg.frame_channels;
+  const int w = h->cfg.window, C = h->cfg.frame_channels;
   C2W_REQUIRE(n_win >= 1 && win_first >= 0 && win_first + n_win <= n_win_global, "window range [%d,%d) outside [0,%d)",
               win_first, win_first + n_win, n_win_global);
   C2W_REQUIRE(win_first >= frame_global0 && win_first + n_win - 1 + w <= frame_global0 + n_frames_local,
               "windows [%d,%d) need frames outside the local range [%d,%d)", win_first, win_first + n_win,
               frame_global0, frame_global0 + n_frames_local);
   C2W_REQUIRE(C >= 1 && C <= 8, "1 to 8 variables per frame (got %d)", C);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  Plan& P = h->plan;
-  const int hw = h->cfg.height * h->cfg.width;
-  int rc = run_modulation(h, t, nullptr, 1, P.h0, P.emb, P.mods, st);
-  if (rc) return rc;
-  for (int c0 = 0; c0 < n_win; c0 += P.n_max) {
-    const int nn = std::min(P.n_max, n_win - c0);
-    const int j0 = win_first + c0;
-    if ((rc = launch_gather(traj, P.xin, nn, hw, C, w, h->cin_pad, j0 - frame_global0, h->sms, st))) return rc;
-    ++g_launches;
-    FinalSpec fs;
-    if (C == 4) {  // the fold is the last conv's epilogue
-      fs.mode = EPI_COMPOSE;
-      fs.eps = eps;
-      fs.order_k = k;
-      fs.win_first = j0;
-      fs.win_last_global = n_win_global - 1;
-      fs.frame_base = frame_global0;
-      if ((rc = run_plan(h, nn, fs, st))) return rc;
-    } else {       // any other variable count: fp32 window outputs, then the fold as its own pass
-      fs.mode = EPI_F32;
-      if ((rc = run_plan(h, nn, fs, st))) return rc;
-      const long long items = static_cast<long long>(nn) * hw * C;
-      compose_generic_kernel<<<grid_for(items, 256, h->sms), 256, 0, st>>>(P.out32, eps, nn, hw, h->levels[0].tail.cout_pad, C,
-                                                                           k, j0, n_win_global - 1, frame_global0, nullptr);
-      ++g_launches;
-      C2W_CUDA(cudaGetLastError());
-    }
-  }
-  return C2W_OK;
+  return window_score_fwd(h, traj, frame_global0, WindowSet{win_first, n_win, nullptr, nullptr}, n_win_global, t, eps,
+                          static_cast<cudaStream_t>(stream));
 }
 
 // Forward of a SELECTION of windows (global indices win_list_dev[0..n_sel)).  With the coarse-graining likelihood the
@@ -1431,39 +1503,9 @@ int c2w_window_score_sel(c2w_handle* h, const float* traj, int32_t n_frames_loca
   C2W_REQUIRE(!P.vjp || n_sel <= P.n_max, "c2w_window_score_sel: %d windows exceed the bound VJP workspace (%d)", n_sel,
               P.n_max);
   C2W_REQUIRE(eps || P.vjp, "c2w_window_score_sel: no output asked for on a plain workspace");
-  const int w = h->cfg.window, k = w / 2, C = h->cfg.frame_channels;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int hw = h->cfg.height * h->cfg.width;
   (void)n_frames_local;
-  int rc = run_modulation(h, t, nullptr, 1, P.h0, P.emb, P.mods, st);
-  if (rc) return rc;
-  for (int c0 = 0; c0 < n_sel; c0 += P.n_max) {
-    const int nn = std::min(P.n_max, n_sel - c0);
-    const long long items = static_cast<long long>(nn) * hw * (h->cin_pad / 8);
-    gather_windows_kernel<<<grid_for(items, 256, h->sms), 256, 0, st>>>(traj, P.xin, nn, hw, C, w * C, h->cin_pad,
-                                                                        frame_global0, win_list_dev + c0);
-    ++g_launches;
-    C2W_CUDA(cudaGetLastError());
-    FinalSpec fs;
-    fs.mode = EPI_F32;
-    if (eps && C == 4) {
-      fs.mode = EPI_COMPOSE;
-      fs.eps = eps;
-      fs.order_k = k;
-      fs.win_last_global = n_win_global - 1;
-      fs.frame_base = frame_global0;
-      fs.win_list = win_list_dev + c0;
-    }
-    if ((rc = run_plan(h, nn, fs, st))) return rc;
-    if (eps && C != 4) {  // the fold as its own pass over the fp32 window outputs
-      const long long it2 = static_cast<long long>(nn) * hw * C;
-      compose_generic_kernel<<<grid_for(it2, 256, h->sms), 256, 0, st>>>(P.out32, eps, nn, hw, h->levels[0].tail.cout_pad, C, k, 0,
-                                                                          n_win_global - 1, frame_global0, win_list_dev + c0);
-      ++g_launches;
-      C2W_CUDA(cudaGetLastError());
-    }
-  }
-  return C2W_OK;
+  return window_score_fwd(h, traj, frame_global0, WindowSet{0, n_sel, win_list_dev, nullptr}, n_win_global, t, eps,
+                          static_cast<cudaStream_t>(stream));
 }
 
 // Adjoint of the selected windows whose stashing forward has JUST run (c2w_window_score_sel, same list): compose adjoint
@@ -1476,35 +1518,8 @@ int c2w_window_score_backward_sel(c2w_handle* h, const float* cot, int32_t n_fra
   Plan& P = h->plan;
   if (P.n_max < 1 || !P.vjp) return fail(C2W_ERR_STATE, "bind a VJP workspace first (c2w_bind_workspace_vjp)");
   C2W_REQUIRE(n_sel <= P.n_max, "backward handles one chunk: %d windows, workspace %d", n_sel, P.n_max);
-  const int w = h->cfg.window, k = w / 2, C = h->cfg.frame_channels;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int hw = h->cfg.height * h->cfg.width;
-  const int cpad = h->levels[0].tail.cout_pad;
-  const long long items = static_cast<long long>(n_sel) * hw * (cpad / 8);
-  if (C == 4)
-    compose_adjoint_kernel<<<grid_for(items, 256, h->sms), 256, 0, st>>>(cot, P.cot, n_sel, hw, cpad, k, 0, n_win_global - 1,
-                                                                           frame_global0, win_list_dev);
-  else
-    compose_adjoint_generic_kernel<<<grid_for(items, 256, h->sms), 256, 0, st>>>(cot, P.cot, n_sel, hw, cpad, C, k, 0,
-                                                                                   n_win_global - 1, frame_global0, win_list_dev);
-  ++g_launches;
-  C2W_CUDA(cudaGetLastError());
-  FinalSpec fs;
-  fs.mode = EPI_F32;
-  int rc = run_ops(h, P.bwd, n_sel, fs, st);
-  if (rc) return rc;
-  if (C == 4) {
-    const long long items2 = static_cast<long long>(n_frames_local) * hw;
-    unfold_adjoint_sel_kernel<<<grid_for(items2, 256, h->sms), 256, 0, st>>>(P.out32, vjp, n_frames_local, hw, h->cin_pad, w,
-                                                                               frame_global0, n_win_global, pos_dev);
-  } else {
-    const long long items2 = static_cast<long long>(n_frames_local) * hw * C;
-    unfold_adjoint_generic_kernel<<<grid_for(items2, 256, h->sms), 256, 0, st>>>(
-        P.out32, vjp, n_sel, n_frames_local, hw, h->cin_pad, C, w, 0, frame_global0, n_win_global, pos_dev);
-  }
-  ++g_launches;
-  C2W_CUDA(cudaGetLastError());
-  return C2W_OK;
+  return window_score_bwd(h, cot, n_frames_local, frame_global0, WindowSet{0, n_sel, win_list_dev, pos_dev}, n_win_global,
+                          vjp, static_cast<cudaStream_t>(stream));
 }
 
 // J^T g of ScoreUNet.forward w.r.t. its input: forward (stashing) + input-gradient pass, n <= max_windows.
@@ -1548,39 +1563,13 @@ int c2w_window_score_backward(c2w_handle* h, const float* cot, int32_t n_frames_
   C2W_REQUIRE(h && cot && vjp, "c2w_window_score_backward: bad argument");
   Plan& P = h->plan;
   if (P.n_max < 1 || !P.vjp) return fail(C2W_ERR_STATE, "bind a VJP workspace first (c2w_bind_workspace_vjp)");
-  const int w = h->cfg.window, k = w / 2, C = h->cfg.frame_channels;
+  const int w = h->cfg.window;
   C2W_REQUIRE(n_win >= 1 && n_win <= P.n_max, "backward handles one chunk: %d windows, workspace %d", n_win, P.n_max);
   C2W_REQUIRE(win_first >= frame_global0 && win_first + n_win - 1 + w <= frame_global0 + n_frames_local,
               "windows [%d,%d) need frames outside the local range [%d,%d)", win_first, win_first + n_win,
               frame_global0, frame_global0 + n_frames_local);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int hw = h->cfg.height * h->cfg.width;
-  const int cpad = h->levels[0].tail.cout_pad;
-  const long long items = static_cast<long long>(n_win) * hw * (cpad / 8);
-  if (C == 4)
-    compose_adjoint_kernel<<<grid_for(items, 256, h->sms), 256, 0, st>>>(cot, P.cot, n_win, hw, cpad, k, win_first,
-                                                                           n_win_global - 1, frame_global0);
-  else
-    compose_adjoint_generic_kernel<<<grid_for(items, 256, h->sms), 256, 0, st>>>(cot, P.cot, n_win, hw, cpad, C, k, win_first,
-                                                                                   n_win_global - 1, frame_global0, nullptr);
-  ++g_launches;
-  C2W_CUDA(cudaGetLastError());
-  FinalSpec fs;
-  fs.mode = EPI_F32;
-  int rc = run_ops(h, P.bwd, n_win, fs, st);
-  if (rc) return rc;
-  if (C == 4) {
-    const long long items2 = static_cast<long long>(n_win + w - 1) * hw;
-    unfold_adjoint_kernel<<<grid_for(items2, 256, h->sms), 256, 0, st>>>(P.out32, vjp, n_win, hw, h->cin_pad, w, win_first,
-                                                                           frame_global0);
-  } else {
-    const long long items2 = static_cast<long long>(n_frames_local) * hw * C;
-    unfold_adjoint_generic_kernel<<<grid_for(items2, 256, h->sms), 256, 0, st>>>(
-        P.out32, vjp, n_win, n_frames_local, hw, h->cin_pad, C, w, win_first, frame_global0, n_win_global, nullptr);
-  }
-  ++g_launches;
-  C2W_CUDA(cudaGetLastError());
-  return C2W_OK;
+  return window_score_bwd(h, cot, n_frames_local, frame_global0, WindowSet{win_first, n_win, nullptr, nullptr},
+                          n_win_global, vjp, static_cast<cudaStream_t>(stream));
 }
 
 int c2w_set_forcing(c2w_handle* h, const float* forcing_dev) {
@@ -1882,19 +1871,19 @@ int c2w_adamw_ema_step(float* p, const float* g, float* m, float* v, float* ema,
   return C2W_OK;
 }
 
-// GuideParams from a c2w_guide: the checks and fields both guidance entry points share (`what` names the caller).
-static int guide_params(const c2w_guide* g, const char* what, GuideParams& p) {
+// GuideParams and the variable count C from a c2w_guide: the checks and fields both guidance entry points share (`what`
+// names the caller).
+static int guide_params(const c2w_guide* g, const char* what, GuideParams& p, int& C) {
   C2W_REQUIRE(g && g->x && g->eps && g->nan_flag, "%s: bad argument", what);
   C2W_REQUIRE(g->mode != 1 || (g->eps_out && g->partials), "mode 1 needs eps_out and partials");
   C2W_REQUIRE(g->own_n >= 1, "own_n must be positive");
-  const int C = g->channels == 0 ? 4 : g->channels;
+  C = g->channels == 0 ? 4 : g->channels;
   C2W_REQUIRE(C >= 1 && C <= C2W_MAX_VARS, "%s: 1 to %d variables per frame (got %d)", what, C2W_MAX_VARS, C);
   C2W_REQUIRE(C == 4 || g->halo == nullptr, "%s: the fused halo push handles 4 variables per frame", what);
   p.x = g->x;
   p.eps = g->eps;
   p.eps_out = g->eps_out;
   p.y = g->y;
-  p.C = C;
   for (int i = 0; i < C2W_MAX_VARS; ++i) {
     p.std2[i] = g->std2[i];
     p.gamma[i] = g->gamma[i];
@@ -1942,14 +1931,13 @@ int c2w_guided_step(const c2w_guide* g, void* stream) {
   C2W_REQUIRE(g->mode != 2 || (g->cot_out && g->y), "mode 2 needs cot_out and an observation");
   C2W_REQUIRE(g->t_step >= 1, "own_n and t_step must be positive");
   GuideParams p;
-  int rc = guide_params(g, "c2w_guided_step", p);
+  int C;
+  int rc = guide_params(g, "c2w_guided_step", p, C);
   if (rc) return rc;
   dim3 grid(g->H / g->s_step, g->own_n);
-  if (p.C == 4) guided_step_kernel<<<grid, 32 * (g->W / g->s_step), 0, static_cast<cudaStream_t>(stream)>>>(p);
-  else guided_step_generic_kernel<<<grid, 32 * (g->W / g->s_step), 0, static_cast<cudaStream_t>(stream)>>>(p);
-  ++g_launches;
-  C2W_CUDA(cudaGetLastError());
-  return C2W_OK;
+  return launch_for_vars(C, [&](auto vars) {
+    guided_step_kernel<decltype(vars)::value><<<grid, 32 * (g->W / g->s_step), 0, static_cast<cudaStream_t>(stream)>>>(p);
+  });
 }
 
 int c2w_guided_step_points(const c2w_guide* g, const c2w_point_obs* obs, void* stream) {
@@ -1960,7 +1948,8 @@ int c2w_guided_step_points(const c2w_guide* g, const c2w_point_obs* obs, void* s
               C2W_POINT_STRIP_PIX);
   C2W_REQUIRE(g->mode != 2 || g->cot_out, "mode 2 needs cot_out");
   GuideParams p;
-  int rc = guide_params(g, "c2w_guided_step_points", p);
+  int C;
+  int rc = guide_params(g, "c2w_guided_step_points", p, C);
   if (rc) return rc;
   PointParams q;
   q.frame_slot = obs->frame_slot;
@@ -1970,11 +1959,9 @@ int c2w_guided_step_points(const c2w_guide* g, const c2w_point_obs* obs, void* s
   q.wsum = obs->wsum;
   q.strip_rows = obs->strip_rows;
   dim3 grid((g->H + obs->strip_rows - 1) / obs->strip_rows, g->own_n);
-  if (p.C == 4) guided_points_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(p, q);
-  else guided_points_generic_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(p, q);
-  ++g_launches;
-  C2W_CUDA(cudaGetLastError());
-  return C2W_OK;
+  return launch_for_vars(C, [&](auto vars) {
+    guided_points_kernel<decltype(vars)::value><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(p, q);
+  });
 }
 
 int c2w_reduce_partials(const float* partials, int32_t n, double* sumsq, void* stream) {
@@ -1991,16 +1978,11 @@ int c2w_corrector_update_c(float* x, const float* eps, const float* z, const dou
   C2W_REQUIRE(x && eps && sumsq && nan_flag && npix >= 1 && count > 0, "c2w_corrector_update: bad argument");
   C2W_REQUIRE(channels >= 1 && channels <= C2W_MAX_VARS, "c2w_corrector_update: 1 to %d variables per frame (got %d)",
               C2W_MAX_VARS, channels);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (channels == 4)
-    corrector_update_kernel<<<grid_for(npix, 256, c2w_num_sms()), 256, 0, st>>>(x, eps, z, sumsq, count, tau, sigma_next,
-                                                                                pix0_global, npix, seed, step_id, nan_flag);
-  else
-    corrector_update_generic_kernel<<<grid_for(npix, 256, c2w_num_sms()), 256, 0, st>>>(
-        x, eps, z, sumsq, count, tau, sigma_next, pix0_global, npix, channels, seed, step_id, nan_flag);
-  ++g_launches;
-  C2W_CUDA(cudaGetLastError());
-  return C2W_OK;
+  return launch_for_vars(channels, [&](auto vars) {
+    corrector_update_kernel<decltype(vars)::value><<<grid_for(npix, 256, c2w_num_sms()), 256, 0,
+                                                     static_cast<cudaStream_t>(stream)>>>(
+        x, eps, z, sumsq, count, tau, sigma_next, pix0_global, npix, seed, step_id, nan_flag);
+  });
 }
 
 int c2w_corrector_update(float* x, const float* eps, const float* z, const double* sumsq, double count, float tau,

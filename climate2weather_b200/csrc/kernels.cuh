@@ -1397,12 +1397,46 @@ __global__ void zero_upsample_kernel(const bf16* __restrict__ in, bf16* __restri
   }
 }
 
+// ------------------------------------------------------------------------------------------------ frame variables
+// The C variables of one pixel of a frame tensor (fp32 [frames, HW, C]).  The frame kernels below are templates on
+// C = 1..8; C = 4 (the shipped configs, exp/downscaling.py:101) moves a pixel as one 16-byte access, any other count
+// as C scalar accesses.
+template <int C>
+struct Vars {
+  float v[C];
+  __device__ __forceinline__ float& operator[](int c) { return v[c]; }
+  __device__ __forceinline__ float operator[](int c) const { return v[c]; }
+};
+template <int C>
+__device__ __forceinline__ Vars<C> load_vars(const float* p) {
+  Vars<C> r;
+  if constexpr (C == 4) {
+    const float4 q = *reinterpret_cast<const float4*>(p);
+    r.v[0] = q.x, r.v[1] = q.y, r.v[2] = q.z, r.v[3] = q.w;
+  } else {
+#pragma unroll
+    for (int c = 0; c < C; ++c) r.v[c] = p[c];
+  }
+  return r;
+}
+template <int C>
+__device__ __forceinline__ void store_vars(float* p, const Vars<C>& r) {
+  if constexpr (C == 4) {
+    *reinterpret_cast<float4*>(p) = make_float4(r.v[0], r.v[1], r.v[2], r.v[3]);
+  } else {
+#pragma unroll
+    for (int c = 0; c < C; ++c) p[c] = r.v[c];
+  }
+}
+
 // Adjoint of the window compose (src/thor/score.py:76-88,111-141): UNet-output cotangent of window i, slot tau is
-// the frame cotangent g[win + tau] where that slot is the frame's source, zero elsewhere.
-// g: fp32 [frames, HW, 4] ; cot: bf16 [n, HW, cpad]
+// the frame cotangent g[win + tau] where that slot is the frame's source, zero elsewhere.  The windows: win_list[i],
+// or win_first + i when win_list is null.
+// g: fp32 [frames, HW, C] ; cot: bf16 [n, HW, cpad]; one thread writes 8 channels (16 B).
+template <int C>
 __global__ void compose_adjoint_kernel(const float* __restrict__ g, bf16* __restrict__ cot, int n, int hw, int cpad,
                                        int order_k, int win_first, int win_last_global, int frame_base,
-                                       const int* __restrict__ win_list = nullptr) {
+                                       const int* __restrict__ win_list) {
   const int groups = cpad >> 3;
   const long long total = static_cast<long long>(n) * hw * groups;
   for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
@@ -1412,128 +1446,49 @@ __global__ void compose_adjoint_kernel(const float* __restrict__ g, bf16* __rest
     const int pix = static_cast<int>(pw % hw);
     const int i = static_cast<int>(pw / hw);
     const int win = win_list ? win_list[i] : win_first + i;
+    const auto take = [&](int tau) {
+      return tau <= 2 * order_k &&
+             ((tau == order_k) || (win == 0 && tau < order_k) || (win == win_last_global && tau > order_k));
+    };
+    const auto frame = [&](int tau) { return g + (static_cast<long long>(win + tau - frame_base) * hw + pix) * C; };
     float v[8];
+    if constexpr (8 % C == 0) {  // the 8 channels are 8 / C whole slots
 #pragma unroll
-    for (int hf = 0; hf < 2; ++hf) {
-      const int tau = 2 * gq + hf;
-      const bool take = (tau == order_k) || (win == 0 && tau < order_k) ||
-                        (win == win_last_global && tau > order_k && tau <= 2 * order_k);
-      float4 q = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (take) q = __ldg(reinterpret_cast<const float4*>(g + (static_cast<long long>(win + tau - frame_base) * hw + pix) * 4));
-      v[4 * hf + 0] = q.x;
-      v[4 * hf + 1] = q.y;
-      v[4 * hf + 2] = q.z;
-      v[4 * hf + 3] = q.w;
+      for (int hf = 0; hf < 8 / C; ++hf) {
+        const int tau = (8 / C) * gq + hf;
+        const Vars<C> q = take(tau) ? load_vars<C>(frame(tau)) : Vars<C>{};
+#pragma unroll
+        for (int c = 0; c < C; ++c) v[C * hf + c] = q[c];
+      }
+    } else {  // the 8 channels straddle slots
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        const int ch = 8 * gq + e;
+        const int tau = ch / C, c = ch - tau * C;
+        v[e] = take(tau) ? frame(tau)[c] : 0.f;
+      }
     }
     *reinterpret_cast<uint4*>(cot + (static_cast<long long>(i) * hw + pix) * cpad + 8 * gq) =
         make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
   }
 }
 
-// Adjoint of unfold (src/thor/score.py:68-74): vjp[f] += sum_tau gin[f - tau - win_first][slot tau] over the windows
-// of this launch.  gin: fp32 [n, HW, cpad] ; vjp: fp32 [frames, HW, 4] ; frames f in [win_first, win_first + n + 2k).
-__global__ void unfold_adjoint_kernel(const float* __restrict__ gin, float* __restrict__ vjp, int n, int hw, int cpad,
-                                      int window, int win_first, int frame_base) {
-  const long long total = static_cast<long long>(n + window - 1) * hw;
+// Adjoint of unfold (src/thor/score.py:68-74): vjp[f] += sum_tau gin[window f - tau][slot tau] over the windows of this
+// launch; a frame no such window touches is left as it is.  The windows: pos == null -> the contiguous global windows
+// [win_first, win_first + n); else pos[j] = batch index of global window j or -1 (n_win_global entries).
+// gin: fp32 [n, HW, cpad] ; vjp: fp32 [frames, HW, C] ; one thread per (local frame f_lo + fo, pixel), fo < nf.
+template <int C>
+__global__ void unfold_adjoint_kernel(const float* __restrict__ gin, float* __restrict__ vjp, int n, int f_lo, int nf,
+                                      int hw, int cpad, int window, int win_first, int frame_base, int n_win_global,
+                                      const int* __restrict__ pos) {
+  const long long total = static_cast<long long>(nf) * hw;
   for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
        idx += static_cast<long long>(gridDim.x) * blockDim.x) {
     const int pix = static_cast<int>(idx % hw);
-    const int fo = static_cast<int>(idx / hw);  // frame offset from win_first
-    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-    for (int tau = 0; tau < window; ++tau) {
-      const int i = fo - tau;
-      if (i < 0 || i >= n) continue;
-      const float4 q = *reinterpret_cast<const float4*>(gin + (static_cast<long long>(i) * hw + pix) * cpad + 4 * tau);
-      acc.x += q.x;
-      acc.y += q.y;
-      acc.z += q.z;
-      acc.w += q.w;
-    }
-    float4* dst = reinterpret_cast<float4*>(vjp + (static_cast<long long>(win_first + fo - frame_base) * hw + pix) * 4);
-    float4 o = *dst;
-    o.x += acc.x;
-    o.y += acc.y;
-    o.z += acc.z;
-    o.w += acc.w;
-    *dst = o;
-  }
-}
-
-// The same for a SELECTION of windows: pos[j] = index of global window j in this launch's batch or -1.  One thread per
-// (local frame, pixel); vjp is accumulated.
-__global__ void unfold_adjoint_sel_kernel(const float* __restrict__ gin, float* __restrict__ vjp, int n_frames, int hw,
-                                          int cpad, int window, int frame_base, int n_win_global,
-                                          const int* __restrict__ pos) {
-  const long long total = static_cast<long long>(n_frames) * hw;
-  for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
-       idx += static_cast<long long>(gridDim.x) * blockDim.x) {
-    const int pix = static_cast<int>(idx % hw);
-    const int fl = static_cast<int>(idx / hw);
+    const int fl = f_lo + static_cast<int>(idx / hw);
     const int fg = frame_base + fl;
-    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    Vars<C> acc{};
     bool any = false;
-    for (int tau = 0; tau < window; ++tau) {
-      const int j = fg - tau;
-      if (j < 0 || j >= n_win_global) continue;
-      const int i = pos[j];
-      if (i < 0) continue;
-      const float4 q = *reinterpret_cast<const float4*>(gin + (static_cast<long long>(i) * hw + pix) * cpad + 4 * tau);
-      acc.x += q.x;
-      acc.y += q.y;
-      acc.z += q.z;
-      acc.w += q.w;
-      any = true;
-    }
-    if (!any) continue;
-    float4* dst = reinterpret_cast<float4*>(vjp + (static_cast<long long>(fl) * hw + pix) * 4);
-    float4 o = *dst;
-    o.x += acc.x;
-    o.y += acc.y;
-    o.z += acc.z;
-    o.w += acc.w;
-    *dst = o;
-  }
-}
-
-// The three adjoints above for any number of variables per frame (C != 4; g / vjp: fp32 [frames, HW, C]).
-__global__ void compose_adjoint_generic_kernel(const float* __restrict__ g, bf16* __restrict__ cot, int n, int hw, int cpad,
-                                               int C, int order_k, int win_first, int win_last_global, int frame_base,
-                                               const int* __restrict__ win_list) {
-  const int groups = cpad >> 3;
-  const long long total = static_cast<long long>(n) * hw * groups;
-  for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
-       idx += static_cast<long long>(gridDim.x) * blockDim.x) {
-    const int gq = static_cast<int>(idx % groups);
-    const long long pw = idx / groups;
-    const int pix = static_cast<int>(pw % hw);
-    const int i = static_cast<int>(pw / hw);
-    const int win = win_list ? win_list[i] : win_first + i;
-    float v[8];
-#pragma unroll
-    for (int e = 0; e < 8; ++e) {
-      const int ch = 8 * gq + e;
-      const int tau = ch / C, c = ch - tau * C;
-      const bool take = tau <= 2 * order_k && ((tau == order_k) || (win == 0 && tau < order_k) ||
-                                               (win == win_last_global && tau > order_k));
-      v[e] = take ? __ldg(g + (static_cast<long long>(win + tau - frame_base) * hw + pix) * C + c) : 0.f;
-    }
-    *reinterpret_cast<uint4*>(cot + (static_cast<long long>(i) * hw + pix) * cpad + 8 * gq) =
-        make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
-  }
-}
-// pos == null: the contiguous windows [win_first, win_first + n); else pos[j] = batch index of global window j or -1
-__global__ void unfold_adjoint_generic_kernel(const float* __restrict__ gin, float* __restrict__ vjp, int n, int n_frames,
-                                              int hw, int cpad, int C, int window, int win_first, int frame_base,
-                                              int n_win_global, const int* __restrict__ pos) {
-  const long long total = static_cast<long long>(n_frames) * hw * C;
-  for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
-       idx += static_cast<long long>(gridDim.x) * blockDim.x) {
-    const int c = static_cast<int>(idx % C);
-    const long long fp = idx / C;
-    const int pix = static_cast<int>(fp % hw);
-    const int fl = static_cast<int>(fp / hw);
-    const int fg = frame_base + fl;
-    float acc = 0.f;
     for (int tau = 0; tau < window; ++tau) {
       const int j = fg - tau;  // global window whose slot tau is this frame
       int i;
@@ -1542,17 +1497,25 @@ __global__ void unfold_adjoint_generic_kernel(const float* __restrict__ gin, flo
         i = pos[j];
       } else {
         i = j - win_first;
-        if (i >= n) i = -1;
+        if (i >= n) continue;
       }
       if (i < 0) continue;
-      acc += gin[(static_cast<long long>(i) * hw + pix) * cpad + tau * C + c];
+      const Vars<C> q = load_vars<C>(gin + (static_cast<long long>(i) * hw + pix) * cpad + tau * C);
+#pragma unroll
+      for (int c = 0; c < C; ++c) acc[c] += q[c];
+      any = true;
     }
-    vjp[idx] += acc;
+    if (!any) continue;
+    float* dst = vjp + (static_cast<long long>(fl) * hw + pix) * C;
+    Vars<C> o = load_vars<C>(dst);
+#pragma unroll
+    for (int c = 0; c < C; ++c) o[c] += acc[c];
+    store_vars<C>(dst, o);
   }
 }
 
 // ------------------------------------------------------------------------------------------------ K6 / K7
-// State layout: x, eps, z are fp32 [frames, H, W, 4] (one float4 per pixel).  Observation y: fp32 [n_obs, 4, Hs, Ws]
+// State layout: x, eps, z are fp32 [frames, H, W, C] (Vars<C> per pixel).  Observation y: fp32 [n_obs, C, Hs, Ws]
 // exactly as the reference builds it (exp/downscaling.py:129-132: every t_step-th frame, s x s tile means).
 struct GuideParams {
   float* x;
@@ -1561,7 +1524,6 @@ struct GuideParams {
   const float* y;    // null => unconditioned
   float std2[8];     // likelihood std^2 per variable
   float gamma[8];
-  int C;             // variables per frame: 4 -> guided_step_kernel (one float4 per pixel), else the generic kernel
   float mu, sigma;            // at the time the score was evaluated
   float mu_next, sigma_next;  // mode 0: target of the predictor step
   int t_step, s_step, H, W;
@@ -1572,9 +1534,9 @@ struct GuideParams {
   int* nan_flag;
   const float* vjp;   // exact_grad: J_eps^T g per pixel (UNet vector-Jacobian product), null = closed-form guidance
   float* cot_out;     // mode 2: g = A^T((y - A x0) / var), the cotangent fed to the UNet VJP
-  // mode 0, time-sharded: the halo PUSH fused into the predictor update (K8, csrc/halo.cu) — the updated pixels of the
-  // first / last k owned frames are also stored into the left / right neighbour's mailbox over NVLink, and the last CTA
-  // publishes the step counter.  Null pointers: no neighbour on that side / not sharded.
+  // mode 0, time-sharded, C = 4: the halo PUSH fused into the predictor update (K8, csrc/halo.cu) — the updated pixels
+  // of the first / last k owned frames are also stored into the left / right neighbour's mailbox over NVLink, and the
+  // last CTA publishes the step counter.  Null pointers: no neighbour on that side / not sharded.
   float4* push_l;          // left neighbour's mailbox slot (receives local frames [own_lo, own_lo + halo_k))
   float4* push_r;          // right neighbour's slot (receives local frames [own_lo + own_n - halo_k, own_lo + own_n))
   unsigned int* flag_l;    // neighbours' step counters
@@ -1601,55 +1563,66 @@ __device__ __forceinline__ void block_partial(const GuideParams& p, float sq) {
 // The dense tail of the guidance pass, shared by K6 (coarse-grained observations) and K6p (point observations).  Per
 // pixel: grad_x log p = (g - sigma J_eps^T g) / mu  (src/thor/score.py:48-60; the second term only with exact_grad);
 // eps_guided = eps - sigma * grad  =>  per-pixel correction sigma (g - sigma vjp) / mu.  Mode 0 then updates x in place
-// (and stores the boundary frames into the neighbours' halo mailboxes), mode 1 writes eps_guided and the CTA's partial
-// sum of its squares.  The observation policy `Obs` walks this thread's pixels (first / end / step, pixel(i) = index
-// within the frame) and gives the likelihood cotangent g of pixel i: g4 for float4 pixels, entry + g for scalar lanes.
-template <class Obs>
-__device__ __forceinline__ void guide_tail4(const GuideParams& p, const Obs& obs, long long fbase) {
+// (and, C = 4, stores the boundary frames into the neighbours' halo mailboxes), mode 1 writes eps_guided and the CTA's
+// partial sum of its squares, mode 2 writes g alone to cot_out.  The observation policy `Obs` walks this thread's pixels
+// (first / end / step, pixel(i) = index within the frame) and gives the likelihood cotangent g(p, i, o) of pixel i at
+// element offset o.
+template <int C, class Obs>
+__device__ __forceinline__ void guide_tail(const GuideParams& p, const Obs& obs, long long fbase) {
+  if (p.mode == 2) {
+    for (int i = obs.first(); i < obs.end(); i += obs.step()) {
+      const long long o = (fbase + obs.pixel(i)) * C;
+      store_vars<C>(p.cot_out + o, obs.g(p, i, o));
+    }
+    return;
+  }
   const int lane = threadIdx.x & 31;
   const float inv_mu = 1.0f / p.mu;
   const float sg_mu = p.sigma * inv_mu;
   float sq = 0.f;
   bool bad = false;
+#pragma unroll 1  // unrolled, K6p for C = 1 spills around the division slow path; C = 4 is not unrolled either way
   for (int i = obs.first(); i < obs.end(); i += obs.step()) {
     const long long pix_in_frame = obs.pixel(i);
-    const long long o = (fbase + pix_in_frame) * 4;
-    float4 ev = *reinterpret_cast<const float4*>(p.eps + o);
-    float4 gv = obs.g4(p, i, o, ev);
+    const long long o = (fbase + pix_in_frame) * C;
+    Vars<C> ev = load_vars<C>(p.eps + o);
+    Vars<C> gv = obs.g(p, i, o);
     if (p.vjp != nullptr) {
-      const float4 jv = *reinterpret_cast<const float4*>(p.vjp + o);
-      gv.x -= p.sigma * jv.x;
-      gv.y -= p.sigma * jv.y;
-      gv.z -= p.sigma * jv.z;
-      gv.w -= p.sigma * jv.w;
+      const Vars<C> jv = load_vars<C>(p.vjp + o);
+#pragma unroll
+      for (int c = 0; c < C; ++c) gv[c] -= p.sigma * jv[c];
     }
-    ev.x -= sg_mu * gv.x;
-    ev.y -= sg_mu * gv.y;
-    ev.z -= sg_mu * gv.z;
-    ev.w -= sg_mu * gv.w;
+#pragma unroll
+    for (int c = 0; c < C; ++c) ev[c] = __fmaf_rn(-sg_mu, gv[c], ev[c]);  // fused even where g is uniform (K6, no vjp)
     if (p.mode == 0) {
-      float4 xv = *reinterpret_cast<const float4*>(p.x + o);
-      // x0 = (x - sigma eps)/mu ; x <- mu' x0 + sigma' eps     (src/thor/pipelines.py:41-46)
-      xv.x = p.mu_next * ((xv.x - p.sigma * ev.x) * inv_mu) + p.sigma_next * ev.x;
-      xv.y = p.mu_next * ((xv.y - p.sigma * ev.y) * inv_mu) + p.sigma_next * ev.y;
-      xv.z = p.mu_next * ((xv.z - p.sigma * ev.z) * inv_mu) + p.sigma_next * ev.z;
-      xv.w = p.mu_next * ((xv.w - p.sigma * ev.w) * inv_mu) + p.sigma_next * ev.w;
-      bad |= !(isfinite(xv.x) && isfinite(xv.y) && isfinite(xv.z) && isfinite(xv.w));
-      *reinterpret_cast<float4*>(p.x + o) = xv;
-      // boundary frames also go straight into the neighbours' halo mailboxes (peer stores through NVLink)
-      const long long hw = static_cast<long long>(p.H) * p.W;
-      const int own_idx = static_cast<int>(blockIdx.y);
-      if (p.push_l != nullptr && own_idx < p.halo_k) p.push_l[own_idx * hw + pix_in_frame] = xv;
-      if (p.push_r != nullptr && own_idx >= p.own_n - p.halo_k)
-        p.push_r[(own_idx - (p.own_n - p.halo_k)) * hw + pix_in_frame] = xv;
+      Vars<C> xv = load_vars<C>(p.x + o);
+#pragma unroll
+      for (int c = 0; c < C; ++c) {
+        // x0 = (x - sigma eps)/mu ; x <- mu' x0 + sigma' eps     (src/thor/pipelines.py:41-46)
+        xv[c] = p.mu_next * ((xv[c] - p.sigma * ev[c]) * inv_mu) + p.sigma_next * ev[c];
+        bad |= !isfinite(xv[c]);
+      }
+      store_vars<C>(p.x + o, xv);
+      if constexpr (C == 4) {
+        // boundary frames also go straight into the neighbours' halo mailboxes (peer stores through NVLink)
+        const float4 xq = make_float4(xv[0], xv[1], xv[2], xv[3]);
+        const long long hw = static_cast<long long>(p.H) * p.W;
+        const int own_idx = static_cast<int>(blockIdx.y);
+        if (p.push_l != nullptr && own_idx < p.halo_k) p.push_l[own_idx * hw + pix_in_frame] = xq;
+        if (p.push_r != nullptr && own_idx >= p.own_n - p.halo_k)
+          p.push_r[(own_idx - (p.own_n - p.halo_k)) * hw + pix_in_frame] = xq;
+      }
     } else {
-      sq += ev.x * ev.x + ev.y * ev.y + ev.z * ev.z + ev.w * ev.w;
-      *reinterpret_cast<float4*>(p.eps_out + o) = ev;
+      float s = ev[0] * ev[0];  // the pixel's sum first, then the thread's
+#pragma unroll
+      for (int c = 1; c < C; ++c) s += ev[c] * ev[c];
+      sq += s;
+      store_vars<C>(p.eps_out + o, ev);
     }
   }
   if (p.mode == 0) {
     if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(p.nan_flag, 1);
-    if (p.push_done != nullptr) {  // fused halo push: fence this CTA's peer stores, the last CTA publishes the step
+    if (C == 4 && p.push_done != nullptr) {  // fused halo push: fence this CTA's peer stores, the last CTA publishes
       __threadfence_system();
       __syncthreads();
       if (threadIdx.x == 0) {
@@ -1667,162 +1640,50 @@ __device__ __forceinline__ void guide_tail4(const GuideParams& p, const Obs& obs
   }
 }
 
-template <class Obs>
-__device__ __forceinline__ void guide_tail_generic(const GuideParams& p, const Obs& obs, long long fbase) {
-  constexpr int MC = 8;
-  const int C = p.C;
-  const int lane = threadIdx.x & 31;
-  const float inv_mu = 1.0f / p.mu;
-  const float sg_mu = p.sigma * inv_mu;
-  float sq = 0.f;
-  bool bad = false;
-  for (int i = obs.first(); i < obs.end(); i += obs.step()) {
-    const long long o = (fbase + obs.pixel(i)) * C;
-    const int e = obs.entry(i);
-#pragma unroll
-    for (int c = 0; c < MC; ++c) {
-      if (c < C) {
-        float gv = obs.g(p, e, o, c);
-        if (p.vjp != nullptr) gv -= p.sigma * p.vjp[o + c];
-        const float ev = p.eps[o + c] - sg_mu * gv;
-        if (p.mode == 0) {
-          const float xv = p.mu_next * ((p.x[o + c] - p.sigma * ev) * inv_mu) + p.sigma_next * ev;
-          bad |= !isfinite(xv);
-          p.x[o + c] = xv;
-        } else {
-          sq += ev * ev;
-          p.eps_out[o + c] = ev;
-        }
-      }
-    }
-  }
-  if (p.mode == 0) {
-    if (__any_sync(0xffffffffu, bad) && lane == 0) atomicOr(p.nan_flag, 1);
-  } else {
-    block_partial(p, sq);
-  }
-}
-
 // K6's observation policy: the warp's s x s tile, whose pixels all get the same cotangent (the tile's residual / s^2).
-struct TileObs4 {
+template <int C>
+struct TileObs {
   int s, h0, w0, W;
-  float4 corr;
+  Vars<C> corr;
   __device__ int first() const { return threadIdx.x & 31; }
   __device__ int end() const { return s * s; }
   __device__ int step() const { return 32; }
   __device__ long long pixel(int i) const { return static_cast<long long>(h0 + i / s) * W + (w0 + i % s); }
-  __device__ float4 g4(const GuideParams&, int, long long, float4) const { return corr; }
-};
-struct TileObsC {
-  int s, h0, w0, W;
-  float corr[8];
-  __device__ int first() const { return threadIdx.x & 31; }
-  __device__ int end() const { return s * s; }
-  __device__ int step() const { return 32; }
-  __device__ long long pixel(int i) const { return static_cast<long long>(h0 + i / s) * W + (w0 + i % s); }
-  __device__ int entry(int) const { return 0; }
-  __device__ float g(const GuideParams&, int, long long, int c) const { return corr[c]; }
+  __device__ Vars<C> g(const GuideParams&, int, long long) const { return corr; }
 };
 
 // CTA = one s-row strip of one frame; one warp per s x s observation tile (warp-shuffle tile mean, deterministic).
+template <int C>
 __global__ void guided_step_kernel(const GuideParams p) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int s = p.s_step;
   const int fl = p.own_lo + blockIdx.y;
   const int fg = p.frame_global0 + fl;
-  const int h0 = blockIdx.x * s, w0 = warp * s;
   const long long fbase = (static_cast<long long>(fl) * p.H) * p.W;
   const bool observed = (p.y != nullptr) && (fg % p.t_step == 0);
   const float inv_mu = 1.0f / p.mu;
-  float4 corr = make_float4(0.f, 0.f, 0.f, 0.f);  // eps_guided = eps - corr   (src/thor/score.py:35)
+  TileObs<C> obs{s, static_cast<int>(blockIdx.x) * s, warp * s, p.W, {}};  // eps_guided = eps - corr (score.py:35)
   if (observed) {
-    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    Vars<C> acc{};
     for (int i = lane; i < s * s; i += 32) {
-      const long long o = (fbase + static_cast<long long>(h0 + i / s) * p.W + (w0 + i % s)) * 4;
-      const float4 xv = *reinterpret_cast<const float4*>(p.x + o);
-      const float4 ev = *reinterpret_cast<const float4*>(p.eps + o);
-      acc.x += (xv.x - p.sigma * ev.x) * inv_mu;
-      acc.y += (xv.y - p.sigma * ev.y) * inv_mu;
-      acc.z += (xv.z - p.sigma * ev.z) * inv_mu;
-      acc.w += (xv.w - p.sigma * ev.w) * inv_mu;
+      const long long o = (fbase + obs.pixel(i)) * C;
+      const Vars<C> xv = load_vars<C>(p.x + o), ev = load_vars<C>(p.eps + o);
+#pragma unroll
+      for (int c = 0; c < C; ++c) acc[c] += (xv[c] - p.sigma * ev[c]) * inv_mu;
     }
     const float inv_area = 1.0f / static_cast<float>(s * s);
-    const float mean[4] = {warp_sum(acc.x) * inv_area, warp_sum(acc.y) * inv_area, warp_sum(acc.z) * inv_area,
-                           warp_sum(acc.w) * inv_area};
     const int Hs = p.H / s, Ws = p.W / s;
     const int m = fg / p.t_step;
     const float r2 = (p.sigma * inv_mu) * (p.sigma * inv_mu);
-    float c[4];
 #pragma unroll
-    for (int ch = 0; ch < 4; ++ch) {
-      const float yv = __ldg(p.y + ((static_cast<long long>(m) * 4 + ch) * Hs + blockIdx.x) * Ws + warp);
-      const float err = yv - mean[ch];
-      const float var = p.std2[ch] + p.gamma[ch] * r2;
+    for (int c = 0; c < C; ++c) {
+      const float mean = warp_sum(acc[c]) * inv_area;
+      const float yv = __ldg(p.y + ((static_cast<long long>(m) * C + c) * Hs + blockIdx.x) * Ws + warp);
       // g = A^T(err / var): each pixel of the tile gets err/var / s^2
-      c[ch] = (err / var) * inv_area;
-    }
-    corr = make_float4(c[0], c[1], c[2], c[3]);
-  }
-  if (p.mode == 2) {
-    for (int i = lane; i < s * s; i += 32) {
-      const long long o = (fbase + static_cast<long long>(h0 + i / s) * p.W + (w0 + i % s)) * 4;
-      *reinterpret_cast<float4*>(p.cot_out + o) = corr;
-    }
-    return;
-  }
-  guide_tail4(p, TileObs4{s, h0, w0, p.W, corr}, fbase);
-}
-
-// ---- any number of variables per frame (1 <= C <= 8, C != 4): the same arithmetic on [frames, H, W, C] with scalar
-// lanes.  The shipped configs have C = 4 (exp/downscaling.py:101) and never launch these; they keep the reference's
-// generality (src/thor/score.py:68-88 is written for any C) at HBM-bound-kernel cost, without the fused halo push.
-__global__ void guided_step_generic_kernel(const GuideParams p) {
-  constexpr int MC = 8;
-  const int C = p.C;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int s = p.s_step;
-  const int fl = p.own_lo + blockIdx.y;
-  const int fg = p.frame_global0 + fl;
-  const int h0 = blockIdx.x * s, w0 = warp * s;
-  const long long fbase = (static_cast<long long>(fl) * p.H) * p.W;
-  const bool observed = (p.y != nullptr) && (fg % p.t_step == 0);
-  const float inv_mu = 1.0f / p.mu;
-  TileObsC obs{s, h0, w0, p.W, {}};
-#pragma unroll
-  for (int c = 0; c < MC; ++c) obs.corr[c] = 0.f;
-  if (observed) {
-    float acc[MC];
-#pragma unroll
-    for (int c = 0; c < MC; ++c) acc[c] = 0.f;
-    for (int i = lane; i < s * s; i += 32) {
-      const long long o = (fbase + static_cast<long long>(h0 + i / s) * p.W + (w0 + i % s)) * C;
-#pragma unroll
-      for (int c = 0; c < MC; ++c)
-        if (c < C) acc[c] += (p.x[o + c] - p.sigma * p.eps[o + c]) * inv_mu;
-    }
-    const float inv_area = 1.0f / static_cast<float>(s * s);
-    const int Hs = p.H / s, Ws = p.W / s;
-    const int m = fg / p.t_step;
-    const float r2 = (p.sigma * inv_mu) * (p.sigma * inv_mu);
-#pragma unroll
-    for (int c = 0; c < MC; ++c) {
-      if (c < C) {  // C is uniform over the warp: every lane takes part in the shuffle
-        const float mean = warp_sum(acc[c]) * inv_area;
-        const float yv = __ldg(p.y + ((static_cast<long long>(m) * C + c) * Hs + blockIdx.x) * Ws + warp);
-        obs.corr[c] = ((yv - mean) / (p.std2[c] + p.gamma[c] * r2)) * inv_area;
-      }
+      obs.corr[c] = ((yv - mean) / (p.std2[c] + p.gamma[c] * r2)) * inv_area;
     }
   }
-  if (p.mode == 2) {
-    for (int i = lane; i < s * s; i += 32) {
-      const long long o = (fbase + static_cast<long long>(h0 + i / s) * p.W + (w0 + i % s)) * C;
-#pragma unroll
-      for (int c = 0; c < MC; ++c)
-        if (c < C) p.cot_out[o + c] = obs.corr[c];
-    }
-    return;
-  }
-  guide_tail_generic(p, obs, fbase);
+  guide_tail<C>(p, obs, fbase);
 }
 
 // ---- K6p: point observations (PointObservation: variables observed at single grid points of chosen frames).  The
@@ -1848,37 +1709,35 @@ __device__ __forceinline__ float point_g(const GuideParams& p, float ys, float w
 }
 
 // The CTA's pixels: `npix` pixels from `pix0` on; slot == nullptr on a frame without observations.
+template <int C>
 struct StripObs {
   const int* slot;
   const float* ysum;
   const float* wsum;
   long long pix0;
-  int npix, C;
+  int npix;
   __device__ int first() const { return threadIdx.x; }
   __device__ int end() const { return npix; }
   __device__ int step() const { return blockDim.x; }
   __device__ long long pixel(int i) const { return pix0 + i; }
-  __device__ float4 g4(const GuideParams& p, int i, long long o, float4 ev) const {
+  __device__ Vars<C> g(const GuideParams& p, int i, long long o) const {
+    Vars<C> r{};
     const int e = slot ? slot[i] : -1;
-    if (e < 0) return make_float4(0.f, 0.f, 0.f, 0.f);
-    const float4 xv = *reinterpret_cast<const float4*>(p.x + o);
-    const float4 ys = *reinterpret_cast<const float4*>(ysum + 4ll * e);
-    const float4 ws = *reinterpret_cast<const float4*>(wsum + 4ll * e);
-    return make_float4(point_g(p, ys.x, ws.x, xv.x, ev.x, 0), point_g(p, ys.y, ws.y, xv.y, ev.y, 1),
-                       point_g(p, ys.z, ws.z, xv.z, ev.z, 2), point_g(p, ys.w, ws.w, xv.w, ev.w, 3));
-  }
-  __device__ int entry(int i) const { return slot ? slot[i] : -1; }
-  __device__ float g(const GuideParams& p, int e, long long o, int c) const {
-    if (e < 0) return 0.f;
-    const long long k = static_cast<long long>(e) * C + c;
-    return point_g(p, ysum[k], wsum[k], p.x[o + c], p.eps[o + c], c);
+    if (e < 0) return r;
+    const Vars<C> xv = load_vars<C>(p.x + o), ev = load_vars<C>(p.eps + o);
+    const Vars<C> ys = load_vars<C>(ysum + static_cast<long long>(C) * e);
+    const Vars<C> ws = load_vars<C>(wsum + static_cast<long long>(C) * e);
+#pragma unroll
+    for (int c = 0; c < C; ++c) r[c] = point_g(p, ys[c], ws[c], xv[c], ev[c], c);
+    return r;
   }
 };
 
-// Shared by both point kernels: this CTA's strip and, on an observed frame, its pixel -> entry map in `slot`.
-__device__ __forceinline__ StripObs point_strip(const GuideParams& p, const PointParams& q, int* slot) {
+// This CTA's strip and, on an observed frame, its pixel -> entry map in `slot`.
+template <int C>
+__device__ __forceinline__ StripObs<C> point_strip(const GuideParams& p, const PointParams& q, int* slot) {
   const int h0 = blockIdx.x * q.strip_rows;
-  StripObs obs{nullptr, q.ysum, q.wsum, static_cast<long long>(h0) * p.W, min(q.strip_rows, p.H - h0) * p.W, p.C};
+  StripObs<C> obs{nullptr, q.ysum, q.wsum, static_cast<long long>(h0) * p.W, min(q.strip_rows, p.H - h0) * p.W};
   const int os = q.frame_slot[blockIdx.y];
   if (os >= 0) {  // uniform over the CTA
     for (int i = threadIdx.x; i < obs.npix; i += blockDim.x) slot[i] = -1;
@@ -1893,38 +1752,11 @@ __device__ __forceinline__ StripObs point_strip(const GuideParams& p, const Poin
   return obs;
 }
 
+template <int C>
 __global__ void __launch_bounds__(256) guided_points_kernel(const GuideParams p, const PointParams q) {
   __shared__ int slot[C2W_POINT_STRIP_PIX];
   const long long fbase = (static_cast<long long>(p.own_lo + blockIdx.y) * p.H) * p.W;
-  const StripObs obs = point_strip(p, q, slot);
-  if (p.mode == 2) {  // g on the observed pixels, zero elsewhere
-    for (int i = obs.first(); i < obs.end(); i += obs.step()) {
-      const long long o = (fbase + obs.pixel(i)) * 4;
-      float4 gv = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (obs.entry(i) >= 0) gv = obs.g4(p, i, o, *reinterpret_cast<const float4*>(p.eps + o));
-      *reinterpret_cast<float4*>(p.cot_out + o) = gv;
-    }
-    return;
-  }
-  guide_tail4(p, obs, fbase);
-}
-
-__global__ void __launch_bounds__(256) guided_points_generic_kernel(const GuideParams p, const PointParams q) {
-  __shared__ int slot[C2W_POINT_STRIP_PIX];
-  const int C = p.C;
-  const long long fbase = (static_cast<long long>(p.own_lo + blockIdx.y) * p.H) * p.W;
-  const StripObs obs = point_strip(p, q, slot);
-  if (p.mode == 2) {
-    for (int i = obs.first(); i < obs.end(); i += obs.step()) {
-      const long long o = (fbase + obs.pixel(i)) * C;
-      const int e = obs.entry(i);
-#pragma unroll
-      for (int c = 0; c < 8; ++c)
-        if (c < C) p.cot_out[o + c] = obs.g(p, e, o, c);
-    }
-    return;
-  }
-  guide_tail_generic(p, obs, fbase);
+  guide_tail<C>(p, point_strip<C>(p, q, slot), fbase);
 }
 
 // Fold of the window outputs (fp32 [n, hw, cpad], EPI_F32 of the last conv) into the composed score [frames, hw, C]:
@@ -2024,7 +1856,9 @@ __device__ __forceinline__ float2 box_muller(uint32_t a, uint32_t b) {
 
 // x <- x - (delta * eps + sqrt(2 delta) z) * sigma' ,  delta = tau / mean(eps^2)   (src/thor/pipelines.py:84-87)
 // sumsq: the trajectory-global sum of eps^2 (already all-reduced when time-sharded); count = L*C*H*W.
-// z == null: draw z on chip with Philox keyed by the GLOBAL pixel index (identical for any sharding).
+// z == null: draw z on chip with Philox keyed by the GLOBAL pixel index (identical for any sharding): one block of four
+// normals per group of four variables, counter word 3 = group index.
+template <int C>
 __global__ void corrector_update_kernel(float* __restrict__ x, const float* __restrict__ eps,
                                         const float* __restrict__ z, const double* __restrict__ sumsq, double count,
                                         float tau, float sigma_next, long long pix0_global, long long npix,
@@ -2034,56 +1868,30 @@ __global__ void corrector_update_kernel(float* __restrict__ x, const float* __re
   bool bad = false;
   for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < npix;
        i += static_cast<long long>(gridDim.x) * blockDim.x) {
-    float4 xv = *reinterpret_cast<const float4*>(x + i * 4);
-    const float4 ev = *reinterpret_cast<const float4*>(eps + i * 4);
-    float4 zv;
+    Vars<C> xv = load_vars<C>(x + i * C);
+    const Vars<C> ev = load_vars<C>(eps + i * C);
+    Vars<C> zv;
     if (z) {
-      zv = *reinterpret_cast<const float4*>(z + i * 4);
+      zv = load_vars<C>(z + i * C);
     } else {
       const unsigned long long g = static_cast<unsigned long long>(pix0_global + i);
-      const uint4 r = philox4x32_10(make_uint4(static_cast<uint32_t>(g), static_cast<uint32_t>(g >> 32), step_id, 0u),
-                                    make_uint2(static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32)));
-      const float2 n0 = box_muller(r.x, r.y), n1 = box_muller(r.z, r.w);
-      zv = make_float4(n0.x, n0.y, n1.x, n1.y);
-    }
-    xv.x -= (delta * ev.x + zs * zv.x) * sigma_next;
-    xv.y -= (delta * ev.y + zs * zv.y) * sigma_next;
-    xv.z -= (delta * ev.z + zs * zv.z) * sigma_next;
-    xv.w -= (delta * ev.w + zs * zv.w) * sigma_next;
-    bad |= !(isfinite(xv.x) && isfinite(xv.y) && isfinite(xv.z) && isfinite(xv.w));
-    *reinterpret_cast<float4*>(x + i * 4) = xv;
-  }
-  if (bad) atomicOr(nan_flag, 1);
-}
-// The same for C != 4 variables per pixel: one Philox block of four normals per group of four variables (counter word 3
-// = group index, so C = 4 would draw exactly what the kernel above draws).
-__global__ void corrector_update_generic_kernel(float* __restrict__ x, const float* __restrict__ eps,
-                                                const float* __restrict__ z, const double* __restrict__ sumsq, double count,
-                                                float tau, float sigma_next, long long pix0_global, long long npix, int C,
-                                                unsigned long long seed, unsigned int step_id, int* nan_flag) {
-  const float delta = tau / static_cast<float>(sumsq[0] / count);
-  const float zs = sqrtf(2.0f * delta);
-  bool bad = false;
-  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < npix;
-       i += static_cast<long long>(gridDim.x) * blockDim.x) {
-    const unsigned long long g = static_cast<unsigned long long>(pix0_global + i);
-    for (int b = 0; 4 * b < C; ++b) {
-      float zv[4] = {0.f, 0.f, 0.f, 0.f};
-      if (!z) {
+#pragma unroll
+      for (int b = 0; 4 * b < C; ++b) {
         const uint4 r = philox4x32_10(make_uint4(static_cast<uint32_t>(g), static_cast<uint32_t>(g >> 32), step_id,
                                                  static_cast<uint32_t>(b)),
                                       make_uint2(static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32)));
         const float2 n0 = box_muller(r.x, r.y), n1 = box_muller(r.z, r.w);
-        zv[0] = n0.x, zv[1] = n0.y, zv[2] = n1.x, zv[3] = n1.y;
-      }
-      for (int e = 0; e < 4 && 4 * b + e < C; ++e) {
-        const long long o = i * C + 4 * b + e;
-        const float zz = z ? z[o] : zv[e];
-        const float xv = x[o] - (delta * eps[o] + zs * zz) * sigma_next;
-        bad |= !isfinite(xv);
-        x[o] = xv;
+        const float n[4] = {n0.x, n0.y, n1.x, n1.y};
+#pragma unroll
+        for (int e = 0; e < 4 && 4 * b + e < C; ++e) zv[4 * b + e] = n[e];
       }
     }
+#pragma unroll
+    for (int c = 0; c < C; ++c) {
+      xv[c] -= (delta * ev[c] + zs * zv[c]) * sigma_next;
+      bad |= !isfinite(xv[c]);
+    }
+    store_vars<C>(x + i * C, xv);
   }
   if (bad) atomicOr(nan_flag, 1);
 }

@@ -684,13 +684,14 @@ def test_sampler_vs_reference_golden(dev, golden_dir):
     assert relerr(s2, torch.from_numpy(g["sample_one_window"])) < 5e-2
 
 
-@pytest.mark.parametrize("C", [1, 3, 6])
+@pytest.mark.parametrize("C", [1, 2, 3, 6, 8])
 def test_other_variable_counts_vs_oracle(dev, C):
     """The reference's score functions and sampler are written for any number of variables per frame
     (src/thor/score.py:68-88, :111-154); the shipped configs have C = 4 (exp/downscaling.py:101), which is the fused
-    float4 path.  C != 4 runs the generic fold / guidance / corrector / adjoint kernels: composed score, closed-form and
-    exact-gradient guided score and a short predictor-corrector run against the fp32 oracle, same tolerances as the
-    4-variable tests; the fold is index work -> chunk-invariant to the bit."""
+    float4 path.  C != 4 runs the separate fold kernel and the scalar-access instances of the guidance / corrector /
+    adjoint kernels: composed score, closed-form and exact-gradient guided score and a short predictor-corrector run
+    against the fp32 oracle, same tolerances as the 4-variable tests; the fold is index work -> chunk-invariant to the
+    bit; the backward over a window range equals the backward over the same windows as a list."""
     import climate2weather_b200 as c2w
     k, L, H, W = 2, 11, 32, 32
     cfg = dict(SMALL, channels=C * (2 * k + 1))
@@ -743,6 +744,7 @@ def test_other_variable_counts_vs_oracle(dev, C):
         sfe.condition_on(A=c2w.CoarseGrain(3, 8), y=y, std=std, gamma=GAMMA, exact_grad=True)
         ee = relerr(sfe(x.to(dev), t).cpu(), want_e)
         assert ee < 4e-2 and ee < 0.5 * relerr(want_g, want_e), (mw, ee)
+    _assert_backward_range_equals_list(net, x, k, t, dev)
 
 
 def test_per_sample_times_and_dsm_loss(dev, golden_dir):
@@ -981,6 +983,33 @@ def test_unet_vjp_full_arch_vs_oracle_autograd(dev):
     assert e_out < 3e-2 and e < 5e-2
 
 
+def _assert_backward_range_equals_list(net, x, k, t, dev):
+    """c2w_window_score_backward over the contiguous windows [1, nw - 1) and c2w_window_score_backward_sel over the same
+    windows as a list accumulate the same vjp to the bit, and leave the frames no window touches (the first and the
+    last) as they were."""
+    L, C, H, W = x.shape
+    nw = L - 2 * k
+    wins = list(range(1, nw - 1))
+    eng = net.engine(C, 2 * k + 1, H, W, dev, max_windows=len(wins), vjp=True)
+    g = torch.Generator().manual_seed(77 + C)
+    xd = x.permute(0, 2, 3, 1).contiguous().to(dev)
+    cot = torch.randn(L, H, W, C, generator=g).to(dev)
+    base = torch.randn(L, H, W, C, generator=g).to(dev)
+    v_range, v_list = base.clone(), base.clone()
+    eng.window_score(xd, 0, wins[0], len(wins), nw, float(t), torch.empty_like(xd))
+    eng.window_score_backward(cot, 0, wins[0], len(wins), nw, v_range)
+    win_list = torch.tensor(wins, dtype=torch.int32, device=dev)
+    pos = torch.full((nw,), -1, dtype=torch.int32)
+    pos[wins] = torch.arange(len(wins), dtype=torch.int32)
+    pos = pos.to(dev)
+    eng.window_score_sel(xd, 0, win_list, float(t), nw)
+    eng.window_score_backward_sel(cot, 0, win_list, pos, nw, v_list)
+    torch.cuda.synchronize()
+    assert torch.equal(v_range, v_list)
+    assert torch.equal(v_range[[0, L - 1]], base[[0, L - 1]])
+    assert not torch.equal(v_range[1:L - 1], base[1:L - 1])
+
+
 def test_exact_grad_guided_score_vs_oracle(dev):
     """condition_on(exact_grad=True): eps - sigma * d log p / dx with the gradient THROUGH the UNet
     (src/thor/score.py:28-35,48-60), against the oracle's autograd formulation; the chunked backward (2 or 3 windows
@@ -1011,6 +1040,7 @@ def test_exact_grad_guided_score_vs_oracle(dev):
     assert relerr(outs[2], outs[1]) < 1e-5
     for o in outs[1:]:
         assert relerr(o, want) < 4e-2 and relerr(o, outs[0]) < 2e-2
+    _assert_backward_range_equals_list(net, x, k, t, dev)
     # a short exact-grad sampling run stays finite and differs from the approximate one
     pipe = c2w.SDAPipeline()
     sf = c2w.DefaultScoreFunction(net, markov_order=k, noise_process=pipe)

@@ -63,7 +63,7 @@ def _std(C):
     return torch.tensor([0.1 + 0.05 * c for c in range(C)]).reshape(1, C, 1)
 
 
-@pytest.mark.parametrize("C", [4, 3])
+@pytest.mark.parametrize("C", [4, 3, 1, 8])
 def test_point_guidance_kernel_vs_closed_form(C):
     """sf(x, t) - eps (the kernel's correction) against the oracle's A^T((y - A x0)/var) through torch.func.vjp of the
     same operator, from the same GPU eps: fp32 elementwise -> 1e-5; one predictor step the same way; the correction is
