@@ -587,7 +587,9 @@ int build_plan(c2w_handle* h, int n, bool vjp, bool per_t, void* base, size_t* b
     op->spec.mode = mode;
     op->spec.out = out;
     op->spec.stride = stride;
-    const int bn = bn_force ? bn_force : conv_pick_bn_tiled(cout_pad, c3, n, H, W, stride, h->sms);
+    // the fp32 / compose epilogues (the last conv of a pass) store 64-wide tiles only; a wider frame (C * window > 64
+    // channels) takes several of them
+    const int bn = bn_force ? bn_force : mode == EPI_F32 ? 64 : conv_pick_bn_tiled(cout_pad, c3, n, H, W, stride, h->sms);
     if (!conv_launch_init(&op->conv, c3, in, n, H, W, cin, wts, cout_pad, bn, h->sms, stride))
       return fail(C2W_ERR_INVALID, "cannot build conv launch (n=%d H=%d W=%d cin=%d cout=%d stride=%d) %s", n, H, W, cin,
                   cout_pad, stride, tmap_error_slot());

@@ -32,7 +32,7 @@ int c2w_op_conv_ex(const c2w_conv_desc* d, void* stream) {
               "c2w_op_conv_ex: unsupported mode %d", d->mode);
   const int sms = c2w_num_sms();
   C2W_REQUIRE(sms > 0, "c2w_op_conv_ex: no CUDA device");
-  const int bn = d->bn ? d->bn : conv_pick_bn(d->cout_pad);
+  const int bn = d->bn ? d->bn : d->mode == EPI_F32 ? 64 : conv_pick_bn(d->cout_pad);  // fp32 output: 64-wide tiles only
   const int stride = d->stride ? d->stride : 1;
   ConvLaunch L;
   if (!conv_launch_init(&L, d->conv3x3 != 0, static_cast<const __nv_bfloat16*>(d->x), d->n_img, d->H, d->W, d->cin,

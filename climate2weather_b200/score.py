@@ -180,10 +180,42 @@ def _per_channel(v, C: int, name: str):
     return out + [1.0] * (4 - len(out))
 
 
+def _check_observation_shape(op: CoarseGrain, y_shape, L: int, C: int, H: int, W: int) -> tuple:
+    """The shape of A(x) for x of [L, C, H, W], [ceil(L / t), C, H / s, W / s], after two checks.  A (t, s) the
+    guidance kernel cannot run raises NotImplementedError: t or s below 1, s not dividing H and W, more than 32 tiles
+    per row.  A y that does not broadcast to A(x) raises ValueError naming both shapes: the reference computes
+    `y - A(x0)`, while the kernel would read y out of bounds or at the wrong offsets."""
+    t, s = op.t_step, op.s_step
+    if t < 1 or s < 1:
+        raise NotImplementedError(f"{op}: t_step and s_step must be at least 1")
+    if H % s or W % s:
+        raise NotImplementedError(f"{op}: s_step={s} must divide the {H}x{W} grid")
+    if W // s > 32:
+        raise NotImplementedError(f"{op}: {W // s} tiles per row of a {H}x{W} grid; the guidance kernel handles at "
+                                  f"most 32 (s_step >= {-(-W // 32)})")
+    want = (-(-L // t), C, H // s, W // s)
+    try:
+        ok = torch.broadcast_shapes(tuple(y_shape), want) == want
+    except RuntimeError:
+        ok = False
+    if not ok:
+        raise ValueError(f"{op}: observation y of shape {tuple(y_shape)} does not broadcast to A(x) of shape {want} "
+                         f"for a trajectory of [{L}, {C}, {H}, {W}]")
+    return want
+
+
+def coarse_grain_observation(op: CoarseGrain, y, L: int, C: int, H: int, W: int) -> Tensor:
+    """y broadcast to the shape of A(x) and made contiguous: the tensor the guidance kernel reads."""
+    y = torch.as_tensor(y)
+    return torch.broadcast_to(y, _check_observation_shape(op, y.shape, L, C, H, W)).contiguous()
+
+
 def _recognise_operator(A: Callable, L: int, C: int, H: int, W: int, y_shape) -> CoarseGrain:
     """`A` is an opaque Python callable in the reference API.  The fused path implements exactly one operator
-    family (every t-th frame, s x s mean); identify (t, s) from the shapes and verify on a random probe."""
+    family (every t-th frame, s x s mean); identify (t, s) from the shapes and verify on a random probe.  A
+    CoarseGrain is taken as it is.  Either way the operator's limits and y's shape are checked."""
     if isinstance(A, CoarseGrain):
+        _check_observation_shape(A, y_shape, L, C, H, W)
         return A
     Lo, Cy, Hs, Ws = y_shape
     if Cy != C or H % Hs or W % Ws or H // Hs != W // Ws:
@@ -198,6 +230,7 @@ def _recognise_operator(A: Callable, L: int, C: int, H: int, W: int, y_shape) ->
         cand = CoarseGrain(t, s)
         ref = cand(probe)
         if ref.shape == got.shape and torch.allclose(ref, got, rtol=1e-5, atol=1e-6):
+            _check_observation_shape(cand, y_shape, L, C, H, W)
             return cand
     raise NotImplementedError("observation operator A was not recognised as `AvgPool2d(s)(x[::t])`; the fused "
                               "guidance kernel supports only that family (pass climate2weather_b200.CoarseGrain)")
@@ -682,7 +715,10 @@ class AbstractScoreFunction:
                         lk["op"] = _recognise_operator(lk["A"], L, C, H, W, lk["y"].shape)
                     lk["std_c"] = _per_channel(lk["std"], C, "std")
                     lk["gamma_c"] = _per_channel(lk["gamma"], C, "gamma")
-                rt.set_condition(dict(op=lk["op"], y=lk["y"], std=lk["std_c"], gamma=lk["gamma_c"]))
+                y = lk["y"]
+                if isinstance(lk["op"], CoarseGrain):  # checked against this trajectory's geometry, every time
+                    y = coarse_grain_observation(lk["op"], y, L, C, H, W)
+                rt.set_condition(dict(op=lk["op"], y=y, std=lk["std_c"], gamma=lk["gamma_c"]))
             self._runtimes = {key: rt}  # one live trajectory geometry at a time
         else:
             rt.refresh_engine()  # once per score call / sampling run: catches in-place parameter updates

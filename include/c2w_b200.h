@@ -65,13 +65,13 @@ typedef struct c2w_guide {
   int32_t* nan_flag;     /* set to 1 if any updated value is not finite (src/thor/pipelines.py:90-91)      */
   const float* vjp;      /* exact_grad=True: J_eps^T g from c2w_window_score_backward (src/thor/score.py:28-35,
                             48-60 with grad enabled); NULL = closed-form guidance (exact_grad=False)        */
-  float* cot_out;        /* mode 2 output, [frames_local, H, W, 4]                                         */
+  float* cot_out;        /* mode 2 output, [frames_local, H, W, C]                                         */
   void* halo;            /* c2w_halo* or NULL.  mode 0, time-sharded: the halo PUSH is fused into this kernel — the
                             updated pixels of the first / last k owned frames are also stored into the neighbours'
                             mailboxes over NVLink and the last CTA publishes the step; complete with c2w_halo_pull  */
   int32_t halo_k;        /* Markov order k (frames per side)                                                       */
-  int32_t channels;      /* C, variables per frame: 0 or 4 = the shipped configs (one float4 per pixel, every fused
-                            path); 1..8 otherwise run the generic kernels (no fused halo push)                     */
+  int32_t channels;      /* C, variables per frame, 1..8 (0 = 4, the shipped configs); every count runs the same
+                            kernels, instantiated per C; the fused halo push needs C = 4                           */
 } c2w_guide;
 
 /* ---- lifecycle ------------------------------------------------------------------------------------------ */

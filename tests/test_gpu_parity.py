@@ -106,14 +106,15 @@ def test_conv3x3_vs_torch(lib, dev, n, H, W, cin, cout, mode):
 
 
 def test_gemm_mode_vs_torch(lib, dev):
-    """Plain GEMM mode (1x1 Conv1d of the attention blocks): bf16 output 2^-7; fp32 output (64-wide tiles only) 1e-4."""
+    """Plain GEMM mode (1x1 Conv1d of the attention blocks): bf16 output 2^-7; fp32 output 1e-4, in 64-wide tiles, one or
+    several per row (the picked tile for mode 4 with bn = 0)."""
     from climate2weather_b200 import _lib
     g = torch.Generator().manual_seed(7)
-    for M, K, N in [(256, 128, 128), (64, 512, 1536), (200, 576, 64), (384, 512, 512)]:
+    for M, K, N, f32 in [(256, 128, 128, False), (64, 512, 1536, False), (200, 576, 64, True), (384, 512, 512, False),
+                         (200, 128, 192, True)]:
         a = torch.randn(M, K, generator=g).to(dev).to(torch.bfloat16)
         w = (torch.randn(N, K, generator=g) / math.sqrt(K)).to(dev).to(torch.bfloat16)
         b = torch.randn(N, generator=g).to(dev)
-        f32 = N == 64
         out32 = torch.empty(M, N, device=dev) if f32 else None
         out = torch.empty(M, N, device=dev, dtype=torch.bfloat16)
         _lib.check(lib.c2w_op_conv(a.data_ptr(), 1, 1, M, K, w.data_ptr(), N, b.data_ptr(), 4 if f32 else 0, None,
@@ -303,19 +304,22 @@ def test_attention_core(lib, dev, T, C):
 
 @pytest.mark.parametrize("L,k,first,n", [(16, 6, 0, 4), (16, 6, 2, 2), (9, 2, 1, 4)])
 @pytest.mark.parametrize("H,W", [(4, 8), (16, 16), (8, 24)])  # 256 pixels: the tiled kernel (64-pixel tiles); others: generic
-def test_gather_windows_bit_exact(lib, dev, L, k, first, n, H, W):
-    """K0 vs the oracle unfold index map (src/thor/score.py:68-74): pure indexing + one bf16 rounding."""
+@pytest.mark.parametrize("C", [1, 3, 4, 5, 8])  # C != 4: the scalar lanes; k = 6, C = 5 -> 65 channels straddle 64
+def test_gather_windows_bit_exact(lib, dev, C, L, k, first, n, H, W):
+    """K0 vs the oracle unfold index map (src/thor/score.py:68-74): pure indexing + one bf16 rounding; the channels
+    past w*C up to cin_pad = 64 * ceil(w*C / 64) are zero."""
     from climate2weather_b200 import _lib
-    C = 4
     w = 2 * k + 1
+    cin_pad = 64 * -(-w * C // 64)
     x = torch.randn(L, C, H, W, generator=torch.Generator().manual_seed(L))
     traj = x.permute(0, 2, 3, 1).contiguous().to(dev)
-    out = torch.full((n, H * W, 64), 7.0, device=dev, dtype=torch.bfloat16)
-    _lib.check(lib.c2w_op_gather_windows(traj.data_ptr(), out.data_ptr(), n, H * W, C, w, 64, first, stream()), "gather")
+    out = torch.full((n, H * W, cin_pad), 7.0, device=dev, dtype=torch.bfloat16)
+    _lib.check(lib.c2w_op_gather_windows(traj.data_ptr(), out.data_ptr(), n, H * W, C, w, cin_pad, first, stream()),
+               "gather")
     torch.cuda.synchronize()
     ref = score_ref.unfold(x, k)[first:first + n].reshape(n, w * C, H * W).permute(0, 2, 1).to(torch.bfloat16)
     assert torch.equal(out[..., :w * C].cpu(), ref)
-    assert float(out[..., w * C:].abs().max()) == 0.0
+    assert float(out[..., w * C:].abs().max()) == 0.0  # w * C is never a multiple of 64 here
 
 
 # ------------------------------------------------------------------------------------------------ whole network
@@ -437,7 +441,9 @@ def _index_coded_net(dev, k, C, mode):
         "window": out[(tau, c)] = in[(0, c)]        -> with x[f] = f the UNet output is the WINDOW index j
         "slot"  : weights 0, bias[(tau, c)] = tau*C + c   -> the output is the window-CHANNEL index
         "pixel" : out[(tau, c)] = in[(tau, c)]      -> the output is the input pixel (fold o unfold = id)
-    All values are small integers, exact in bf16 operands and fp32 accumulators."""
+        "centre-sum": out[(k, c)] = sum_tau in[(tau, c)], every other output zero
+    All values are small integers, exact in bf16 operands and fp32 accumulators.  The residual branch ends in a zero
+    conv, so its input gradient is exactly 0 and the input-gradient pass is the transpose of the tail alone."""
     import climate2weather_b200 as c2w
     w = 2 * k + 1
     net = c2w.ScoreUNet(channels=C * w, embedding_dim=64, hidden_channels=[128], hidden_blocks=[1], attention_levels=[], activation=torch.nn.SiLU)
@@ -448,26 +454,33 @@ def _index_coded_net(dev, k, C, mode):
             sd["unet.tails.0.weight"][ch, ch % C, 1, 1] = 1.0
         elif mode == "pixel":
             sd["unet.tails.0.weight"][ch, ch, 1, 1] = 1.0
+        elif mode == "centre-sum":
+            sd["unet.tails.0.weight"][k * C + ch % C, ch, 1, 1] = 1.0
         else:
             sd["unet.tails.0.bias"][ch] = float(ch)
     net.load_state_dict(sd)
     return net.to(dev)
 
 
-@pytest.mark.parametrize("L,H,W,chunks", [
+_COMPOSE_CASES = [
     (13, 128, 128, (None, 1)),             # one window: head, centre and tail slots all come from window 0
     (14, 128, 128, (None, 1, 2)),          # two windows; chunk 1 -> first batch != last batch
     (26, 128, 128, (None, 1, 3, 5, 14)),   # ragged last batch (3, 5), first == last (14)
-    (168, 128, 128, (None, 32, 100)),      # BASELINE config 2 geometry: 156 windows
     (40, 16, 64, (None, 7)),
-])
-def test_compose_index_bit_exact(dev, golden_dir, L, H, W, chunks):
-    """K0 gather + K5 compose epilogue (src/thor/score.py:68-88, :111-154) through c2w_window_score on index-coded
-    networks at k = 6: the composed output must equal, as INTEGERS, the (window, window-channel, pixel) the oracle's
-    fold map names — for every chunking of the window range (the batched variant emits the head slots with the first
-    batch and the tail slots with the last, src/thor/score.py:124-141)."""
+]
+_COMPOSE_L168 = (168, 128, 128, (None, 32, 100))  # BASELINE config 2 geometry: 156 windows (C = 4 and one other count)
+
+
+@pytest.mark.parametrize("C,L,H,W,chunks", [(C,) + case for C in range(1, 9) for case in _COMPOSE_CASES] +
+                         [(C,) + _COMPOSE_L168 for C in (4, 3)])
+def test_compose_index_bit_exact(dev, golden_dir, C, L, H, W, chunks):
+    """K0 gather + the fold (K5 compose epilogue for C = 4, compose_generic_kernel for any other count;
+    src/thor/score.py:68-88, :111-154) through c2w_window_score on index-coded networks at k = 6: the composed output
+    must equal, as INTEGERS, the (window, window-channel, pixel) the oracle's fold map names — for every chunking of the
+    window range (the batched variant emits the head slots with the first batch and the tail slots with the last,
+    src/thor/score.py:124-141)."""
     import climate2weather_b200 as c2w
-    k, C = 6, 4
+    k = 6
     f = score_ref.fold_index(L, k, C)  # [L, C, (window, window-channel)], pinned against the reference (index_maps.npz)
     key = f"fold_{L}_{k}_{C}"
     idx = np.load(golden_dir / "index_maps.npz")
@@ -495,13 +508,16 @@ def test_compose_index_bit_exact(dev, golden_dir, L, H, W, chunks):
             assert torch.equal(got, want[mode]), (mode, mw, (got != want[mode]).nonzero()[:4].tolist())
 
 
-@pytest.mark.parametrize("L,split", [(13, "all"), (14, "halves"), (26, "every3"), (168, "observed")])
-def test_compose_by_window_lists_bit_exact(dev, L, split):
+@pytest.mark.parametrize("C,L,split", [(C, L, split) for C in range(1, 9) for L, split in
+                                        ((13, "all"), (14, "halves"), (26, "every3"))] +
+                         [(C, 168, "observed") for C in (4, 3)])
+def test_compose_by_window_lists_bit_exact(dev, C, L, split):
     """c2w_window_score_sel with a score output (exact_grad: the observed selection on the stashing engine, the others on
     the plain one): two window LISTS fold into one eps exactly like the contiguous c2w_window_score — integers out of
-    index-coded networks at k = 6, H = W = 128; lists shorter and longer than a chunk, first / last window in either."""
+    index-coded networks at k = 6, H = W = 128, C variables per frame; lists shorter and longer than a chunk, first /
+    last window in either."""
     import climate2weather_b200 as c2w
-    k, C, H, W = 6, 4, 128, 128
+    k, H, W = 6, 128, 128
     nw = L - 2 * k
     f = score_ref.fold_index(L, k, C)
     frame_code = torch.arange(L, dtype=torch.float32).reshape(L, 1, 1, 1).expand(L, C, H, W).contiguous()
@@ -521,6 +537,59 @@ def test_compose_by_window_lists_bit_exact(dev, L, split):
         got = eps.permute(0, 3, 1, 2).cpu()
         want = torch.from_numpy(f[..., 0 if mode == "window" else 1]).float().reshape(L, C, 1, 1).expand(L, C, H, W)
         assert torch.equal(got, want), (mode, split, (got != want).nonzero()[:4].tolist())
+
+
+@pytest.mark.parametrize("C,k", [(C, 2) for C in range(1, 9)] + [(5, 6), (8, 6)])  # k = 6: C * w > 64 channels
+def test_window_adjoint_index_bit_exact(dev, C, k):
+    """The window adjoints (compose_adjoint_kernel -> input-gradient pass -> unfold_adjoint_kernel) as exact integers,
+    through c2w_window_score_backward (range form) and c2w_window_score_backward_sel (list form), each right after its
+    stashing forward; integer cot and base in [-8, 8] (vjp accumulates onto base):
+      "pixel" (identity Jacobian): vjp[f] = base[f] + cot[f] if the source window of frame f (score_ref.fold_index:
+          centre slot, or the head / tail slots of the first / last window) is in the set, else base[f] to the bit;
+      "centre-sum": vjp[f] = base[f] + sum over windows j of the set with j <= f <= j + 2k of cot[j + k].
+    On the whole trajectory (first / last window in and out of the set) and on time-sharded local slices
+    (frame_global0 > 0)."""
+    nw, H, W = 8, 32, 32
+    w, L = 2 * k + 1, nw + 2 * k
+    src = score_ref.fold_index(L, k, C)[:, 0, 0]  # source window of each global frame
+    g = torch.Generator().manual_seed(90 + C)
+    x, cot, base = (torch.randint(-8, 9, (L, H, W, C), generator=g).float() for _ in range(3))
+    # (local slice [lo, hi), window sets: ranges (first, n) and lists); a set's windows lie inside the slice
+    cases = [((0, L), [(0, nw), (0, 3), (5, 3), (2, 4)], [[0, 2, 5, 7], [1, 4, 6], [7], [0]]),
+             ((3, L), [(3, 5), (4, 2)], [[3, 5, 7], [4, 6]]),   # the last rank's slice: holds the last window
+             ((2, 6 + 2 * k), [(2, 4)], [[2, 5], [3, 4, 5]])]   # a middle rank's slice
+    for mode in ("pixel", "centre-sum"):
+        net = _index_coded_net(dev, k, C, mode)
+        eng = net.engine(C, w, H, W, dev, max_windows=nw, vjp=True)
+        for (lo, hi), ranges, lists in cases:
+            xd, cd = (v[lo:hi].contiguous().to(dev) for v in (x, cot))
+            for wins, contiguous in [(list(range(a, a + n)), True) for a, n in ranges] + [(li, False) for li in lists]:
+                want = base.clone()
+                for f in range(L):
+                    if mode == "pixel":
+                        want[f] += cot[f] if src[f] in wins else 0.0
+                    else:
+                        for j in wins:
+                            if j <= f <= j + 2 * k:
+                                want[f] += cot[j + k]
+                want = want[lo:hi]
+                got = []
+                if contiguous:
+                    v = base[lo:hi].contiguous().to(dev)
+                    eng.window_score(xd, lo, wins[0], len(wins), nw, 0.5, torch.empty_like(xd))
+                    eng.window_score_backward(cd, lo, wins[0], len(wins), nw, v)
+                    got.append(("range", v))
+                wl = torch.tensor(wins, dtype=torch.int32, device=dev)
+                pos = torch.full((nw,), -1, dtype=torch.int32)
+                pos[wins] = torch.arange(len(wins), dtype=torch.int32)
+                v = base[lo:hi].contiguous().to(dev)
+                eng.window_score_sel(xd, lo, wl, 0.5, nw)
+                eng.window_score_backward_sel(cd, lo, wl, pos.to(dev), nw, v)
+                got.append(("list", v))
+                torch.cuda.synchronize()
+                for form, v in got:
+                    v = v.cpu()
+                    assert torch.equal(v, want), (mode, form, (lo, hi), wins, (v != want).nonzero()[:4].tolist())
 
 
 # ------------------------------------------------------------------------------------------------ K6 / K7

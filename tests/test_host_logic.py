@@ -404,3 +404,54 @@ def test_observed_window_selection_is_exactly_the_fold_preimage_of_the_observed_
             p = make_plan(L, k, r, world)
             got += observed_windows(p.win_lo, p.win_hi, p.n_win_global, L, k, t_step)
         assert got == want, world
+
+
+# ------------------------------------------------------------------------------------------------ CoarseGrain conditioning
+def test_coarse_grain_observation_shape_is_checked():
+    """A CoarseGrain passed as `A` is checked against y like a recognised operator: y must broadcast to A(x), which is
+    [ceil(L / t), C, H / s, W / s].  Too few observed frames would make the guidance kernel read past y, too large
+    tiles would make it read y at the wrong offsets; both raise ValueError naming the two shapes."""
+    import re
+
+    from climate2weather_b200 import score as sc
+    L, C, H, W = 11, 4, 32, 32
+    op = sc.CoarseGrain(3, 8)
+    assert sc._recognise_operator(op, L, C, H, W, (4, 4, 4, 4)) is op
+    for bad in ((2, 4, 4, 4), (4, 4, 8, 8), (4, 3, 4, 4)):
+        with pytest.raises(ValueError, match=re.escape(f"{bad}") + ".*" + re.escape("(4, 4, 4, 4)")):
+            sc._recognise_operator(op, L, C, H, W, bad)
+        with pytest.raises(ValueError, match=re.escape(f"{bad}")):
+            sc.coarse_grain_observation(op, torch.zeros(bad), L, C, H, W)
+    # a y that broadcasts (one observation for every observed frame) is uploaded as the full, contiguous A(x) shape
+    y1 = torch.randn(1, C, 4, 4)
+    assert sc._recognise_operator(op, L, C, H, W, tuple(y1.shape)) is op
+    y = sc.coarse_grain_observation(op, y1, L, C, H, W)
+    assert y.shape == (4, C, 4, 4) and y.is_contiguous() and all(torch.equal(y[m], y1[0]) for m in range(4))
+    y4 = torch.randn(4, C, 4, 4)
+    assert torch.equal(sc.coarse_grain_observation(op, y4, L, C, H, W), y4)
+    # an opaque operator of the same family, recognised from the shapes, gets the same checks
+    A = lambda x: torch.nn.functional.avg_pool2d(x[..., ::3, :, :, :], 8, stride=8)
+    got = sc._recognise_operator(A, L, C, H, W, (4, 4, 4, 4))
+    assert (got.t_step, got.s_step) == (3, 8)
+
+
+@pytest.mark.parametrize("t,s,what", [(6, 1, "at most 32"), (6, 2, "at most 32"), (6, 5, "must divide"),
+                                      (0, 16, "at least 1"), (6, 0, "at least 1"), (-1, 16, "at least 1")])
+def test_coarse_grain_limits_raise_at_set_up(t, s, what):
+    """(t, s) the guidance kernel cannot run are refused when the operator is recognised, not at the first guided step:
+    s must divide H and W, leave at most 32 tiles per row (s >= 4 at 128 x 128), and t, s must be at least 1.  The same
+    holds for an opaque operator recognised as that family."""
+    from climate2weather_b200 import score as sc
+    L, C, H, W = 13, 4, 128, 128
+    op = sc.CoarseGrain(t, s)
+    shape = (-(-L // t) if t >= 1 else 1, C, H // s if s >= 1 else 1, W // s if s >= 1 else 1)
+    with pytest.raises(NotImplementedError, match=what):
+        sc._recognise_operator(op, L, C, H, W, shape)
+    with pytest.raises(NotImplementedError, match=what):
+        sc.coarse_grain_observation(op, torch.zeros(shape), L, C, H, W)
+    if t >= 1 and s in (1, 2):
+        A = lambda x: torch.nn.functional.avg_pool2d(x[..., ::t, :, :, :], s, stride=s)
+        with pytest.raises(NotImplementedError, match=what):
+            sc._recognise_operator(A, L, C, H, W, shape)
+    for ok in (4, 8, 16, 32, 64, 128):
+        assert sc._recognise_operator(sc.CoarseGrain(6, ok), L, C, H, W, (3, C, H // ok, W // ok)).s_step == ok
