@@ -6,12 +6,13 @@ Public API mirrors the reference's classes on this path (SURVEY.md §8(b)):
     SDAPipeline                                 <- thor.pipelines.SDAPipeline (alias: VPSDE)
     CoarseGrain                                 <- the observation operator of exp/downscaling.py:129-132
     PointObservation                            <- observations at single grid points (stations, masked data)
+    CombinedObservation                         <- a coarse field and point observations in one likelihood
 The arithmetic lives in libc2w_b200.so (csrc/, C ABI in include/c2w_b200.h); importing this package on a machine
 without the built library works, calling into the path raises.
 """
 from .model import ScoreUNet, build_from_reference
 from .pipelines import SDAPipeline
-from .score import (AbstractScoreFunction, BatchedScoreFunction, CoarseGrain, DefaultScoreFunction,
+from .score import (AbstractScoreFunction, BatchedScoreFunction, CoarseGrain, CombinedObservation, DefaultScoreFunction,
                     PointObservation)
 from .sharding import ShardPlan, make_plan
 
@@ -20,4 +21,4 @@ MCScoreNet = DefaultScoreFunction
 VPSDE = SDAPipeline
 
 __all__ = ["ScoreUNet", "build_from_reference", "SDAPipeline", "AbstractScoreFunction", "DefaultScoreFunction",
-           "BatchedScoreFunction", "CoarseGrain", "PointObservation", "ShardPlan", "make_plan", "MCScoreNet", "VPSDE"]
+           "BatchedScoreFunction", "CoarseGrain", "PointObservation", "CombinedObservation", "ShardPlan", "make_plan", "MCScoreNet", "VPSDE"]

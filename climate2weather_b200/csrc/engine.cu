@@ -1926,6 +1926,17 @@ static int guide_params(const c2w_guide* g, const char* what, GuideParams& p, in
   return C2W_OK;
 }
 
+static PointParams point_params(const c2w_point_obs* obs) {
+  PointParams q;
+  q.frame_slot = obs->frame_slot;
+  q.strip_off = obs->strip_off;
+  q.pix = obs->pix;
+  q.ysum = obs->ysum;
+  q.wsum = obs->wsum;
+  q.strip_rows = obs->strip_rows;
+  return q;
+}
+
 int c2w_guided_step(const c2w_guide* g, void* stream) {
   C2W_REQUIRE(g, "c2w_guided_step: bad argument");
   C2W_REQUIRE(g->s_step >= 1 && g->H % g->s_step == 0 && g->W % g->s_step == 0 && g->W / g->s_step <= 32,
@@ -1953,17 +1964,43 @@ int c2w_guided_step_points(const c2w_guide* g, const c2w_point_obs* obs, void* s
   int C;
   int rc = guide_params(g, "c2w_guided_step_points", p, C);
   if (rc) return rc;
-  PointParams q;
-  q.frame_slot = obs->frame_slot;
-  q.strip_off = obs->strip_off;
-  q.pix = obs->pix;
-  q.ysum = obs->ysum;
-  q.wsum = obs->wsum;
-  q.strip_rows = obs->strip_rows;
+  PointParams q = point_params(obs);
   dim3 grid((g->H + obs->strip_rows - 1) / obs->strip_rows, g->own_n);
   return launch_for_vars(C, [&](auto vars) {
     guided_points_kernel<decltype(vars)::value><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(p, q);
   });
+}
+
+int c2w_guided_step_combined(const c2w_guide* g, const c2w_point_obs* obs, const float* point_std2, void* stream) {
+  C2W_REQUIRE(g && obs && point_std2 && obs->frame_slot && obs->strip_off, "c2w_guided_step_combined: bad argument");
+  C2W_REQUIRE(obs->n_slots == 0 || (obs->pix && obs->ysum && obs->wsum), "c2w_guided_step_combined: entries missing");
+  C2W_REQUIRE(g->y, "c2w_guided_step_combined: needs the coarse observation y");
+  C2W_REQUIRE(g->H >= 1 && g->W >= 1, "c2w_guided_step_combined: empty %dx%d grid", g->H, g->W);
+  C2W_REQUIRE(g->s_step >= 1 && g->H % g->s_step == 0 && g->W % g->s_step == 0 && g->W / g->s_step <= 32,
+              "s_step=%d must divide %dx%d with at most 32 tiles per row", g->s_step, g->H, g->W);
+  C2W_REQUIRE(g->t_step >= 1, "own_n and t_step must be positive");
+  C2W_REQUIRE(obs->strip_rows >= 1 && obs->strip_rows % g->s_step == 0 &&
+                  static_cast<long long>(obs->strip_rows) * g->W <= C2W_COMBINED_STRIP_PIX,
+              "c2w_guided_step_combined: strip of %d rows of %d pixels must be a multiple of s_step=%d and at most %d "
+              "pixels", obs->strip_rows, g->W, g->s_step, C2W_COMBINED_STRIP_PIX);
+  C2W_REQUIRE(g->mode != 2 || g->cot_out, "mode 2 needs cot_out");
+  GuideParams p;
+  int C;
+  int rc = guide_params(g, "c2w_guided_step_combined", p, C);
+  if (rc) return rc;
+  PointParams q = point_params(obs);
+  PointStd2 ps;
+  for (int i = 0; i < C2W_MAX_VARS; ++i) ps.v[i] = i < C ? point_std2[i] : 0.f;
+  const int smem = combined_smem_bytes(obs->strip_rows, g->W, g->s_step, C);
+  dim3 grid((g->H + obs->strip_rows - 1) / obs->strip_rows, g->own_n);
+  cudaError_t attr = cudaSuccess;
+  rc = launch_for_vars(C, [&](auto vars) {
+    const auto kernel = guided_combined_kernel<decltype(vars)::value>;
+    if (smem > 48 * 1024) attr = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (attr == cudaSuccess) kernel<<<grid, 256, smem, static_cast<cudaStream_t>(stream)>>>(p, q, ps);
+  });
+  C2W_CUDA(attr);
+  return rc;
 }
 
 int c2w_reduce_partials(const float* partials, int32_t n, double* sumsq, void* stream) {

@@ -1652,18 +1652,17 @@ struct TileObs {
   __device__ Vars<C> g(const GuideParams&, int, long long) const { return corr; }
 };
 
-// CTA = one s-row strip of one frame; one warp per s x s observation tile (warp-shuffle tile mean, deterministic).
+// If observed: obs.corr <- the cotangent of observation tile (ty, tx) (obs's pixels) of global frame fg at fbase,
+// computed by one warp (every lane gets it): the warp-shuffle tile mean of x0 (lane order, deterministic), then
+// g = A^T(err / var) = err / var / s^2 on each pixel of the tile.  Shared by K6 and K6c: both give a tile the same bits.
+// The test is taken here rather than by the caller so that K6's 1/mu is computed ahead of the branch and shared with
+// guide_tail, as before the block moved here: K6 keeps its instruction schedule and register count.
 template <int C>
-__global__ void guided_step_kernel(const GuideParams p) {
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int s = p.s_step;
-  const int fl = p.own_lo + blockIdx.y;
-  const int fg = p.frame_global0 + fl;
-  const long long fbase = (static_cast<long long>(fl) * p.H) * p.W;
-  const bool observed = (p.y != nullptr) && (fg % p.t_step == 0);
-  const float inv_mu = 1.0f / p.mu;
-  TileObs<C> obs{s, static_cast<int>(blockIdx.x) * s, warp * s, p.W, {}};  // eps_guided = eps - corr (score.py:35)
+__device__ __forceinline__ void tile_cotangent(const GuideParams& p, bool observed, float inv_mu, long long fbase, int fg,
+                                               unsigned ty, int tx, TileObs<C>& obs) {
   if (observed) {
+    const int lane = threadIdx.x & 31;
+    const int s = obs.s;
     Vars<C> acc{};
     for (int i = lane; i < s * s; i += 32) {
       const long long o = (fbase + obs.pixel(i)) * C;
@@ -1678,11 +1677,24 @@ __global__ void guided_step_kernel(const GuideParams p) {
 #pragma unroll
     for (int c = 0; c < C; ++c) {
       const float mean = warp_sum(acc[c]) * inv_area;
-      const float yv = __ldg(p.y + ((static_cast<long long>(m) * C + c) * Hs + blockIdx.x) * Ws + warp);
-      // g = A^T(err / var): each pixel of the tile gets err/var / s^2
+      const float yv = __ldg(p.y + ((static_cast<long long>(m) * C + c) * Hs + ty) * Ws + tx);
       obs.corr[c] = ((yv - mean) / (p.std2[c] + p.gamma[c] * r2)) * inv_area;
     }
   }
+}
+
+// CTA = one s-row strip of one frame; one warp per s x s observation tile.
+template <int C>
+__global__ void guided_step_kernel(const GuideParams p) {
+  const int warp = threadIdx.x >> 5;
+  const int s = p.s_step;
+  const int fl = p.own_lo + blockIdx.y;
+  const int fg = p.frame_global0 + fl;
+  const long long fbase = (static_cast<long long>(fl) * p.H) * p.W;
+  const bool observed = (p.y != nullptr) && (fg % p.t_step == 0);
+  const float inv_mu = 1.0f / p.mu;
+  TileObs<C> obs{s, static_cast<int>(blockIdx.x) * s, warp * s, p.W, {}};  // eps_guided = eps - corr (score.py:35)
+  tile_cotangent<C>(p, observed, inv_mu, fbase, fg, blockIdx.x, warp, obs);
   guide_tail<C>(p, obs, fbase);
 }
 
@@ -1701,11 +1713,12 @@ struct PointParams {
   int strip_rows;
 };
 
-__device__ __forceinline__ float point_g(const GuideParams& p, float ys, float ws, float x, float e, int c) {
+__device__ __forceinline__ float point_g(const GuideParams& p, float ys, float ws, float x, float e, float std2,
+                                         float gamma) {
   const float inv_mu = 1.0f / p.mu;
   const float r2 = (p.sigma * inv_mu) * (p.sigma * inv_mu);
   const float x0 = (x - p.sigma * e) * inv_mu;
-  return (ys - ws * x0) / (p.std2[c] + p.gamma[c] * r2);
+  return (ys - ws * x0) / (std2 + gamma * r2);
 }
 
 // The CTA's pixels: `npix` pixels from `pix0` on; slot == nullptr on a frame without observations.
@@ -1728,7 +1741,7 @@ struct StripObs {
     const Vars<C> ys = load_vars<C>(ysum + static_cast<long long>(C) * e);
     const Vars<C> ws = load_vars<C>(wsum + static_cast<long long>(C) * e);
 #pragma unroll
-    for (int c = 0; c < C; ++c) r[c] = point_g(p, ys[c], ws[c], xv[c], ev[c], c);
+    for (int c = 0; c < C; ++c) r[c] = point_g(p, ys[c], ws[c], xv[c], ev[c], p.std2[c], p.gamma[c]);
     return r;
   }
 };
@@ -1757,6 +1770,79 @@ __global__ void __launch_bounds__(256) guided_points_kernel(const GuideParams p,
   __shared__ int slot[C2W_POINT_STRIP_PIX];
   const long long fbase = (static_cast<long long>(p.own_lo + blockIdx.y) * p.H) * p.W;
   guide_tail<C>(p, point_strip<C>(p, q, slot), fbase);
+}
+
+// ---- K6c: a coarse field and point observations in one likelihood (CombinedObservation).  The cotangent is the sum
+// of the two terms' own, g = A_c^T((y_c - A_c x0)/var_c) + A_p^T((y_p - A_p x0)/var_p), each with its own std^2 per
+// variable (the point term's in PointStd2, gamma shared).  CTA = a strip of q.strip_rows full rows of one owned frame,
+// a multiple of s_step so that every observation tile lies inside one strip.  Phase 1, on a frame with f % t_step == 0:
+// the strip's tile cotangents (tile_cotangent, one warp per tile in turn) go to shared memory.  Phase 2: point_strip's
+// pixel -> entry map, then the dense tail with g = tile term + point term, in that order, each 0 where absent.  Dynamic
+// shared memory: [strip_rows * W] ints of map rounded up to 16 bytes, then [(strip_rows / s) * (W / s)][C] floats of
+// tile cotangents (combined_smem_bytes).
+struct PointStd2 {
+  float v[C2W_MAX_VARS];
+};
+
+__host__ __device__ __forceinline__ int combined_map_ints(int strip_rows, int W) { return (strip_rows * W + 3) & ~3; }
+__host__ __device__ __forceinline__ int combined_smem_bytes(int strip_rows, int W, int s, int C) {
+  return 4 * (combined_map_ints(strip_rows, W) + (strip_rows / s) * (W / s) * C);
+}
+
+template <int C>
+struct CombinedObs {
+  StripObs<C> pts;
+  const float* corr;  // [tiles][C] of this strip; null on a frame without a coarse observation
+  const PointStd2& std2;
+  int s, tiles_w, W;
+  __device__ int first() const { return pts.first(); }
+  __device__ int end() const { return pts.end(); }
+  __device__ int step() const { return pts.step(); }
+  __device__ long long pixel(int i) const { return pts.pixel(i); }
+  __device__ Vars<C> g(const GuideParams& p, int i, long long o) const {
+    Vars<C> r{};
+    if (corr) {
+      const int row = i / W;
+      const Vars<C> t = load_vars<C>(corr + ((row / s) * tiles_w + (i - row * W) / s) * C);
+#pragma unroll
+      for (int c = 0; c < C; ++c) r[c] = t[c];
+    }
+    const int e = pts.slot ? pts.slot[i] : -1;
+    if (e < 0) return r;
+    const Vars<C> xv = load_vars<C>(p.x + o), ev = load_vars<C>(p.eps + o);
+    const Vars<C> ys = load_vars<C>(pts.ysum + static_cast<long long>(C) * e);
+    const Vars<C> ws = load_vars<C>(pts.wsum + static_cast<long long>(C) * e);
+#pragma unroll
+    for (int c = 0; c < C; ++c) r[c] += point_g(p, ys[c], ws[c], xv[c], ev[c], std2.v[c], p.gamma[c]);
+    return r;
+  }
+};
+
+template <int C>
+__global__ void __launch_bounds__(256) guided_combined_kernel(const GuideParams p, const PointParams q,
+                                                              const PointStd2 pstd2) {
+  extern __shared__ __align__(16) int combined_smem[];
+  const int s = p.s_step, tiles_w = p.W / s;
+  const int fl = p.own_lo + blockIdx.y;
+  const int fg = p.frame_global0 + fl;
+  const long long fbase = (static_cast<long long>(fl) * p.H) * p.W;
+  float* corr = reinterpret_cast<float*>(combined_smem + combined_map_ints(q.strip_rows, p.W));
+  const bool coarse = fg % p.t_step == 0;
+  if (coarse) {  // uniform over the CTA
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const float inv_mu = 1.0f / p.mu;
+    const int ty0 = blockIdx.x * (q.strip_rows / s);
+    const int tiles = (min(q.strip_rows, p.H - static_cast<int>(blockIdx.x) * q.strip_rows) / s) * tiles_w;
+    for (int t = warp; t < tiles; t += blockDim.x >> 5) {
+      const int ty = ty0 + t / tiles_w, tx = t % tiles_w;
+      TileObs<C> tile{s, ty * s, tx * s, p.W, {}};
+      tile_cotangent<C>(p, true, inv_mu, fbase, fg, ty, tx, tile);
+      if (lane == 0) store_vars<C>(corr + t * C, tile.corr);
+    }
+    __syncthreads();
+  }
+  const CombinedObs<C> obs{point_strip<C>(p, q, combined_smem), coarse ? corr : nullptr, pstd2, s, tiles_w, p.W};
+  guide_tail<C>(p, obs, fbase);
 }
 
 // Fold of the window outputs (fp32 [n, hw, cpad], EPI_F32 of the last conv) into the composed score [frames, hw, C]:

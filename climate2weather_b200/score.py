@@ -8,6 +8,7 @@ include/c2w_b200.h.  Nothing here computes on the CPU and nothing falls back to 
 from __future__ import annotations
 
 import ctypes
+import math
 from typing import Callable, Optional, Sequence, Union
 
 import numpy as np
@@ -116,6 +117,109 @@ class PointObservation:
         return f"PointObservation(frames={self.n_frames}, points={self.n_points}, masked={self.mask is not None})"
 
 
+class CombinedObservation:
+    """A coarse field and point observations in one likelihood (downscaling with station records):
+
+        A(x) = cat([coarse(x).reshape(-1), points(x).reshape(-1)])
+
+    The terms are independent, so log p(y | x) is the sum of the two terms' own.  Calling the object is the plain torch
+    operator, so the same instance, a flat y and a flat std condition the reference unchanged.  Build y (and a std
+    that differs between the terms) with `pack`; the point block may be NaN under the point mask.
+
+    `condition_on(A=CombinedObservation(...), y=flat, std=..., gamma=...)`: std is a scalar or C per-variable values
+    shared by both terms, or a flat tensor in y's layout that is constant per (term, variable) — a std per individual
+    observation is not supported; gamma is a scalar or C per-variable values shared by both terms."""
+
+    def __init__(self, coarse: CoarseGrain, points: PointObservation):
+        if isinstance(coarse, CombinedObservation) or isinstance(points, CombinedObservation):
+            raise NotImplementedError("CombinedObservation: a set of observation operators cannot hold another set")
+        if type(coarse) is type(points) and isinstance(coarse, (CoarseGrain, PointObservation)):
+            raise NotImplementedError(f"CombinedObservation: at most one operator of each kind, got two "
+                                      f"{type(coarse).__name__}")
+        if not isinstance(coarse, CoarseGrain) or not isinstance(points, PointObservation):
+            raise TypeError(f"CombinedObservation(coarse: CoarseGrain, points: PointObservation), got "
+                            f"({type(coarse).__name__}, {type(points).__name__})")
+        self.coarse, self.points = coarse, points
+
+    def __call__(self, x: Tensor) -> Tensor:
+        return torch.cat([self.coarse(x).reshape(-1), self.points(x).reshape(-1)])
+
+    def term_shapes(self, x_shape) -> tuple:
+        """Shapes of the two terms' observations for a trajectory of x_shape = (L, C, H, W)."""
+        L, C, H, W = (int(v) for v in x_shape)
+        s = self.coarse.s_step
+        return (-(-L // self.coarse.t_step), C, H // s, W // s), (self.points.n_frames, C, self.points.n_points)
+
+    def pack(self, coarse_part, point_part, x_shape) -> Tensor:
+        """The flat tensor in y's layout from the per-term parts, for a trajectory of x_shape = (L, C, H, W).  Each part
+        is a tensor of its term's shape ([ceil(L / t), C, H / s, W / s] and [F, C, P]), a scalar, or C per-variable
+        values; the last two are expanded to the term's shape (an observation std per term)."""
+        parts = []
+        for part, shape, name in zip((coarse_part, point_part), self.term_shapes(x_shape), ("coarse", "point")):
+            t = torch.as_tensor(part).cpu()
+            t = t if t.is_floating_point() else t.float()
+            C = shape[1]
+            if t.numel() == 1:
+                t = t.reshape(-1).expand(math.prod(shape))
+            elif t.numel() == C and math.prod(shape) != C:
+                t = t.reshape(1, C, *([1] * (len(shape) - 2))).expand(shape)
+            elif tuple(t.shape) != shape:
+                raise ValueError(f"{self}: {name} part of shape {tuple(t.shape)} is neither {shape}, a scalar nor "
+                                 f"{C} per-variable values")
+            parts.append(t.reshape(-1))
+        return torch.cat(parts)
+
+    def split(self, flat, x_shape) -> tuple:
+        """The per-term parts (coarse [ceil(L / t), C, H / s, W / s], point [F, C, P]) of a flat tensor in y's layout.
+        Its length must be exactly the sum of both terms' sizes (the coarse block is not broadcast)."""
+        flat = torch.as_tensor(flat)
+        cs, ps = self.term_shapes(x_shape)
+        nc, n = math.prod(cs), math.prod(cs) + math.prod(ps)
+        if flat.dim() != 1 or flat.numel() != n:
+            raise ValueError(f"{self}: y of shape {tuple(flat.shape)} is not 1-D of length {n} ({nc} coarse "
+                             f"{cs} + {n - nc} point {ps} entries) for a trajectory of {list(x_shape)}")
+        return flat[:nc].reshape(cs), flat[nc:].reshape(ps)
+
+    def std_per_term(self, std, x_shape) -> tuple:
+        """(coarse std, point std), C floats each: a scalar or C per-variable values serve both terms; a flat tensor in
+        y's layout must be constant per (term, variable)."""
+        C = int(x_shape[1])
+        t = torch.as_tensor(std, dtype=torch.float32).reshape(-1).cpu()
+        if t.numel() in (1, C):
+            v = _per_channel(t, C, "std")[:C]
+            return v, list(v)
+        cs, ps = self.term_shapes(x_shape)
+        if t.numel() != math.prod(cs) + math.prod(ps):
+            raise ValueError(f"{self}: std has {t.numel()} values; expected a scalar, {C} per-variable values or "
+                             f"{math.prod(cs) + math.prod(ps)} in y's layout")
+        out = []
+        for name, block in zip(("coarse", "point"), self.split(t, x_shape)):
+            per_var = block.transpose(0, 1).reshape(C, -1)
+            if not bool((per_var == per_var[:, :1]).all()):
+                raise ValueError(f"{self}: std varies within the {name} term of a variable; it must be constant per "
+                                 f"(term, variable) (a std per observation is not supported)")
+            out.append([float(v) for v in per_var[:, 0]])
+        return out[0], out[1]
+
+    def observed_frames(self, L: int, C: int) -> list:
+        """Global frames either term observes, ascending."""
+        return sorted(set(range(0, L, self.coarse.t_step)) | set(self.points.observed_frames(C)))
+
+    def __repr__(self):
+        return f"CombinedObservation({self.coarse}, {self.points})"
+
+
+def combined_strip_rows(H: int, W: int, s: int) -> int:
+    """Rows per CTA of the combined guidance kernel: a multiple of s, so that every observation tile lies in one strip,
+    and near POINT_STRIP_PIX pixels — s * max(1, min(H / s, floor(2048 / (s W)))), 16 rows at 128 x 128 with s = 16.
+    The strip's pixel map must fit COMBINED_STRIP_PIX ints (c2w_b200.h: C2W_COMBINED_STRIP_PIX)."""
+    R = s * max(1, min(H // s, POINT_STRIP_PIX // (s * W)))
+    if R * W > COMBINED_STRIP_PIX:
+        raise NotImplementedError(f"CombinedObservation: a strip of {R} rows of {W} pixels (s_step={s}) exceeds the "
+                                  f"{COMBINED_STRIP_PIX} pixels the combined guidance kernel maps")
+    return R
+
+
 def point_strip_rows(H: int, W: int) -> int:
     """Rows per CTA of the point-guidance kernel: the strip's pixel -> entry map fits C2W_POINT_STRIP_PIX ints of static
     shared memory (c2w_b200.h) — 16 rows, 8 KB at 128 x 128."""
@@ -123,9 +227,11 @@ def point_strip_rows(H: int, W: int) -> int:
 
 
 POINT_STRIP_PIX = 2048  # C2W_POINT_STRIP_PIX
+COMBINED_STRIP_PIX = 16384  # C2W_COMBINED_STRIP_PIX
 
 
-def point_plan(op: PointObservation, y, L: int, C: int, H: int, W: int, frame_lo: int, frame_hi: int, strip: int) -> dict:
+def point_plan(op: PointObservation, y, L: int, C: int, H: int, W: int, frame_lo: int, frame_hi: int, strip: int,
+               max_strip_pix: int = POINT_STRIP_PIX) -> dict:
     """The device form of a point observation for the owned global frames [frame_lo, frame_hi) (c2w_point_obs).
 
     Observations of one (frame, pixel) merge into one entry: per variable ysum = sum(mask * y), wsum = sum(mask), summed
@@ -138,8 +244,8 @@ def point_plan(op: PointObservation, y, L: int, C: int, H: int, W: int, frame_lo
     op.check_geometry(L, C, H, W)
     if y.shape[1] != C:
         raise ValueError(f"PointObservation: y has {y.shape[1]} variables, the trajectory {C}")
-    if strip < 1 or strip * W > POINT_STRIP_PIX:
-        raise ValueError(f"strip of {strip} rows of {W} pixels exceeds {POINT_STRIP_PIX} pixels")
+    if strip < 1 or strip * W > max_strip_pix:
+        raise ValueError(f"strip of {strip} rows of {W} pixels exceeds {max_strip_pix} pixels")
     n_own = frame_hi - frame_lo
     frames = op.frames.numpy()
     pix = (op.rows * W + op.cols).numpy()
@@ -326,7 +432,10 @@ class _Runtime:
         """Global indices of this rank's windows whose OUTPUT carries a non-zero cotangent (see `observed_windows`)."""
         p = self.plan
         op = self.cond["op"]
-        obs = op.observed_frames(self.C) if isinstance(op, PointObservation) else op.t_step
+        if isinstance(op, CombinedObservation):
+            obs = op.observed_frames(self.L, self.C)
+        else:
+            obs = op.observed_frames(self.C) if isinstance(op, PointObservation) else op.t_step
         return observed_windows(p.win_lo, p.win_hi, p.n_win_global, self.L, self.sf.markov_order, obs)
 
     def _selection(self):
@@ -422,11 +531,14 @@ class _Runtime:
         self.cond = cond
         self._sel = None
         self.points = None
-        if cond is not None and isinstance(cond["op"], PointObservation):
+        if cond is not None and isinstance(cond["op"], (PointObservation, CombinedObservation)):
             # this rank's owned frames only, built once per conditioning and trajectory geometry
             p = self.plan
-            pl = point_plan(cond["op"], cond["y"], self.L, self.C, self.H, self.W, p.own_lo, p.own_lo + p.own_n,
-                            point_strip_rows(self.H, self.W))
+            op, y, strip, max_pix = cond["op"], cond["y"], point_strip_rows(self.H, self.W), POINT_STRIP_PIX
+            if isinstance(op, CombinedObservation):  # strips of whole observation tiles (guided_combined_kernel)
+                op, y, max_pix = op.points, cond["point_y"], COMBINED_STRIP_PIX
+                strip = combined_strip_rows(self.H, self.W, cond["op"].coarse.s_step)
+            pl = point_plan(op, y, self.L, self.C, self.H, self.W, p.own_lo, p.own_lo + p.own_n, strip, max_pix)
             dev = {n: torch.as_tensor(pl[n]).to(self.device) for n in ("frame_slot", "strip_off", "pix", "ysum", "wsum")}
             for n in ("pix", "ysum", "wsum"):  # no entries on this rank: still a valid pointer
                 if dev[n].numel() == 0:
@@ -438,7 +550,7 @@ class _Runtime:
             self.points = dict(obs=ob, tensors=dev, n_strips=pl["n_strips"])
         if cond is not None and self.exact:
             self.refresh_engine()  # the stashing workspace is sized by the selection
-        if cond is not None and self.points is None:
+        if cond is not None and not isinstance(cond["op"], PointObservation):
             self.y_dev = cond["y"].to(device=self.device, dtype=torch.float32).contiguous()
 
     def _guide(self, mode: int, mu: float, sigma: float, mu_next: float, sigma_next: float, frames=None) -> None:
@@ -447,13 +559,14 @@ class _Runtime:
         g.x, g.eps = self.x.data_ptr(), self.eps.data_ptr()
         s = self.s_tile
         pts = self.points if self.cond is not None else None
-        if pts is not None:  # point observations: y, t_step and s_step are not read
+        combined = pts is not None and isinstance(self.cond["op"], CombinedObservation)
+        if pts is not None and not combined:  # point observations: y, t_step and s_step are not read
             g.y, g.t_step = None, 1
             for i in range(self.C):
                 g.std2[i] = self.cond["std"][i] ** 2
                 g.gamma[i] = self.cond["gamma"][i]
-        elif self.cond is not None:
-            cg: CoarseGrain = self.cond["op"]
+        elif self.cond is not None:  # the coarse term (of a CombinedObservation: the point term is in pts)
+            cg: CoarseGrain = self.cond["op"].coarse if combined else self.cond["op"]
             s = cg.s_step
             g.y = self.y_dev.data_ptr()
             g.t_step = cg.t_step
@@ -488,7 +601,11 @@ class _Runtime:
             g.eps_out, g.partials = self.eps_g.data_ptr(), self.partials.data_ptr()
             self._n_part = n_part
         with torch.cuda.device(self.device):
-            if pts is not None:
+            if combined:
+                pstd2 = (ctypes.c_float * self.C)(*(v ** 2 for v in self.cond["point_std"]))
+                _lib.check(self.lib.c2w_guided_step_combined(ctypes.byref(g), ctypes.byref(pts["obs"]), pstd2, self.stream),
+                           "c2w_guided_step_combined")
+            elif pts is not None:
                 _lib.check(self.lib.c2w_guided_step_points(ctypes.byref(g), ctypes.byref(pts["obs"]), self.stream),
                            "c2w_guided_step_points")
             else:
@@ -632,6 +749,9 @@ class AbstractScoreFunction:
         J = (g - sigma J_eps^T g)/mu with g = A^T((y - A x0)/var), computed by the UNet input-gradient kernels."""
         if isinstance(A, PointObservation):
             A.check_observation(torch.as_tensor(y))
+        if isinstance(A, CombinedObservation) and torch.as_tensor(y).dim() != 1:
+            raise ValueError(f"{A}: y must be the flat tensor A(x) gives (CombinedObservation.pack), got shape "
+                             f"{tuple(torch.as_tensor(y).shape)}")
         if self.likelihood is not None:
             print("Warning: Overwriting old conditioning")
         self.likelihood = dict(A=A, y=torch.as_tensor(y), std=std, gamma=gamma, op=None, exact=bool(exact_grad))
@@ -709,16 +829,23 @@ class AbstractScoreFunction:
             if self.likelihood is not None:
                 lk = self.likelihood
                 if lk["op"] is None:
-                    if isinstance(lk["A"], PointObservation):  # geometry checks run in point_plan (set_condition)
+                    # geometry checks run in point_plan (set_condition) and, for the coarse term, below
+                    if isinstance(lk["A"], (PointObservation, CombinedObservation)):
                         lk["op"] = lk["A"]
                     else:
                         lk["op"] = _recognise_operator(lk["A"], L, C, H, W, lk["y"].shape)
-                    lk["std_c"] = _per_channel(lk["std"], C, "std")
                     lk["gamma_c"] = _per_channel(lk["gamma"], C, "gamma")
-                y = lk["y"]
-                if isinstance(lk["op"], CoarseGrain):  # checked against this trajectory's geometry, every time
-                    y = coarse_grain_observation(lk["op"], y, L, C, H, W)
-                rt.set_condition(dict(op=lk["op"], y=y, std=lk["std_c"], gamma=lk["gamma_c"]))
+                op, y = lk["op"], lk["y"]
+                cond = dict(op=op, gamma=lk["gamma_c"])
+                if isinstance(op, CombinedObservation):  # split and checked against this trajectory's geometry
+                    _check_observation_shape(op.coarse, op.term_shapes(x.shape)[0], L, C, H, W)
+                    y, cond["point_y"] = op.split(y, x.shape)
+                    cond["std"], cond["point_std"] = op.std_per_term(lk["std"], x.shape)
+                else:
+                    cond["std"] = _per_channel(lk["std"], C, "std")
+                if isinstance(op, CoarseGrain):  # checked against this trajectory's geometry, every time
+                    y = coarse_grain_observation(op, y, L, C, H, W)
+                rt.set_condition(dict(cond, y=y))
             self._runtimes = {key: rt}  # one live trajectory geometry at a time
         else:
             rt.refresh_engine()  # once per score call / sampling run: catches in-place parameter updates

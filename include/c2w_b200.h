@@ -199,6 +199,13 @@ typedef struct c2w_point_obs {
  * (modes 0/1/2, vjp, cot_out, nan_flag, halo for C = 4, channels).  Mode 1 writes own_n * ceil(H / strip_rows)
  * partials. */
 int c2w_guided_step_points(const c2w_guide* g, const c2w_point_obs* obs, void* stream);
+/* A coarse field and point observations in one likelihood (CombinedObservation in climate2weather_b200/score.py):
+ * g carries the coarse term (y, t_step, s_step, std2: c2w_guided_step), obs the point term, point_std2 (HOST, channels
+ * floats) the point term's std^2 per variable; gamma is shared.  The cotangent is the sum of the two terms'.  obs is
+ * built with strip_rows a multiple of s_step and strip_rows * W <= C2W_COMBINED_STRIP_PIX (the host library picks
+ * s * max(1, min(H / s, floor(C2W_POINT_STRIP_PIX / (s * W))))).  Mode 1 writes own_n * ceil(H / strip_rows) partials. */
+#define C2W_COMBINED_STRIP_PIX 16384
+int c2w_guided_step_combined(const c2w_guide* g, const c2w_point_obs* obs, const float* point_std2, void* stream);
 int c2w_reduce_partials(const float* partials, int32_t n, double* sumsq, void* stream);
 /* x <- x - (delta eps + sqrt(2 delta) z) sigma_next, delta = tau / (sumsq / count)  (src/thor/pipelines.py:84-87).
  * z == NULL: on-chip Philox4x32-10 keyed by (seed, step_id, global pixel index). */
