@@ -131,6 +131,7 @@ SIGNATURES = {
     "c2w_guided_step": (_i, [C.POINTER(Guide), _vp]),
     "c2w_guided_step_points": (_i, [C.POINTER(Guide), C.POINTER(PointObs), _vp]),
     "c2w_guided_step_combined": (_i, [C.POINTER(Guide), C.POINTER(PointObs), C.POINTER(C.c_float), _vp]),
+    "c2w_guided_step_obs_std": (_i, [C.POINTER(Guide), C.POINTER(PointObs), _vp, _vp, _vp]),
     "c2w_reduce_partials": (_i, [_vp, C.c_int32, _vp, _vp]),
     "c2w_corrector_update": (_i, [_vp, _vp, _vp, _vp, _d, _f, _f, _i64, _i64, C.c_uint64, C.c_uint32, _vp, _vp]),
     "c2w_corrector_update_c": (_i, [_vp, _vp, _vp, _vp, _d, _f, _f, _i64, _i64, C.c_int32, C.c_uint64, C.c_uint32, _vp,

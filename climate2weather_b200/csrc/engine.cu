@@ -1937,8 +1937,11 @@ static PointParams point_params(const c2w_point_obs* obs) {
   return q;
 }
 
-int c2w_guided_step(const c2w_guide* g, void* stream) {
-  C2W_REQUIRE(g, "c2w_guided_step: bad argument");
+// The bodies of c2w_guided_step, c2w_guided_step_points and c2w_guided_step_combined: their argument checks, then
+// the per-variable (PerObs = false) or per-observation (c2w_guided_step_obs_std) instance of K6, K6p or K6c.
+extern "C++" {
+template <bool PerObs>
+static int guided_coarse(const c2w_guide* g, const ObsStd2& v, void* stream) {
   C2W_REQUIRE(g->s_step >= 1 && g->H % g->s_step == 0 && g->W % g->s_step == 0 && g->W / g->s_step <= 32,
               "s_step=%d must divide %dx%d with at most 32 tiles per row", g->s_step, g->H, g->W);
   C2W_REQUIRE(g->mode != 2 || (g->cot_out && g->y), "mode 2 needs cot_out and an observation");
@@ -1949,12 +1952,14 @@ int c2w_guided_step(const c2w_guide* g, void* stream) {
   if (rc) return rc;
   dim3 grid(g->H / g->s_step, g->own_n);
   return launch_for_vars(C, [&](auto vars) {
-    guided_step_kernel<decltype(vars)::value><<<grid, 32 * (g->W / g->s_step), 0, static_cast<cudaStream_t>(stream)>>>(p);
+    guided_step_kernel<decltype(vars)::value, PerObs>
+        <<<grid, 32 * (g->W / g->s_step), 0, static_cast<cudaStream_t>(stream)>>>(p, v);
   });
 }
 
-int c2w_guided_step_points(const c2w_guide* g, const c2w_point_obs* obs, void* stream) {
-  C2W_REQUIRE(g && obs && obs->frame_slot && obs->strip_off, "c2w_guided_step_points: bad argument");
+template <bool PerObs>
+static int guided_points(const c2w_guide* g, const c2w_point_obs* obs, const ObsStd2& v, void* stream) {
+  C2W_REQUIRE(obs->frame_slot && obs->strip_off, "c2w_guided_step_points: bad argument");
   C2W_REQUIRE(obs->n_slots == 0 || (obs->pix && obs->ysum && obs->wsum), "c2w_guided_step_points: entries missing");
   C2W_REQUIRE(g->H >= 1 && g->W >= 1 && obs->strip_rows >= 1 && obs->strip_rows * g->W <= C2W_POINT_STRIP_PIX,
               "c2w_guided_step_points: strip of %d rows of %d pixels exceeds %d pixels", obs->strip_rows, g->W,
@@ -1967,12 +1972,14 @@ int c2w_guided_step_points(const c2w_guide* g, const c2w_point_obs* obs, void* s
   PointParams q = point_params(obs);
   dim3 grid((g->H + obs->strip_rows - 1) / obs->strip_rows, g->own_n);
   return launch_for_vars(C, [&](auto vars) {
-    guided_points_kernel<decltype(vars)::value><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(p, q);
+    guided_points_kernel<decltype(vars)::value, PerObs><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(p, q, v);
   });
 }
 
-int c2w_guided_step_combined(const c2w_guide* g, const c2w_point_obs* obs, const float* point_std2, void* stream) {
-  C2W_REQUIRE(g && obs && point_std2 && obs->frame_slot && obs->strip_off, "c2w_guided_step_combined: bad argument");
+template <bool PerObs>
+static int guided_combined(const c2w_guide* g, const c2w_point_obs* obs, const float* point_std2, const ObsStd2& v,
+                           void* stream) {
+  C2W_REQUIRE(obs->frame_slot && obs->strip_off, "c2w_guided_step_combined: bad argument");
   C2W_REQUIRE(obs->n_slots == 0 || (obs->pix && obs->ysum && obs->wsum), "c2w_guided_step_combined: entries missing");
   C2W_REQUIRE(g->y, "c2w_guided_step_combined: needs the coarse observation y");
   C2W_REQUIRE(g->H >= 1 && g->W >= 1, "c2w_guided_step_combined: empty %dx%d grid", g->H, g->W);
@@ -1990,17 +1997,47 @@ int c2w_guided_step_combined(const c2w_guide* g, const c2w_point_obs* obs, const
   if (rc) return rc;
   PointParams q = point_params(obs);
   PointStd2 ps;
-  for (int i = 0; i < C2W_MAX_VARS; ++i) ps.v[i] = i < C ? point_std2[i] : 0.f;
+  for (int i = 0; i < C2W_MAX_VARS; ++i) ps.v[i] = i < C && !PerObs ? point_std2[i] : 0.f;
   const int smem = combined_smem_bytes(obs->strip_rows, g->W, g->s_step, C);
   dim3 grid((g->H + obs->strip_rows - 1) / obs->strip_rows, g->own_n);
   cudaError_t attr = cudaSuccess;
   rc = launch_for_vars(C, [&](auto vars) {
-    const auto kernel = guided_combined_kernel<decltype(vars)::value>;
+    const auto kernel = guided_combined_kernel<decltype(vars)::value, PerObs>;
     if (smem > 48 * 1024) attr = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (attr == cudaSuccess) kernel<<<grid, 256, smem, static_cast<cudaStream_t>(stream)>>>(p, q, ps);
+    if (attr == cudaSuccess) kernel<<<grid, 256, smem, static_cast<cudaStream_t>(stream)>>>(p, q, ps, v);
   });
   C2W_CUDA(attr);
   return rc;
+}
+}  // extern "C++"
+
+int c2w_guided_step(const c2w_guide* g, void* stream) {
+  C2W_REQUIRE(g, "c2w_guided_step: bad argument");
+  return guided_coarse<false>(g, ObsStd2{}, stream);
+}
+
+int c2w_guided_step_points(const c2w_guide* g, const c2w_point_obs* obs, void* stream) {
+  C2W_REQUIRE(g && obs, "c2w_guided_step_points: bad argument");
+  return guided_points<false>(g, obs, ObsStd2{}, stream);
+}
+
+int c2w_guided_step_combined(const c2w_guide* g, const c2w_point_obs* obs, const float* point_std2, void* stream) {
+  C2W_REQUIRE(g && obs && point_std2, "c2w_guided_step_combined: bad argument");
+  return guided_combined<false>(g, obs, point_std2, ObsStd2{}, stream);
+}
+
+int c2w_guided_step_obs_std(const c2w_guide* g, const c2w_point_obs* obs, const float* coarse_std2,
+                            const float* entry_std2, void* stream) {
+  C2W_REQUIRE(g, "c2w_guided_step_obs_std: bad argument");
+  C2W_REQUIRE((g->y == nullptr) == (coarse_std2 == nullptr),
+              "c2w_guided_step_obs_std: the coarse term needs both g->y and coarse_std2, or neither");
+  C2W_REQUIRE((obs == nullptr) == (entry_std2 == nullptr),
+              "c2w_guided_step_obs_std: the point term needs both obs and entry_std2, or neither");
+  C2W_REQUIRE(g->y || obs, "c2w_guided_step_obs_std: no observation term (needs g->y or obs)");
+  const ObsStd2 v{coarse_std2, entry_std2};
+  if (obs == nullptr) return guided_coarse<true>(g, v, stream);
+  if (g->y == nullptr) return guided_points<true>(g, obs, v, stream);
+  return guided_combined<true>(g, obs, nullptr, v, stream);
 }
 
 int c2w_reduce_partials(const float* partials, int32_t n, double* sumsq, void* stream) {

@@ -1652,14 +1652,24 @@ struct TileObs {
   __device__ Vars<C> g(const GuideParams&, int, long long) const { return corr; }
 };
 
+// The variance source of a guidance kernel.  Per variable (PerObs = false, the default instances): GuideParams::std2,
+// and for K6c's point term PointStd2.  Per observation (PerObs = true, c2w_guided_step_obs_std): std^2 of every
+// observation tile in y's layout [n_obs, C, Hs, Ws], and of every point entry [n_entries, C]; the per-variable std2
+// fields are not read.  Null where the kernel has no such term.
+struct ObsStd2 {
+  const float* tile;
+  const float* entry;
+};
+
 // If observed: obs.corr <- the cotangent of observation tile (ty, tx) (obs's pixels) of global frame fg at fbase,
 // computed by one warp (every lane gets it): the warp-shuffle tile mean of x0 (lane order, deterministic), then
 // g = A^T(err / var) = err / var / s^2 on each pixel of the tile.  Shared by K6 and K6c: both give a tile the same bits.
 // The test is taken here rather than by the caller so that K6's 1/mu is computed ahead of the branch and shared with
-// guide_tail, as before the block moved here: K6 keeps its instruction schedule and register count.
-template <int C>
+// guide_tail, as before the block moved here: K6 keeps its instruction schedule and register count.  PerObs: the tile's
+// std^2 is read from tile_std2 at y's offset, in the same expression.
+template <int C, bool PerObs = false>
 __device__ __forceinline__ void tile_cotangent(const GuideParams& p, bool observed, float inv_mu, long long fbase, int fg,
-                                               unsigned ty, int tx, TileObs<C>& obs) {
+                                               unsigned ty, int tx, TileObs<C>& obs, const float* tile_std2 = nullptr) {
   if (observed) {
     const int lane = threadIdx.x & 31;
     const int s = obs.s;
@@ -1677,15 +1687,17 @@ __device__ __forceinline__ void tile_cotangent(const GuideParams& p, bool observ
 #pragma unroll
     for (int c = 0; c < C; ++c) {
       const float mean = warp_sum(acc[c]) * inv_area;
-      const float yv = __ldg(p.y + ((static_cast<long long>(m) * C + c) * Hs + ty) * Ws + tx);
-      obs.corr[c] = ((yv - mean) / (p.std2[c] + p.gamma[c] * r2)) * inv_area;
+      const long long yi = ((static_cast<long long>(m) * C + c) * Hs + ty) * Ws + tx;
+      const float yv = __ldg(p.y + yi);
+      const float std2 = PerObs ? __ldg(tile_std2 + yi) : p.std2[c];
+      obs.corr[c] = ((yv - mean) / (std2 + p.gamma[c] * r2)) * inv_area;
     }
   }
 }
 
 // CTA = one s-row strip of one frame; one warp per s x s observation tile.
-template <int C>
-__global__ void guided_step_kernel(const GuideParams p) {
+template <int C, bool PerObs>
+__global__ void guided_step_kernel(const GuideParams p, const ObsStd2 v) {
   const int warp = threadIdx.x >> 5;
   const int s = p.s_step;
   const int fl = p.own_lo + blockIdx.y;
@@ -1694,7 +1706,7 @@ __global__ void guided_step_kernel(const GuideParams p) {
   const bool observed = (p.y != nullptr) && (fg % p.t_step == 0);
   const float inv_mu = 1.0f / p.mu;
   TileObs<C> obs{s, static_cast<int>(blockIdx.x) * s, warp * s, p.W, {}};  // eps_guided = eps - corr (score.py:35)
-  tile_cotangent<C>(p, observed, inv_mu, fbase, fg, blockIdx.x, warp, obs);
+  tile_cotangent<C, PerObs>(p, observed, inv_mu, fbase, fg, blockIdx.x, warp, obs, v.tile);
   guide_tail<C>(p, obs, fbase);
 }
 
@@ -1704,6 +1716,9 @@ __global__ void guided_step_kernel(const GuideParams p) {
 // `strip_rows` full rows of one owned frame; an observed frame first scatters the strip's entries (CSR by frame slot
 // and strip) into a shared-memory map pixel -> entry, then runs the dense tail above with g computed from the x and
 // eps it loads anyway.  Entries are unique per pixel: no atomics, bit-identical from run to run and under sharding.
+// PerObs (a std per observation): observations merge only where their std^2 agree, so a pixel may hold a run of
+// consecutive entries (never crossing a strip), each with its own std^2 per variable.  The map holds the run's head;
+// g adds the run's entries in entry order, still without atomics.
 struct PointParams {
   const int* frame_slot;  // [own_n] observed slot of owned frame own_lo + i, or -1
   const int* strip_off;   // [n_slots * n_strips + 1] CSR offsets into the entries
@@ -1721,14 +1736,18 @@ __device__ __forceinline__ float point_g(const GuideParams& p, float ys, float w
   return (ys - ws * x0) / (std2 + gamma * r2);
 }
 
-// The CTA's pixels: `npix` pixels from `pix0` on; slot == nullptr on a frame without observations.
-template <int C>
+// The CTA's pixels: `npix` pixels from `pix0` on; slot == nullptr on a frame without observations.  PerObs: also the
+// entries' pixels, their std^2 [n_entries][C] and the strip's end entry, to walk a run.
+template <int C, bool PerObs = false>
 struct StripObs {
   const int* slot;
   const float* ysum;
   const float* wsum;
   long long pix0;
   int npix;
+  const int* pix = nullptr;
+  const float* std2 = nullptr;
+  int e_end = 0;
   __device__ int first() const { return threadIdx.x; }
   __device__ int end() const { return npix; }
   __device__ int step() const { return blockDim.x; }
@@ -1738,19 +1757,38 @@ struct StripObs {
     const int e = slot ? slot[i] : -1;
     if (e < 0) return r;
     const Vars<C> xv = load_vars<C>(p.x + o), ev = load_vars<C>(p.eps + o);
-    const Vars<C> ys = load_vars<C>(ysum + static_cast<long long>(C) * e);
-    const Vars<C> ws = load_vars<C>(wsum + static_cast<long long>(C) * e);
+    if constexpr (PerObs) {
 #pragma unroll
-    for (int c = 0; c < C; ++c) r[c] = point_g(p, ys[c], ws[c], xv[c], ev[c], p.std2[c], p.gamma[c]);
+      for (int c = 0; c < C; ++c) r[c] = -0.0f;  // -0 + v == v for every v: the run's first term is taken as it is
+      add_run(p, e, xv, ev, r);
+    } else {
+      const Vars<C> ys = load_vars<C>(ysum + static_cast<long long>(C) * e);
+      const Vars<C> ws = load_vars<C>(wsum + static_cast<long long>(C) * e);
+#pragma unroll
+      for (int c = 0; c < C; ++c) r[c] = point_g(p, ys[c], ws[c], xv[c], ev[c], p.std2[c], p.gamma[c]);
+    }
     return r;
+  }
+  // PerObs: r += the point term of every entry of the run headed by e (same pixel, within the strip), in entry order.
+  __device__ void add_run(const GuideParams& p, int e, const Vars<C>& xv, const Vars<C>& ev, Vars<C>& r) const {
+    const int px = pix[e];
+#pragma unroll 1
+    for (int k = e; k < e_end && pix[k] == px; ++k) {
+      const Vars<C> ys = load_vars<C>(ysum + static_cast<long long>(C) * k);
+      const Vars<C> ws = load_vars<C>(wsum + static_cast<long long>(C) * k);
+      const Vars<C> s2 = load_vars<C>(std2 + static_cast<long long>(C) * k);
+#pragma unroll
+      for (int c = 0; c < C; ++c) r[c] += point_g(p, ys[c], ws[c], xv[c], ev[c], s2[c], p.gamma[c]);
+    }
   }
 };
 
-// This CTA's strip and, on an observed frame, its pixel -> entry map in `slot`.
-template <int C>
-__device__ __forceinline__ StripObs<C> point_strip(const GuideParams& p, const PointParams& q, int* slot) {
+// This CTA's strip and, on an observed frame, its pixel -> entry map in `slot` (PerObs: run heads only).
+template <int C, bool PerObs = false>
+__device__ __forceinline__ StripObs<C, PerObs> point_strip(const GuideParams& p, const PointParams& q, int* slot,
+                                                           const float* entry_std2 = nullptr) {
   const int h0 = blockIdx.x * q.strip_rows;
-  StripObs<C> obs{nullptr, q.ysum, q.wsum, static_cast<long long>(h0) * p.W, min(q.strip_rows, p.H - h0) * p.W};
+  StripObs<C, PerObs> obs{nullptr, q.ysum, q.wsum, static_cast<long long>(h0) * p.W, min(q.strip_rows, p.H - h0) * p.W};
   const int os = q.frame_slot[blockIdx.y];
   if (os >= 0) {  // uniform over the CTA
     for (int i = threadIdx.x; i < obs.npix; i += blockDim.x) slot[i] = -1;
@@ -1758,18 +1796,23 @@ __device__ __forceinline__ StripObs<C> point_strip(const GuideParams& p, const P
     const int* off = q.strip_off + static_cast<long long>(os) * gridDim.x + blockIdx.x;
     const int e0 = off[0], e1 = off[1];
     for (int e = e0 + static_cast<int>(threadIdx.x); e < e1; e += blockDim.x)
-      slot[q.pix[e] - static_cast<int>(obs.pix0)] = e;
+      if (!PerObs || e == e0 || q.pix[e - 1] != q.pix[e]) slot[q.pix[e] - static_cast<int>(obs.pix0)] = e;
     __syncthreads();
     obs.slot = slot;
+    if constexpr (PerObs) {
+      obs.pix = q.pix;
+      obs.std2 = entry_std2;
+      obs.e_end = e1;
+    }
   }
   return obs;
 }
 
-template <int C>
-__global__ void __launch_bounds__(256) guided_points_kernel(const GuideParams p, const PointParams q) {
+template <int C, bool PerObs>
+__global__ void __launch_bounds__(256) guided_points_kernel(const GuideParams p, const PointParams q, const ObsStd2 v) {
   __shared__ int slot[C2W_POINT_STRIP_PIX];
   const long long fbase = (static_cast<long long>(p.own_lo + blockIdx.y) * p.H) * p.W;
-  guide_tail<C>(p, point_strip<C>(p, q, slot), fbase);
+  guide_tail<C>(p, point_strip<C, PerObs>(p, q, slot, v.entry), fbase);
 }
 
 // ---- K6c: a coarse field and point observations in one likelihood (CombinedObservation).  The cotangent is the sum
@@ -1789,9 +1832,10 @@ __host__ __device__ __forceinline__ int combined_smem_bytes(int strip_rows, int 
   return 4 * (combined_map_ints(strip_rows, W) + (strip_rows / s) * (W / s) * C);
 }
 
-template <int C>
+// PerObs: the tile term with tile_cotangent's per-tile std^2, the point term over the pixel's run (StripObs::add_run).
+template <int C, bool PerObs = false>
 struct CombinedObs {
-  StripObs<C> pts;
+  StripObs<C, PerObs> pts;
   const float* corr;  // [tiles][C] of this strip; null on a frame without a coarse observation
   const PointStd2& std2;
   int s, tiles_w, W;
@@ -1810,17 +1854,22 @@ struct CombinedObs {
     const int e = pts.slot ? pts.slot[i] : -1;
     if (e < 0) return r;
     const Vars<C> xv = load_vars<C>(p.x + o), ev = load_vars<C>(p.eps + o);
-    const Vars<C> ys = load_vars<C>(pts.ysum + static_cast<long long>(C) * e);
-    const Vars<C> ws = load_vars<C>(pts.wsum + static_cast<long long>(C) * e);
+    if constexpr (PerObs) {
+      pts.add_run(p, e, xv, ev, r);
+    } else {
+      const Vars<C> ys = load_vars<C>(pts.ysum + static_cast<long long>(C) * e);
+      const Vars<C> ws = load_vars<C>(pts.wsum + static_cast<long long>(C) * e);
 #pragma unroll
-    for (int c = 0; c < C; ++c) r[c] += point_g(p, ys[c], ws[c], xv[c], ev[c], std2.v[c], p.gamma[c]);
+      for (int c = 0; c < C; ++c) r[c] += point_g(p, ys[c], ws[c], xv[c], ev[c], std2.v[c], p.gamma[c]);
+    }
     return r;
   }
 };
 
-template <int C>
+// PerObs: pstd2 is not read; the variances come from v.
+template <int C, bool PerObs>
 __global__ void __launch_bounds__(256) guided_combined_kernel(const GuideParams p, const PointParams q,
-                                                              const PointStd2 pstd2) {
+                                                              const PointStd2 pstd2, const ObsStd2 v) {
   extern __shared__ __align__(16) int combined_smem[];
   const int s = p.s_step, tiles_w = p.W / s;
   const int fl = p.own_lo + blockIdx.y;
@@ -1836,12 +1885,13 @@ __global__ void __launch_bounds__(256) guided_combined_kernel(const GuideParams 
     for (int t = warp; t < tiles; t += blockDim.x >> 5) {
       const int ty = ty0 + t / tiles_w, tx = t % tiles_w;
       TileObs<C> tile{s, ty * s, tx * s, p.W, {}};
-      tile_cotangent<C>(p, true, inv_mu, fbase, fg, ty, tx, tile);
+      tile_cotangent<C, PerObs>(p, true, inv_mu, fbase, fg, ty, tx, tile, v.tile);
       if (lane == 0) store_vars<C>(corr + t * C, tile.corr);
     }
     __syncthreads();
   }
-  const CombinedObs<C> obs{point_strip<C>(p, q, combined_smem), coarse ? corr : nullptr, pstd2, s, tiles_w, p.W};
+  const CombinedObs<C, PerObs> obs{point_strip<C, PerObs>(p, q, combined_smem, v.entry), coarse ? corr : nullptr, pstd2,
+                                   s, tiles_w, p.W};
   guide_tail<C>(p, obs, fbase);
 }
 

@@ -127,8 +127,9 @@ class CombinedObservation:
     that differs between the terms) with `pack`; the point block may be NaN under the point mask.
 
     `condition_on(A=CombinedObservation(...), y=flat, std=..., gamma=...)`: std is a scalar or C per-variable values
-    shared by both terms, or a flat tensor in y's layout that is constant per (term, variable) — a std per individual
-    observation is not supported; gamma is a scalar or C per-variable values shared by both terms."""
+    shared by both terms, or a flat tensor in y's layout (`pack` builds it from per-term parts): constant per (term,
+    variable), or a std per observation (NaN allowed under the point mask, +inf for an observation that should not
+    count); gamma is a scalar or C per-variable values shared by both terms."""
 
     def __init__(self, coarse: CoarseGrain, points: PointObservation):
         if isinstance(coarse, CombinedObservation) or isinstance(points, CombinedObservation):
@@ -201,6 +202,23 @@ class CombinedObservation:
             out.append([float(v) for v in per_var[:, 0]])
         return out[0], out[1]
 
+    def std_per_observation(self, std, x_shape) -> tuple:
+        """(coarse std^2 [ceil(L / t), C, H / s, W / s], point std [F, C, P]), fp32, from a scalar, C per-variable values
+        or a flat tensor in y's layout.  std^2 is fp32(std) * fp32(std) rounded to fp32, as the reference's `std ** 2`.
+        A std that is negative or NaN at an observation (under the point mask it is ignored) raises ValueError."""
+        C = int(x_shape[1])
+        t = torch.as_tensor(std, dtype=torch.float32).reshape(-1).cpu()
+        cs, ps = self.term_shapes(x_shape)
+        if t.numel() in (1, C):
+            t = self.pack(t, t, x_shape)
+        elif t.numel() != math.prod(cs) + math.prod(ps):
+            raise ValueError(f"{self}: std has {t.numel()} values; expected a scalar, {C} per-variable values or "
+                             f"{math.prod(cs) + math.prod(ps)} in y's layout")
+        coarse, point = (b.contiguous() for b in self.split(t, x_shape))
+        _check_std_values(coarse, None, f"{self}: coarse term")
+        _check_std_values(point, self.points.mask_for(C), f"{self}: point term")
+        return coarse * coarse, point
+
     def observed_frames(self, L: int, C: int) -> list:
         """Global frames either term observes, ascending."""
         return sorted(set(range(0, L, self.coarse.t_step)) | set(self.points.observed_frames(C)))
@@ -231,14 +249,20 @@ COMBINED_STRIP_PIX = 16384  # C2W_COMBINED_STRIP_PIX
 
 
 def point_plan(op: PointObservation, y, L: int, C: int, H: int, W: int, frame_lo: int, frame_hi: int, strip: int,
-               max_strip_pix: int = POINT_STRIP_PIX) -> dict:
+               max_strip_pix: int = POINT_STRIP_PIX, std=None) -> dict:
     """The device form of a point observation for the owned global frames [frame_lo, frame_hi) (c2w_point_obs).
 
     Observations of one (frame, pixel) merge into one entry: per variable ysum = sum(mask * y), wsum = sum(mask), summed
     in fp64 in point order and rounded to fp32 once — exact, since sum_p mask_p (y_p - x0) / var = (ysum - wsum x0) / var.
     Entries with wsum = 0 for every variable are dropped.  Entries are sorted by (frame, strip, pixel); frame_slot maps
     owned frame i (global frame_lo + i) to its observed slot or -1, strip_off is the CSR over (slot, strip).  Frames
-    outside [frame_lo, frame_hi) are not kept."""
+    outside [frame_lo, frame_hi) are not kept.
+
+    With `std` (a std per observation, [F, C, P] or broadcasting to it), only observations of one (frame, pixel,
+    variable) with the same fp32 std^2 merge: a pixel's distinct std^2 become a run of consecutive entries, entry j of
+    the run holding the j-th smallest std^2 of every variable (wsum = ysum = 0, std2 = 1 in the slots of a variable
+    with fewer).  An observation with std^2 = inf contributes exactly zero and is left out, as if masked.  The plan then
+    also holds std2 [n_entries, C] fp32."""
     y = torch.as_tensor(y)
     op.check_observation(y)
     op.check_geometry(L, C, H, W)
@@ -255,13 +279,16 @@ def point_plan(op: PointObservation, y, L: int, C: int, H: int, W: int, frame_lo
     yv = np.where(mask[sel], y.detach().cpu().double().numpy()[sel], 0.0)      # [n_sel, C, P]; NaN under the mask -> 0
     wv = mask[sel].astype(np.float64)
     key = ((frames[sel] - frame_lo)[:, None] * (H * W) + pix[None, :]).reshape(-1)  # (local frame, pixel)
-    uk, inv = np.unique(key, return_inverse=True)                                  # sorted: frame, then pixel
-    ysum = np.zeros((uk.size, C))
-    wsum = np.zeros((uk.size, C))
-    np.add.at(ysum, inv, yv.transpose(0, 2, 1).reshape(-1, C))
-    np.add.at(wsum, inv, wv.transpose(0, 2, 1).reshape(-1, C))
-    keep = (wsum > 0).any(1)
-    uk, ysum, wsum = uk[keep], ysum[keep], wsum[keep]
+    if std is None:
+        uk, inv = np.unique(key, return_inverse=True)                              # sorted: frame, then pixel
+        ysum = np.zeros((uk.size, C))
+        wsum = np.zeros((uk.size, C))
+        np.add.at(ysum, inv, yv.transpose(0, 2, 1).reshape(-1, C))
+        np.add.at(wsum, inv, wv.transpose(0, 2, 1).reshape(-1, C))
+        keep = (wsum > 0).any(1)
+        uk, ysum, wsum = uk[keep], ysum[keep], wsum[keep]
+    else:
+        uk, ysum, wsum, std2 = _plan_runs(op, std, key, sel, mask, yv, C)
     fr, px = uk // (H * W), uk % (H * W)
     n_strips = -(-H // strip)
     obs_frames = np.unique(fr)
@@ -270,9 +297,41 @@ def point_plan(op: PointObservation, y, L: int, C: int, H: int, W: int, frame_lo
     cell = frame_slot[fr].astype(np.int64) * n_strips + (px // W) // strip  # non-decreasing: the keys are sorted
     counts = np.bincount(cell, minlength=obs_frames.size * n_strips)
     strip_off = np.concatenate([[0], np.cumsum(counts)]).astype(np.int32)
-    return dict(frame_slot=frame_slot, strip_off=strip_off, pix=px.astype(np.int32), ysum=ysum.astype(np.float32),
-                wsum=wsum.astype(np.float32), n_slots=int(obs_frames.size), strip_rows=int(strip), n_strips=n_strips,
-                frames=[int(frame_lo + f) for f in obs_frames])
+    out = dict(frame_slot=frame_slot, strip_off=strip_off, pix=px.astype(np.int32), ysum=ysum.astype(np.float32),
+               wsum=wsum.astype(np.float32), n_slots=int(obs_frames.size), strip_rows=int(strip), n_strips=n_strips,
+               frames=[int(frame_lo + f) for f in obs_frames])
+    if std is not None:
+        out["std2"] = std2
+    return out
+
+
+def _plan_runs(op: PointObservation, std, key, sel, mask, yv, C: int) -> tuple:
+    """point_plan's entries with a std per observation: (entry keys, local frame * H W + pixel, repeated over a pixel's
+    run; ysum, wsum (fp64) and std2 (fp32), each [n_entries, C]).  The sums run in point order, as without std."""
+    s = torch.broadcast_to(torch.as_tensor(std, dtype=torch.float32).cpu(), (op.n_frames, C, op.n_points))
+    s2 = (s * s).numpy()[sel].transpose(0, 2, 1).reshape(-1, C)      # fp32 std^2 per (observation, variable)
+    live = mask[sel].transpose(0, 2, 1).reshape(-1, C) & np.isfinite(s2)  # std = inf: contributes exactly 0
+    o, c = np.nonzero(live)                                            # point order, then variable
+    k, v = key[o], s2[o, c]
+    # the class of an observation: the rank of its std^2 among the distinct ones of its (frame, pixel, variable)
+    order = np.lexsort((v, c, k))
+    ks, cs, vs = k[order], c[order], v[order]
+    new_group = np.ones(order.size, dtype=bool)
+    new_group[1:] = (ks[1:] != ks[:-1]) | (cs[1:] != cs[:-1])
+    new_value = new_group.copy()
+    new_value[1:] |= vs[1:] != vs[:-1]
+    value_id = np.cumsum(new_value) - 1
+    cls = np.empty(order.size, dtype=np.int64)
+    cls[order] = value_id - np.maximum.accumulate(np.where(new_group, value_id, 0))
+    n_cls = int(cls.max()) + 1 if cls.size else 1
+    uk, inv = np.unique(k * n_cls + cls, return_inverse=True)          # sorted: frame, pixel, then class
+    ysum = np.zeros((uk.size, C))
+    wsum = np.zeros((uk.size, C))
+    std2 = np.ones((uk.size, C), dtype=np.float32)
+    np.add.at(ysum, (inv, c), yv.transpose(0, 2, 1).reshape(-1, C)[o, c])
+    np.add.at(wsum, (inv, c), 1.0)
+    std2[inv, c] = v
+    return uk // n_cls, ysum, wsum, std2
 
 
 def _per_channel(v, C: int, name: str):
@@ -284,6 +343,46 @@ def _per_channel(v, C: int, name: str):
         raise ValueError(f"{name}: expected a scalar or {C} per-variable values, got {t.numel()}")
     out = [float(x) for x in t]
     return out + [1.0] * (4 - len(out))
+
+
+def _check_std_values(std: Tensor, mask, what: str) -> None:
+    """A std per observation is >= 0 (+inf allowed: that observation contributes exactly zero) and not NaN wherever
+    mask is set (mask None: everywhere)."""
+    v = std if mask is None else std[mask]
+    if bool((torch.isnan(v) | (v < 0)).any()):
+        raise ValueError(f"{what}: std (A(x)'s shape {tuple(std.shape)}) is negative or NaN at an unmasked observation")
+
+
+def _std_per_observation(std, shape, C: int, mask, what: str) -> Optional[Tensor]:
+    """A std given per observation, broadcast to A(x)'s `shape`, fp32 and contiguous, after its checks; None for the
+    per-variable forms, a scalar or C values, which `_per_channel` reads.  So a [1, 1, P] std with P == C is per
+    variable: expand it to [F, C, P] to give each of the P stations its own."""
+    t = torch.as_tensor(std, dtype=torch.float32).cpu()
+    if t.numel() in (1, C):
+        return None
+    try:
+        b = torch.broadcast_to(t, tuple(shape)).contiguous()
+    except RuntimeError:
+        raise ValueError(f"{what}: std of shape {tuple(t.shape)} does not broadcast to A(x) of shape {tuple(shape)}; "
+                         f"expected a scalar, {C} per-variable values or a tensor that broadcasts to {tuple(shape)}") \
+            from None
+    _check_std_values(b, mask, what)
+    return b
+
+
+def _collapse_per_variable(std: Tensor, mask) -> Optional[list]:
+    """The C per-variable values of a std [M, C, ...] that is constant per variable over its observations (where mask
+    is set; 1.0 for a variable without any), else None.  Such a std runs on the per-variable kernels."""
+    C = std.shape[1]
+    per_var = std.transpose(0, 1).reshape(C, -1)
+    keep = None if mask is None else mask.transpose(0, 1).reshape(C, -1)
+    out = []
+    for c in range(C):
+        v = per_var[c] if keep is None else per_var[c][keep[c]]
+        if v.numel() and not bool((v == v[0]).all()):
+            return None
+        out.append(float(v[0]) if v.numel() else 1.0)
+    return out
 
 
 def _check_observation_shape(op: CoarseGrain, y_shape, L: int, C: int, H: int, W: int) -> tuple:
@@ -531,6 +630,8 @@ class _Runtime:
         self.cond = cond
         self._sel = None
         self.points = None
+        # a std per observation (cond["obs_std"]): the coarse std^2 block next to y_dev, the point std in the plan
+        obs_std = cond.get("obs_std") if cond is not None else None
         if cond is not None and isinstance(cond["op"], (PointObservation, CombinedObservation)):
             # this rank's owned frames only, built once per conditioning and trajectory geometry
             p = self.plan
@@ -538,9 +639,11 @@ class _Runtime:
             if isinstance(op, CombinedObservation):  # strips of whole observation tiles (guided_combined_kernel)
                 op, y, max_pix = op.points, cond["point_y"], COMBINED_STRIP_PIX
                 strip = combined_strip_rows(self.H, self.W, cond["op"].coarse.s_step)
-            pl = point_plan(op, y, self.L, self.C, self.H, self.W, p.own_lo, p.own_lo + p.own_n, strip, max_pix)
-            dev = {n: torch.as_tensor(pl[n]).to(self.device) for n in ("frame_slot", "strip_off", "pix", "ysum", "wsum")}
-            for n in ("pix", "ysum", "wsum"):  # no entries on this rank: still a valid pointer
+            std = obs_std["point_std"] if obs_std is not None else None
+            pl = point_plan(op, y, self.L, self.C, self.H, self.W, p.own_lo, p.own_lo + p.own_n, strip, max_pix, std)
+            names = ("frame_slot", "strip_off", "pix", "ysum", "wsum") + (("std2",) if std is not None else ())
+            dev = {n: torch.as_tensor(pl[n]).to(self.device) for n in names}
+            for n in names[2:]:  # no entries on this rank: still a valid pointer
                 if dev[n].numel() == 0:
                     dev[n] = torch.zeros(max(1, self.C), dtype=dev[n].dtype, device=self.device)
             ob = _lib.PointObs()
@@ -552,6 +655,9 @@ class _Runtime:
             self.refresh_engine()  # the stashing workspace is sized by the selection
         if cond is not None and not isinstance(cond["op"], PointObservation):
             self.y_dev = cond["y"].to(device=self.device, dtype=torch.float32).contiguous()
+        self.coarse_std2_dev = None
+        if obs_std is not None and obs_std["coarse_std2"] is not None:
+            self.coarse_std2_dev = obs_std["coarse_std2"].to(device=self.device, dtype=torch.float32).contiguous()
 
     def _guide(self, mode: int, mu: float, sigma: float, mu_next: float, sigma_next: float, frames=None) -> None:
         p = self.plan
@@ -560,10 +666,11 @@ class _Runtime:
         s = self.s_tile
         pts = self.points if self.cond is not None else None
         combined = pts is not None and isinstance(self.cond["op"], CombinedObservation)
+        per_obs = self.cond is not None and self.cond.get("obs_std") is not None  # g.std2 is not read
         if pts is not None and not combined:  # point observations: y, t_step and s_step are not read
             g.y, g.t_step = None, 1
             for i in range(self.C):
-                g.std2[i] = self.cond["std"][i] ** 2
+                g.std2[i] = 1.0 if per_obs else self.cond["std"][i] ** 2
                 g.gamma[i] = self.cond["gamma"][i]
         elif self.cond is not None:  # the coarse term (of a CombinedObservation: the point term is in pts)
             cg: CoarseGrain = self.cond["op"].coarse if combined else self.cond["op"]
@@ -571,7 +678,7 @@ class _Runtime:
             g.y = self.y_dev.data_ptr()
             g.t_step = cg.t_step
             for i in range(self.C):
-                g.std2[i] = self.cond["std"][i] ** 2
+                g.std2[i] = 1.0 if per_obs else self.cond["std"][i] ** 2
                 g.gamma[i] = self.cond["gamma"][i]
         else:
             g.y = None
@@ -601,7 +708,13 @@ class _Runtime:
             g.eps_out, g.partials = self.eps_g.data_ptr(), self.partials.data_ptr()
             self._n_part = n_part
         with torch.cuda.device(self.device):
-            if combined:
+            if per_obs:
+                obs = ctypes.byref(pts["obs"]) if pts is not None else None
+                entry = pts["tensors"]["std2"].data_ptr() if pts is not None else None
+                coarse = self.coarse_std2_dev.data_ptr() if self.coarse_std2_dev is not None else None
+                _lib.check(self.lib.c2w_guided_step_obs_std(ctypes.byref(g), obs, coarse, entry, self.stream),
+                           "c2w_guided_step_obs_std")
+            elif combined:
                 pstd2 = (ctypes.c_float * self.C)(*(v ** 2 for v in self.cond["point_std"]))
                 _lib.check(self.lib.c2w_guided_step_combined(ctypes.byref(g), ctypes.byref(pts["obs"]), pstd2, self.stream),
                            "c2w_guided_step_combined")
@@ -748,7 +861,9 @@ class AbstractScoreFunction:
         J = A^T((y - A x0)/var)/mu; `exact_grad=True` adds the term through the network,
         J = (g - sigma J_eps^T g)/mu with g = A^T((y - A x0)/var), computed by the UNet input-gradient kernels."""
         if isinstance(A, PointObservation):
-            A.check_observation(torch.as_tensor(y))
+            yt = torch.as_tensor(y)
+            A.check_observation(yt)
+            _std_per_observation(std, yt.shape, yt.shape[1], A.mask_for(yt.shape[1]), repr(A))
         if isinstance(A, CombinedObservation) and torch.as_tensor(y).dim() != 1:
             raise ValueError(f"{A}: y must be the flat tensor A(x) gives (CombinedObservation.pack), got shape "
                              f"{tuple(torch.as_tensor(y).shape)}")
@@ -840,16 +955,47 @@ class AbstractScoreFunction:
                 if isinstance(op, CombinedObservation):  # split and checked against this trajectory's geometry
                     _check_observation_shape(op.coarse, op.term_shapes(x.shape)[0], L, C, H, W)
                     y, cond["point_y"] = op.split(y, x.shape)
-                    cond["std"], cond["point_std"] = op.std_per_term(lk["std"], x.shape)
+                    if torch.as_tensor(lk["std"]).numel() in (1, C):
+                        cond["std"], cond["point_std"] = op.std_per_term(lk["std"], x.shape)
+                    else:
+                        cond.update(_combined_std(op, lk["std"], x.shape))
                 else:
-                    cond["std"] = _per_channel(lk["std"], C, "std")
-                if isinstance(op, CoarseGrain):  # checked against this trajectory's geometry, every time
-                    y = coarse_grain_observation(op, y, L, C, H, W)
+                    if isinstance(op, CoarseGrain):  # checked against this trajectory's geometry, every time
+                        y = coarse_grain_observation(op, y, L, C, H, W)
+                    cond.update(_single_std(op, lk["std"], y.shape, C))
                 rt.set_condition(dict(cond, y=y))
             self._runtimes = {key: rt}  # one live trajectory geometry at a time
         else:
             rt.refresh_engine()  # once per score call / sampling run: catches in-place parameter updates
         return rt
+
+
+def _single_std(op, std, obs_shape, C: int) -> dict:
+    """The std entries of a CoarseGrain's or PointObservation's conditioning: per variable ({"std": C values}) when
+    std is a scalar, C values or constant per variable, else per observation ({"obs_std": coarse std^2 block or
+    point std, the other None})."""
+    mask = op.mask_for(C) if isinstance(op, PointObservation) else None
+    b = _std_per_observation(std, obs_shape, C, mask, repr(op))
+    if b is None:
+        return {"std": _per_channel(std, C, "std")}
+    v = _collapse_per_variable(b, mask)
+    if v is not None:
+        return {"std": v}
+    if mask is not None:
+        return {"obs_std": dict(coarse_std2=None, point_std=b)}
+    return {"obs_std": dict(coarse_std2=b * b, point_std=None)}
+
+
+def _combined_std(op: CombinedObservation, std, x_shape) -> dict:
+    """The std entries of a CombinedObservation's conditioning from a flat std in y's layout: per (term, variable)
+    ({"std", "point_std"}) when each term's block is constant per variable, else per observation ({"obs_std"})."""
+    coarse_std2, point_std = op.std_per_observation(std, x_shape)
+    mask = op.points.mask_for(int(x_shape[1]))
+    coarse = op.split(torch.as_tensor(std, dtype=torch.float32).reshape(-1).cpu(), x_shape)[0]
+    cv, pv = _collapse_per_variable(coarse, None), _collapse_per_variable(point_std, mask)
+    if cv is not None and pv is not None:
+        return {"std": cv, "point_std": pv}
+    return {"obs_std": dict(coarse_std2=coarse_std2, point_std=point_std)}
 
 
 def _mu_sigma(noise_process, t) -> tuple:

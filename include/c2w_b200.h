@@ -190,7 +190,8 @@ int c2w_guided_step(const c2w_guide* g, void* stream);
 typedef struct c2w_point_obs {
   const int32_t* frame_slot; /* [own_n] observed slot of the updated frame own_lo + i, or -1                      */
   const int32_t* strip_off;  /* [n_slots * ceil(H / strip_rows) + 1] CSR offsets into the entries                */
-  const int32_t* pix;        /* [n_entries] pixel index within the frame (h * W + w), unique per (slot, strip)    */
+  const int32_t* pix;        /* [n_entries] pixel index within the frame (h * W + w), unique per (slot, strip);
+                              * c2w_guided_step_obs_std: runs of one pixel allowed, see there                   */
   const float* ysum;         /* [n_entries, C] sum of mask * y                                                    */
   const float* wsum;         /* [n_entries, C] number of unmasked observations                                    */
   int32_t n_slots, strip_rows;
@@ -206,6 +207,13 @@ int c2w_guided_step_points(const c2w_guide* g, const c2w_point_obs* obs, void* s
  * s * max(1, min(H / s, floor(C2W_POINT_STRIP_PIX / (s * W))))).  Mode 1 writes own_n * ceil(H / strip_rows) partials. */
 #define C2W_COMBINED_STRIP_PIX 16384
 int c2w_guided_step_combined(const c2w_guide* g, const c2w_point_obs* obs, const float* point_std2, void* stream);
+/* A std per observation: the guidance step of the three entry points above with each observation's own std^2.
+ * g->std2 is ignored; gamma comes from g.  Coarse term: g->y and coarse_std2 (device, y's layout), both or neither.
+ * Point term: obs and entry_std2 (device, [n_entries, C]), both or neither; an obs here may hold runs of entries
+ * with the same pixel (consecutive, within one strip).  At least one term.  Launches K6, K6p or K6c accordingly,
+ * with the argument checks of c2w_guided_step, c2w_guided_step_points or c2w_guided_step_combined. */
+int c2w_guided_step_obs_std(const c2w_guide* g, const c2w_point_obs* obs, const float* coarse_std2,
+                            const float* entry_std2, void* stream);
 int c2w_reduce_partials(const float* partials, int32_t n, double* sumsq, void* stream);
 /* x <- x - (delta eps + sqrt(2 delta) z) sigma_next, delta = tau / (sumsq / count)  (src/thor/pipelines.py:84-87).
  * z == NULL: on-chip Philox4x32-10 keyed by (seed, step_id, global pixel index). */
