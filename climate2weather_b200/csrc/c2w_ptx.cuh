@@ -285,14 +285,17 @@ __device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {
 }
 
 // ---------------------------------------------------------------- descriptors
-// Shared-memory matrix descriptor, K-major operand, 128-byte swizzle, rows of 128 B (64 bf16),
-// 8-row groups 1024 B apart.  Field layout: see cute/arch/mma_sm100_desc.hpp (SmemDescriptor).
-__device__ __forceinline__ uint64_t umma_desc_kmajor_sw128(uint32_t smem_addr) {
+// Shared-memory matrix descriptor, K-major operand, 128-byte swizzle, rows of 128 B (64 bf16), 8-row groups `sbo`
+// bytes apart (1024 for a dense tile).  `base_offset` is the matrix base-offset field (bits 49-51).  Field layout:
+// see cute/arch/mma_sm100_desc.hpp (SmemDescriptor).
+__device__ __forceinline__ uint64_t umma_desc_kmajor_sw128(uint32_t smem_addr, uint32_t sbo = 1024,
+                                                           uint32_t base_offset = 0) {
   uint64_t d = 0;
   d |= static_cast<uint64_t>((smem_addr >> 4) & 0x3FFF);  // start address
   d |= static_cast<uint64_t>(1) << 16;                    // leading byte offset (unused for swizzled K-major)
-  d |= static_cast<uint64_t>(1024 >> 4) << 32;            // stride byte offset: 8 rows * 128 B
+  d |= static_cast<uint64_t>((sbo >> 4) & 0x3FFF) << 32;  // stride byte offset: from one 8-row group to the next
   d |= static_cast<uint64_t>(1) << 46;                    // descriptor version (sm_100)
+  d |= static_cast<uint64_t>(base_offset & 7) << 49;      // matrix base offset
   d |= static_cast<uint64_t>(2) << 61;                    // SWIZZLE_128B
   return d;
 }

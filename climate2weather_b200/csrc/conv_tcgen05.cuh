@@ -10,16 +10,18 @@
 //            (c0, s-1, h0+r-1, n0); out-of-bounds rows/columns are zero-filled by the TMA unit, which is exactly
 //            padding=1 / padding_mode=zeros (configs/sda_unet.yml:16).  Stride-2 convs use the same box with element
 //            strides {1, 2, 2, 1}.  Activation-reuse path (AR; stride-1 convs with 64/128-wide N tiles): the M tile is
-//            a 16 x 8 spatial block and ONE halo'd box [18 x 8 px][64 ch] per (channel block, filter column) serves
-//            the three filter rows as sub-views r * 8 rows into it.
-//            B (packed weights [Cout, 9*Cin], K-major) is a 2-D TMA load {64, BN}.
+//            a 16 x 8 spatial block and ONE halo'd box [18 rows x 10 px][64 ch] per channel block serves all nine
+//            taps: tap (r, s) is the sub-view r rows and s pixels into it, addressed by the MMA descriptor alone.
+//            B (packed weights [Cout, 9*Cin], K-major) is a 2-D TMA load {64, BN} (AR: one box holds the three
+//            filter rows' tiles of one filter column).
 //            Both land in 128B-swizzled K-major tiles that tcgen05.mma consumes directly.
 // Roles:     warp 0 = TMA producer, warp 1 = MMA issuer (single thread), warp 2 = TMEM allocator + TMA stores of the
 //            finished tiles + residual prefetch, warps 4..11 = epilogue, warps 12..15 (fused-LayerNorm kernels only)
 //            = LayerNorm pass; the register file is re-split per warpgroup with setmaxnreg in those kernels.
 //            Persistent CTAs (grid = #SMs, static round-robin tiles), a ring of operand stages (full/empty
-//            mbarriers), two TMEM accumulators (tmem_full/tmem_empty; released as soon as the epilogue's tcgen05.ld
-//            have landed), staging tiles handed between epilogue, LayerNorm and store warps by mbarriers only.
+//            mbarriers; AR: a ring of activation units and a ring of weight stages), two TMEM accumulators
+//            (tmem_full/tmem_empty; released as soon as the epilogue's tcgen05.ld have landed), staging tiles handed
+//            between epilogue, LayerNorm and store warps by mbarriers only.
 //            Two CTAs (a cluster) share one MMA (cta_group::2, 256 x BN tile) whenever there are two M tiles.
 // Epilogue:  TMEM -> registers (tcgen05.ld 32x32b.x32) -> +bias [-> SiLU | + residual] -> bf16 -> 128B-swizzled
 //            staging tile in shared memory -> TMA store (per-thread row stores cost 8x the L1 wavefronts of the
@@ -76,12 +78,13 @@ struct ConvParams {
   int tiles_w;      // AR: 16 x 8 spatial tiles per image row (W / 8); tiles_per_img = (H / 16) * tiles_w
   int img_h, img_w; // AR: output image size
   // AR on 8-row images (ar2): the 16 x 8 M tile is two images stacked row-interleaved — tile row = (image row, image,
-  // pixel) — so that filter row r is still one contiguous sub-view of the halo'd unit ([10 rows][2 img][8 px][64 ch],
-  // 20 KB): the tensor maps list the image dimension BEFORE the row dimension.  tiles_per_img = tiles per image pair.
+  // pixel) — so that tap (r, s) is still one strided sub-view of the halo'd unit ([10 rows][2 img][10 px][64 ch],
+  // 25 KB): the tensor maps list the image dimension BEFORE the row dimension.  tiles_per_img = tiles per image pair.
   int ar2;
-  int ar_row_step16;  // (bytes >> 4) from filter row r to r + 1 inside the unit: 64 (ar2: 128)
-  int ar_tx_bytes;    // bytes one CTA's loads of a stage deliver
-  int num_stages;   // depth of the A/B ring
+  int ar_row_step16;  // (bytes >> 4) from filter row r to r + 1 inside the unit: 80 (ar2: 160)
+  int ar_tx_a;        // bytes one CTA's activation unit delivers
+  int ar_tx_b;        // bytes one CTA's three weight tiles of a filter column deliver
+  int num_stages;   // depth of the A/B ring (AR: of the weight ring)
   int num_staging;  // epilogue staging tiles (2: used alternately)
   // epilogue
   int mode;
@@ -121,12 +124,14 @@ constexpr int kConvThreads = 128 + kEpiThreads;  // + kLnThreads in kernels with
 constexpr int kLnWarps = 4;                      // LayerNorm warps (one warpgroup) of those kernels
 constexpr int kLnThreads = kLnWarps * 32;
 constexpr int kSmemLimit = 232448;  // 227 KB
+constexpr int kARUnitW = 10;        // AR: pixel columns of a unit (8 + the halo on either side)
 
 // BN   : N tile (output channels per tile).
 // CG   : CTAs per MMA (tcgen05 cta_group).  CG == 2: a cluster of two CTAs computes a 256 x BN tile, each CTA
 //        holding its own 128 A rows and HALF of the B rows in shared memory.
 // Shared memory: [A ring][B ring][1 or 2 staging tiles][barriers]; the ring depth is a launch-time number (what is
-// left after the staging tiles: residual convs double-buffer them so the residual prefetch runs a tile ahead).
+// left after the staging tiles: residual convs double-buffer them so the residual prefetch runs a tile ahead).  AR:
+// [kARUnits activation units][weight stages of three B tiles][staging][barriers], the weight ring taking what is left.
 template <int BN, int CG>
 struct ConvCfg {
   // A pipeline stage holds kSub K-sub-blocks of 64 (one 128 B swizzle row each).  With BN <= 128 a 64-wide
@@ -138,24 +143,30 @@ struct ConvCfg {
   static constexpr int kSubBytes = kATileBytes + kBTileBytes;
   static constexpr int kStageBytes = kSub * kSubBytes;
   static constexpr int kStagingBytes = (BN / 64) * kATileBytes;  // bf16 [BN/64 boxes][128 rows][64 ch], swizzled
-  static constexpr int kBarrierBytes = 256 + 4096;  // mbarriers, TMEM slot; LN row statistics float2[2 tiles][2][128]
+  static constexpr int kBarrierBytes = 512 + 4096;  // mbarriers, TMEM slot; LN row statistics float2[2 tiles][2][128]
   static constexpr int kMaxStages = 8;
-  // AR (activation reuse, 3x3 stride 1): the M tile is a 16 x 8 spatial block; a stage holds, for one (channel
-  // block, filter column s), the block's input with a one-row halo above and below shifted by s-1 columns
-  // ([18 x 8 pixels][64 ch] = 18 KB) and the three B tiles of filter rows r = 0..2.  Filter row r is the sub-view
-  // starting r * 8 rows (r KB) into the unit, so the unit is loaded once and multiplied three times: 6 KB of A per
-  // K block instead of 16 KB.  (K1 with streamed operands is bound by the chip-wide L2 -> SM TMA throughput,
-  // ~12 TB/s: profiles/r01c_*.)
+  // AR (activation reuse, 3x3 stride 1): the M tile is a 16 x 8 spatial block.  One UNIT per channel block holds the
+  // block's input with a one-pixel halo on every side ([18 rows][10 px][64 ch] = 22.5 KB), loaded by one TMA box.
+  // Tap (r, s) is the sub-view starting r rows and s pixels into it: an MMA descriptor whose start address is
+  // r * 1280 + s * 128 bytes into the unit and whose 8-row groups (one tile row of 8 pixels each) are 1280 B apart.
+  // So the unit is loaded once and multiplied nine times: 2.5 KB of A per K block instead of 16 KB.  The units have
+  // their own ring; the weight ring holds, per stage, the three B tiles (r = 0..2) of one filter column s, loaded by
+  // one TMA box too.
+  // (K1 with streamed operands is bound by the chip-wide L2 -> SM TMA throughput, ~12 TB/s: profiles/r01c_*.)
   static constexpr int kARTileH = 16, kARTileW = 8;
-  // unit slot: 18 KB; 20 KB for 128-wide tiles, which also run the two-image form (ConvParams::ar2)
-  static constexpr int kARUnitBytes = (BN == 128 ? 20 : 18) * kARTileW * kBlockK * 2;
-  static constexpr int kARStageBytes = kARUnitBytes + 3 * kBTileBytes;
+  // unit slot, 1024-aligned: 23 KB; 25 KB for 128-wide tiles, which also run the two-image form (ConvParams::ar2)
+  static constexpr int kARUnitBytes = ((BN == 128 ? 20 : 18) * kARUnitW * kBlockK * 2 + 1023) / 1024 * 1024;
+  // units in flight (the weight ring takes what is left; 64-wide tiles, whose weight ring is at kMaxStages, take three)
+  static constexpr int kARUnits = BN == 64 ? 3 : 2;
+  static constexpr int kARBStageBytes = 3 * kBTileBytes;
   static constexpr int ar_stages_for(int num_staging) {
-    const int n = (kSmemLimit - 1024 - kBarrierBytes - num_staging * kStagingBytes) / kARStageBytes;
+    const int n = (kSmemLimit - 1024 - kBarrierBytes - num_staging * kStagingBytes - kARUnits * kARUnitBytes) /
+                  kARBStageBytes;
     return n > kMaxStages ? kMaxStages : n;
   }
   static constexpr int ar_smem_bytes(int num_staging) {
-    return ar_stages_for(num_staging) * kARStageBytes + num_staging * kStagingBytes + kBarrierBytes + 1024;
+    return kARUnits * kARUnitBytes + ar_stages_for(num_staging) * kARBStageBytes + num_staging * kStagingBytes +
+           kBarrierBytes + 1024;
   }
   static constexpr int kTmemCols = (2 * BN <= 128) ? 128 : (2 * BN <= 256) ? 256 : 512;
   static constexpr int stages_for(int num_staging) {
@@ -168,7 +179,7 @@ struct ConvCfg {
   static_assert(BN % 64 == 0 && BN >= 64 && BN <= 256, "BN must be 64..256, multiple of 64");
   static_assert(CG == 1 || CG == 2, "cta_group is 1 or 2");
   static_assert(stages_for(2) >= 1 && stages_for(1) >= 2, "pipeline too shallow");
-  static_assert(2 * kMaxStages + 10 <= 256 / 8 - 1, "barrier block too small");
+  static_assert(2 * kMaxStages + 2 * kARUnits + 10 <= 512 / 8 - 1, "barrier block too small");
 };
 
 // SiLU = x * sigmoid(x) = h + h * tanh(h), h = x / 2: one MUFU op per element (tanh.approx, rel. error 2^-11, far
@@ -324,11 +335,13 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
   // every staging-tile access becomes a generic LD/ST with 64-bit address math instead of LDS/STS)
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   const int num_stages = p.num_stages;
+  constexpr int num_units = AR ? Cfg::kARUnits : 0;
+  // AR: [A units][B stages of [r0][r1][r2]]; otherwise [A ring][B ring]
   uint8_t* smA = smem;
-  uint8_t* smB = smem + num_stages * Cfg::kSub * kATileBytes;  // (AR: stages are [A unit][B r0][B r1][B r2])
-  uint8_t* stg0 = smem + num_stages * (AR ? Cfg::kARStageBytes : Cfg::kStageBytes);  // epilogue staging tile(s)
+  uint8_t* smB = smem + (AR ? num_units * Cfg::kARUnitBytes : num_stages * Cfg::kSub * kATileBytes);
+  uint8_t* stg0 = smB + num_stages * (AR ? Cfg::kARBStageBytes : Cfg::kSub * Cfg::kBTileBytes);  // staging tile(s)
   uint64_t* bars = reinterpret_cast<uint64_t*>(stg0 + p.num_staging * Cfg::kStagingBytes);
-  uint64_t* full = bars;
+  uint64_t* full = bars;  // [kMaxStages] operand stage landed (AR: weight stage)
   uint64_t* empty = bars + Cfg::kMaxStages;
   uint64_t* tmem_full = bars + 2 * Cfg::kMaxStages;
   uint64_t* tmem_empty = tmem_full + 2;
@@ -336,8 +349,10 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
   uint64_t* stg_full = res_full + 2;    // [2] staging[b] written by the epilogue warps
   uint64_t* stg_free = stg_full + 2;    // [2] staging[b] read by its store (and the LayerNorm pass)
   uint64_t* ln_done = stg_free + 2;     // [2] LayerNorm pass over staging[b] finished (all epilogue warps)
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(ln_done + 2);
-  float2* ln_stats = reinterpret_cast<float2*>(reinterpret_cast<uint8_t*>(bars) + 256);  // [2][2][128]
+  uint64_t* a_full = ln_done + 2;       // [kARUnits] AR: activation unit landed
+  uint64_t* a_empty = a_full + Cfg::kARUnits;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(a_empty + Cfg::kARUnits);
+  float2* ln_stats = reinterpret_cast<float2*>(reinterpret_cast<uint8_t*>(bars) + 512);  // [2][2][128]
 
   const int warp_idx = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -366,6 +381,10 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
     for (int s = 0; s < num_stages; ++s) {
       mbar_init(&full[s], 1);
       mbar_init(&empty[s], 1);
+    }
+    for (int u = 0; u < num_units; ++u) {
+      mbar_init(&a_full[u], 1);
+      mbar_init(&a_empty[u], 1);
     }
     for (int a = 0; a < 2; ++a) {
       mbar_init(&tmem_full[a], 1);
@@ -417,6 +436,9 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
       int stage = 0;
       uint32_t phase = 0;
       int issued = 0;
+      int unit = 0;
+      uint32_t a_phase = 0;
+      int a_issued = 0;
       [[maybe_unused]] long long w_empty = 0;
       [[maybe_unused]] const long long t_begin = C2W_DIAG_CLOCK();
       for (int tile = group_id; AR && tile < num_tiles; tile += num_groups) {
@@ -424,48 +446,64 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
         const int mt = (tile / p.num_n_tiles) * CG + rank;
         const int img = mt / p.tiles_per_img, tt = mt % p.tiles_per_img;
         const int h0 = (tt / p.tiles_w) * Cfg::kARTileH, w0 = (tt % p.tiles_w) * Cfg::kARTileW;
-        for (int kb = 0; kb < 3 * p.cin_blocks; ++kb) {  // kb = cb * 3 + s
-          const int cb = kb / 3, s3 = kb - cb * 3;
-          C2W_TIMED_WAIT(w_empty, &empty[stage], phase ^ 1);
+        const int a2 = p.ar2 ? 2 * img : h0 - 1, a3 = p.ar2 ? -1 : img;
+        for (int cb = 0; cb < p.cin_blocks; ++cb) {
+          // ---- the channel block's halo'd unit
+          C2W_TIMED_WAIT(w_empty, &a_empty[unit], a_phase ^ 1);
           if (elect_one()) {
-            const uint32_t full_bar = (CG == 2) ? mapa_shared(smem_u32(&full[stage]), 0) : smem_u32(&full[stage]);
-            uint8_t* sbase = smem + stage * Cfg::kARStageBytes;
+            // timing experiments (diagnostics build): after the rings are primed, 4 and 1 signal the unit as landed
+            // without loading it
 #ifdef C2W_DIAG
-            if (p.dbg_skip_loads == 1 && issued >= num_stages) {
-              if (rank == 0) mbar_arrive(&full[stage]);
-            } else
-#endif
-            {
-#ifdef C2W_DIAG
-              // timing experiment (dbg_skip_loads == 2): every other tile reuses stale weights — the operand traffic
-              // of a 256-row M tile sharing one B load, without its data flow
-              // (3: no weight loads at all, 4: no activation loads at all — which latency does the ring cover?)
-              const bool skip_b = ((p.dbg_skip_loads == 2 && ((tile / num_groups) & 1)) || p.dbg_skip_loads == 3) &&
-                                  issued >= num_stages;
-              const bool skip_a = p.dbg_skip_loads == 4 && issued >= num_stages;
+            const bool skip_a = (p.dbg_skip_loads == 4 || p.dbg_skip_loads == 1) && a_issued >= num_units;
 #else
-              constexpr bool skip_b = false, skip_a = false;
+            constexpr bool skip_a = false;
 #endif
-              if (rank == 0)
-                mbar_arrive_expect_tx(&full[stage], CG * (p.ar_tx_bytes - (skip_b ? 3 * Cfg::kBTileBytes : 0) -
-                                                          (skip_a ? p.ar_tx_bytes - 3 * Cfg::kBTileBytes : 0)));
-              const int a2 = p.ar2 ? 2 * img : h0 - 1, a3 = p.ar2 ? -1 : img;
-              if (skip_a) {
-              } else if (CG == 2) tma_load_4d_pair(&tmA, full_bar, sbase, cb * kBlockK, w0 + s3 - 1, a2, a3);
-              else tma_load_4d(&tmA, &full[stage], sbase, cb * kBlockK, w0 + s3 - 1, a2, a3);
-              for (int r = 0; r < 3 && !skip_b; ++r) {
-                const int kk = (r * 3 + s3) * p.cin_blocks + cb;  // K block of tap (r, s) in the packed weights
-                uint8_t* bdst = sbase + Cfg::kARUnitBytes + r * Cfg::kBTileBytes;
-                if (CG == 2) tma_load_2d_pair(&tmB, full_bar, bdst, kk * kBlockK, nt * BN + rank * Cfg::kBRows);
-                else tma_load_2d(&tmB, &full[stage], bdst, kk * kBlockK, nt * BN);
-              }
+            if (rank == 0) mbar_arrive_expect_tx(&a_full[unit], skip_a ? 0 : CG * p.ar_tx_a);
+            uint8_t* adst = smA + unit * Cfg::kARUnitBytes;
+            if (skip_a) {
+            } else if (CG == 2) {
+              tma_load_4d_pair(&tmA, mapa_shared(smem_u32(&a_full[unit]), 0), adst, cb * kBlockK, w0 - 1, a2, a3);
+            } else {
+              tma_load_4d(&tmA, &a_full[unit], adst, cb * kBlockK, w0 - 1, a2, a3);
             }
           }
           __syncwarp();
-          ++issued;
-          if (++stage == num_stages) {
-            stage = 0;
-            phase ^= 1;
+          ++a_issued;
+          if (++unit == num_units) {
+            unit = 0;
+            a_phase ^= 1;
+          }
+          // ---- the weights of filter columns s = 0..2, one stage each
+          for (int s3 = 0; s3 < 3; ++s3) {
+            C2W_TIMED_WAIT(w_empty, &empty[stage], phase ^ 1);
+            if (elect_one()) {
+#ifdef C2W_DIAG
+              // 2: every other tile reuses stale weights — the operand traffic of a 256-row M tile sharing one B
+              // load, without its data flow; 3 and 1: no weight loads at all
+              const bool skip_b = ((p.dbg_skip_loads == 2 && ((tile / num_groups) & 1)) || p.dbg_skip_loads == 3 ||
+                                   p.dbg_skip_loads == 1) &&
+                                  issued >= num_stages;
+#else
+              constexpr bool skip_b = false;
+#endif
+              if (rank == 0) mbar_arrive_expect_tx(&full[stage], skip_b ? 0 : CG * p.ar_tx_b);
+              // one box {64 ch, B rows, r = 0..2} at channel s * Cin + cb * 64 of the [Cout][r][s * Cin] weight view
+              uint8_t* bdst = smB + stage * Cfg::kARBStageBytes;
+              const int kc = (s3 * p.cin_blocks + cb) * kBlockK;
+              if (skip_b) {
+              } else if (CG == 2) {
+                tma_load_4d_pair(&tmB, mapa_shared(smem_u32(&full[stage]), 0), bdst, kc, nt * BN + rank * Cfg::kBRows,
+                                 0, 0);
+              } else {
+                tma_load_4d(&tmB, &full[stage], bdst, kc, nt * BN, 0, 0);
+              }
+            }
+            __syncwarp();
+            ++issued;
+            if (++stage == num_stages) {
+              stage = 0;
+              phase ^= 1;
+            }
           }
         }
       }
@@ -529,10 +567,13 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
     } else if (warp_idx == 1 && rank == 0) {
       // ------------------------------------------------------------ MMA issuer (leader CTA, one elected lane issues)
       constexpr uint32_t idesc = umma_idesc_bf16(kBlockM * CG, BN);
-      const uint64_t adesc0 = umma_desc_kmajor_sw128(smem_u32(smA));
+      // AR: 8-row groups = tile rows of 8 pixels, one unit row (kARUnitW pixels) apart
+      const uint64_t adesc0 = umma_desc_kmajor_sw128(smem_u32(smA), AR ? kARUnitW * 128 : 1024);
       const uint64_t bdesc0 = umma_desc_kmajor_sw128(smem_u32(smB));
       int stage = 0;
       uint32_t phase = 0;
+      int unit = 0;
+      uint32_t a_phase = 0;
       int acc = 0;
       uint32_t acc_phase = 0;
       [[maybe_unused]] long long w_full = 0, w_tmem = 0;
@@ -542,35 +583,50 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
         tc_fence_after();
         const uint32_t tmem_d = tmem_base + acc * BN;
         const uint32_t ar_row_step = static_cast<uint32_t>(p.ar_row_step16);
-        for (int kb = 0; AR && kb < 3 * p.cin_blocks; ++kb) {
-          C2W_TIMED_WAIT(w_full, &full[stage], phase);
-          tc_fence_after();
-          if (elect_one()) {
-            const uint64_t adesc = adesc0 + static_cast<uint64_t>(stage * (Cfg::kARStageBytes >> 4));
-            const uint64_t bdesc = adesc + static_cast<uint64_t>(Cfg::kARUnitBytes >> 4);
+        // K order cb -> s -> r -> k: each filter column's weight stage is released as soon as its nine MMAs are issued
+        for (int cb = 0; AR && cb < p.cin_blocks; ++cb) {
+          C2W_TIMED_WAIT(w_full, &a_full[unit], a_phase);
+          const uint64_t adesc_u = adesc0 + static_cast<uint64_t>(unit * (Cfg::kARUnitBytes >> 4));
+          for (int s3 = 0; s3 < 3; ++s3) {
+            C2W_TIMED_WAIT(w_full, &full[stage], phase);
+            tc_fence_after();
+            if (elect_one()) {
+              const uint64_t bdesc = bdesc0 + static_cast<uint64_t>(stage * (Cfg::kARBStageBytes >> 4));
   #pragma unroll
-            for (int r = 0; r < 3; ++r) {
+              for (int r = 0; r < 3; ++r) {
+                // tap (r, s) = the unit from its r-th pixel row and s-th pixel column on.  The 128B swizzle is a
+                // function of the absolute shared-memory address for the MMA's reads as for TMA's writes, so a start
+                // address s * 128 B into a swizzle atom with 1280 B between 8-row groups reads what TMA wrote; the
+                // descriptor's base-offset field stays 0 (set to (start >> 7) & 7 it gives wrong results).
+                const uint64_t adesc = adesc_u + r * ar_row_step + s3 * 8;
   #pragma unroll
-              for (int k = 0; k < kBlockK / 16; ++k) {
-                // filter row r = the unit from its r-th pixel row on: + r * 8 rows * 128 B (keeps the swizzle phase)
-                const uint64_t a = adesc + r * ar_row_step + 2 * k;
-                const uint64_t b = bdesc + r * (Cfg::kBTileBytes >> 4) + 2 * k;
-                if (CG == 2) umma_bf16_pair(tmem_d, a, b, idesc, (kb | r | k) != 0);
-                else umma_bf16(tmem_d, a, b, idesc, (kb | r | k) != 0);
+                for (int k = 0; k < kBlockK / 16; ++k) {
+                  const uint64_t a = adesc + 2 * k;
+                  const uint64_t b = bdesc + r * (Cfg::kBTileBytes >> 4) + 2 * k;
+                  if (CG == 2) umma_bf16_pair(tmem_d, a, b, idesc, (cb | s3 | r | k) != 0);
+                  else umma_bf16(tmem_d, a, b, idesc, (cb | s3 | r | k) != 0);
+                }
+              }
+              const bool last = s3 == 2 && cb + 1 == p.cin_blocks;
+              if (CG == 2) {
+                umma_commit_pair(&empty[stage]);
+                if (s3 == 2) umma_commit_pair(&a_empty[unit]);
+                if (last) umma_commit_pair(&tmem_full[acc]);
+              } else {
+                umma_commit(&empty[stage]);
+                if (s3 == 2) umma_commit(&a_empty[unit]);
+                if (last) umma_commit(&tmem_full[acc]);
               }
             }
-            if (CG == 2) {
-              umma_commit_pair(&empty[stage]);
-              if (kb + 1 >= 3 * p.cin_blocks) umma_commit_pair(&tmem_full[acc]);
-            } else {
-              umma_commit(&empty[stage]);
-              if (kb + 1 >= 3 * p.cin_blocks) umma_commit(&tmem_full[acc]);
+            __syncwarp();
+            if (++stage == num_stages) {
+              stage = 0;
+              phase ^= 1;
             }
           }
-          __syncwarp();
-          if (++stage == num_stages) {
-            stage = 0;
-            phase ^= 1;
+          if (++unit == num_units) {
+            unit = 0;
+            a_phase ^= 1;
           }
         }
         for (int kb = 0; !AR && kb < num_kb; kb += Cfg::kSub) {
@@ -984,8 +1040,10 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
 #endif
   if (warp_idx == 2) {
     tc_fence_after();
-    if (CG == 2) tmem_dealloc_pair(tmem_base, Cfg::kTmemCols);
-    else tmem_dealloc(tmem_base, Cfg::kTmemCols);
+    // AR: the TMEM base is read back from shared memory rather than kept live through the whole kernel, which would
+    // take a register from the 56 of the producer / MMA warps of the LayerNorm kernels (ptxas spills it otherwise)
+    if (CG == 2) tmem_dealloc_pair(AR ? *tmem_slot : tmem_base, Cfg::kTmemCols);
+    else tmem_dealloc(AR ? *tmem_slot : tmem_base, Cfg::kTmemCols);
   }
 }
 
@@ -1131,11 +1189,11 @@ inline bool conv_launch_init(ConvLaunch* L, bool is_conv3x3, const __nv_bfloat16
       p.tiles_per_img = (H / 16) * p.tiles_w;
       p.img_h = H;
       p.img_w = W;
-      p.ar_row_step16 = (8 * 128) >> 4;
-      const int b_bytes = 3 * (bn / L->cg) * kBlockK * 2;
-      p.ar_tx_bytes = 18 * 8 * kBlockK * 2 + b_bytes;
+      p.ar_row_step16 = (kARUnitW * 128) >> 4;
+      p.ar_tx_a = 18 * kARUnitW * kBlockK * 2;
+      p.ar_tx_b = 3 * (bn / L->cg) * kBlockK * 2;
       const uint64_t dims[4] = {(uint64_t)cin, (uint64_t)W, (uint64_t)H, (uint64_t)n_img};
-      const uint32_t box[4] = {(uint32_t)kBlockK, 8u, 18u, 1u};
+      const uint32_t box[4] = {(uint32_t)kBlockK, (uint32_t)kARUnitW, 18u, 1u};
       if (!make_tmap_bf16(&L->tmA, x, 4, dims, box)) return false;
     } else if (want_ar && stride == 1 && bn == 128 && L->cg == 2 && H == 8 && W % 8 == 0 && n_img >= 2) {
       // two 8-row images per M tile, image dimension inside the row dimension (see ConvParams::ar2)
@@ -1146,12 +1204,13 @@ inline bool conv_launch_init(ConvLaunch* L, bool is_conv3x3, const __nv_bfloat16
       p.num_m_tiles = ((n_img + 1) / 2) * p.tiles_w;
       p.img_h = H;
       p.img_w = W;
-      p.ar_row_step16 = (2 * 8 * 128) >> 4;
-      p.ar_tx_bytes = 10 * 2 * 8 * kBlockK * 2 + 3 * (bn / L->cg) * kBlockK * 2;
+      p.ar_row_step16 = (2 * kARUnitW * 128) >> 4;
+      p.ar_tx_a = 10 * 2 * kARUnitW * kBlockK * 2;
+      p.ar_tx_b = 3 * (bn / L->cg) * kBlockK * 2;
       const uint64_t row_b = (uint64_t)W * cin * 2;
       const uint64_t dims[4] = {(uint64_t)cin, (uint64_t)W, (uint64_t)n_img, (uint64_t)H};
       const uint64_t strides[3] = {(uint64_t)cin * 2, row_b * H, row_b};
-      const uint32_t box[4] = {(uint32_t)kBlockK, 8u, 2u, 10u};
+      const uint32_t box[4] = {(uint32_t)kBlockK, (uint32_t)kARUnitW, 2u, 10u};
       if (!make_tmap_bf16(&L->tmA, x, 4, dims, box, nullptr, strides)) return false;
     } else {
       if (variant >= 0 && (variant & 4)) return false;  // AR was requested explicitly but does not apply
@@ -1169,7 +1228,14 @@ inline bool conv_launch_init(ConvLaunch* L, bool is_conv3x3, const __nv_bfloat16
     const uint32_t box[4] = {(uint32_t)kBlockK, (uint32_t)kBlockM, 1, 1};
     if (!make_tmap_bf16(&L->tmA, x, 4, dims, box)) return false;
   }
-  {
+  if (L->ar) {
+    // the three B tiles (r = 0..2) of one (filter column s, channel block) in one box: the packed weights
+    // [Cout][r][s][Cin] viewed as {s * Cin + c, Cout, r}, the r tiles landing one after the other in the stage
+    const uint64_t dims[4] = {(uint64_t)3 * cin, (uint64_t)cout_pad, 3, 1};
+    const uint64_t strides[3] = {(uint64_t)9 * cin * 2, (uint64_t)3 * cin * 2, (uint64_t)9 * cin * 2 * cout_pad};
+    const uint32_t box[4] = {(uint32_t)kBlockK, (uint32_t)(bn / L->cg), 3u, 1u};
+    if (!make_tmap_bf16(&L->tmB, w_packed, 4, dims, box, nullptr, strides)) return false;
+  } else {
     const uint64_t dims[2] = {(uint64_t)p.taps * cin, (uint64_t)cout_pad};
     const uint32_t box[2] = {(uint32_t)kBlockK, (uint32_t)(bn / L->cg)};
     if (!make_tmap_bf16(&L->tmB, w_packed, 2, dims, box)) return false;
@@ -1243,6 +1309,7 @@ inline bool conv_use_pdl() {
 template <int BN, int CG, bool LN, bool AR>
 inline cudaError_t conv_launch_variant(const ConvLaunch& L, cudaStream_t stream) {
   using Cfg = ConvCfg<BN, CG>;
+  static_assert(!AR || Cfg::ar_stages_for(2) >= 3, "activation-reuse weight ring too shallow");
   // the attribute is per device: remember which devices of this process have it
   static unsigned long long attr_done = 0;
   int dev = 0;

@@ -208,6 +208,18 @@ def main():
             timeit(f"G2 cg2+AR res skip={sk}", 32, 128, 128, 128, 128, variant=5, skip_loads=sk, res=True, cudnn=False)
             timeit(f"G2 cg2+AR res+LN skip={sk}", 32, 128, 128, 128, 128, variant=5, skip_loads=sk, ln=True, cudnn=False)
         return 0
+    if "--ar" in sys.argv:  # the activation-reuse instances at the step's layer shapes, timing only
+        for _ in range(2):
+            timeit("G2 128x128x128 AR", 32, 128, 128, 128, 128, variant=5, cudnn=False)
+            timeit("G2 128x128x128 AR res", 32, 128, 128, 128, 128, variant=5, res=True, cudnn=False)
+            timeit("G2 128x128x128 AR res+LN", 32, 128, 128, 128, 128, variant=5, ln=True, cudnn=False)
+            timeit("G5 64x64x128 AR res+LN", 64, 64, 64, 128, 128, variant=5, ln=True, cudnn=False)
+            timeit("G6 64x64 256->128 AR", 64, 64, 64, 256, 128, variant=5, cudnn=False)
+            timeit("L2 32x32x256 bn128 AR", 156, 32, 32, 256, 256, variant=5, bn=128, cudnn=False)
+            timeit("L3 16x16x384 bn128 AR", 156, 16, 16, 384, 384, variant=5, bn=128, cudnn=False)
+            timeit("L4 8x8x512 bn128 AR (two-image)", 156, 8, 8, 512, 512, variant=5, bn=128, cudnn=False)
+            timeit("G2 128x128x128 AR bn64", 32, 128, 128, 128, 64, variant=5, bn=64, cudnn=False)
+        return 0
     if "--tiles" in sys.argv:  # N-tile choice per level at the real window count (conv_pick_bn_tiled's cost model)
         n = 156
         for res in (False, True):
