@@ -113,6 +113,10 @@ struct ConvParams {
                             // %globaltimer ns for THIS launch (tools/timeline.py: kernel-inside time vs gaps)
   long long* dbg_stats;  // diagnostics only: per-CTA wait cycles [grid][12] (see tools/bringup_conv.py --stats)
   int dbg_skip_loads;  // diagnostics only: after the ring is primed, signal `full` without issuing TMA loads
+  // EPI_COMPOSE over an ensemble stored member-major (0: one trajectory): windows per member Nw.  Window G is window
+  // G mod Nw of member G div Nw, whose frames start at frame G + 2k (G div Nw); head / tail tests are member-local.
+  // Last, in the struct's tail padding, so that the fields above keep their offsets.
+  int member_win;
 };
 
 constexpr int kBlockM = 128;
@@ -207,13 +211,20 @@ __device__ __forceinline__ void epilogue_chunk_direct(const ConvParams& p, const
     const int n_img = m / p.hw;
     const int pix = m - n_img * p.hw;
     const int win = p.win_list ? __ldg(p.win_list + n_img) : p.win_first + n_img;
+    int j = win, last = p.win_last_global, f0 = win - p.frame_base;  // window within its member, its first frame
+    if (p.member_win > 0) {
+      const int m = win / p.member_win;
+      j = win - m * p.member_win;
+      last = p.member_win - 1;
+      f0 += 2 * p.order_k * m;
+    }
 #pragma unroll
     for (int g = 0; g < 8; ++g) {
       const int tau = (col0 >> 2) + g;  // window slot of channels [4*tau, 4*tau+4)
-      const bool take = (tau == p.order_k) || (win == 0 && tau < p.order_k) ||
-                        (win == p.win_last_global && tau > p.order_k && tau <= 2 * p.order_k);
+      const bool take = (tau == p.order_k) || (j == 0 && tau < p.order_k) ||
+                        (j == last && tau > p.order_k && tau <= 2 * p.order_k);
       if (take) {
-        const long long fl = static_cast<long long>(win + tau - p.frame_base);
+        const long long fl = static_cast<long long>(f0 + tau);
         float4 o = make_float4(f[4 * g], f[4 * g + 1], f[4 * g + 2], f[4 * g + 3]);
         *reinterpret_cast<float4*>(p.eps + (fl * p.hw + pix) * 4) = o;
       }

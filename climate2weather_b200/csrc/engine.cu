@@ -144,6 +144,7 @@ struct c2w_handle {
   int sms = 0;
   bool timing = false;
   bool fuse_ln = true;  // C2W_NO_FUSE_LN=1 keeps every LayerNorm a separate kernel (A/B runs)
+  int tile_windows = 0;  // c2w_bind_workspace_members: K1 tile widths picked for this many windows (0: the bound count)
   bool fuse_dsilu = true;  // C2W_NO_FUSE_DSILU=1: silu' of the input-gradient pass as a separate elementwise kernel
   bool fuse_dual = true;   // C2W_NO_FUSE_DUAL=1: stashing forward with a separate SiLU pass after conv1
   std::vector<TimedSpan> spans;
@@ -412,10 +413,10 @@ int launch_attention(const bf16* qkv, bf16* out, int n, int T, int C, cudaStream
 
 int grid_for(long long items, int threads, int sms);
 
-// K0: window batch [n, hw, cin_pad] bf16 from the resident trajectory (tiled form for 4-variable frames); f0 and
-// win_list as gather_windows_kernel takes them.
+// K0: window batch [n, hw, cin_pad] bf16 from the resident trajectory (tiled form for 4-variable frames); f0,
+// win_list and member_win as gather_windows_kernel takes them.
 int launch_gather(const float* traj, bf16* out, int n, int hw, int C, int w, int cin_pad, int f0, int sms, cudaStream_t st,
-                  const int* win_list = nullptr) {
+                  const int* win_list = nullptr, int member_win = 0) {
   static int tiled = -1;
   if (tiled < 0) {
     const char* e = getenv("C2W_GATHER_TILED");
@@ -423,11 +424,16 @@ int launch_gather(const float* traj, bf16* out, int n, int hw, int C, int w, int
   }
   if (!win_list && tiled && C == 4 && hw % kGatherPix == 0 && w <= 64) {
     const size_t smem = static_cast<size_t>(kGatherWin + w - 1) * kGatherPix * sizeof(uint2);
-    gather_windows_tiled_kernel<<<dim3(hw / kGatherPix, (n + kGatherWin - 1) / kGatherWin), 256, smem, st>>>(traj, out, n, hw, w,
-                                                                                                       cin_pad, f0);
+    // tiles per member times the members [f0, f0 + n) touches, or tiles of the launch
+    const int tiles = member_win > 0 ? ((member_win + kGatherWin - 1) / kGatherWin) *
+                                           ((f0 + n - 1) / member_win - f0 / member_win + 1)
+                                     : (n + kGatherWin - 1) / kGatherWin;
+    gather_windows_tiled_kernel<<<dim3(hw / kGatherPix, tiles), 256, smem, st>>>(traj, out, n, hw, w, cin_pad, f0,
+                                                                                  member_win);
   } else {
     const long long items = static_cast<long long>(n) * hw * (cin_pad / 8);
-    gather_windows_kernel<<<grid_for(items, 256, sms), 256, 0, st>>>(traj, out, n, hw, C, w * C, cin_pad, f0, win_list);
+    gather_windows_kernel<<<grid_for(items, 256, sms), 256, 0, st>>>(traj, out, n, hw, C, w * C, cin_pad, f0, win_list,
+                                                                     member_win);
   }
   C2W_CUDA(cudaGetLastError());
   return C2W_OK;
@@ -589,8 +595,22 @@ int build_plan(c2w_handle* h, int n, bool vjp, bool per_t, void* base, size_t* b
     op->spec.stride = stride;
     // the fp32 / compose epilogues (the last conv of a pass) store 64-wide tiles only; a wider frame (C * window > 64
     // channels) takes several of them
-    const int bn = bn_force ? bn_force : mode == EPI_F32 ? 64 : conv_pick_bn_tiled(cout_pad, c3, n, H, W, stride, h->sms);
-    if (!conv_launch_init(&op->conv, c3, in, n, H, W, cin, wts, cout_pad, bn, h->sms, stride))
+    // The tile width, the CTA pair and the main loop (streamed, activation reuse, its two-image form) are picked from the
+    // window count; the main loop fixes the order of the fp32 sums, the two-image form also whether the LayerNorm is
+    // fused.  An ensemble workspace (h->tile_windows: a member's own window count) makes every one of these choices as
+    // the member's own workspace would, so that its launches compute what the member's run computes.
+    const int n_pick = h->tile_windows > 0 ? h->tile_windows : n;
+    const int bn = bn_force ? bn_force
+                            : mode == EPI_F32 ? 64 : conv_pick_bn_tiled(cout_pad, c3, n_pick, H, W, stride, h->sms);
+    int variant = -1;
+    if (n_pick != n) {  // the member's plan of this conv decides the variant (bit 0 CTA pair, bit 2 activation reuse)
+      ConvLaunch member;
+      if (!conv_launch_init(&member, c3, in, n_pick, H, W, cin, wts, cout_pad, bn, h->sms, stride))
+        return fail(C2W_ERR_INVALID, "cannot build conv launch (n=%d H=%d W=%d cin=%d cout=%d stride=%d) %s", n_pick, H, W,
+                    cin, cout_pad, stride, tmap_error_slot());
+      variant = (member.cg == 2 ? 1 : 0) | (member.ar ? 4 : 0);
+    }
+    if (!conv_launch_init(&op->conv, c3, in, n, H, W, cin, wts, cout_pad, bn, h->sms, stride, variant))
       return fail(C2W_ERR_INVALID, "cannot build conv launch (n=%d H=%d W=%d cin=%d cout=%d stride=%d) %s", n, H, W, cin,
                   cout_pad, stride, tmap_error_slot());
     op->conv.p.mode = mode;
@@ -940,6 +960,7 @@ struct FinalSpec {
   float* eps = nullptr;
   int order_k = 0, win_first = 0, win_last_global = 0, frame_base = 0;
   const int* win_list = nullptr;  // EPI_COMPOSE over a selection of windows
+  int member_win = 0;             // EPI_COMPOSE over an ensemble: windows per member (ConvParams::member_win)
 };
 
 // Runs an op list (the forward pass, or the input-gradient pass) on the first nn windows of the plan.
@@ -973,6 +994,7 @@ int run_ops(c2w_handle* h, std::vector<Op>& ops, int nn, const FinalSpec& fs, cu
           L.p.win_last_global = fs.win_last_global;
           L.p.frame_base = fs.frame_base;
           L.p.win_list = fs.win_list;
+          L.p.member_win = fs.member_win;
         }
 #ifdef C2W_DIAG
         if (h->timeline != nullptr && h->timeline_used < h->timeline_cap) L.p.dbg_timeline = h->timeline + 2 * h->timeline_used++;
@@ -1082,11 +1104,13 @@ int launch_for_vars(int C, F&& launch) {
 
 // The windows of a window-score call: the contiguous global windows [first, first + n) when list is null, else the
 // global windows list[0..n) (device array).  pos (device, n_win_global entries, backward of a list only): the place of
-// global window j in the list, or -1.
+// global window j in the list, or -1.  member_win > 0: the contiguous windows of an ensemble stored member-major, with
+// member_win windows per member (c2w_window_score_members; frame_global0 = 0, no list).
 struct WindowSet {
   int first, n;
   const int* list;
   const int* pos;
+  int member_win = 0;
 };
 
 // Gather -> UNet -> fold into eps, in chunks of the bound workspace.  eps == null: no fold, the window outputs stay
@@ -1103,7 +1127,7 @@ int window_score_fwd(c2w_handle* h, const float* traj, int frame_global0, const 
     const int j0 = ws.first + c0;  // first window of the chunk (contiguous windows)
     const int* list = ws.list ? ws.list + c0 : nullptr;
     if ((rc = launch_gather(traj, P.xin, nn, hw, C, w, h->cin_pad, list ? frame_global0 : j0 - frame_global0, h->sms, st,
-                            list)))
+                            list, ws.member_win)))
       return rc;
     ++g_launches;
     FinalSpec fs;
@@ -1116,12 +1140,14 @@ int window_score_fwd(c2w_handle* h, const float* traj, int frame_global0, const 
       fs.win_last_global = n_win_global - 1;
       fs.frame_base = frame_global0;
       fs.win_list = list;
+      fs.member_win = ws.member_win;
     }
     if ((rc = run_plan(h, nn, fs, st))) return rc;
     if (eps && C != 4) {  // any other variable count: the fold as its own pass over the fp32 window outputs
       const long long items = static_cast<long long>(nn) * hw * C;
       compose_generic_kernel<<<grid_for(items, 256, h->sms), 256, 0, st>>>(P.out32, eps, nn, hw, h->levels[0].tail.cout_pad,
-                                                                           C, k, j0, n_win_global - 1, frame_global0, list);
+                                                                           C, k, j0, n_win_global - 1, frame_global0, list,
+                                                                           ws.member_win);
       ++g_launches;
       C2W_CUDA(cudaGetLastError());
     }
@@ -1410,6 +1436,14 @@ int c2w_bind_workspace_ex(c2w_handle* h, int32_t max_windows, void* dev_ptr, int
   return build_plan(h, max_windows, vjp, per_t, aligned, &need_bytes, train);
 }
 
+int c2w_bind_workspace_members(c2w_handle* h, int32_t max_windows, int32_t tile_windows, void* dev_ptr, int64_t bytes) {
+  C2W_REQUIRE(h && tile_windows >= 1, "c2w_bind_workspace_members: bad argument");
+  h->tile_windows = tile_windows;
+  const int rc = c2w_bind_workspace_ex(h, max_windows, dev_ptr, bytes, 0);
+  h->tile_windows = 0;  // a later bind plans for its own window count again
+  return rc;
+}
+
 int64_t c2w_workspace_bytes(c2w_handle* h, int32_t max_windows) { return c2w_workspace_bytes_ex(h, max_windows, 0); }
 int c2w_bind_workspace(c2w_handle* h, int32_t max_windows, void* dev_ptr, int64_t bytes) {
   return c2w_bind_workspace_ex(h, max_windows, dev_ptr, bytes, 0);
@@ -1487,6 +1521,26 @@ int c2w_window_score(c2w_handle* h, const float* traj, int32_t n_frames_local, i
   C2W_REQUIRE(C >= 1 && C <= 8, "1 to 8 variables per frame (got %d)", C);
   return window_score_fwd(h, traj, frame_global0, WindowSet{win_first, n_win, nullptr, nullptr}, n_win_global, t, eps,
                           static_cast<cudaStream_t>(stream));
+}
+
+// An ensemble stored member-major: window_score_fwd with the member mapping (WindowSet::member_win), whose chunks may
+// mix members; each window folds with its member's own head / tail test.
+int c2w_window_score_members(c2w_handle* h, const float* traj, int32_t n_members, int32_t member_frames,
+                             int32_t win_first, int32_t n_win, float t, float* eps, void* stream) {
+  C2W_REQUIRE(h && traj && eps, "c2w_window_score_members: bad argument");
+  if (h->plan.n_max < 1) return fail(C2W_ERR_STATE, "bind a workspace first");
+  if (h->plan.per_t) return fail(C2W_ERR_STATE, "window scores use one diffusion time: bind a plain workspace");
+  const int w = h->cfg.window, C = h->cfg.frame_channels;
+  C2W_REQUIRE(C >= 1 && C <= 8, "1 to 8 variables per frame (got %d)", C);
+  const int nw = member_frames - (w - 1);
+  C2W_REQUIRE(n_members >= 1 && nw >= 1, "c2w_window_score_members: %d members of %d frames (a window has %d)",
+              n_members, member_frames, w);
+  C2W_REQUIRE(n_win >= 1 && win_first >= 0 && static_cast<long long>(win_first) + n_win <= static_cast<long long>(n_members) * nw,
+              "c2w_window_score_members: window range [%d,%d) outside [0,%lld)", win_first, win_first + n_win,
+              static_cast<long long>(n_members) * nw);
+  WindowSet ws{win_first, n_win, nullptr, nullptr};
+  ws.member_win = nw;
+  return window_score_fwd(h, traj, 0, ws, nw, t, eps, static_cast<cudaStream_t>(stream));
 }
 
 // Forward of a SELECTION of windows (global indices win_list_dev[0..n_sel)).  With the coarse-graining likelihood the
@@ -1910,6 +1964,7 @@ static int guide_params(const c2w_guide* g, const char* what, GuideParams& p, in
   p.publish = 0;
   p.halo_k = g->halo_k;
   p.own_n = g->own_n;
+  p.member_frames = 0;
   if (g->halo != nullptr && g->mode == 0) {  // fused halo push (csrc/halo.cu)
     C2W_REQUIRE(g->halo_k >= 1 && g->own_n >= g->halo_k, "%s: fused halo push needs 1 <= halo_k <= own_n", what);
     void *sl, *sr, *fl, *fr, *dn;
@@ -1939,9 +1994,11 @@ static PointParams point_params(const c2w_point_obs* obs) {
 
 // The bodies of c2w_guided_step, c2w_guided_step_points and c2w_guided_step_combined: their argument checks, then
 // the per-variable (PerObs = false) or per-observation (c2w_guided_step_obs_std) instance of K6, K6p or K6c.
+// member_frames > 0 (c2w_guided_step_members): the Members instances of K6 and K6c, which observe frame f as member
+// frame f mod member_frames; K6p reads the frame's slot from obs->frame_slot either way.
 extern "C++" {
 template <bool PerObs>
-static int guided_coarse(const c2w_guide* g, const ObsStd2& v, void* stream) {
+static int guided_coarse(const c2w_guide* g, const ObsStd2& v, void* stream, int member_frames = 0) {
   C2W_REQUIRE(g->s_step >= 1 && g->H % g->s_step == 0 && g->W % g->s_step == 0 && g->W / g->s_step <= 32,
               "s_step=%d must divide %dx%d with at most 32 tiles per row", g->s_step, g->H, g->W);
   C2W_REQUIRE(g->mode != 2 || (g->cot_out && g->y), "mode 2 needs cot_out and an observation");
@@ -1950,10 +2007,12 @@ static int guided_coarse(const c2w_guide* g, const ObsStd2& v, void* stream) {
   int C;
   int rc = guide_params(g, "c2w_guided_step", p, C);
   if (rc) return rc;
+  p.member_frames = member_frames;
   dim3 grid(g->H / g->s_step, g->own_n);
   return launch_for_vars(C, [&](auto vars) {
-    guided_step_kernel<decltype(vars)::value, PerObs>
-        <<<grid, 32 * (g->W / g->s_step), 0, static_cast<cudaStream_t>(stream)>>>(p, v);
+    const auto kernel = member_frames > 0 ? guided_step_kernel<decltype(vars)::value, PerObs, true>
+                                          : guided_step_kernel<decltype(vars)::value, PerObs>;
+    kernel<<<grid, 32 * (g->W / g->s_step), 0, static_cast<cudaStream_t>(stream)>>>(p, v);
   });
 }
 
@@ -1978,7 +2037,7 @@ static int guided_points(const c2w_guide* g, const c2w_point_obs* obs, const Obs
 
 template <bool PerObs>
 static int guided_combined(const c2w_guide* g, const c2w_point_obs* obs, const float* point_std2, const ObsStd2& v,
-                           void* stream) {
+                           void* stream, int member_frames = 0) {
   C2W_REQUIRE(obs->frame_slot && obs->strip_off, "c2w_guided_step_combined: bad argument");
   C2W_REQUIRE(obs->n_slots == 0 || (obs->pix && obs->ysum && obs->wsum), "c2w_guided_step_combined: entries missing");
   C2W_REQUIRE(g->y, "c2w_guided_step_combined: needs the coarse observation y");
@@ -1995,6 +2054,7 @@ static int guided_combined(const c2w_guide* g, const c2w_point_obs* obs, const f
   int C;
   int rc = guide_params(g, "c2w_guided_step_combined", p, C);
   if (rc) return rc;
+  p.member_frames = member_frames;
   PointParams q = point_params(obs);
   PointStd2 ps;
   for (int i = 0; i < C2W_MAX_VARS; ++i) ps.v[i] = i < C && !PerObs ? point_std2[i] : 0.f;
@@ -2002,7 +2062,8 @@ static int guided_combined(const c2w_guide* g, const c2w_point_obs* obs, const f
   dim3 grid((g->H + obs->strip_rows - 1) / obs->strip_rows, g->own_n);
   cudaError_t attr = cudaSuccess;
   rc = launch_for_vars(C, [&](auto vars) {
-    const auto kernel = guided_combined_kernel<decltype(vars)::value, PerObs>;
+    const auto kernel = member_frames > 0 ? guided_combined_kernel<decltype(vars)::value, PerObs, true>
+                                          : guided_combined_kernel<decltype(vars)::value, PerObs>;
     if (smem > 48 * 1024) attr = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (attr == cudaSuccess) kernel<<<grid, 256, smem, static_cast<cudaStream_t>(stream)>>>(p, q, ps, v);
   });
@@ -2040,12 +2101,71 @@ int c2w_guided_step_obs_std(const c2w_guide* g, const c2w_point_obs* obs, const 
   return guided_combined<true>(g, obs, nullptr, v, stream);
 }
 
+int c2w_guided_step_members(const c2w_guide* g, int32_t member_frames, const c2w_point_obs* obs, const float* point_std2,
+                            const float* coarse_std2, const float* entry_std2, void* stream) {
+  C2W_REQUIRE(g, "c2w_guided_step_members: bad argument");
+  C2W_REQUIRE(member_frames >= 1 && g->own_n % member_frames == 0,
+              "c2w_guided_step_members: own_n=%d is not a whole number of members of %d frames", g->own_n, member_frames);
+  C2W_REQUIRE((g->frame_global0 + g->own_lo) % member_frames == 0,
+              "c2w_guided_step_members: frame_global0 + own_lo = %d is not the first frame of a member of %d frames",
+              g->frame_global0 + g->own_lo, member_frames);
+  C2W_REQUIRE(g->halo == nullptr, "c2w_guided_step_members: an ensemble is not time-sharded (halo must be NULL)");
+  if (coarse_std2 || entry_std2) {  // a std per observation: the checks of c2w_guided_step_obs_std
+    C2W_REQUIRE((g->y == nullptr) == (coarse_std2 == nullptr),
+                "c2w_guided_step_members: the coarse term needs both g->y and coarse_std2, or neither");
+    C2W_REQUIRE((obs == nullptr) == (entry_std2 == nullptr),
+                "c2w_guided_step_members: the point term needs both obs and entry_std2, or neither");
+    C2W_REQUIRE(point_std2 == nullptr, "c2w_guided_step_members: point_std2 with a std per observation");
+    const ObsStd2 v{coarse_std2, entry_std2};
+    if (obs == nullptr) return guided_coarse<true>(g, v, stream, member_frames);
+    if (g->y == nullptr) return guided_points<true>(g, obs, v, stream);
+    return guided_combined<true>(g, obs, nullptr, v, stream, member_frames);
+  }
+  if (obs == nullptr) {
+    C2W_REQUIRE(point_std2 == nullptr, "c2w_guided_step_members: point_std2 without obs");
+    return guided_coarse<false>(g, ObsStd2{}, stream, member_frames);
+  }
+  if (g->y == nullptr) {
+    C2W_REQUIRE(point_std2 == nullptr, "c2w_guided_step_members: point_std2 without a coarse term (the point term's "
+                "std^2 is g->std2)");
+    return guided_points<false>(g, obs, ObsStd2{}, stream);
+  }
+  C2W_REQUIRE(point_std2, "c2w_guided_step_members: a coarse and a point term need point_std2");
+  return guided_combined<false>(g, obs, point_std2, ObsStd2{}, stream, member_frames);
+}
+
 int c2w_reduce_partials(const float* partials, int32_t n, double* sumsq, void* stream) {
   C2W_REQUIRE(partials && sumsq && n >= 1, "c2w_reduce_partials: bad argument");
   reduce_partials_kernel<<<1, 256, 0, static_cast<cudaStream_t>(stream)>>>(partials, n, sumsq);
   ++g_launches;
   C2W_CUDA(cudaGetLastError());
   return C2W_OK;
+}
+
+int c2w_reduce_partials_members(const float* partials, int32_t n_members, int32_t member_partials, double* sumsq,
+                                void* stream) {
+  C2W_REQUIRE(partials && sumsq && n_members >= 1 && member_partials >= 1, "c2w_reduce_partials_members: bad argument");
+  reduce_partials_segments_kernel<<<n_members, 256, 0, static_cast<cudaStream_t>(stream)>>>(partials, member_partials,
+                                                                                            sumsq);
+  ++g_launches;
+  C2W_CUDA(cudaGetLastError());
+  return C2W_OK;
+}
+
+int c2w_corrector_update_members(float* x, const float* eps, const double* sumsq, double count, float tau,
+                                 float sigma_next, int32_t n_members, int64_t member_pix, int32_t channels,
+                                 const uint64_t* seeds, uint32_t step_id, int32_t* nan_flag, void* stream) {
+  C2W_REQUIRE(x && eps && sumsq && seeds && nan_flag && n_members >= 1 && member_pix >= 1 && count > 0,
+              "c2w_corrector_update_members: bad argument");
+  C2W_REQUIRE(channels >= 1 && channels <= C2W_MAX_VARS,
+              "c2w_corrector_update_members: 1 to %d variables per frame (got %d)", C2W_MAX_VARS, channels);
+  const long long npix = static_cast<long long>(n_members) * member_pix;
+  return launch_for_vars(channels, [&](auto vars) {
+    corrector_members_kernel<decltype(vars)::value><<<grid_for(npix, 256, c2w_num_sms()), 256, 0,
+                                                      static_cast<cudaStream_t>(stream)>>>(
+        x, eps, sumsq, count, tau, sigma_next, member_pix, npix, reinterpret_cast<const unsigned long long*>(seeds),
+        step_id, nan_flag);
+  });
 }
 
 int c2w_corrector_update_c(float* x, const float* eps, const float* z, const double* sumsq, double count, float tau,

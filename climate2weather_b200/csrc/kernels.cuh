@@ -40,8 +40,11 @@ __device__ __forceinline__ float2 unpack_bf16x2(uint32_t w) {
 // One thread writes 8 channels (16 B): writes are fully coalesced, reads are 16 B (C = 4) sectors.
 // win_list (optional): GLOBAL window indices of the n windows (a selection, e.g. the windows whose output carries a
 // non-zero cotangent); window i then starts at local frame win_list[i] - f0 (f0 = global index of local frame 0).
+// member_win > 0 (an ensemble stored member-major, no list): window G = f0 + i is window G mod member_win of member
+// m = G div member_win and starts at frame G + (w - 1) m, so that no window crosses members.
 __global__ void gather_windows_kernel(const float* __restrict__ traj, bf16* __restrict__ out, int n, int hw, int C,
-                                      int wC, int cin_pad, int f0, const int* __restrict__ win_list = nullptr) {
+                                      int wC, int cin_pad, int f0, const int* __restrict__ win_list = nullptr,
+                                      int member_win = 0) {
   const int groups = cin_pad >> 3;
   const long long total = static_cast<long long>(n) * hw * groups;
   for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
@@ -50,7 +53,8 @@ __global__ void gather_windows_kernel(const float* __restrict__ traj, bf16* __re
     const long long pw = idx / groups;
     const int pix = static_cast<int>(pw % hw);
     const int i = static_cast<int>(pw / hw);
-    const int fw = win_list ? (win_list[i] - f0) : (f0 + i);  // first local frame of window i
+    int fw = win_list ? (win_list[i] - f0) : (f0 + i);  // first local frame of window i
+    if (member_win > 0) fw += (wC / C - 1) * (fw / member_win);
     float v[8];
     if (C == 4) {
 #pragma unroll
@@ -81,16 +85,31 @@ __global__ void gather_windows_kernel(const float* __restrict__ traj, bf16* __re
 // Tiled form for C = 4 (the shipped 4-variable frames): a CTA owns 64 pixels x kGatherWin consecutive windows, reads the
 // kGatherWin + w - 1 frames they span ONCE (coalesced float4 -> packed bf16x4 in shared memory) and writes every
 // window's 128-byte pixel rows from there: each frame pixel leaves L2 1.75 times (w = 13) instead of 13 times.
+// member_win > 0 (an ensemble, windows numbered as in gather_windows_kernel): the tiles are cut per member, so that a
+// CTA's windows are consecutive windows of one member and its frames are still nwin + w - 1 consecutive frames.  The
+// grid then has ceil(member_win / kGatherWin) tiles per member the launch touches; a tile outside [f0, f0 + n) exits.
 constexpr int kGatherWin = 16, kGatherPix = 64;
 __global__ void __launch_bounds__(256) gather_windows_tiled_kernel(const float* __restrict__ traj, bf16* __restrict__ out,
-                                                                   int n, int hw, int w, int cin_pad, int f0) {
+                                                                   int n, int hw, int w, int cin_pad, int f0,
+                                                                   int member_win = 0) {
   extern __shared__ uint2 gtile[];  // [frames][kGatherPix] bf16x4
-  const int pix0 = blockIdx.x * kGatherPix, i0 = blockIdx.y * kGatherWin;
-  const int nwin = (n - i0) < kGatherWin ? (n - i0) : kGatherWin;
+  const int pix0 = blockIdx.x * kGatherPix;
+  int i0 = blockIdx.y * kGatherWin, nwin = (n - i0) < kGatherWin ? (n - i0) : kGatherWin, fr0 = f0 + i0;
+  if (member_win > 0) {
+    const int tiles = (member_win + kGatherWin - 1) / kGatherWin;
+    const int m = f0 / member_win + static_cast<int>(blockIdx.y) / tiles;
+    const int lo = max(f0, m * member_win + (static_cast<int>(blockIdx.y) % tiles) * kGatherWin);
+    const int hi = min(min(m * member_win + (static_cast<int>(blockIdx.y) % tiles + 1) * kGatherWin, (m + 1) * member_win),
+                       f0 + n);
+    if (lo >= hi) return;  // uniform over the CTA
+    i0 = lo - f0;
+    nwin = hi - lo;
+    fr0 = lo + (w - 1) * m;
+  }
   const int nfr = nwin + w - 1;
   for (int idx = threadIdx.x; idx < nfr * kGatherPix; idx += blockDim.x) {
     const int fr = idx / kGatherPix, px = idx - fr * kGatherPix;
-    const float4 q = __ldg(reinterpret_cast<const float4*>(traj + (static_cast<long long>(f0 + i0 + fr) * hw + pix0 + px) * 4));
+    const float4 q = __ldg(reinterpret_cast<const float4*>(traj + (static_cast<long long>(fr0 + fr) * hw + pix0 + px) * 4));
     gtile[idx] = make_uint2(pack_bf16x2(q.x, q.y), pack_bf16x2(q.z, q.w));
   }
   __syncthreads();
@@ -1544,7 +1563,18 @@ struct GuideParams {
   unsigned int* push_done; // CTA counter (local)
   unsigned int publish;    // value to publish: step + 1
   int halo_k, own_n;
+  // Members instances (an ensemble stored member-major, c2w_guided_step_members): frames per member L.  The frame test
+  // and y's offset use the member frame f mod L.  Last, in the struct's tail padding: the fields above keep their
+  // offsets and the kernels' parameter blocks their size.
+  int member_frames;
 };
+
+// The frame the observation operator sees for local frame fl: the global frame, or with Members its frame within its
+// member.
+template <bool Members>
+__device__ __forceinline__ int observed_frame(const GuideParams& p, int fl) {
+  return Members ? (p.frame_global0 + fl) % p.member_frames : p.frame_global0 + fl;
+}
 
 // mode 1: the CTA's sum of eps_guided^2 -> partials[blockIdx.y * gridDim.x + blockIdx.x] (fixed order, no atomics)
 __device__ __forceinline__ void block_partial(const GuideParams& p, float sq) {
@@ -1696,12 +1726,12 @@ __device__ __forceinline__ void tile_cotangent(const GuideParams& p, bool observ
 }
 
 // CTA = one s-row strip of one frame; one warp per s x s observation tile.
-template <int C, bool PerObs>
+template <int C, bool PerObs, bool Members = false>
 __global__ void guided_step_kernel(const GuideParams p, const ObsStd2 v) {
   const int warp = threadIdx.x >> 5;
   const int s = p.s_step;
   const int fl = p.own_lo + blockIdx.y;
-  const int fg = p.frame_global0 + fl;
+  const int fg = observed_frame<Members>(p, fl);
   const long long fbase = (static_cast<long long>(fl) * p.H) * p.W;
   const bool observed = (p.y != nullptr) && (fg % p.t_step == 0);
   const float inv_mu = 1.0f / p.mu;
@@ -1867,13 +1897,13 @@ struct CombinedObs {
 };
 
 // PerObs: pstd2 is not read; the variances come from v.
-template <int C, bool PerObs>
+template <int C, bool PerObs, bool Members = false>
 __global__ void __launch_bounds__(256) guided_combined_kernel(const GuideParams p, const PointParams q,
                                                               const PointStd2 pstd2, const ObsStd2 v) {
   extern __shared__ __align__(16) int combined_smem[];
   const int s = p.s_step, tiles_w = p.W / s;
   const int fl = p.own_lo + blockIdx.y;
-  const int fg = p.frame_global0 + fl;
+  const int fg = observed_frame<Members>(p, fl);
   const long long fbase = (static_cast<long long>(fl) * p.H) * p.W;
   float* corr = reinterpret_cast<float*>(combined_smem + combined_map_ints(q.strip_rows, p.W));
   const bool coarse = fg % p.t_step == 0;
@@ -1897,10 +1927,10 @@ __global__ void __launch_bounds__(256) guided_combined_kernel(const GuideParams 
 
 // Fold of the window outputs (fp32 [n, hw, cpad], EPI_F32 of the last conv) into the composed score [frames, hw, C]:
 // the centre slot of every window, the head slots of window 0 and the tail slots of the last window
-// (src/thor/score.py:76-88) — what the K1 compose epilogue does for C = 4.
+// (src/thor/score.py:76-88) — what the K1 compose epilogue does for C = 4.  member_win: as ConvParams::member_win.
 __global__ void compose_generic_kernel(const float* __restrict__ out32, float* __restrict__ eps, int n, int hw, int cpad,
                                        int C, int k, int win_first, int win_last_global, int frame_base,
-                                       const int* __restrict__ win_list) {
+                                       const int* __restrict__ win_list, int member_win = 0) {
   const long long total = static_cast<long long>(n) * hw * C;
   for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
        idx += static_cast<long long>(gridDim.x) * blockDim.x) {
@@ -1908,10 +1938,17 @@ __global__ void compose_generic_kernel(const float* __restrict__ out32, float* _
     const long long ip = idx / C;
     const int pix = static_cast<int>(ip % hw), i = static_cast<int>(ip / hw);
     const int win = win_list ? win_list[i] : win_first + i;
+    int j = win, last = win_last_global, f0 = win - frame_base;  // window within its member, its first frame
+    if (member_win > 0) {
+      const int m = win / member_win;
+      j = win - m * member_win;
+      last = member_win - 1;
+      f0 += 2 * k * m;
+    }
     const float* src = out32 + (static_cast<long long>(i) * hw + pix) * cpad + c;
-    const int t0 = (win == 0) ? 0 : k, t1 = (win == win_last_global) ? 2 * k : k;
+    const int t0 = (j == 0) ? 0 : k, t1 = (j == last) ? 2 * k : k;
     for (int tau = t0; tau <= t1; ++tau)
-      eps[((static_cast<long long>(win + tau - frame_base)) * hw + pix) * C + c] = src[tau * C];
+      eps[((static_cast<long long>(f0 + tau)) * hw + pix) * C + c] = src[tau * C];
   }
 }
 
@@ -1955,8 +1992,9 @@ __global__ void adamw_ema_kernel(float* __restrict__ p, const float* __restrict_
     adamw_ema_one(p[i], g[i], m[i], v[i], ema ? ema + i : nullptr, h);
 }
 
-// Deterministic final reduction of the per-CTA partials (fixed order, double accumulate).
-__global__ void reduce_partials_kernel(const float* __restrict__ partials, int n, double* __restrict__ out) {
+// Deterministic final reduction of the per-CTA partials (fixed order, double accumulate): 256 strided lanes, then the
+// tree.  One block of 256 threads per reduction.
+__device__ __forceinline__ void reduce_partials_block(const float* __restrict__ partials, int n, double* __restrict__ out) {
   __shared__ double sh[256];
   double acc = 0.0;
   for (int i = threadIdx.x; i < n; i += blockDim.x) acc += static_cast<double>(partials[i]);
@@ -1967,6 +2005,14 @@ __global__ void reduce_partials_kernel(const float* __restrict__ partials, int n
     __syncthreads();
   }
   if (threadIdx.x == 0) out[0] = sh[0];
+}
+__global__ void reduce_partials_kernel(const float* __restrict__ partials, int n, double* __restrict__ out) {
+  reduce_partials_block(partials, n, out);
+}
+// One reduction per member of an ensemble: block m sums partials [m seg, (m + 1) seg) into out[m], in the order above,
+// so that each value equals reduce_partials_kernel's over that segment alone.
+__global__ void reduce_partials_segments_kernel(const float* __restrict__ partials, int seg, double* __restrict__ out) {
+  reduce_partials_block(partials + static_cast<long long>(blockIdx.x) * seg, seg, out + blockIdx.x);
 }
 
 // Philox4x32-10 (counter-based; keyed by seed, counter = (global pixel index, step id)).
@@ -2021,6 +2067,44 @@ __global__ void corrector_update_kernel(float* __restrict__ x, const float* __re
 #pragma unroll
         for (int e = 0; e < 4 && 4 * b + e < C; ++e) zv[4 * b + e] = n[e];
       }
+    }
+#pragma unroll
+    for (int c = 0; c < C; ++c) {
+      xv[c] -= (delta * ev[c] + zs * zv[c]) * sigma_next;
+      bad |= !isfinite(xv[c]);
+    }
+    store_vars<C>(x + i * C, xv);
+  }
+  if (bad) atomicOr(nan_flag, 1);
+}
+
+// The corrector of an ensemble stored member-major, member_pix pixels per member: pixel i of member m gets m's delta
+// (sumsq[m], one reduce_partials_segments_kernel value each) and z keyed by (seeds[m], step_id, i) — exactly what
+// corrector_update_kernel gives member m alone with seed seeds[m].
+template <int C>
+__global__ void corrector_members_kernel(float* __restrict__ x, const float* __restrict__ eps,
+                                         const double* __restrict__ sumsq, double count, float tau, float sigma_next,
+                                         long long member_pix, long long npix, const unsigned long long* __restrict__ seeds,
+                                         unsigned int step_id, int* nan_flag) {
+  bool bad = false;
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < npix;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long m = i / member_pix;
+    const float delta = tau / static_cast<float>(sumsq[m] / count);
+    const float zs = sqrtf(2.0f * delta);
+    const unsigned long long g = static_cast<unsigned long long>(i - m * member_pix), seed = seeds[m];
+    Vars<C> xv = load_vars<C>(x + i * C);
+    const Vars<C> ev = load_vars<C>(eps + i * C);
+    Vars<C> zv;
+#pragma unroll
+    for (int b = 0; 4 * b < C; ++b) {
+      const uint4 r = philox4x32_10(make_uint4(static_cast<uint32_t>(g), static_cast<uint32_t>(g >> 32), step_id,
+                                               static_cast<uint32_t>(b)),
+                                    make_uint2(static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32)));
+      const float2 n0 = box_muller(r.x, r.y), n1 = box_muller(r.z, r.w);
+      const float n[4] = {n0.x, n0.y, n1.x, n1.y};
+#pragma unroll
+      for (int e = 0; e < 4 && 4 * b + e < C; ++e) zv[4 * b + e] = n[e];
     }
 #pragma unroll
     for (int c = 0; c < C; ++c) {

@@ -83,7 +83,7 @@ class Engine:
 
     def __init__(self, net: "ScoreUNet", frame_channels: int, window: int, height: int, width: int,
                  device: torch.device, max_windows: int, vjp: bool = False, per_sample_t: bool = False,
-                 train: bool = False):
+                 train: bool = False, tile_windows: int = 0):
         self.lib = _lib.load()
         self.device = torch.device(device)
         if self.device.type != "cuda":
@@ -108,6 +108,7 @@ class Engine:
                            f"c2w_load_weight({name})")
             _lib.check(self.lib.c2w_finalize_weights(self.handle), "c2w_finalize_weights")
             self.max_windows = 0
+            self.tile_windows = 0
             self.workspace = None
             self.vjp = bool(vjp) or bool(train)
             self.per_sample_t = bool(per_sample_t) or bool(train)
@@ -121,9 +122,12 @@ class Engine:
                 self.layout[name] = (int(off.value), int(num.value))
             self._flat_scratch: Optional[Tensor] = None
             self._train_token = None
-            self.bind(max_windows)
+            self.bind(max_windows, tile_windows)
 
-    def bind(self, max_windows: int) -> None:
+    def bind(self, max_windows: int, tile_windows: int = 0) -> None:
+        """Binds a workspace of max_windows windows.  tile_windows > 0 (an ensemble, plain workspace only): the convs are
+        planned (tile width, CTA pair, main loop) as for tile_windows windows, a member's own workspace
+        (c2w_bind_workspace_members)."""
         flags = _lib.WS_TRAIN if self.train else ((_lib.WS_VJP if self.vjp else 0) |
                                                   (_lib.WS_PER_SAMPLE_T if self.per_sample_t else 0))
         with torch.cuda.device(self.device):
@@ -132,9 +136,16 @@ class Engine:
                 _lib.check(-1, "c2w_workspace_bytes")
             self.workspace = None  # release the old arena before taking the new one
             self.workspace = torch.empty(nbytes + 1024, dtype=torch.uint8, device=self.device)
-            _lib.check(self.lib.c2w_bind_workspace_ex(self.handle, max_windows, self.workspace.data_ptr(),
-                                                      self.workspace.numel(), flags), "c2w_bind_workspace")
-            self.max_windows = max_windows
+            if tile_windows:
+                if flags:
+                    raise _lib.C2WError("an ensemble workspace is a plain one (no VJP / per-sample times)")
+                _lib.check(self.lib.c2w_bind_workspace_members(self.handle, max_windows, tile_windows,
+                                                               self.workspace.data_ptr(), self.workspace.numel()),
+                           "c2w_bind_workspace_members")
+            else:
+                _lib.check(self.lib.c2w_bind_workspace_ex(self.handle, max_windows, self.workspace.data_ptr(),
+                                                          self.workspace.numel(), flags), "c2w_bind_workspace")
+            self.max_windows, self.tile_windows = max_windows, tile_windows
 
     @property
     def stream(self) -> int:
@@ -252,6 +263,15 @@ class Engine:
                                                  n_win, n_win_global, float(t), eps.data_ptr(), self.stream),
                        "c2w_window_score")
 
+    def window_score_members(self, traj: Tensor, n_members: int, member_frames: int, win_first: int, n_win: int,
+                             t: float, eps: Tensor) -> None:
+        """Windows [win_first, win_first + n_win) of an ensemble stored member-major: traj / eps fp32
+        [n_members * member_frames, H, W, C] (c2w_window_score_members)."""
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.c2w_window_score_members(self.handle, traj.data_ptr(), n_members, member_frames,
+                                                         win_first, n_win, float(t), eps.data_ptr(), self.stream),
+                       "c2w_window_score_members")
+
     def __del__(self):
         try:
             if getattr(self, "handle", None) and self.handle.value:
@@ -356,15 +376,19 @@ class ScoreUNet(nn.Module):
         return (getattr(self, "_weights_epoch", 0),) + tuple((p.data_ptr(), p._version) for p in self.parameters())
 
     def engine(self, frame_channels: int, window: int, height: int, width: int, device, max_windows: Optional[int] = None,
-               vjp: bool = False, per_sample_t: bool = False, train: bool = False) -> Engine:
+               vjp: bool = False, per_sample_t: bool = False, train: bool = False, tile_windows: int = 0) -> Engine:
         """Packed-weight engine for this geometry; if the parameters changed since it was packed (and still live on its
-        device) the weights are re-packed in place on the device, otherwise the engine is rebuilt."""
+        device) the weights are re-packed in place on the device, otherwise the engine is rebuilt.  tile_windows: see
+        Engine.bind (an ensemble's workspace); 0 plans the tiles for the bound window count."""
         device = torch.device(device)
         if device.type == "cuda" and device.index is None:
             device = torch.device("cuda", torch.cuda.current_device())
         if frame_channels * window != self.channels:
             raise ValueError(f"frame_channels*window = {frame_channels * window} != channels = {self.channels}")
-        key = (frame_channels, window, height, width, str(device), bool(vjp), bool(per_sample_t), bool(train))
+        # an ensemble's engine (tile_windows > 0) is kept apart from the plain one: alternating ensemble and single runs
+        # then rebind neither
+        key = (frame_channels, window, height, width, str(device), bool(vjp), bool(per_sample_t), bool(train),
+               bool(tile_windows))
         fp = self._fingerprint()
         hit = self._engines.get(key)
         want = max_windows or self.DEFAULT_MAX_WINDOWS
@@ -377,11 +401,11 @@ class ScoreUNet(nn.Module):
                     eng.refresh_weights(self)
                     self._engines[key] = (eng, fp)
             if hit is not None:
-                if max_windows is not None and eng.max_windows != max_windows:
-                    eng.bind(max_windows)
+                if (max_windows is not None and eng.max_windows != max_windows) or eng.tile_windows != tile_windows:
+                    eng.bind(max_windows or eng.max_windows, tile_windows)
                 return eng
         eng = Engine(self, frame_channels, window, height, width, device, want, vjp=vjp, per_sample_t=per_sample_t,
-                     train=train)
+                     train=train, tile_windows=tile_windows)
         self._engines[key] = (eng, fp)
         return eng
 

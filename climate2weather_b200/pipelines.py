@@ -10,7 +10,7 @@ from __future__ import annotations
 
 import math
 import time
-from typing import Optional
+from typing import Optional, Sequence
 
 import torch
 from torch import Tensor
@@ -77,23 +77,64 @@ class SDAPipeline:
                             f"got {type(score_fn).__name__}.  There is no generic torch-op sampling loop here.")
         return self._sample_resident(score_fn, noise, steps, corrections, tau, device, show_progressbar, seed, proc_x0)
 
+    def sample_ensemble(self, score_fn, noise, steps: int = 64, corrections: int = 0, tau: float = 1.0, proc_x0=None,
+                        device=None, show_progressbar=True, seeds: Optional[Sequence[int]] = None):
+        """M members sampled together: noise [M, L, C, H, W] -> [M, L, C, H, W], every member conditioned on the score
+        function's one `condition_on` (the reference's ensemble: the same observation, different noise).  The members
+        share one device-resident state, so each UNet launch holds windows of several members.
+
+        Member m is bit-identical to `sample(score_fn, noise[m], ..., seed=seeds[m])`, whatever `max_windows` is.
+        `seeds`: M corrector seeds; by default M draws from the global generator in member order, as M sequential
+        `sample` calls would make.  `proc_x0` is called once per member on its [L, C, H, W] x0; `trace_at` traces are
+        [M, L, C, H, W].  Closed-form guidance only (exact_grad=False), not with time sharding, and not with
+        `rng = "reference"` corrections."""
+        if not isinstance(score_fn, AbstractScoreFunction):
+            raise TypeError("SDAPipeline.sample_ensemble drives this package's score functions "
+                            f"(Default/BatchedScoreFunction); got {type(score_fn).__name__}")
+        if noise.dim() != 5:
+            raise ValueError(f"sample_ensemble: noise must be [M, L, C, H, W], got shape {tuple(noise.shape)}")
+        M = int(noise.shape[0])
+        if M < 1:
+            raise ValueError("sample_ensemble: noise holds no member (M = 0)")
+        if seeds is not None:
+            seeds = [int(v) for v in seeds]
+            if len(seeds) != M:
+                raise ValueError(f"sample_ensemble: {len(seeds)} seeds for {M} members (one per member)")
+        if corrections > 0 and self.rng == "reference":
+            raise NotImplementedError("sample_ensemble: rng='reference' with corrections draws z on the host from the "
+                                      "global CPU generator, member after member; drawing it for all members step by "
+                                      "step cannot reproduce that stream, so it is refused (use rng='device' or sample)")
+        return self._sample_resident(score_fn, noise, steps, corrections, tau, device, show_progressbar, seeds, proc_x0,
+                                     members=M)
+
+    def _draw_seed(self, corrections: int) -> int:
+        """The corrector seed of a run without one: one draw from the global generator when the corrector draws its
+        noise on chip, else 0.  rng == "reference" replays the reference's draws (z.normal_() only,
+        src/thor/pipelines.py:82): nothing else may touch the global CPU generator, or the stream is shifted by one draw."""
+        if corrections > 0 and self.rng != "reference":
+            return int(torch.empty((), dtype=torch.int64).random_().item())
+        return 0
+
     def _sample_resident(self, sf: AbstractScoreFunction, noise: Tensor, steps: int, corrections: int, tau: float,
-                         device, show_progressbar: bool, seed: Optional[int], proc_x0=None) -> Optional[Tensor]:
+                         device, show_progressbar: bool, seed, proc_x0=None, members: int = 0) -> Optional[Tensor]:
+        """The sampler on the resident state: one trajectory (`seed` an int or None), or an ensemble of `members`
+        (`seed` a list of M ints or None)."""
         if device is not None and torch.device(device).type == "cuda":
             sf.device = torch.device(device)
-        rt = sf.runtime(noise)
+        rt = sf.runtime(noise, members=members)
         group = sf.shard[2] if sf.shard else None
         rt.reset_finite_check()
         rt.load(noise)
         time_steps = torch.linspace(1, 0, steps + 1).to(dtype=torch.float32)
         dt = 1 / steps
         z_dev = None
-        if seed is None:
-            # rng == "reference" replays the reference's draws (z.normal_() only, src/thor/pipelines.py:82): nothing else
-            # may touch the global CPU generator, or the stream is shifted by one draw
-            device_rng = corrections > 0 and self.rng != "reference"
-            seed = int(torch.empty((), dtype=torch.int64).random_().item()) if device_rng else 0
-            if sf.shard and device_rng:
+        if members:
+            if seed is None:  # one draw per member, in member order: what M sequential sample() calls draw
+                seed = [self._draw_seed(corrections) for _ in range(members)]
+            seed = rt.member_seeds(seed)
+        elif seed is None:
+            seed = self._draw_seed(corrections)
+            if sf.shard and corrections > 0 and self.rng != "reference":
                 # the on-chip Philox stream is keyed by (seed, step, GLOBAL pixel): every rank must use rank 0's draw,
                 # otherwise the result would depend on the sharding
                 s_t = torch.tensor([seed], dtype=torch.int64, device=rt.device)
@@ -143,7 +184,7 @@ class SDAPipeline:
                 tr = rt.owned(rt.x)
                 if sf.shard:
                     tr = all_gather_frames(tr, rt.plan, group)
-                self.traces[istep + 1] = tr.cpu()
+                self.traces[istep + 1] = tr.reshape(noise.shape).cpu() if members else tr.cpu()
         rt.check_finite()
         out = rt.owned(rt.x)
         if sf.shard:

@@ -249,7 +249,7 @@ COMBINED_STRIP_PIX = 16384  # C2W_COMBINED_STRIP_PIX
 
 
 def point_plan(op: PointObservation, y, L: int, C: int, H: int, W: int, frame_lo: int, frame_hi: int, strip: int,
-               max_strip_pix: int = POINT_STRIP_PIX, std=None) -> dict:
+               max_strip_pix: int = POINT_STRIP_PIX, std=None, members: int = 0) -> dict:
     """The device form of a point observation for the owned global frames [frame_lo, frame_hi) (c2w_point_obs).
 
     Observations of one (frame, pixel) merge into one entry: per variable ysum = sum(mask * y), wsum = sum(mask), summed
@@ -262,7 +262,10 @@ def point_plan(op: PointObservation, y, L: int, C: int, H: int, W: int, frame_lo
     variable) with the same fp32 std^2 merge: a pixel's distinct std^2 become a run of consecutive entries, entry j of
     the run holding the j-th smallest std^2 of every variable (wsum = ysum = 0, std2 = 1 in the slots of a variable
     with fewer).  An observation with std^2 = inf contributes exactly zero and is left out, as if masked.  The plan then
-    also holds std2 [n_entries, C] fp32."""
+    also holds std2 [n_entries, C] fp32.
+
+    `members` = M > 0: the plan of an ensemble of M trajectories stored member-major, all conditioned on y — one
+    member's plan with frame_slot repeated M times, so that every member's frames point at the same entries."""
     y = torch.as_tensor(y)
     op.check_observation(y)
     op.check_geometry(L, C, H, W)
@@ -297,8 +300,8 @@ def point_plan(op: PointObservation, y, L: int, C: int, H: int, W: int, frame_lo
     cell = frame_slot[fr].astype(np.int64) * n_strips + (px // W) // strip  # non-decreasing: the keys are sorted
     counts = np.bincount(cell, minlength=obs_frames.size * n_strips)
     strip_off = np.concatenate([[0], np.cumsum(counts)]).astype(np.int32)
-    out = dict(frame_slot=frame_slot, strip_off=strip_off, pix=px.astype(np.int32), ysum=ysum.astype(np.float32),
-               wsum=wsum.astype(np.float32), n_slots=int(obs_frames.size), strip_rows=int(strip), n_strips=n_strips,
+    out = dict(frame_slot=np.tile(frame_slot, members) if members else frame_slot, strip_off=strip_off,
+               pix=px.astype(np.int32), ysum=ysum.astype(np.float32), wsum=wsum.astype(np.float32), n_slots=int(obs_frames.size), strip_rows=int(strip), n_strips=n_strips,
                frames=[int(frame_lo + f) for f in obs_frames])
     if std is not None:
         out["std2"] = std2
@@ -466,20 +469,29 @@ def observed_windows(win_lo: int, win_hi: int, n_win_global: int, L: int, k: int
 
 
 class _Runtime:
-    """Device-resident state of one trajectory (or of this rank's time shard of it)."""
+    """Device-resident state of one trajectory (or of this rank's time shard of it), or of an ensemble of `members`
+    trajectories of L frames stored member-major in one state [members * L, H, W, C] (members = 0: one trajectory).
+    An ensemble's plan is that of one member; every kernel call covers all members at once (the *_members entry
+    points), and every member is conditioned on the same observation."""
 
     def __init__(self, sf: "AbstractScoreFunction", L: int, C: int, H: int, W: int, device: torch.device,
-                 plan: ShardPlan, max_windows: int, exact: bool = False):
+                 plan: ShardPlan, max_windows: int, exact: bool = False, members: int = 0):
         if not 1 <= C <= 8:
             raise NotImplementedError(f"1 to 8 variables per frame (c2w_b200.h: C2W_MAX_VARS); got C={C}")
         self.sf, self.L, self.C, self.H, self.W, self.device, self.plan = sf, L, C, H, W, device, plan
+        self.members = int(members)
         self.lib = _lib.load()
         k = sf.markov_order
         self.exact = bool(exact)  # exact_grad=True: guidance through the UNet VJP (src/thor/score.py:28-33,51-52)
         self.cond = None
         self.points = None        # PointObservation: this rank's device plan (c2w_point_obs), see set_condition
         self._engine_args = (C, 2 * k + 1, H, W, device)
-        self._engine_windows = min(max_windows, plan.win_hi - plan.win_lo)
+        self._engine_windows = min(max_windows, self.n_windows)
+        # an ensemble's convs are planned as a member's own run plans them (its window count per launch): tile width,
+        # CTA pair and main loop, and with them the order of the fp32 sums, match that run's, so each member is computed
+        # bit for bit as alone
+        self._tile_windows = min(sf.max_windows or sf._default_windows(plan.n_win_global), plan.n_win_global) \
+            if self.members else 0
         self._engine = None
         self._engine_vjp = None   # exact_grad: the stashing engine for the windows that need a backward pass
         self._engine_epoch = None
@@ -487,13 +499,13 @@ class _Runtime:
         self._rest = None         # exact_grad: the other local windows (int32 device list)
         self.refresh_engine()
         f32 = dict(dtype=torch.float32, device=device)
-        self.x = torch.zeros(plan.n_local, H, W, C, **f32)
+        self.x = torch.zeros(self.n_frames, H, W, C, **f32)
         self.eps = torch.zeros_like(self.x)
         self.eps_g: Optional[Tensor] = None
         self.vjp = torch.zeros_like(self.x) if self.exact else None   # J_eps^T g, accumulated per score evaluation
         self.cot = torch.zeros_like(self.x) if self.exact else None   # g = A^T((y - A x0)/var)
         self.nan_flag = torch.zeros(1, dtype=torch.int32, device=device)
-        self.sumsq = torch.zeros(1, dtype=torch.float64, device=device)
+        self.sumsq = torch.zeros(max(1, self.members), dtype=torch.float64, device=device)  # one per member
         self.partials: Optional[Tensor] = None
         self.cond = None
         self.s_tile = next(s for s in (16, 8, 32, 4, 64, 2, 128, 1) if H % s == 0 and W % s == 0 and W // s <= 32)
@@ -501,11 +513,29 @@ class _Runtime:
         self._peer_halo_ok = True
         self._halo_pushed = False  # the last update kernel already stored the boundary frames into the neighbours' mailboxes
 
+    @property
+    def n_frames(self) -> int:
+        """Frames of the resident state: this rank's (with halos), or every member's."""
+        return self.members * self.L if self.members else self.plan.n_local
+
+    @property
+    def n_windows(self) -> int:
+        """Windows one score evaluation runs: this rank's, or every member's (members x (L - 2k))."""
+        p = self.plan
+        return self.members * p.n_win_global if self.members else p.win_hi - p.win_lo
+
+    @property
+    def own(self) -> tuple:
+        """(first local frame, frames) this runtime updates: this rank's owned frames, or every member's."""
+        p = self.plan
+        return (0, self.n_frames) if self.members else (p.own_lo - p.frame_lo, p.own_n)
+
     # ------------------------------------------------------------------------------------------------ engine
     def refresh_engine(self) -> None:
         """(Re)binds the packed-weight engine; `ScoreUNet.engine` re-packs if the parameters changed since (full
         fingerprint: data pointers, autograd versions, and the explicit epoch raw-pointer optimisers bump)."""
-        self._engine = self.sf.unet.engine(*self._engine_args, max_windows=self._engine_windows, vjp=False)
+        self._engine = self.sf.unet.engine(*self._engine_args, max_windows=self._engine_windows, vjp=False,
+                                           tile_windows=self._tile_windows)
         if self.exact and self.cond is not None:  # sized by the selection, so only once the operator is known
             nsel = max(1, len(self._selected_list()))
             self._engine_vjp = self.sf.unet.engine(*self._engine_args, max_windows=min(nsel, self._engine_windows), vjp=True)
@@ -572,11 +602,13 @@ class _Runtime:
         return torch.cuda.current_stream(self.device).cuda_stream
 
     def load(self, x_nchw: Tensor) -> None:
-        """x_nchw: the FULL trajectory [L, C, H, W] (any device); keeps this rank's frames (with halos)."""
+        """x_nchw: the FULL trajectory [L, C, H, W] (any device); keeps this rank's frames (with halos).  An ensemble:
+        every member, [members, L, C, H, W]."""
         p = self.plan
-        src = x_nchw[p.frame_lo:p.frame_hi].to(device=self.device, dtype=torch.float32, non_blocking=True).contiguous()
+        src = x_nchw.reshape(self.n_frames, self.C, self.H, self.W) if self.members else x_nchw[p.frame_lo:p.frame_hi]
+        src = src.to(device=self.device, dtype=torch.float32, non_blocking=True).contiguous()
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.c2w_traj_pack(src.data_ptr(), self.x.data_ptr(), p.n_local, self.C, self.H * self.W,
+            _lib.check(self.lib.c2w_traj_pack(src.data_ptr(), self.x.data_ptr(), self.n_frames, self.C, self.H * self.W,
                                               self.stream), "c2w_traj_pack")
 
     def unpack(self, buf: Tensor, lo: int, n: int) -> Tensor:
@@ -587,15 +619,17 @@ class _Runtime:
         return out
 
     def owned(self, buf: Tensor) -> Tensor:
-        """NCHW copy of this rank's owned frames of `buf`."""
-        p = self.plan
-        return self.unpack(buf, p.own_lo - p.frame_lo, p.own_n)
+        """NCHW copy of this rank's owned frames of `buf` (an ensemble: every member's, [members * L, C, H, W])."""
+        return self.unpack(buf, *self.own)
 
     # ------------------------------------------------------------------------------------------------ kernels
     def score(self, t: float, group=None) -> None:
         """eps <- composed window score of x at time t (src/thor/score.py:90-93 / :156-185).  With exact_grad the
         likelihood cotangent is pushed back through the same windows chunk by chunk: vjp <- J_eps^T g."""
         p = self.plan
+        if self.members:  # every member's windows, chunked by the workspace: a launch may hold several members'
+            self.engine.window_score_members(self.x, self.members, self.L, 0, self.n_windows, t, self.eps)
+            return
         if not (self.exact and self.cond is not None):
             self.engine.window_score(self.x, p.frame_lo, p.win_lo, p.win_hi - p.win_lo, p.n_win_global, t, self.eps)
             return
@@ -640,7 +674,8 @@ class _Runtime:
                 op, y, max_pix = op.points, cond["point_y"], COMBINED_STRIP_PIX
                 strip = combined_strip_rows(self.H, self.W, cond["op"].coarse.s_step)
             std = obs_std["point_std"] if obs_std is not None else None
-            pl = point_plan(op, y, self.L, self.C, self.H, self.W, p.own_lo, p.own_lo + p.own_n, strip, max_pix, std)
+            pl = point_plan(op, y, self.L, self.C, self.H, self.W, p.own_lo, p.own_lo + p.own_n, strip, max_pix, std,
+                            members=cond.get("members", 0))
             names = ("frame_slot", "strip_off", "pix", "ysum", "wsum") + (("std2",) if std is not None else ())
             dev = {n: torch.as_tensor(pl[n]).to(self.device) for n in names}
             for n in names[2:]:  # no entries on this rank: still a valid pointer
@@ -685,7 +720,7 @@ class _Runtime:
             g.t_step = 1
         g.s_step, g.H, g.W = s, self.H, self.W
         g.mu, g.sigma, g.mu_next, g.sigma_next = mu, sigma, mu_next, sigma_next
-        g.frame_global0, g.own_lo, g.own_n = p.frame_lo, p.own_lo - p.frame_lo, p.own_n
+        g.frame_global0, (g.own_lo, g.own_n) = p.frame_lo, self.own
         if frames is not None:
             g.own_lo, g.own_n = frames
         g.mode = mode
@@ -700,7 +735,7 @@ class _Runtime:
                 g.halo = ph.handle
                 self._halo_pushed = True
         if mode == 1:
-            n_part = p.own_n * (pts["n_strips"] if pts is not None else self.H // s)
+            n_part = g.own_n * (pts["n_strips"] if pts is not None else self.H // s)
             if self.partials is None or self.partials.numel() < n_part:
                 self.partials = torch.zeros(n_part, dtype=torch.float32, device=self.device)
             if self.eps_g is None:
@@ -708,7 +743,15 @@ class _Runtime:
             g.eps_out, g.partials = self.eps_g.data_ptr(), self.partials.data_ptr()
             self._n_part = n_part
         with torch.cuda.device(self.device):
-            if per_obs:
+            if self.members:  # the same operands; the entry point observes every member's frames as one member's
+                obs = ctypes.byref(pts["obs"]) if pts is not None else None
+                pstd2 = (ctypes.c_float * self.C)(*(v ** 2 for v in self.cond["point_std"])) \
+                    if (combined and not per_obs) else None
+                entry = pts["tensors"]["std2"].data_ptr() if (per_obs and pts is not None) else None
+                coarse = self.coarse_std2_dev.data_ptr() if (per_obs and self.coarse_std2_dev is not None) else None
+                _lib.check(self.lib.c2w_guided_step_members(ctypes.byref(g), self.L, obs, pstd2, coarse, entry,
+                                                            self.stream), "c2w_guided_step_members")
+            elif per_obs:
                 obs = ctypes.byref(pts["obs"]) if pts is not None else None
                 entry = pts["tensors"]["std2"].data_ptr() if pts is not None else None
                 coarse = self.coarse_std2_dev.data_ptr() if self.coarse_std2_dev is not None else None
@@ -732,32 +775,45 @@ class _Runtime:
         """The predictor with a user `proc_x0` callable (src/thor/pipelines.py:43-45).  The fused update is split around
         the hook: the guided score comes from the kernel (mode 1); x0 = (x - sigma eps)/mu is handed to the callable as
         an NCHW device tensor and `mu' proc(x0) + sigma' eps` written back — elementwise torch ops on the resident
-        tensors, because the hook itself is an arbitrary torch callable (no shipped config passes one)."""
-        p = self.plan
+        tensors, because the hook itself is an arbitrary torch callable (no shipped config passes one).  An ensemble
+        calls the hook once per member, on that member's [L, C, H, W], as a run of that member alone would."""
         self._guide(1, mu, sigma, 0.0, 0.0)
-        lo = p.own_lo - p.frame_lo
-        x_own, e_own = self.x[lo:lo + p.own_n], self.eps_g[lo:lo + p.own_n]
-        x0 = proc_x0(((x_own - sigma * e_own) / mu).permute(0, 3, 1, 2))
-        if tuple(x0.shape) != (p.own_n, self.C, self.H, self.W):
-            raise ValueError(f"proc_x0 returned shape {tuple(x0.shape)}")
-        x_own.copy_(mu_next * x0.permute(0, 2, 3, 1) + sigma_next * e_own)
-        self.nan_flag |= (~torch.isfinite(x_own)).any().to(torch.int32)
+        lo, n = self.own
+        parts = [(m * self.L, self.L) for m in range(self.members)] if self.members else [(lo, n)]
+        for lo, n in parts:  # (first frame, frames) of each member, or of this rank's owned frames
+            x_own, e_own = self.x[lo:lo + n], self.eps_g[lo:lo + n]
+            x0 = proc_x0(((x_own - sigma * e_own) / mu).permute(0, 3, 1, 2))
+            if tuple(x0.shape) != (n, self.C, self.H, self.W):
+                raise ValueError(f"proc_x0 returned shape {tuple(x0.shape)}")
+            x_own.copy_(mu_next * x0.permute(0, 2, 3, 1) + sigma_next * e_own)
+            self.nan_flag |= (~torch.isfinite(x_own)).any().to(torch.int32)
 
     def guided_eps(self, mu: float, sigma: float) -> None:
         """eps_g <- eps - sigma * grad_x log p(y | x) (src/thor/score.py:24-35) and the partial sums of eps_g^2."""
         self._guide(1, mu, sigma, 0.0, 0.0)
 
-    def corrector(self, tau: float, sigma_next: float, z: Optional[Tensor], seed: int, step_id: int,
+    def corrector(self, tau: float, sigma_next: float, z: Optional[Tensor], seed, step_id: int,
                   group=None) -> None:
-        """One Langevin correction with eps_g already computed (src/thor/pipelines.py:81-88)."""
+        """One Langevin correction with eps_g already computed (src/thor/pipelines.py:81-88).  An ensemble: `seed` is
+        the members' seeds (int64 device tensor, `member_seeds`), each member has its own mean(eps^2) and noise."""
         p = self.plan
+        hw = self.H * self.W
+        if self.members:
+            with torch.cuda.device(self.device):
+                _lib.check(self.lib.c2w_reduce_partials_members(self.partials.data_ptr(), self.members,
+                                                                self._n_part // self.members, self.sumsq.data_ptr(),
+                                                                self.stream), "c2w_reduce_partials_members")
+                _lib.check(self.lib.c2w_corrector_update_members(
+                    self.x.data_ptr(), self.eps_g.data_ptr(), self.sumsq.data_ptr(), float(self.L * self.C * hw),
+                    float(tau), float(sigma_next), self.members, self.L * hw, self.C, seed.data_ptr(), int(step_id),
+                    self.nan_flag.data_ptr(), self.stream), "c2w_corrector_update_members")
+            return
         with torch.cuda.device(self.device):
             _lib.check(self.lib.c2w_reduce_partials(self.partials.data_ptr(), self._n_part, self.sumsq.data_ptr(),
                                                     self.stream), "c2w_reduce_partials")
             if p.world > 1:
                 dist.all_reduce(self.sumsq, group=group)  # trajectory-global mean(eps^2): one scalar per correction
             lo = p.own_lo - p.frame_lo
-            hw = self.H * self.W
             zp = None
             if z is not None:
                 zl = z[lo:lo + p.own_n]
@@ -767,6 +823,12 @@ class _Runtime:
                 self.x[lo:].data_ptr(), self.eps_g[lo:].data_ptr(), zp, self.sumsq.data_ptr(),
                 float(self.L * self.C * hw), float(tau), float(sigma_next), p.own_lo * hw, p.own_n * hw, self.C, int(seed),
                 int(step_id), self.nan_flag.data_ptr(), self.stream), "c2w_corrector_update_c")
+
+    def member_seeds(self, seeds: Sequence[int]) -> Tensor:
+        """The members' corrector seeds as the device array c2w_corrector_update_members reads: each taken modulo 2^64,
+        as the single-trajectory call takes its uint64 seed."""
+        u = np.array([int(s) & 0xFFFF_FFFF_FFFF_FFFF for s in seeds], dtype=np.uint64).view(np.int64)
+        return torch.from_numpy(u).to(self.device)
 
     def _ensure_peer_halo(self) -> Optional[PeerHalo]:
         """The peer-memory mailboxes (set up collectively on first use by every rank at the same point)."""
@@ -928,19 +990,31 @@ class AbstractScoreFunction:
     def _default_windows(self, n_win: int) -> int:
         return min(n_win, self.DEFAULT_WINDOWS)
 
-    def runtime(self, x: Tensor) -> _Runtime:
-        L, C, H, W = x.shape
+    def runtime(self, x: Tensor, members: int = 0) -> _Runtime:
+        """The device state for a trajectory x [L, C, H, W], or with members = M an ensemble x [M, L, C, H, W] (closed-
+        form guidance only, not time-sharded; one plan over M L frames and M (L - 2k) windows)."""
+        shape = tuple(x.shape[1:]) if members else tuple(x.shape)
+        L, C, H, W = shape
+        exact = bool(self.likelihood is not None and self.likelihood.get("exact"))
+        if members and exact:
+            raise NotImplementedError("ensemble sampling runs closed-form guidance only: condition_on(..., "
+                                      "exact_grad=False); exact_grad=True needs member-aware window selection and "
+                                      "adjoints, which are not implemented")
+        if members and self.shard:
+            raise NotImplementedError("ensemble sampling does not run on a time-sharded score function "
+                                      "(enable_time_sharding); run one ensemble per rank instead")
         dev = self._compute_device(x)
         rank, world = (self.shard[0], self.shard[1]) if self.shard else (0, 1)
-        exact = bool(self.likelihood is not None and self.likelihood.get("exact"))
-        key = (L, C, H, W, str(dev), rank, world, exact)
+        key = (L, C, H, W, str(dev), rank, world, exact, members)
         rt = self._runtimes.get(key)
         if rt is None:
             plan = make_plan(L, self.markov_order, rank, world)
-            mw = self.max_windows or self._default_windows(plan.win_hi - plan.win_lo)
+            n_win = members * plan.n_win_global if members else plan.win_hi - plan.win_lo
+            mw = self.max_windows or self._default_windows(n_win)
             if exact:
                 mw = min(mw, self.VJP_WINDOWS)  # the stash costs ~110 MiB per window at the reference shapes
-            rt = _Runtime(self, L, C, H, W, dev, plan, mw, exact=exact)
+            args = (self, L, C, H, W, dev, plan, mw)
+            rt = _Runtime(*args, exact=exact, members=members) if members else _Runtime(*args, exact=exact)
             if self.likelihood is not None:
                 lk = self.likelihood
                 if lk["op"] is None:
@@ -952,13 +1026,15 @@ class AbstractScoreFunction:
                     lk["gamma_c"] = _per_channel(lk["gamma"], C, "gamma")
                 op, y = lk["op"], lk["y"]
                 cond = dict(op=op, gamma=lk["gamma_c"])
+                if members:  # the point plan repeats its frame slots per member
+                    cond["members"] = members
                 if isinstance(op, CombinedObservation):  # split and checked against this trajectory's geometry
-                    _check_observation_shape(op.coarse, op.term_shapes(x.shape)[0], L, C, H, W)
-                    y, cond["point_y"] = op.split(y, x.shape)
+                    _check_observation_shape(op.coarse, op.term_shapes(shape)[0], L, C, H, W)
+                    y, cond["point_y"] = op.split(y, shape)
                     if torch.as_tensor(lk["std"]).numel() in (1, C):
-                        cond["std"], cond["point_std"] = op.std_per_term(lk["std"], x.shape)
+                        cond["std"], cond["point_std"] = op.std_per_term(lk["std"], shape)
                     else:
-                        cond.update(_combined_std(op, lk["std"], x.shape))
+                        cond.update(_combined_std(op, lk["std"], shape))
                 else:
                     if isinstance(op, CoarseGrain):  # checked against this trajectory's geometry, every time
                         y = coarse_grain_observation(op, y, L, C, H, W)

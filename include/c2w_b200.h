@@ -149,6 +149,22 @@ int c2w_window_score_backward_sel(c2w_handle* h, const float* cot, int32_t n_fra
                                   const int32_t* win_list_dev, const int32_t* pos_dev, int32_t n_sel, int32_t n_win_global,
                                   float* vjp, void* stream);
 
+/* An ensemble of n_members trajectories of member_frames frames each, stored member-major in one resident state
+ * traj / eps: [n_members * member_frames, H, W, C] (the reference's ensemble: one score function, one sample() per
+ * member).  Nw = member_frames - 2k windows per member; ensemble window G in [0, n_members * Nw) is window G mod Nw of
+ * member m = G div Nw and reads frames m * member_frames + (G mod Nw) + [0, 2k].  Computes windows
+ * [win_first, win_first + n_win), chunked by the bound workspace so that one launch may hold windows of several
+ * members; each window folds its centre slot, and its member's head / tail slots when it is its member's first / last
+ * window, so member m's part of eps equals c2w_window_score over that member alone. */
+int c2w_window_score_members(c2w_handle* h, const float* traj, int32_t n_members, int32_t member_frames,
+                             int32_t win_first, int32_t n_win, float t, float* eps, void* stream);
+/* A plain workspace of max_windows windows (c2w_workspace_bytes(max_windows) bytes) whose convs are planned as for a
+ * workspace of tile_windows windows: the same N-tile width, CTA pair and main loop (streamed, activation reuse or its
+ * two-image form, which also decides whether the LayerNorm is fused).  These choices fix the order of the fp32 sums,
+ * so an ensemble bound with tile_windows = the window count of one member's own workspace computes every member
+ * bit for bit as c2w_window_score does on that member alone, however its launches mix members. */
+int c2w_bind_workspace_members(c2w_handle* h, int32_t max_windows, int32_t tile_windows, void* dev_ptr, int64_t bytes);
+
 /* ---- layout: reference NCHW fp32 [frames, C, H, W] <-> device [frames, H, W, C] --------------------------- */
 int c2w_traj_pack(const float* nchw, float* fhwc, int64_t frames, int32_t C, int32_t hw, void* stream);
 int c2w_traj_unpack(const float* fhwc, float* nchw, int64_t frames, int32_t C, int32_t hw, void* stream);
@@ -215,6 +231,20 @@ int c2w_guided_step_combined(const c2w_guide* g, const c2w_point_obs* obs, const
 int c2w_guided_step_obs_std(const c2w_guide* g, const c2w_point_obs* obs, const float* coarse_std2,
                             const float* entry_std2, void* stream);
 int c2w_reduce_partials(const float* partials, int32_t n, double* sumsq, void* stream);
+/* The guidance step of an ensemble stored member-major (see c2w_window_score_members): g covers all members' frames
+ * (own_n a multiple of member_frames, frame_global0 + own_lo the first frame of a member, halo NULL) and every member
+ * is conditioned on the same observation.  Frame f is observed as member frame f mod member_frames: the coarse term's
+ * frame test and y's offset use it; a point term's obs->frame_slot lists the slots of every member's frames (the slot
+ * array of one member, repeated).  The terms as in c2w_guided_step (g->y), c2w_guided_step_points (obs) and
+ * c2w_guided_step_combined (g->y, obs, point_std2), or, with coarse_std2 / entry_std2, c2w_guided_step_obs_std; neither
+ * term: unconditioned.  Same checks as those entries.  Mode 1 writes the partials in (frame, strip) order, so member
+ * m's are the m-th of n_members equal segments. */
+int c2w_guided_step_members(const c2w_guide* g, int32_t member_frames, const c2w_point_obs* obs, const float* point_std2,
+                            const float* coarse_std2, const float* entry_std2, void* stream);
+/* sumsq[m] = the sum of partials [m * member_partials, (m + 1) * member_partials), m < n_members, each summed exactly as
+ * c2w_reduce_partials sums that segment alone. */
+int c2w_reduce_partials_members(const float* partials, int32_t n_members, int32_t member_partials, double* sumsq,
+                                void* stream);
 /* x <- x - (delta eps + sqrt(2 delta) z) sigma_next, delta = tau / (sumsq / count)  (src/thor/pipelines.py:84-87).
  * z == NULL: on-chip Philox4x32-10 keyed by (seed, step_id, global pixel index). */
 int c2w_corrector_update(float* x, const float* eps, const float* z, const double* sumsq, double count, float tau,
@@ -224,6 +254,13 @@ int c2w_corrector_update(float* x, const float* eps, const float* z, const doubl
 int c2w_corrector_update_c(float* x, const float* eps, const float* z, const double* sumsq, double count, float tau,
                            float sigma_next, int64_t pix0_global, int64_t npix, int32_t channels, uint64_t seed,
                            uint32_t step_id, int32_t* nan_flag, void* stream);
+/* The corrector of an ensemble stored member-major, member_pix = member_frames * H * W pixels per member: pixel i of
+ * member m is updated with delta_m = tau / (sumsq[m] / count) and on-chip Philox z keyed by (seeds[m], step_id, i),
+ * i.e. bit for bit what c2w_corrector_update_c(pix0_global = 0, seed = seeds[m]) does to member m alone.  seeds:
+ * DEVICE array of n_members. */
+int c2w_corrector_update_members(float* x, const float* eps, const double* sumsq, double count, float tau,
+                                 float sigma_next, int32_t n_members, int64_t member_pix, int32_t channels,
+                                 const uint64_t* seeds, uint32_t step_id, int32_t* nan_flag, void* stream);
 
 /* ---- op-level hooks (parity tests of single kernels; same kernels the calls above launch) ----------------- */
 /* One launch of K1 (Conv2d 3x3 pad 1, stride 1 or 2 — model/nn.py:155,157,169,185,193,194 — or a plain GEMM for the
