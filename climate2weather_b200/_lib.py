@@ -144,6 +144,8 @@ SIGNATURES = {
     "c2w_corrector_update_c": (_i, [_vp, _vp, _vp, _vp, _d, _f, _f, _i64, _i64, C.c_int32, C.c_uint64, C.c_uint32, _vp,
                                     _vp]),
     "c2w_op_conv_ex": (_i, [C.POINTER(ConvDesc), _vp]),
+    "c2w_op_conv_phase": (_i, [C.POINTER(ConvDesc), _vp]),
+    "c2w_pack_phase_weights": (_i, [_vp, _i, _i, _i, _i, _vp]),
     "c2w_conv_tile_width": (_i, [_i, _i, _i, _i, _i, _i, _i]),
     "c2w_op_wgrad": (_i, [_vp, _vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _vp, _i64,
                           _vp, _vp, C.c_int32, C.c_int32, C.c_int32, _vp]),

@@ -131,6 +131,13 @@ __device__ __forceinline__ void tma_store_4d(const CUtensorMap* m, const void* s
                "r"(smem_u32(src)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
                : "memory");
 }
+__device__ __forceinline__ void tma_store_5d(const CUtensorMap* m, const void* src, int c0, int c1, int c2, int c3,
+                                             int c4) {
+  asm volatile("cp.async.bulk.tensor.5d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5, %6}], [%1];" ::"l"(
+                   reinterpret_cast<uint64_t>(m)),
+               "r"(smem_u32(src)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4)
+               : "memory");
+}
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 // all bulk groups of this thread have finished READING their shared-memory source
 __device__ __forceinline__ void bulk_wait_read_all() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }

@@ -335,12 +335,28 @@ __device__ __forceinline__ void epilogue_chunk_staged(const ConvParams& p, const
   }
 }
 
-template <int BN, int CG, bool LN, bool AR>
+// Phase form (PH) of the activation-reuse kernels: the conv3x3 of a nearest x2 upsampled input (the ascent tails,
+// model/nn.py:184-185) computed at the LOW resolution.  Output pixel (2i + a, 2j + b) reads upsampled rows 2i + a - 1
+// .. 2i + a + 1, i.e. low-res rows {i - 1, i} (a = 0) or {i, i + 1} (a = 1), and the same for columns: so each output
+// phase (a, b) is an exact 2x2 conv of the low-res input with merged weights (conv_pack_phase_weights), 16 instead of
+// 36 tap-MACs per low-res pixel, and the upsampled input is never written.  The M tile is a 16 x 8 block of low-res
+// pixels and one phase; its taps (tr, ts) are the sub-views a + tr rows and b + ts pixels into the same halo'd unit.
+// The two CTAs of a pair share the weights, hence the phase: M tile mt -> pair g = mt / 2, phase g % 4, low-res tile
+// 2 (g / 4) + mt % 2 (the four phases of a low-res pair run back to back and find its input in L2).
+__device__ __forceinline__ int ph_split(int mt, int& phase) {
+  const int g = mt >> 1;
+  phase = g & 3;
+  return ((g >> 2) << 1) | (mt & 1);
+}
+
+template <int BN, int CG, bool LN, bool AR, bool PH = false>
 __global__ void __launch_bounds__(kConvThreads + (LN ? kLnThreads : 0), 1)
 conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                          const __grid_constant__ CUtensorMap tmOut, const __grid_constant__ CUtensorMap tmOut2,
                          const ConvParams p) {
   using Cfg = ConvCfg<BN, CG>;
+  static_assert(!PH || (AR && CG == 2), "the phase form is an activation-reuse main loop of a CTA pair");
+  constexpr int kCols = PH ? 2 : 3;  // filter columns (= rows) of the main loop: 2x2 phase taps or 3x3
   extern __shared__ uint8_t smem_raw[];
   // 1024 B alignment by POINTER arithmetic (an integer round trip hides the address space from the compiler and
   // every staging-tile access becomes a generic LD/ST with 64-bit address math instead of LDS/STS)
@@ -454,7 +470,9 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
       [[maybe_unused]] const long long t_begin = C2W_DIAG_CLOCK();
       for (int tile = group_id; AR && tile < num_tiles; tile += num_groups) {
         const int nt = tile % p.num_n_tiles;
-        const int mt = (tile / p.num_n_tiles) * CG + rank;
+        int mt = (tile / p.num_n_tiles) * CG + rank;
+        int ph = 0;
+        if (PH) mt = ph_split(mt, ph);
         const int img = mt / p.tiles_per_img, tt = mt % p.tiles_per_img;
         const int h0 = (tt / p.tiles_w) * Cfg::kARTileH, w0 = (tt % p.tiles_w) * Cfg::kARTileW;
         const int a2 = p.ar2 ? 2 * img : h0 - 1, a3 = p.ar2 ? -1 : img;
@@ -484,8 +502,8 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
             unit = 0;
             a_phase ^= 1;
           }
-          // ---- the weights of filter columns s = 0..2, one stage each
-          for (int s3 = 0; s3 < 3; ++s3) {
+          // ---- the weights of filter columns s = 0..2 (PH: 0..1), one stage each
+          for (int s3 = 0; s3 < kCols; ++s3) {
             C2W_TIMED_WAIT(w_empty, &empty[stage], phase ^ 1);
             if (elect_one()) {
 #ifdef C2W_DIAG
@@ -499,12 +517,13 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
 #endif
               if (rank == 0) mbar_arrive_expect_tx(&full[stage], skip_b ? 0 : CG * p.ar_tx_b);
               // one box {64 ch, B rows, r = 0..2} at channel s * Cin + cb * 64 of the [Cout][r][s * Cin] weight view
+              // (PH: {64 ch, B rows, r = 0..1, 1} of the [phase][Cout][r][s * Cin] view)
               uint8_t* bdst = smB + stage * Cfg::kARBStageBytes;
               const int kc = (s3 * p.cin_blocks + cb) * kBlockK;
               if (skip_b) {
               } else if (CG == 2) {
                 tma_load_4d_pair(&tmB, mapa_shared(smem_u32(&full[stage]), 0), bdst, kc, nt * BN + rank * Cfg::kBRows,
-                                 0, 0);
+                                 0, ph);
               } else {
                 tma_load_4d(&tmB, &full[stage], bdst, kc, nt * BN, 0, 0);
               }
@@ -594,17 +613,24 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
         tc_fence_after();
         const uint32_t tmem_d = tmem_base + acc * BN;
         const uint32_t ar_row_step = static_cast<uint32_t>(p.ar_row_step16);
+        // PH: output phase (a, b) = the unit from its a-th row and b-th pixel on (leader: rank 0 = even M tile)
+        uint32_t ph_off = 0;
+        if (PH) {
+          int ph;
+          ph_split((tile / p.num_n_tiles) * CG, ph);
+          ph_off = (ph >> 1) * ar_row_step + (ph & 1) * 8;
+        }
         // K order cb -> s -> r -> k: each filter column's weight stage is released as soon as its nine MMAs are issued
         for (int cb = 0; AR && cb < p.cin_blocks; ++cb) {
           C2W_TIMED_WAIT(w_full, &a_full[unit], a_phase);
-          const uint64_t adesc_u = adesc0 + static_cast<uint64_t>(unit * (Cfg::kARUnitBytes >> 4));
-          for (int s3 = 0; s3 < 3; ++s3) {
+          const uint64_t adesc_u = adesc0 + static_cast<uint64_t>(unit * (Cfg::kARUnitBytes >> 4)) + ph_off;
+          for (int s3 = 0; s3 < kCols; ++s3) {
             C2W_TIMED_WAIT(w_full, &full[stage], phase);
             tc_fence_after();
             if (elect_one()) {
               const uint64_t bdesc = bdesc0 + static_cast<uint64_t>(stage * (Cfg::kARBStageBytes >> 4));
   #pragma unroll
-              for (int r = 0; r < 3; ++r) {
+              for (int r = 0; r < kCols; ++r) {
                 // tap (r, s) = the unit from its r-th pixel row and s-th pixel column on.  The 128B swizzle is a
                 // function of the absolute shared-memory address for the MMA's reads as for TMA's writes, so a start
                 // address s * 128 B into a swizzle atom with 1280 B between 8-row groups reads what TMA wrote; the
@@ -618,14 +644,14 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
                   else umma_bf16(tmem_d, a, b, idesc, (cb | s3 | r | k) != 0);
                 }
               }
-              const bool last = s3 == 2 && cb + 1 == p.cin_blocks;
+              const bool last = s3 == kCols - 1 && cb + 1 == p.cin_blocks;
               if (CG == 2) {
                 umma_commit_pair(&empty[stage]);
-                if (s3 == 2) umma_commit_pair(&a_empty[unit]);
+                if (s3 == kCols - 1) umma_commit_pair(&a_empty[unit]);
                 if (last) umma_commit_pair(&tmem_full[acc]);
               } else {
                 umma_commit(&empty[stage]);
-                if (s3 == 2) umma_commit(&a_empty[unit]);
+                if (s3 == kCols - 1) umma_commit(&a_empty[unit]);
                 if (last) umma_commit(&tmem_full[acc]);
               }
             }
@@ -689,6 +715,17 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
       // TMA store of the finished tile and the prefetch of the auxiliary tile of the staging tile's next user; the
       // epilogue warps never wait for a TMA transfer.
       const bool leader = lane == 0;                // owns every bulk async-group of this CTA
+      // PH: the box {64 ch, b, 8 px, a, 16 rows} at (b, j0, a, n * H + i0) of the {C, b, j, a, n * H + i} view of the
+      // [n, 2H, 2W, C] output (H x W the low-res image): c1 = b, c2 = j0, c3 = a, c4 = n * H + i0
+      auto ph_coords = [&](int mt, int& c1, int& c2, int& c3, int& c4) {
+        int ph;
+        mt = ph_split(mt, ph);
+        const int img = mt / p.tiles_per_img, tt = mt % p.tiles_per_img;
+        c1 = ph & 1;
+        c2 = (tt % p.tiles_w) * Cfg::kARTileW;
+        c3 = ph >> 1;
+        c4 = img * p.img_h + (tt / p.tiles_w) * Cfg::kARTileH;
+      };
       auto box_coords = [&](int mt, int& c1, int& c2, int& c3) {
         const int img = mt / p.tiles_per_img, tt = mt % p.tiles_per_img;
         c1 = (tt % p.tiles_w) * Cfg::kARTileW;
@@ -708,7 +745,11 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
         mbar_arrive_expect_tx(&res_full[buf], Cfg::kStagingBytes);
   #pragma unroll
         for (int b = 0; b < BN / 64; ++b) {
-          if (AR) {
+          if (PH) {
+            int c1, c2, c3, c4;
+            ph_coords(mt, c1, c2, c3, c4);
+            tma_load_5d(&tmOut, &res_full[buf], dst + b * kATileBytes, nt * BN + b * 64, c1, c2, c3, c4);
+          } else if (AR) {
             int c1, c2, c3;
             box_coords(mt, c1, c2, c3);
             if (p.ar2) {
@@ -737,7 +778,11 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
         if (leader) {
   #pragma unroll
           for (int b = 0; b < BN / 64; ++b) {
-            if (AR) {
+            if (PH) {
+              int c1, c2, c3, c4;
+              ph_coords(mt, c1, c2, c3, c4);
+              tma_store_5d(&tmOut, stg + b * kATileBytes, nt * BN + b * 64, c1, c2, c3, c4);
+            } else if (AR) {
               int c1, c2, c3;
               box_coords(mt, c1, c2, c3);
               tma_store_4d(&tmOut, stg + b * kATileBytes, nt * BN + b * 64, c1, c2, c3);
@@ -802,8 +847,11 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
         const bool valid = m < p.m_total;
         // modulation vector of this tile's image (per-sample diffusion times) or of the whole batch
         const float* ln_mod_t = nullptr;
-        if (LN && p.ln_mod != nullptr)
-          ln_mod_t = p.ln_mod + static_cast<size_t>(p.ln_mod_stride) * (mt / p.tiles_per_img);
+        if (LN && p.ln_mod != nullptr) {
+          int ph, mt_img = mt;
+          if (PH) mt_img = ph_split(mt, ph);
+          ln_mod_t = p.ln_mod + static_cast<size_t>(p.ln_mod_stride) * (mt_img / p.tiles_per_img);
+        }
         C2W_TIMED_WAIT(w_tfull, &tmem_full[acc], acc_phase);
         tc_fence_after();
         const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc * BN + col_base;
@@ -899,7 +947,9 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
       [[maybe_unused]] long long w_lnfull = 0, c_ln = 0;
       int it_local = 0;
       for (int tile = group_id; tile < num_tiles; tile += num_groups) {
-        const int mt = (tile / p.num_n_tiles) * CG + rank;
+        int mt = (tile / p.num_n_tiles) * CG + rank;
+        int ph = 0;  // PH: output phase of the tile; mt becomes its low-res tile
+        if (PH) mt = ph_split(mt, ph);
         const int buf = two_bufs ? (it_local & 1) : 0;
         const int use = two_bufs ? (it_local >> 1) : it_local;
         uint8_t* stg = stg0 + buf * Cfg::kStagingBytes;
@@ -929,8 +979,14 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
             const int tt = mt % p.tiles_per_img, img = mt / p.tiles_per_img;
             const int th0 = (tt / p.tiles_w) * Cfg::kARTileH, tw0 = (tt % p.tiles_w) * Cfg::kARTileW;
             tile_pix = (static_cast<long long>(img) * p.ln_H + th0) * p.ln_W + tw0;
+            if (PH)  // tile row (i, j) is output pixel (2 (th0 + i) + a, 2 (tw0 + j) + b) of the ln_H x ln_W image
+              tile_pix = (static_cast<long long>(img) * p.ln_H + 2 * th0 + (ph >> 1)) * p.ln_W + 2 * tw0 + (ph & 1);
             tile_valid = tile_pix < p.m_total;
-            if (p.ln_up) {
+            if (PH) {
+              tile_out += tile_pix * BN;
+              row_pitch = 2 * p.ln_W * BN;
+              px_pitch = 2 * BN;
+            } else if (p.ln_up) {
               tile_out += ((static_cast<long long>(img) * 2 * p.ln_H + 2 * th0) * 2 * p.ln_W + 2 * tw0) * BN;
               row_pitch = 4 * p.ln_W * BN;
               px_pitch = 2 * BN;
@@ -992,7 +1048,8 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
                 const bool ok = AR ? tile_valid : (tile_pix + r < p.m_total);
                 if (ok) {
                   if (p.ln_inv != nullptr && ln_chunk == 0)
-                    p.ln_inv[tile_pix + (AR ? (r >> 3) * p.ln_W + (r & 7) : r)] = invv[bb];
+                    p.ln_inv[tile_pix + (PH ? 2 * ((r >> 3) * p.ln_W + (r & 7)) : AR ? (r >> 3) * p.ln_W + (r & 7) : r)] =
+                        invv[bb];
                   __nv_bfloat16* dst = tile_out + eo;
                   *reinterpret_cast<uint4*>(dst) = yv[bb];
                   if (AR && p.ln_up) {
@@ -1128,6 +1185,7 @@ struct ConvLaunch {
   int cg;     // CTAs per MMA (1 or 2)
   int ln;     // fused LayerNorm output
   int ar;     // activation-reuse main loop (16 x 8 spatial tiles)
+  int ph;     // phase form of the activation-reuse main loop (conv_launch_init_phase)
   int grid;   // CTAs (a multiple of cg)
   int n_img, Ho, Wo, cout_pad;
   const void* out_ptr;  // bf16 output bound by conv_launch_set_out (LayerNorm fusion matches on it)
@@ -1160,6 +1218,7 @@ inline bool conv_launch_init(ConvLaunch* L, bool is_conv3x3, const __nv_bfloat16
   memset(&L->tmOut2, 0, sizeof(CUtensorMap));
   L->bn = bn;
   L->ln = 0;
+  L->ph = 0;
   L->out_ptr = nullptr;
   if (cin % kBlockK != 0 || cout_pad % bn != 0) return false;
   if (stride != 1 && !(stride == 2 && is_conv3x3 && H % 2 == 0 && W % 2 == 0)) return false;
@@ -1256,9 +1315,93 @@ inline bool conv_launch_init(ConvLaunch* L, bool is_conv3x3, const __nv_bfloat16
   return true;
 }
 
+// Phase weights of a 3x3 conv applied to a nearest x2 upsampled input (see ph_split): fp32 OIHW [cout, cin, 3, 3] ->
+// bf16 [4 phases][cout_pad][4 taps * cin_pad], phase = 2a + b, tap = 2 tr + ts, k = tap * cin_pad + c (zero padding).
+// Merged weight (a, b, tr, ts) = sum of w[r][s] over the filter rows r that read low-res row offset tr of phase a
+// (a = 0: tr 0 <- r 0, tr 1 <- r 1, 2; a = 1: tr 0 <- r 0, 1, tr 1 <- r 2) and the same for columns, summed in fp32 in
+// the order r -> s (ascending) and rounded to bf16 once.  refresh_weights_kernel repeats this sum in the same order.
+__host__ __device__ inline float conv_phase_weight(const float* w9, int a, int b, int tr, int ts) {
+  const int r0 = tr == 0 ? 0 : 1 + a, r1 = tr == 0 ? a : 2;
+  const int s0 = ts == 0 ? 0 : 1 + b, s1 = ts == 0 ? b : 2;
+  float acc = 0.f;
+  for (int r = r0; r <= r1; ++r)
+    for (int s = s0; s <= s1; ++s) acc += w9[r * 3 + s];
+  return acc;
+}
+inline void conv_pack_phase_weights(const float* w, int cout, int cin, int cin_pad, int cout_pad, __nv_bfloat16* out) {
+  const size_t K = static_cast<size_t>(4) * cin_pad;
+  for (size_t i = 0; i < 4 * static_cast<size_t>(cout_pad) * K; ++i) out[i] = __float2bfloat16_rn(0.f);
+  for (int ph = 0; ph < 4; ++ph)
+    for (int o = 0; o < cout; ++o)
+      for (int c = 0; c < cin; ++c)
+        for (int t = 0; t < 4; ++t)
+          out[(static_cast<size_t>(ph) * cout_pad + o) * K + static_cast<size_t>(t) * cin_pad + c] = __float2bfloat16_rn(
+              conv_phase_weight(w + (static_cast<size_t>(o) * cin + c) * 9, ph >> 1, ph & 1, t >> 1, t & 1));
+}
+
+// The phase form of conv3x3(nearest x2 (x)) (see ph_split): x is the LOW-RES NHWC input [n_img, H, W, cin], w_phase
+// the phase weights (conv_pack_phase_weights), the output [n_img, 2H, 2W, cout_pad].  Needs the activation-reuse
+// geometry at the low resolution with an even number of 16 x 8 tiles per image (the two CTAs of a pair share a phase).
+inline bool conv_phase_geometry_ok(int H, int W) { return H % 16 == 0 && W % 8 == 0 && (H / 16) * (W / 8) % 2 == 0; }
+inline bool conv_launch_init_phase(ConvLaunch* L, const __nv_bfloat16* x, int n_img, int H, int W, int cin,
+                                   const __nv_bfloat16* w_phase, int cout_pad, int bn, int num_sms) {
+  ConvParams& p = L->p;
+  memset(&p, 0, sizeof(p));
+  memset(&L->tmOut, 0, sizeof(CUtensorMap));
+  memset(&L->tmOut2, 0, sizeof(CUtensorMap));
+  L->bn = bn;
+  L->ln = 0;
+  L->out_ptr = nullptr;
+  if (cin % kBlockK != 0 || !(bn == 64 || bn == 128) || cout_pad % bn != 0 || n_img < 1 ||
+      !conv_phase_geometry_ok(H, W))
+    return false;
+  L->cg = 2;
+  L->ar = 1;
+  L->ph = 1;
+  L->n_img = n_img;
+  L->Ho = 2 * H;
+  L->Wo = 2 * W;
+  L->cout_pad = cout_pad;
+  p.taps = 4;
+  p.stride = 1;
+  p.cin_blocks = cin / kBlockK;
+  p.num_n_tiles = cout_pad / bn;
+  p.ln_eps = 1e-5f;
+  p.m_total = 4 * n_img * H * W;
+  p.tiles_w = W / 8;
+  p.tiles_per_img = (H / 16) * p.tiles_w;
+  p.num_m_tiles = 4 * n_img * p.tiles_per_img;
+  p.img_h = H;
+  p.img_w = W;
+  p.ar_row_step16 = (kARUnitW * 128) >> 4;
+  p.ar_tx_a = 18 * kARUnitW * kBlockK * 2;
+  p.ar_tx_b = 2 * (bn / 2) * kBlockK * 2;
+  {
+    const uint64_t dims[4] = {(uint64_t)cin, (uint64_t)W, (uint64_t)H, (uint64_t)n_img};
+    const uint32_t box[4] = {(uint32_t)kBlockK, (uint32_t)kARUnitW, 18u, 1u};
+    if (!make_tmap_bf16(&L->tmA, x, 4, dims, box)) return false;
+  }
+  {  // [phase][Cout][tr][ts * Cin + c] viewed as {ts * Cin + c, Cout, tr, phase}: the two tr tiles of one (ts, cb)
+    const uint64_t dims[4] = {(uint64_t)2 * cin, (uint64_t)cout_pad, 2, 4};
+    const uint64_t strides[3] = {(uint64_t)4 * cin * 2, (uint64_t)2 * cin * 2, (uint64_t)4 * cin * 2 * cout_pad};
+    const uint32_t box[4] = {(uint32_t)kBlockK, (uint32_t)(bn / 2), 2u, 1u};
+    if (!make_tmap_bf16(&L->tmB, w_phase, 4, dims, box, nullptr, strides)) return false;
+  }
+  conv_set_grid(L, num_sms);
+  p.ldc = cout_pad;
+  return true;
+}
+
 // Tensor map of a bf16 [M, cout_pad] epilogue tensor: rows of 128 pixels, or (AR) 16 x 8 spatial blocks of the
-// [n, H, W, cout_pad] view of the same memory.
+// [n, H, W, cout_pad] view of the same memory (PH: the {C, b, j, a, n * H + i} view of [n, 2H, 2W, C], see ph_coords).
 inline bool conv_make_epi_map(const ConvLaunch* L, CUtensorMap* m, const void* ptr) {
+  if (L->ph) {
+    const uint64_t C = L->cout_pad, Wl = L->Wo / 2, Hl = L->Ho / 2;
+    const uint64_t dims[5] = {C, 2, Wl, 2, (uint64_t)L->n_img * Hl};
+    const uint64_t strides[4] = {C * 2, 2 * C * 2, 2 * Wl * C * 2, 4 * Wl * C * 2};
+    const uint32_t box[5] = {64u, 1u, 8u, 1u, 16u};
+    return make_tmap_bf16(m, ptr, 5, dims, box, nullptr, strides);
+  }
   if (L->ar) {  // ar2: one 8 x 8 box per image (the staging tile is image-major)
     const uint64_t dims[4] = {(uint64_t)L->cout_pad, (uint64_t)L->Wo, (uint64_t)L->Ho, (uint64_t)L->n_img};
     const uint32_t box[4] = {64u, 8u, L->p.ar2 ? 8u : 16u, 1u};
@@ -1276,7 +1419,7 @@ inline bool conv_launch_set_out(ConvLaunch* L, __nv_bfloat16* out) {
 
 // Second bf16 output of EPI_BIAS_SILU_DUAL (the SiLU of the first)
 inline bool conv_launch_set_out2(ConvLaunch* L, __nv_bfloat16* out2) {
-  if (L->bn > 128) return false;  // two staging tiles of a wider tile leave no operand ring
+  if (L->bn > 128 || L->ph) return false;  // two staging tiles of a wider tile leave no operand ring
   return conv_make_epi_map(L, &L->tmOut2, out2);
 }
 
@@ -1285,7 +1428,7 @@ inline bool conv_launch_can_ln(const ConvLaunch* L, int upsample) {
   const ConvParams& p = L->p;
   if (L->ln || p.ar2 || p.num_n_tiles != 1 || !(L->bn == 64 || L->bn == 128 || L->bn == 256)) return false;
   if (!(p.mode == EPI_BIAS || p.mode == EPI_BIAS_RES)) return false;
-  if (upsample && p.taps != 9) return false;
+  if (upsample && (p.taps != 9 || L->ph)) return false;
   return true;
 }
 
@@ -1317,7 +1460,7 @@ inline bool conv_use_pdl() {
   return pdl != 0;
 }
 
-template <int BN, int CG, bool LN, bool AR>
+template <int BN, int CG, bool LN, bool AR, bool PH = false>
 inline cudaError_t conv_launch_variant(const ConvLaunch& L, cudaStream_t stream) {
   using Cfg = ConvCfg<BN, CG>;
   static_assert(!AR || Cfg::ar_stages_for(2) >= 3, "activation-reuse weight ring too shallow");
@@ -1326,7 +1469,7 @@ inline cudaError_t conv_launch_variant(const ConvLaunch& L, cudaStream_t stream)
   int dev = 0;
   cudaGetDevice(&dev);
   if (!((attr_done >> (dev & 63)) & 1ull)) {
-    cudaError_t e = cudaFuncSetAttribute(conv_gemm_tcgen05_kernel<BN, CG, LN, AR>,
+    cudaError_t e = cudaFuncSetAttribute(conv_gemm_tcgen05_kernel<BN, CG, LN, AR, PH>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit);
     if (e != cudaSuccess) return e;
     attr_done |= 1ull << (dev & 63);
@@ -1362,13 +1505,14 @@ inline cudaError_t conv_launch_variant(const ConvLaunch& L, cudaStream_t stream)
     attr[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.numAttrs = 2;
   }
-  return cudaLaunchKernelEx(&cfg, conv_gemm_tcgen05_kernel<BN, CG, LN, AR>, L.tmA, L.tmB, L.tmOut, L.tmOut2, p);
+  return cudaLaunchKernelEx(&cfg, conv_gemm_tcgen05_kernel<BN, CG, LN, AR, PH>, L.tmA, L.tmB, L.tmOut, L.tmOut2, p);
 }
 
 template <int BN, bool LN>
 inline cudaError_t conv_launch_bn_ln(const ConvLaunch& L, cudaStream_t stream) {
   if (L.cg == 2) {
     if constexpr (BN == 128 || BN == 64) {
+      if (L.ph) return conv_launch_variant<BN, 2, LN, true, true>(L, stream);
       if (L.ar) return conv_launch_variant<BN, 2, LN, true>(L, stream);
     }
     return conv_launch_variant<BN, 2, LN, false>(L, stream);

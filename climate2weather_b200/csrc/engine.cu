@@ -34,6 +34,7 @@ struct ConvW {
   bf16* w = nullptr;   // [cout_pad, taps * cin_pad], k = tap * cin_pad + c
   float* b = nullptr;  // [cout_pad]
   bf16* wd = nullptr;  // input-gradient weights [cin_pad, taps * cout_pad], k = (8 - tap) * cout_pad + o  (flipped)
+  bf16* wph = nullptr;  // ascent tails: phase weights [4][cout_pad, 4 * cin_pad] (conv_pack_phase_weights)
   int cin = 0, cout = 0, cin_pad = 0, cout_pad = 0, taps = 0;
   long long gw = -1, gb = -1;  // offsets of weight / bias in the flat gradient buffer (c2w_param_layout)
 };
@@ -499,6 +500,17 @@ int build_plan(c2w_handle* h, int n, bool vjp, bool per_t, void* base, size_t* b
   float* forc_pad = h->forcing_pad > 0 ? B.take<float>(ns * h->forcing_pad) : nullptr;
   float* fvec = h->forcing_pad > 0 ? B.take<float>(ns * h->cfg.embedding_dim) : nullptr;
   std::vector<bf16*> xs(nl), as(nl), hs(nl), gs(nl), ga(nl), gh(nl);
+  // Forward-only plans run the tail of level l > 0 (LN -> nearest x2 -> conv) as the phase form of K1 at the low
+  // resolution (conv_launch_init_phase): the LayerNorm writes as[l], no upsampled tensor exists.  Stashing plans keep
+  // the upsampled LayerNorm output: the tail's wgrad and input gradient read it.  Tails whose low-res image does not tile
+  // take the upsampled path too.  Above 128 output channels the phase tail has 128-wide N tiles, so the LayerNorm of
+  // its output is a launch of its own (config 2, level 3: 253 us for the upsampled 256-wide tile with the fused
+  // LayerNorm against 146 us for the phase conv and the LayerNorm launch, profiles/r09_tail_timing.txt).
+  auto phase_tail = [&](int l) {
+    const ConvW& t = h->levels[l].tail;
+    return !vjp && l > 0 && t.wph != nullptr && (t.cout_pad <= 128 || t.cout_pad % 128 == 0) &&
+           conv_phase_geometry_ok(h->levels[l].H, h->levels[l].W);
+  };
   size_t up_elems = 0, qkv_elems = 0, att_elems = 0;
   for (int l = 0; l < nl; ++l) {
     const LevelW& L = h->levels[l];
@@ -511,7 +523,7 @@ int build_plan(c2w_handle* h, int n, bool vjp, bool per_t, void* base, size_t* b
       ga[l] = B.take<bf16>(e);
       gh[l] = B.take<bf16>(e);
     }
-    if (l > 0) {
+    if (l > 0 && !phase_tail(l)) {
       const LevelW& U = h->levels[l - 1];
       up_elems = std::max(up_elems, static_cast<size_t>(n) * U.H * U.W * L.C);
     }
@@ -651,7 +663,7 @@ int build_plan(c2w_handle* h, int n, bool vjp, bool per_t, void* base, size_t* b
     if (h->fuse_ln && !P.ops.empty()) {
       Op& prev = P.ops.back();
       if (prev.kind == OP_CONV && !prev.is_final && prev.conv.out_ptr == in && prev.conv.cout_pad == C &&
-          prev.conv.p.num_n_tiles != 1 && (C == 128 || C == 256)) {
+          !prev.conv.ph && prev.conv.p.num_n_tiles != 1 && (C == 128 || C == 256)) {
         // the tile picker split this layer for a fuller last wave; the fused LayerNorm is worth more than that
         Op whole;
         const Op::ConvSpec& sp = prev.spec;
@@ -903,6 +915,23 @@ int build_plan(c2w_handle* h, int n, bool vjp, bool per_t, void* base, size_t* b
     if (l > 0) {
       const LevelW& U = h->levels[l - 1];
       const size_t eu = static_cast<size_t>(n) * U.H * U.W * L.C;
+      if (phase_tail(l)) {
+        add_ln(xs[l], as[l], nullptr, L.C, L.H, L.W, 0, -1);
+        if (real) {
+          Op op;
+          op.kind = OP_CONV;
+          if (!conv_launch_init_phase(&op.conv, as[l], n, L.H, L.W, L.C, L.tail.wph, L.tail.cout_pad,
+                                      std::min(L.tail.cout_pad, 128), h->sms))
+            return fail(C2W_ERR_INVALID, "cannot build the phase-form tail launch (n=%d H=%d W=%d cin=%d cout=%d) %s", n,
+                        L.H, L.W, L.C, L.tail.cout_pad, tmap_error_slot());
+          op.conv.p.mode = EPI_BIAS_RES;
+          op.conv.p.bias = L.tail.b;
+          if (!conv_launch_set_out(&op.conv, xs[l - 1])) return fail(C2W_ERR_CUDA, "cannot encode the output tensor map");
+          op.pix_per_img = U.H * U.W;
+          P.ops.push_back(op);
+        }
+        continue;
+      }
       bf16* upl = vjp ? stash(eu) : up;
       float* invt = vjp ? stash_f(static_cast<size_t>(n) * L.H * L.W) : nullptr;
       add_ln(xs[l], upl, invt, L.C, L.H, L.W, 1, -1);
@@ -1305,6 +1334,11 @@ int c2w_finalize_weights(c2w_handle* h) {
       if ((rc = pack_conv(h, buf, L.C, Cu, 9, &L.head))) return rc;
       snprintf(buf, sizeof buf, "unet.tails.%d.2", rev);
       if ((rc = pack_conv(h, buf, Cu, L.C, 9, &L.tail))) return rc;
+      // the same tail at the low resolution (forward-only plans): four 2x2 phase convs of the un-upsampled LayerNorm
+      std::vector<bf16> ph(static_cast<size_t>(4) * L.tail.cout_pad * 4 * L.tail.cin_pad);
+      conv_pack_phase_weights(h->raw[std::string(buf) + ".weight"].data(), Cu, L.C, L.tail.cin_pad, L.tail.cout_pad,
+                              ph.data());
+      if ((rc = dev_upload(h, ph.data(), ph.size() * sizeof(bf16), reinterpret_cast<void**>(&L.tail.wph)))) return rc;
     }
     const int step = L.attn ? 2 : 1;
     for (int side = 0; side < 2; ++side) {
@@ -1653,7 +1687,8 @@ int c2w_refresh_weights(c2w_handle* h, const float* flat_dev, void* stream) {
     auto conv = [&](const ConvW& w) -> int {
       if (w.gw < 0 || w.gb < 0) return fail(C2W_ERR_MISSING, "a conv has no slot in the flat parameter layout");
       RefreshJob j{};
-      j.src = w.gw, j.n = static_cast<long long>(w.cout) * w.cin * w.taps, j.wp = w.w, j.wd = w.wd, j.kind = 0;
+      j.src = w.gw, j.n = static_cast<long long>(w.cout) * w.cin * w.taps, j.wp = w.w, j.wd = w.wd, j.wph = w.wph;
+      j.kind = 0;
       j.cout = w.cout, j.cin = w.cin, j.taps = w.taps, j.cin_pad = w.cin_pad, j.cout_pad = w.cout_pad;
       if (w.taps > 9) return fail(C2W_ERR_INVALID, "weight re-pack handles up to 9 taps (got %d)", w.taps);
       j.chunks = ((w.cout + kRefreshTile - 1) / kRefreshTile) * ((w.cin + kRefreshTile - 1) / kRefreshTile);

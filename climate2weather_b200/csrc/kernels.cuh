@@ -11,6 +11,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "conv_tcgen05.cuh"  // conv_phase_weight (refresh_weights_kernel)
+
 namespace c2w {
 
 typedef __nv_bfloat16 bf16;
@@ -1154,6 +1156,7 @@ struct RefreshJob {
   long long n;     // copy: floats; padded rows: rows * cols_pad; conv: unused
   bf16* wp;        // conv: forward operand
   bf16* wd;        // conv: input-gradient operand
+  bf16* wph;       // conv: phase operand of an ascent tail (conv_pack_phase_weights), or null
   float* fdst;     // copy / padded rows: destination
   int kind;        // 0 conv weights, 1 fp32 copy, 2 rows of `cin` floats padded to `cin_pad`
   int cout, cin, taps, cin_pad, cout_pad;
@@ -1196,6 +1199,17 @@ refresh_weights_kernel(const RefreshJob* __restrict__ jobs, const int* __restric
         const int o = k % no, ct = k / no, t = ct % jb.taps, c = ct / jb.taps;
         jb.wd[(c0 + c) * Kd + static_cast<size_t>(jb.taps - 1 - t) * jb.cout_pad + o0 + o] =
             __float2bfloat16_rn(tile[o][c * jb.taps + t]);
+      }
+      if (jb.wph != nullptr) {  // (phase, o, tap, c), c fastest; the sums of conv_pack_phase_weights in its order
+        const size_t Kp = static_cast<size_t>(4) * jb.cin_pad;
+        for (int k = threadIdx.x; k < 16 * no * nc; k += blockDim.x) {
+          const int c = k % nc, rest = k / nc, t = rest & 3, o = (rest >> 2) % no, ph = (rest >> 2) / no;
+          float w9[9];
+  #pragma unroll
+          for (int i = 0; i < 9; ++i) w9[i] = tile[o][c * 9 + i];
+          jb.wph[(static_cast<size_t>(ph) * jb.cout_pad + o0 + o) * Kp + static_cast<size_t>(t) * jb.cin_pad + c0 + c] =
+              __float2bfloat16_rn(conv_phase_weight(w9, ph >> 1, ph & 1, t >> 1, t & 1));
+        }
       }
       __syncthreads();
       continue;

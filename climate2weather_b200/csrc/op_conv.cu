@@ -67,6 +67,35 @@ int c2w_op_conv_ex(const c2w_conv_desc* d, void* stream) {
   return C2W_OK;
 }
 
+int c2w_op_conv_phase(const c2w_conv_desc* d, void* stream) {
+  C2W_REQUIRE(d && d->x && d->w_packed && d->bias && d->out, "c2w_op_conv_phase: null argument");
+  C2W_REQUIRE(d->mode == EPI_BIAS || d->mode == EPI_BIAS_RES, "c2w_op_conv_phase: mode 0 or 2 (got %d)", d->mode);
+  C2W_REQUIRE(d->mode != EPI_BIAS_RES || d->res == d->out, "mode 2 works in place: res must equal out");
+  const int sms = c2w_num_sms();
+  C2W_REQUIRE(sms > 0, "c2w_op_conv_phase: no CUDA device");
+  const int bn = d->bn ? d->bn : d->cout_pad <= 128 ? d->cout_pad : 128;
+  ConvLaunch L;
+  if (!conv_launch_init_phase(&L, static_cast<const __nv_bfloat16*>(d->x), d->n_img, d->H, d->W, d->cin,
+                              static_cast<const __nv_bfloat16*>(d->w_packed), d->cout_pad, bn, sms))
+    return fail(C2W_ERR_INVALID, "c2w_op_conv_phase: cannot build launch (n=%d H=%d W=%d cin=%d cout=%d bn=%d) %s",
+                d->n_img, d->H, d->W, d->cin, d->cout_pad, bn, tmap_error_slot());
+  L.p.mode = d->mode;
+  L.p.bias = d->bias;
+  if (!conv_launch_set_out(&L, static_cast<__nv_bfloat16*>(d->out)))
+    return fail(C2W_ERR_CUDA, "c2w_op_conv_phase: cannot encode the output tensor map");
+  if (d->ln_out && !conv_launch_set_ln(&L, static_cast<__nv_bfloat16*>(d->ln_out), d->ln_mod, 0))
+    return fail(C2W_ERR_INVALID, "c2w_op_conv_phase: the fused LayerNorm needs bn == cout_pad");
+  C2W_CUDA(conv_launch(L, static_cast<cudaStream_t>(stream)));
+  return C2W_OK;
+}
+
+int c2w_pack_phase_weights(const float* w, int cout, int cin, int cin_pad, int cout_pad, void* out_bf16) {
+  C2W_REQUIRE(w && out_bf16 && cout >= 1 && cin >= 1 && cin_pad >= cin && cout_pad >= cout,
+              "c2w_pack_phase_weights: bad argument");
+  conv_pack_phase_weights(w, cout, cin, cin_pad, cout_pad, static_cast<__nv_bfloat16*>(out_bf16));
+  return C2W_OK;
+}
+
 // x: bf16 NHWC [n_img, H, W, cin]  (conv3x3 != 0)   or   bf16 [n_img*H*W, cin] row-major (conv3x3 == 0)
 // w_packed: bf16 [cout_pad, taps*cin] with k = (r*3+s)*cin + c ; bias: fp32 [cout_pad]
 // mode: EpiMode (0 bias, 1 bias+silu, 2 bias+residual, 4 fp32 out); res/out: bf16 [M, cout_pad]

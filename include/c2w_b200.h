@@ -295,6 +295,18 @@ int c2w_conv_tile_width(int cout_pad, int conv3x3, int n_img, int H, int W, int 
 int c2w_op_conv(const void* x, int n_img, int H, int W, int cin, const void* w_packed, int cout_pad,
                 const float* bias, int mode, const void* res, void* out, float* out_f32, int conv3x3, int bn,
                 int max_ctas, void* stream);
+/* The phase form of an ascent tail, conv3x3(nearest x2 (x)) + bias [+ residual], computed at the low resolution as four
+ * 2x2 convs (one per output phase (a, b) of pixel (2i + a, 2j + b)) with merged weights.  d->x: LOW-RES input
+ * [n_img, H, W, cin] (H % 16 == 0, W % 8 == 0, an even number of 16 x 8 blocks per image); d->w_packed: the weights of
+ * c2w_pack_phase_weights; out / res: [n_img, 2H, 2W, cout_pad]; mode 0 or 2; bn 64 or 128 (0: cout_pad up to 128,
+ * else 128); ln_out
+ * (optional): the channel LayerNorm of out, [n_img, 2H, 2W, cout_pad], bn == cout_pad, not upsampled.  stride,
+ * conv3x3, variant and max_ctas are not used. */
+int c2w_op_conv_phase(const c2w_conv_desc* d, void* stream);
+/* Host only: the phase weights of a 3x3 conv.  w: fp32 OIHW [cout, cin, 3, 3] -> out: bf16 [4][cout_pad][4 * cin_pad],
+ * phase = 2a + b, tap = 2 tr + ts, k = tap * cin_pad + c; each merged weight is an fp32 sum of the 3x3 weights it
+ * stands for, rounded to bf16 once (the engine packs its ascent tails with this function). */
+int c2w_pack_phase_weights(const float* w, int cout, int cin, int cin_pad, int cout_pad, void* out_bf16);
 int c2w_op_layernorm(const void* x_bf16, const float* mod, void* out_bf16, int64_t npix, int C, int H, int W,
                      int upsample, void* stream);
 int c2w_op_attention(const void* qkv_bf16, void* out_bf16, int n, int T, int C, void* stream);
