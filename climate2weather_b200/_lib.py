@@ -137,6 +137,7 @@ SIGNATURES = {
     "c2w_window_score_members": (_i, [_vp, _vp, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _f, _vp, _vp]),
     "c2w_guided_step_members": (_i, [C.POINTER(Guide), C.c_int32, C.POINTER(PointObs), C.POINTER(C.c_float), _vp, _vp,
                                      _vp]),
+    "c2w_guided_step_batch": (_i, [C.POINTER(Guide), C.c_int32, _vp, _vp, _vp, C.POINTER(PointObs), _vp, _vp, _vp]),
     "c2w_reduce_partials_members": (_i, [_vp, C.c_int32, C.c_int32, _vp, _vp]),
     "c2w_corrector_update_members": (_i, [_vp, _vp, _vp, _d, _f, _f, C.c_int32, _i64, C.c_int32, _vp, C.c_uint32, _vp,
                                           _vp]),

@@ -2169,6 +2169,83 @@ int c2w_guided_step_members(const c2w_guide* g, int32_t member_frames, const c2w
   return guided_combined<false>(g, obs, point_std2, ObsStd2{}, stream, member_frames);
 }
 
+// A batch of independent problems stored member-major: one launch of the single-trajectory K6 / K6p / K6c instance per
+// member, on that member's slice of every operand (x, eps, eps_out, vjp, cot_out, partials, y, coarse_std2,
+// frame_slot) with its own gamma and std^2 in the parameter block.  Each member therefore runs exactly the instance
+// and the parameters its own run uses: a variant of those kernels reading gamma from a register rather than from the
+// parameter block lets ptxas round gamma r^2 + std^2 differently (a separate FMUL and FADD instead of one FFMA), which
+// would break the members' bit identity with their own runs.
+int c2w_guided_step_batch(const c2w_guide* g, int32_t member_frames, const float* gamma, const float* std2,
+                          const float* point_std2, const c2w_point_obs* obs, const float* coarse_std2,
+                          const float* entry_std2, void* stream) {
+  C2W_REQUIRE(g && gamma, "c2w_guided_step_batch: bad argument (gamma is required)");
+  C2W_REQUIRE(member_frames >= 1 && g->own_n % member_frames == 0,
+              "c2w_guided_step_batch: own_n=%d is not a whole number of members of %d frames", g->own_n, member_frames);
+  C2W_REQUIRE((g->frame_global0 + g->own_lo) % member_frames == 0,
+              "c2w_guided_step_batch: frame_global0 + own_lo = %d is not the first frame of a member of %d frames",
+              g->frame_global0 + g->own_lo, member_frames);
+  C2W_REQUIRE(g->halo == nullptr, "c2w_guided_step_batch: a batch is not time-sharded (halo must be NULL)");
+  const bool per_obs = coarse_std2 != nullptr || entry_std2 != nullptr;
+  if (per_obs) {  // a std per observation: the checks of c2w_guided_step_obs_std
+    C2W_REQUIRE((g->y == nullptr) == (coarse_std2 == nullptr),
+                "c2w_guided_step_batch: the coarse term needs both g->y and coarse_std2, or neither");
+    C2W_REQUIRE((obs == nullptr) == (entry_std2 == nullptr),
+                "c2w_guided_step_batch: the point term needs both obs and entry_std2, or neither");
+    C2W_REQUIRE(point_std2 == nullptr, "c2w_guided_step_batch: point_std2 with a std per observation");
+  } else {
+    C2W_REQUIRE((g->y == nullptr && obs == nullptr) || std2 != nullptr,
+                "c2w_guided_step_batch: a per-variable std needs the std2 array");
+    C2W_REQUIRE((g->y != nullptr && obs != nullptr) == (point_std2 != nullptr),
+                "c2w_guided_step_batch: point_std2 is given exactly when there is a coarse and a point term");
+  }
+  C2W_REQUIRE(g->y != nullptr || obs != nullptr, "c2w_guided_step_batch: no observation term (needs g->y or obs)");
+  const int C = g->channels == 0 ? 4 : g->channels;
+  C2W_REQUIRE(C >= 1 && C <= C2W_MAX_VARS, "c2w_guided_step_batch: 1 to %d variables per frame (got %d)", C2W_MAX_VARS,
+              C);
+  C2W_REQUIRE(g->H >= 1 && g->W >= 1 && g->s_step >= 1 && g->t_step >= 1, "c2w_guided_step_batch: bad geometry");
+  const int M = g->own_n / member_frames;
+  const long long frame = static_cast<long long>(g->H) * g->W * C;
+  const long long y_rows = (member_frames + g->t_step - 1) / g->t_step;
+  const long long y_member = g->y ? y_rows * C * (g->H / g->s_step) * (g->W / g->s_step) : 0;
+  // partials per member in mode 1: member_frames CTA rows of the launch's strips
+  const int strips = obs ? (g->H + obs->strip_rows - 1) / obs->strip_rows : g->H / g->s_step;
+  const long long parts = static_cast<long long>(member_frames) * strips;
+  for (int m = 0; m < M; ++m) {
+    c2w_guide gm = *g;
+    const long long off = static_cast<long long>(m) * member_frames * frame;  // member m's first frame, own_lo-relative
+    gm.x = g->x + off;
+    gm.eps = g->eps + off;
+    if (g->eps_out) gm.eps_out = g->eps_out + off;
+    if (g->vjp) gm.vjp = g->vjp + off;
+    if (g->cot_out) gm.cot_out = g->cot_out + off;
+    if (g->partials) gm.partials = g->partials + m * parts;
+    if (g->y) gm.y = g->y + m * y_member;
+    gm.own_n = member_frames;
+    gm.frame_global0 = -g->own_lo;  // local frame own_lo of the member's slice is its frame 0
+    for (int c = 0; c < C; ++c) {
+      gm.gamma[c] = gamma[m * C + c];
+      gm.std2[c] = per_obs || std2 == nullptr ? 1.0f : std2[m * C + c];
+    }
+    c2w_point_obs om;
+    if (obs) {
+      om = *obs;
+      om.frame_slot = obs->frame_slot + static_cast<long long>(m) * member_frames;
+    }
+    int rc;
+    if (per_obs) {
+      const ObsStd2 v{coarse_std2 ? coarse_std2 + m * y_member : nullptr, entry_std2};
+      rc = !obs ? guided_coarse<true>(&gm, v, stream)
+                : !g->y ? guided_points<true>(&gm, &om, v, stream) : guided_combined<true>(&gm, &om, nullptr, v, stream);
+    } else {
+      rc = !obs ? guided_coarse<false>(&gm, ObsStd2{}, stream)
+                : !g->y ? guided_points<false>(&gm, &om, ObsStd2{}, stream)
+                        : guided_combined<false>(&gm, &om, point_std2 + m * C, ObsStd2{}, stream);
+    }
+    if (rc) return rc;
+  }
+  return C2W_OK;
+}
+
 int c2w_reduce_partials(const float* partials, int32_t n, double* sumsq, void* stream) {
   C2W_REQUIRE(partials && sumsq && n >= 1, "c2w_reduce_partials: bad argument");
   reduce_partials_kernel<<<1, 256, 0, static_cast<cudaStream_t>(stream)>>>(partials, n, sumsq);

@@ -16,8 +16,9 @@ import torch
 from torch import Tensor
 
 from . import _lib
-from .score import AbstractScoreFunction, _mu_sigma
-from .sharding import all_gather_frames, gather_frames
+from .score import (AbstractScoreFunction, CoarseGrain, CombinedObservation, PointObservation, _mu_sigma, _Runtime,
+                    condition_for)
+from .sharding import all_gather_frames, gather_frames, make_plan
 
 
 class SDAPipeline:
@@ -107,6 +108,126 @@ class SDAPipeline:
         return self._sample_resident(score_fn, noise, steps, corrections, tau, device, show_progressbar, seeds, proc_x0,
                                      members=M)
 
+    def sample_batch(self, score_fns, noise, steps: int = 64, corrections: int = 0, tau: float = 1.0, proc_x0=None,
+                     device=None, show_progressbar=True, seeds: Optional[Sequence[int]] = None):
+        """M independent problems sampled together: score_fns[m] (each conditioned by its own `condition_on`: its own
+        y, std and gamma, for point terms its own stations, frames and mask) drives noise[m]; noise [M, L, C, H, W] ->
+        [M, L, C, H, W].  The members share one device-resident state and one network, so each UNet launch holds
+        windows of several members, as in `sample_ensemble`.
+
+        Member m is bit-identical to `sample(score_fns[m], noise[m], ..., seed=seeds[m])`, whatever `max_windows` is
+        (the same on every member).  `seeds`, `proc_x0`, `trace_at` and `nan_check_every` behave as in
+        `sample_ensemble`, and `sample_batch([sf] * M, ...)` equals `sample_ensemble(sf, ...)`.  The members must share
+        the ScoreUNet object, markov_order, the windows per launch, the operator family (all CoarseGrain, all
+        PointObservation or all CombinedObservation), the coarse term's (t_step, s_step), and whether they are
+        conditioned at all; closed-form guidance only (exact_grad=False), not time-sharded, and not with
+        `rng = "reference"` corrections.  A disagreement raises before any device work, naming the member."""
+        score_fns = list(score_fns)
+        for m, sf in enumerate(score_fns):
+            if not isinstance(sf, AbstractScoreFunction):
+                raise TypeError(f"sample_batch: member {m}: drives this package's score functions "
+                                f"(Default/BatchedScoreFunction); got {type(sf).__name__}")
+        if noise.dim() != 5:
+            raise ValueError(f"sample_batch: noise must be [M, L, C, H, W], got shape {tuple(noise.shape)}")
+        M = int(noise.shape[0])
+        if M < 1:
+            raise ValueError("sample_batch: noise holds no member (M = 0)")
+        if len(score_fns) != M:
+            raise ValueError(f"sample_batch: {len(score_fns)} score functions for {M} members (one per member)")
+        if seeds is not None:
+            seeds = [int(v) for v in seeds]
+            if len(seeds) != M:
+                raise ValueError(f"sample_batch: {len(seeds)} seeds for {M} members (one per member)")
+        if corrections > 0 and self.rng == "reference":
+            raise NotImplementedError("sample_batch: rng='reference' with corrections draws z on the host from the "
+                                      "global CPU generator, member after member; drawing it for all members step by "
+                                      "step cannot reproduce that stream, so it is refused (use rng='device' or sample)")
+        if device is not None and torch.device(device).type == "cuda":
+            for sf in score_fns:
+                sf.device = torch.device(device)
+        rt = self._batch_runtime(score_fns, noise)
+        return self._sample_resident(score_fns[0], noise, steps, corrections, tau, device, show_progressbar, seeds,
+                                     proc_x0, members=M, rt=rt)
+
+    def _batch_runtime(self, score_fns: list, noise: Tensor) -> _Runtime:
+        """The checks of sample_batch that need the members' score functions, then the batch's runtime: cached while the
+        score functions, the geometry and every member's conditioning (its `likelihood` dict, by identity: condition_on
+        replaces it) stay the same; a new conditioning of any member rebuilds the batch's conditioning only."""
+        M = len(score_fns)
+        shape = tuple(int(v) for v in noise.shape[1:])
+        L = shape[0]
+        sf0 = score_fns[0]
+        k = sf0.markov_order
+        nw = L - 2 * k
+
+        def windows(sf):
+            return min(sf.max_windows or sf._default_windows(nw), nw)
+
+        for m, sf in enumerate(score_fns):
+            lk = sf.likelihood
+            if sf.unet is not sf0.unet:
+                raise ValueError(f"sample_batch: member {m}: its ScoreUNet is not member 0's; the members share one "
+                                 f"network (one engine)")
+            if sf.markov_order != k:
+                raise ValueError(f"sample_batch: member {m}: markov_order {sf.markov_order} differs from member 0's {k}")
+            if windows(sf) != windows(sf0):
+                raise ValueError(f"sample_batch: member {m}: {windows(sf)} windows per launch (max_windows or the class "
+                                 f"default) differ from member 0's {windows(sf0)}; they decide each member's conv plan")
+            if sf.shard:
+                raise NotImplementedError(f"sample_batch: member {m}: a batch does not run on a time-sharded score "
+                                          f"function (enable_time_sharding)")
+            if lk is not None and lk.get("exact"):
+                raise NotImplementedError(f"sample_batch: member {m}: a batch runs closed-form guidance only: "
+                                          f"condition_on(..., exact_grad=False); exact_grad=True needs member-aware window "
+                                          f"selection and adjoints, which are not implemented")
+            if (lk is None) != (sf0.likelihood is None):
+                state = lambda v: "unconditioned" if v is None else "conditioned"
+                raise NotImplementedError(f"sample_batch: member {m}: {state(lk)} while member 0 is "
+                                          f"{state(sf0.likelihood)}; the members are all conditioned or none")
+        likes = tuple(sf.likelihood for sf in score_fns)
+        ident = (tuple(id(sf) for sf in score_fns), shape)
+        hit = getattr(self, "_batch_cache", None)
+        same = hit is not None and hit[0][:2] == ident and all(a is b for a, b in zip(hit[1], likes))
+        conds = None
+        if sf0.likelihood is not None and not same:
+            conds = []
+            for m, lk in enumerate(likes):
+                try:
+                    conds.append(condition_for(lk, shape))
+                except (ValueError, NotImplementedError) as e:
+                    raise type(e)(f"sample_batch: member {m}: {e}") from None
+            family = lambda op: type(op).__name__
+            coarse = lambda op: op.coarse if isinstance(op, CombinedObservation) else op
+            op0 = conds[0]["op"]
+            for m, c in enumerate(conds):
+                op = c["op"]
+                if family(op) != family(op0):
+                    raise NotImplementedError(f"sample_batch: member {m}: operator family {family(op)} differs from "
+                                              f"member 0's {family(op0)}; a batch runs one guidance kernel")
+                if isinstance(op, (CoarseGrain, CombinedObservation)) and \
+                        (coarse(op).t_step, coarse(op).s_step) != (coarse(op0).t_step, coarse(op0).s_step):
+                    raise NotImplementedError(f"sample_batch: member {m}: coarse (t_step, s_step) = "
+                                              f"{(coarse(op).t_step, coarse(op).s_step)} differs from member 0's "
+                                              f"{(coarse(op0).t_step, coarse(op0).s_step)}")
+        dev = sf0._compute_device(noise)
+        key = ident + (str(dev),)
+        if same and hit[0] == key:
+            hit[2].refresh_engine()  # catches in-place parameter updates, as AbstractScoreFunction.runtime does
+            return hit[2]
+        if sf0.likelihood is not None and conds is None:  # the same conditionings on another device
+            conds = [condition_for(lk, shape) for lk in likes]
+        rt = None
+        if hit is not None and hit[0] == key:
+            rt = hit[2]  # the same members and geometry: keep the runtime (and engine), rebuild the conditioning
+            rt.refresh_engine()
+        if rt is None:
+            plan = make_plan(L, k, 0, 1)
+            mw = sf0.max_windows or sf0._default_windows(M * plan.n_win_global)
+            rt = _Runtime(sf0, *shape, dev, plan, mw, members=M)
+        rt.set_condition(conds)
+        self._batch_cache = (key, likes, rt, score_fns)  # the score functions stay alive: their ids stay theirs
+        return rt
+
     def _draw_seed(self, corrections: int) -> int:
         """The corrector seed of a run without one: one draw from the global generator when the corrector draws its
         noise on chip, else 0.  rng == "reference" replays the reference's draws (z.normal_() only,
@@ -116,12 +237,14 @@ class SDAPipeline:
         return 0
 
     def _sample_resident(self, sf: AbstractScoreFunction, noise: Tensor, steps: int, corrections: int, tau: float,
-                         device, show_progressbar: bool, seed, proc_x0=None, members: int = 0) -> Optional[Tensor]:
-        """The sampler on the resident state: one trajectory (`seed` an int or None), or an ensemble of `members`
-        (`seed` a list of M ints or None)."""
+                         device, show_progressbar: bool, seed, proc_x0=None, members: int = 0,
+                         rt: Optional[_Runtime] = None) -> Optional[Tensor]:
+        """The sampler on the resident state: one trajectory (`seed` an int or None), or an ensemble or batch of
+        `members` (`seed` a list of M ints or None; a batch passes its runtime)."""
         if device is not None and torch.device(device).type == "cuda":
             sf.device = torch.device(device)
-        rt = sf.runtime(noise, members=members)
+        if rt is None:
+            rt = sf.runtime(noise, members=members)
         group = sf.shard[2] if sf.shard else None
         rt.reset_finite_check()
         rt.load(noise)

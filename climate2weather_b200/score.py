@@ -337,6 +337,82 @@ def _plan_runs(op: PointObservation, std, key, sel, mask, yv, C: int) -> tuple:
     return uk // n_cls, ysum, wsum, std2
 
 
+def concat_point_plans(plans: Sequence[dict]) -> dict:
+    """One point plan of a batch of independent problems stored member-major from each member's own plan (point_plan
+    over that member's frames [0, L)): member m's slots are offset by the slot count of the members before it, the
+    frame_slot arrays (-1 kept) and the CSR strip_off (member m's entry offsets shifted by the entries before it) are
+    concatenated, and so are the entries (pix, ysum, wsum, std2 where every plan has it).  A member's entries are then
+    byte for byte those of its own plan; a member without an unmasked observation contributes no slot."""
+    slots = entries = 0
+    frame_slot, strip_off = [], [np.zeros(1, dtype=np.int32)]
+    for pl in plans:
+        fs = np.asarray(pl["frame_slot"], dtype=np.int32)
+        frame_slot.append(np.where(fs >= 0, fs + slots, fs).astype(np.int32))
+        strip_off.append((np.asarray(pl["strip_off"][1:], dtype=np.int64) + entries).astype(np.int32))
+        slots += int(pl["n_slots"])
+        entries += int(pl["strip_off"][-1])
+    out = dict(frame_slot=np.concatenate(frame_slot), strip_off=np.concatenate(strip_off), n_slots=slots,
+               strip_rows=plans[0]["strip_rows"], n_strips=plans[0]["n_strips"])
+    names = ("pix", "ysum", "wsum") + (("std2",) if all("std2" in pl for pl in plans) else ())
+    for n in names:
+        out[n] = np.concatenate([np.asarray(pl[n]) for pl in plans])
+    return out
+
+
+def batch_condition(conds: Sequence[dict], shape) -> dict:
+    """The device operands of a batch of independent problems (SDAPipeline.sample_batch) from each member's own
+    conditioning (condition_for), as host arrays, each in the form the member's own run hands its kernel:
+
+    - "y": the coarse term's observations stacked member-major, [M ceil(L / t), C, H / s, W / s] fp32 (None without a
+      coarse term); "coarse_std2": a per-observation tile std^2 block in the same layout, or None;
+    - "plan": the point term's plans, one per member over its frames [0, L), concatenated (concat_point_plans), or None;
+    - "gamma", "std2", "point_std2": [M, C] fp32 per member and variable; the per-variable std^2 is fp32(std^2) as the
+      member's own run rounds it (std2 / point_std2 None with a std per observation).
+
+    When any member has a std per observation the batch runs the per-observation kernels: every other member's
+    per-variable std is expanded to its observations (the same fp32 std^2, and with one std per (pixel, variable) the
+    point entries merge exactly as without a std)."""
+    L, C, H, W = (int(v) for v in shape)
+    M = len(conds)
+    op0 = conds[0]["op"]
+    combined, points = isinstance(op0, CombinedObservation), isinstance(op0, PointObservation)
+    per_obs = any(c.get("obs_std") is not None for c in conds)
+    sq = lambda vals: np.array([np.float64(v) ** 2 for v in vals[:C]], dtype=np.float64).astype(np.float32)
+    out = dict(per_obs=per_obs, kind="combined" if combined else "points" if points else "coarse",
+               gamma=np.array([[float(v) for v in c["gamma"][:C]] for c in conds], dtype=np.float32),
+               std2=None, point_std2=None, y=None, coarse_std2=None, plan=None)
+    if not per_obs:
+        out["std2"] = np.stack([sq(c["std"]) for c in conds])
+        if combined:
+            out["point_std2"] = np.stack([sq(c["point_std"]) for c in conds])
+    if not points:
+        out["y"] = torch.cat([c["y"].to(torch.float32).reshape(-1, C, *c["y"].shape[2:]) for c in conds]).contiguous()
+        if per_obs:
+            blocks = []
+            for c in conds:
+                ob = c.get("obs_std")
+                if ob is not None:
+                    blocks.append(ob["coarse_std2"].to(torch.float32))
+                else:  # per variable: the same fp32 std^2 on each of the member's observation tiles
+                    v = torch.tensor(c["std"][:C], dtype=torch.float32).reshape(1, C, 1, 1)
+                    blocks.append((v * v).expand(c["y"].shape))
+            out["coarse_std2"] = torch.cat(blocks).contiguous()
+    if points or combined:
+        plans = []
+        for c in conds:
+            op, y = (c["op"].points, c["point_y"]) if combined else (c["op"], c["y"])
+            strip, max_pix = (combined_strip_rows(H, W, c["op"].coarse.s_step), COMBINED_STRIP_PIX) if combined \
+                else (point_strip_rows(H, W), POINT_STRIP_PIX)
+            std = None
+            if per_obs:
+                ob = c.get("obs_std")
+                std = ob["point_std"] if ob is not None else \
+                    torch.tensor((c["point_std"] if combined else c["std"])[:C], dtype=torch.float32).reshape(1, C, 1)
+            plans.append(point_plan(op, y, L, C, H, W, 0, L, strip, max_pix, std))
+        out["plan"] = concat_point_plans(plans)
+    return out
+
+
 def _per_channel(v, C: int, name: str):
     """float | Tensor[1,C,1,1] | sequence  ->  4 floats (exp/downscaling.py:218-234)."""
     t = torch.as_tensor(v, dtype=torch.float32).reshape(-1).cpu()
@@ -468,11 +544,26 @@ def observed_windows(win_lo: int, win_hi: int, n_win_global: int, L: int, k: int
     return out
 
 
+def _upload_point_plan(pl: dict, with_std: bool, device, C: int) -> dict:
+    """A point plan on the device: its tensors and the c2w_point_obs that points at them."""
+    names = ("frame_slot", "strip_off", "pix", "ysum", "wsum") + (("std2",) if with_std else ())
+    dev = {n: torch.as_tensor(pl[n]).to(device) for n in names}
+    for n in names[2:]:  # no entries on this rank: still a valid pointer
+        if dev[n].numel() == 0:
+            dev[n] = torch.zeros(max(1, C), dtype=dev[n].dtype, device=device)
+    ob = _lib.PointObs()
+    ob.frame_slot, ob.strip_off, ob.pix = (dev[n].data_ptr() for n in ("frame_slot", "strip_off", "pix"))
+    ob.ysum, ob.wsum = dev["ysum"].data_ptr(), dev["wsum"].data_ptr()
+    ob.n_slots, ob.strip_rows = pl["n_slots"], pl["strip_rows"]
+    return dict(obs=ob, tensors=dev, n_strips=pl["n_strips"])
+
+
 class _Runtime:
     """Device-resident state of one trajectory (or of this rank's time shard of it), or of an ensemble of `members`
     trajectories of L frames stored member-major in one state [members * L, H, W, C] (members = 0: one trajectory).
     An ensemble's plan is that of one member; every kernel call covers all members at once (the *_members entry
-    points), and every member is conditioned on the same observation."""
+    points), and every member is conditioned on the same observation, or, for a batch of independent problems
+    (set_condition with one conditioning per member), on its own (c2w_guided_step_batch)."""
 
     def __init__(self, sf: "AbstractScoreFunction", L: int, C: int, H: int, W: int, device: torch.device,
                  plan: ShardPlan, max_windows: int, exact: bool = False, members: int = 0):
@@ -485,6 +576,7 @@ class _Runtime:
         self.exact = bool(exact)  # exact_grad=True: guidance through the UNet VJP (src/thor/score.py:28-33,51-52)
         self.cond = None
         self.points = None        # PointObservation: this rank's device plan (c2w_point_obs), see set_condition
+        self.batch = None         # a batch of independent problems: its per-member operands, see set_condition
         self._engine_args = (C, 2 * k + 1, H, W, device)
         self._engine_windows = min(max_windows, self.n_windows)
         # an ensemble's convs are planned as a member's own run plans them (its window count per launch): tile width,
@@ -661,6 +753,12 @@ class _Runtime:
         exchange_halos_adjoint(self.vjp, p, group)
 
     def set_condition(self, cond) -> None:
+        """One conditioning (condition_for), None, or for a batch of independent problems (members > 0) a list of
+        every member's own conditioning."""
+        self.batch = None
+        if isinstance(cond, list):
+            self._set_batch_condition(cond)
+            return
         self.cond = cond
         self._sel = None
         self.points = None
@@ -676,16 +774,7 @@ class _Runtime:
             std = obs_std["point_std"] if obs_std is not None else None
             pl = point_plan(op, y, self.L, self.C, self.H, self.W, p.own_lo, p.own_lo + p.own_n, strip, max_pix, std,
                             members=cond.get("members", 0))
-            names = ("frame_slot", "strip_off", "pix", "ysum", "wsum") + (("std2",) if std is not None else ())
-            dev = {n: torch.as_tensor(pl[n]).to(self.device) for n in names}
-            for n in names[2:]:  # no entries on this rank: still a valid pointer
-                if dev[n].numel() == 0:
-                    dev[n] = torch.zeros(max(1, self.C), dtype=dev[n].dtype, device=self.device)
-            ob = _lib.PointObs()
-            ob.frame_slot, ob.strip_off, ob.pix = (dev[n].data_ptr() for n in ("frame_slot", "strip_off", "pix"))
-            ob.ysum, ob.wsum = dev["ysum"].data_ptr(), dev["wsum"].data_ptr()
-            ob.n_slots, ob.strip_rows = pl["n_slots"], pl["strip_rows"]
-            self.points = dict(obs=ob, tensors=dev, n_strips=pl["n_strips"])
+            self.points = _upload_point_plan(pl, std is not None, self.device, self.C)
         if cond is not None and self.exact:
             self.refresh_engine()  # the stashing workspace is sized by the selection
         if cond is not None and not isinstance(cond["op"], PointObservation):
@@ -694,15 +783,42 @@ class _Runtime:
         if obs_std is not None and obs_std["coarse_std2"] is not None:
             self.coarse_std2_dev = obs_std["coarse_std2"].to(device=self.device, dtype=torch.float32).contiguous()
 
+    def _set_batch_condition(self, conds: list) -> None:
+        """A batch of independent problems: member m conditioned on conds[m] (condition_for of its own score function,
+        one family, one coarse (t, s)).  Stacks the coarse blocks, concatenates the point plans and keeps the [M, C]
+        gamma / std^2 arrays on the host (batch_condition), for c2w_guided_step_batch."""
+        if not self.members or len(conds) != self.members:
+            raise ValueError(f"a batch conditioning needs one conditioning per member ({self.members}), got {len(conds)}")
+        b = batch_condition(conds, (self.L, self.C, self.H, self.W))
+        self.cond, self._sel = conds, None
+        f32 = lambda a: None if a is None else \
+            torch.as_tensor(a).to(device=self.device, dtype=torch.float32).contiguous()
+        self.y_dev, self.coarse_std2_dev = f32(b["y"]), f32(b["coarse_std2"])
+        self.points = _upload_point_plan(b["plan"], b["per_obs"], self.device, self.C) if b["plan"] is not None else None
+        op0 = conds[0]["op"]
+        cg = op0.coarse if isinstance(op0, CombinedObservation) else op0 if isinstance(op0, CoarseGrain) else None
+        host = lambda a: None if a is None else (ctypes.c_float * a.size)(*a.reshape(-1).tolist())  # [M, C] fp32
+        self.batch = dict(kind=b["kind"], per_obs=b["per_obs"], gamma=host(b["gamma"]), std2=host(b["std2"]),
+                          point_std2=host(b["point_std2"]), t_step=cg.t_step if cg else 1,
+                          s_step=cg.s_step if cg else None)
+
     def _guide(self, mode: int, mu: float, sigma: float, mu_next: float, sigma_next: float, frames=None) -> None:
         p = self.plan
         g = _lib.Guide()
         g.x, g.eps = self.x.data_ptr(), self.eps.data_ptr()
         s = self.s_tile
         pts = self.points if self.cond is not None else None
-        combined = pts is not None and isinstance(self.cond["op"], CombinedObservation)
-        per_obs = self.cond is not None and self.cond.get("obs_std") is not None  # g.std2 is not read
-        if pts is not None and not combined:  # point observations: y, t_step and s_step are not read
+        bt = self.batch
+        if bt is not None:
+            combined, per_obs = bt["kind"] == "combined", bt["per_obs"]
+        else:
+            combined = pts is not None and isinstance(self.cond["op"], CombinedObservation)
+            per_obs = self.cond is not None and self.cond.get("obs_std") is not None  # g.std2 is not read
+        if bt is not None:  # a batch: every member's y block, std^2 and gamma come from the batch's arrays
+            g.y = self.y_dev.data_ptr() if self.y_dev is not None else None
+            g.t_step = bt["t_step"]
+            s = bt["s_step"] or s
+        elif pts is not None and not combined:  # point observations: y, t_step and s_step are not read
             g.y, g.t_step = None, 1
             for i in range(self.C):
                 g.std2[i] = 1.0 if per_obs else self.cond["std"][i] ** 2
@@ -743,7 +859,14 @@ class _Runtime:
             g.eps_out, g.partials = self.eps_g.data_ptr(), self.partials.data_ptr()
             self._n_part = n_part
         with torch.cuda.device(self.device):
-            if self.members:  # the same operands; the entry point observes every member's frames as one member's
+            if bt is not None:
+                obs = ctypes.byref(pts["obs"]) if pts is not None else None
+                entry = pts["tensors"]["std2"].data_ptr() if (per_obs and pts is not None) else None
+                coarse = self.coarse_std2_dev.data_ptr() if self.coarse_std2_dev is not None else None
+                _lib.check(self.lib.c2w_guided_step_batch(ctypes.byref(g), self.L, bt["gamma"], bt["std2"],
+                                                          bt["point_std2"], obs, coarse, entry, self.stream),
+                           "c2w_guided_step_batch")
+            elif self.members:  # the same operands; the entry point observes every member's frames as one member's
                 obs = ctypes.byref(pts["obs"]) if pts is not None else None
                 pstd2 = (ctypes.c_float * self.C)(*(v ** 2 for v in self.cond["point_std"])) \
                     if (combined and not per_obs) else None
@@ -1016,34 +1139,42 @@ class AbstractScoreFunction:
             args = (self, L, C, H, W, dev, plan, mw)
             rt = _Runtime(*args, exact=exact, members=members) if members else _Runtime(*args, exact=exact)
             if self.likelihood is not None:
-                lk = self.likelihood
-                if lk["op"] is None:
-                    # geometry checks run in point_plan (set_condition) and, for the coarse term, below
-                    if isinstance(lk["A"], (PointObservation, CombinedObservation)):
-                        lk["op"] = lk["A"]
-                    else:
-                        lk["op"] = _recognise_operator(lk["A"], L, C, H, W, lk["y"].shape)
-                    lk["gamma_c"] = _per_channel(lk["gamma"], C, "gamma")
-                op, y = lk["op"], lk["y"]
-                cond = dict(op=op, gamma=lk["gamma_c"])
-                if members:  # the point plan repeats its frame slots per member
-                    cond["members"] = members
-                if isinstance(op, CombinedObservation):  # split and checked against this trajectory's geometry
-                    _check_observation_shape(op.coarse, op.term_shapes(shape)[0], L, C, H, W)
-                    y, cond["point_y"] = op.split(y, shape)
-                    if torch.as_tensor(lk["std"]).numel() in (1, C):
-                        cond["std"], cond["point_std"] = op.std_per_term(lk["std"], shape)
-                    else:
-                        cond.update(_combined_std(op, lk["std"], shape))
-                else:
-                    if isinstance(op, CoarseGrain):  # checked against this trajectory's geometry, every time
-                        y = coarse_grain_observation(op, y, L, C, H, W)
-                    cond.update(_single_std(op, lk["std"], y.shape, C))
-                rt.set_condition(dict(cond, y=y))
+                rt.set_condition(condition_for(self.likelihood, shape, members))
             self._runtimes = {key: rt}  # one live trajectory geometry at a time
         else:
             rt.refresh_engine()  # once per score call / sampling run: catches in-place parameter updates
         return rt
+
+
+def condition_for(lk: dict, shape, members: int = 0) -> dict:
+    """The conditioning of a trajectory of shape (L, C, H, W) from a score function's `likelihood` (condition_on): the
+    operator recognised (cached in lk) and checked against the geometry, y in the form the guidance kernels read (a
+    CombinedObservation's split into its terms), gamma and std per variable, or a std per observation ("obs_std").
+    members = M: an ensemble's, whose point plan repeats its frame slots per member."""
+    L, C, H, W = (int(v) for v in shape)
+    if lk["op"] is None:
+        # geometry checks run in point_plan (set_condition) and, for the coarse term, below
+        if isinstance(lk["A"], (PointObservation, CombinedObservation)):
+            lk["op"] = lk["A"]
+        else:
+            lk["op"] = _recognise_operator(lk["A"], L, C, H, W, lk["y"].shape)
+        lk["gamma_c"] = _per_channel(lk["gamma"], C, "gamma")
+    op, y = lk["op"], lk["y"]
+    cond = dict(op=op, gamma=lk["gamma_c"])
+    if members:  # the point plan repeats its frame slots per member
+        cond["members"] = members
+    if isinstance(op, CombinedObservation):  # split and checked against this trajectory's geometry
+        _check_observation_shape(op.coarse, op.term_shapes(shape)[0], L, C, H, W)
+        y, cond["point_y"] = op.split(y, shape)
+        if torch.as_tensor(lk["std"]).numel() in (1, C):
+            cond["std"], cond["point_std"] = op.std_per_term(lk["std"], shape)
+        else:
+            cond.update(_combined_std(op, lk["std"], shape))
+    else:
+        if isinstance(op, CoarseGrain):  # checked against this trajectory's geometry, every time
+            y = coarse_grain_observation(op, y, L, C, H, W)
+        cond.update(_single_std(op, lk["std"], y.shape, C))
+    return dict(cond, y=y)
 
 
 def _single_std(op, std, obs_shape, C: int) -> dict:

@@ -241,6 +241,25 @@ int c2w_reduce_partials(const float* partials, int32_t n, double* sumsq, void* s
  * m's are the m-th of n_members equal segments. */
 int c2w_guided_step_members(const c2w_guide* g, int32_t member_frames, const c2w_point_obs* obs, const float* point_std2,
                             const float* coarse_std2, const float* entry_std2, void* stream);
+/* The guidance step of a batch of independent problems stored member-major like an ensemble: member m (frames
+ * [m * member_frames, (m + 1) * member_frames) from own_lo on) has its own observation, std^2 and gamma, and is updated
+ * bit for bit as c2w_guided_step, c2w_guided_step_points, c2w_guided_step_combined or c2w_guided_step_obs_std update
+ * that member alone with its own operands: the library launches those entry points' kernels once per member, on the
+ * member's slice of every operand.  The argument checks are those of c2w_guided_step_members, plus at least one term;
+ * g->std2 and g->gamma are ignored.  Per member and variable (HOST arrays [M, C], M = own_n / member_frames):
+ *   gamma       required;
+ *   std2        the coarse term's std^2 (or a point term's alone) per variable; NULL with a std per observation;
+ *   point_std2  a coarse and a point term: the point term's std^2 per variable; else NULL.
+ * Coarse term: g->y is the [M * ceil(member_frames / t_step), C, H / s_step, W / s_step] block, member m's y at rows
+ * [m * ceil(member_frames / t_step), (m + 1) * ceil(member_frames / t_step)); coarse_std2 (a std per observation,
+ * device) has y's layout.  Point term: obs is the concatenation of every member's own plan (c2w_point_obs over that
+ * member's frames): frame_slot [M * member_frames] names member m's slots, offset by the slot count of the members
+ * before it, strip_off is the concatenated CSR with member m's entry offsets shifted, and the entries (pix, ysum, wsum,
+ * entry_std2) are concatenated.  Mode 1 writes the partials in (frame, strip) order, member m's in the m-th of M equal
+ * segments (c2w_reduce_partials_members). */
+int c2w_guided_step_batch(const c2w_guide* g, int32_t member_frames, const float* gamma, const float* std2,
+                          const float* point_std2, const c2w_point_obs* obs, const float* coarse_std2,
+                          const float* entry_std2, void* stream);
 /* sumsq[m] = the sum of partials [m * member_partials, (m + 1) * member_partials), m < n_members, each summed exactly as
  * c2w_reduce_partials sums that segment alone. */
 int c2w_reduce_partials_members(const float* partials, int32_t n_members, int32_t member_partials, double* sumsq,
