@@ -138,6 +138,8 @@ SIGNATURES = {
     "c2w_guided_step_members": (_i, [C.POINTER(Guide), C.c_int32, C.POINTER(PointObs), C.POINTER(C.c_float), _vp, _vp,
                                      _vp]),
     "c2w_guided_step_batch": (_i, [C.POINTER(Guide), C.c_int32, _vp, _vp, _vp, C.POINTER(PointObs), _vp, _vp, _vp]),
+    "c2w_x0_nchw": (_i, [_vp, _vp, _f, _f, _vp, _i64, C.c_int32, C.c_int32, _vp]),
+    "c2w_guided_step_dense": (_i, [C.POINTER(Guide), _vp, _vp]),
     "c2w_reduce_partials_members": (_i, [_vp, C.c_int32, C.c_int32, _vp, _vp]),
     "c2w_corrector_update_members": (_i, [_vp, _vp, _vp, _d, _f, _f, C.c_int32, _i64, C.c_int32, _vp, C.c_uint32, _vp,
                                           _vp]),

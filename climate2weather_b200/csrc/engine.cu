@@ -2246,6 +2246,33 @@ int c2w_guided_step_batch(const c2w_guide* g, int32_t member_frames, const float
   return C2W_OK;
 }
 
+int c2w_x0_nchw(const float* x, const float* eps, float mu, float sigma, float* x0_out, int64_t frames, int32_t C,
+                int32_t hw, void* stream) {
+  C2W_REQUIRE(x && eps && x0_out && frames >= 1 && hw >= 1, "c2w_x0_nchw: bad argument");
+  C2W_REQUIRE(C >= 1 && C <= C2W_MAX_VARS, "c2w_x0_nchw: 1 to %d variables per frame (got %d)", C2W_MAX_VARS, C);
+  return launch_for_vars(C, [&](auto vars) {
+    x0_nchw_kernel<decltype(vars)::value><<<grid_for(frames * hw, 256, c2w_num_sms()), 256, 0,
+                                            static_cast<cudaStream_t>(stream)>>>(x, eps, mu, sigma, x0_out, frames, hw);
+  });
+}
+
+int c2w_guided_step_dense(const c2w_guide* g, const float* grad_nchw, void* stream) {
+  C2W_REQUIRE(g && grad_nchw, "c2w_guided_step_dense: bad argument");
+  C2W_REQUIRE(g->mode == 0 || g->mode == 1,
+              "c2w_guided_step_dense: modes 0 and 1 only (mode 2's cotangent is grad_nchw itself: c2w_traj_pack)");
+  C2W_REQUIRE(g->halo == nullptr, "c2w_guided_step_dense: not time-sharded (halo must be NULL)");
+  C2W_REQUIRE(g->H >= 1 && g->W >= 1, "c2w_guided_step_dense: empty %dx%d grid", g->H, g->W);
+  GuideParams p;
+  int C;
+  int rc = guide_params(g, "c2w_guided_step_dense", p, C);
+  if (rc) return rc;
+  const int strip = std::max(1, std::min(g->H, C2W_POINT_STRIP_PIX / g->W));  // point_strip_rows
+  dim3 grid((g->H + strip - 1) / strip, g->own_n);
+  return launch_for_vars(C, [&](auto vars) {
+    guided_dense_kernel<decltype(vars)::value><<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(p, grad_nchw, strip);
+  });
+}
+
 int c2w_reduce_partials(const float* partials, int32_t n, double* sumsq, void* stream) {
   C2W_REQUIRE(partials && sumsq && n >= 1, "c2w_reduce_partials: bad argument");
   reduce_partials_kernel<<<1, 256, 0, static_cast<cudaStream_t>(stream)>>>(partials, n, sumsq);

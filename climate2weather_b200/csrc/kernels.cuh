@@ -1859,6 +1859,54 @@ __global__ void __launch_bounds__(256) guided_points_kernel(const GuideParams p,
   guide_tail<C>(p, point_strip<C, PerObs>(p, q, slot, v.entry), fbase);
 }
 
+// ---- K6g: any differentiable observation operator.  The host evaluates A and its VJP in torch on x0 (c2w_x0_nchw
+// writes x0 as NCHW) and hands the dense likelihood cotangent g = A^T((y - A x0)/var) in, fp32 NCHW [own_n, C, H, W];
+// this kernel is the guidance + predictor pass of guide_tail on it.  CTA = a strip of strip_rows full rows of one owned
+// frame (point_strip_rows); thread i reads g of its pixel per variable, coalesced over the strip.
+template <int C>
+struct DenseObs {
+  const float* grad;  // this frame's g: [C, H W]
+  long long hw, pix0;
+  int npix;
+  __device__ int first() const { return threadIdx.x; }
+  __device__ int end() const { return npix; }
+  __device__ int step() const { return blockDim.x; }
+  __device__ long long pixel(int i) const { return pix0 + i; }
+  __device__ Vars<C> g(const GuideParams&, int i, long long) const {
+    Vars<C> r;
+#pragma unroll
+    for (int c = 0; c < C; ++c) r[c] = __ldg(grad + c * hw + pix0 + i);
+    return r;
+  }
+};
+
+template <int C>
+__global__ void __launch_bounds__(256) guided_dense_kernel(const GuideParams p, const float* __restrict__ grad_nchw,
+                                                           int strip_rows) {
+  const long long hw = static_cast<long long>(p.H) * p.W;
+  const int h0 = blockIdx.x * strip_rows;
+  const DenseObs<C> obs{grad_nchw + static_cast<long long>(blockIdx.y) * C * hw, hw, static_cast<long long>(h0) * p.W,
+                        min(strip_rows, p.H - h0) * p.W};
+  guide_tail<C>(p, obs, static_cast<long long>(p.own_lo + blockIdx.y) * hw);
+}
+
+// x0 = (x - sigma eps) / mu of the state [F, H W, C] into NCHW [F, C, H W] (the tensor the generic operator A is called
+// on), rounded as the reference's `(x - sigma * eps) / mu` rounds it: a product, a difference and a division, each to
+// fp32.  One thread per pixel; the C stores of a warp are coalesced per variable.
+template <int C>
+__global__ void x0_nchw_kernel(const float* __restrict__ x, const float* __restrict__ eps, float mu, float sigma,
+                               float* __restrict__ out, long long F, int hw) {
+  const long long total = F * hw;
+  for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
+       idx += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long f = idx / hw;
+    const int pix = static_cast<int>(idx - f * hw);
+    const Vars<C> xv = load_vars<C>(x + idx * C), ev = load_vars<C>(eps + idx * C);
+#pragma unroll
+    for (int c = 0; c < C; ++c) out[(f * C + c) * hw + pix] = __fdiv_rn(__fsub_rn(xv[c], __fmul_rn(sigma, ev[c])), mu);
+  }
+}
+
 // ---- K6c: a coarse field and point observations in one likelihood (CombinedObservation).  The cotangent is the sum
 // of the two terms' own, g = A_c^T((y_c - A_c x0)/var_c) + A_p^T((y_p - A_p x0)/var_p), each with its own std^2 per
 // variable (the point term's in PointStd2, gamma shared).  CTA = a strip of q.strip_rows full rows of one owned frame,

@@ -119,7 +119,8 @@ class SDAPipeline:
         (the same on every member).  `seeds`, `proc_x0`, `trace_at` and `nan_check_every` behave as in
         `sample_ensemble`, and `sample_batch([sf] * M, ...)` equals `sample_ensemble(sf, ...)`.  The members must share
         the ScoreUNet object, markov_order, the windows per launch, the operator family (all CoarseGrain, all
-        PointObservation or all CombinedObservation), the coarse term's (t_step, s_step), and whether they are
+        PointObservation, all CombinedObservation, or all generic: each member then runs its own A, y, std and gamma
+        through torch's VJP), the coarse term's (t_step, s_step), and whether they are
         conditioned at all; closed-form guidance only (exact_grad=False), not time-sharded, and not with
         `rng = "reference"` corrections.  A disagreement raises before any device work, naming the member."""
         score_fns = list(score_fns)

@@ -3,10 +3,12 @@ DefaultScoreFunction, BatchedScoreFunction — same constructors, `condition_on`
 
 What differs is where the work happens: the trajectory lives in HBM as fp32 [frames, H, W, C]; unfold, the UNet,
 the centre-pick compose, the likelihood guidance and the predictor/corrector updates are CUDA kernels behind
-include/c2w_b200.h.  Nothing here computes on the CPU and nothing falls back to torch ops.
+include/c2w_b200.h.  Nothing here computes on the CPU and nothing falls back to torch ops; the one computation torch
+runs is a user's own observation operator A and its VJP on the generic observation path (GenericObservation).
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes
 import math
 from typing import Callable, Optional, Sequence, Union
@@ -520,6 +522,77 @@ def _recognise_operator(A: Callable, L: int, C: int, H: int, W: int, y_shape) ->
                               "guidance kernel supports only that family (pass climate2weather_b200.CoarseGrain)")
 
 
+class GenericObservation:
+    """The operator record of the generic observation path: a differentiable callable `A` that is none of the operators
+    the fused guidance kernels implement.  Each score evaluation runs the reference's log_p through it
+    (src/thor/score.py:44-60): x0 = (x - sigma eps)/mu, then A and its vector-Jacobian product in torch on the device,
+    g = A^T((y - A x0)/var), then the fused guidance and state update on g (c2w_guided_step_dense)."""
+
+    def __init__(self, A: Callable):
+        self.A = A
+
+    def __repr__(self):
+        return f"GenericObservation({self.A!r})"
+
+
+def _route_operator(A: Callable, L: int, C: int, H: int, W: int, y_shape):
+    """The operator record of `A` for a trajectory [L, C, H, W] and an observation of y_shape.  PointObservation and
+    CombinedObservation as they are, a CoarseGrain checked by `_recognise_operator` (its errors raise).  Any other
+    callable is recognised as the coarse family if it can be and the fused kernel runs its (t, s); otherwise (y not
+    4-D, not a tile average, no (t, s) matching, (t, s) outside the kernel's limits, or A failing on the CPU probe) it
+    takes the generic path."""
+    if isinstance(A, (PointObservation, CombinedObservation)):
+        return A
+    if isinstance(A, CoarseGrain):
+        return _recognise_operator(A, L, C, H, W, y_shape)
+    if len(y_shape) != 4:
+        return GenericObservation(A)
+    try:
+        return _recognise_operator(A, L, C, H, W, y_shape)
+    except Exception:  # not recognised, outside the kernel's limits, or A cannot run on a CPU tensor
+        return GenericObservation(A)
+
+
+def _generic_autograd() -> contextlib.ExitStack:
+    """The mode A and its VJP run in: autograd on (also inside a caller's no_grad or inference_mode) and fp32 (also
+    inside a caller's autocast, as the reference driver's `fabric.autocast()`)."""
+    stack = contextlib.ExitStack()
+    stack.enter_context(torch.inference_mode(False))
+    stack.enter_context(torch.enable_grad())
+    stack.enter_context(torch.autocast("cuda", enabled=False))
+    return stack
+
+
+def generic_operands(A: Callable, y, std, gamma, x: Tensor) -> dict:
+    """The operands of the generic observation path for trajectories shaped like x ([L, C, H, W] fp32 on the compute
+    device): A evaluated once on x for the shape of A(x); y, std^2 (fp32(std) * fp32(std)) and gamma as fp32 tensors on
+    x's device that broadcast to that shape.  A raising is re-raised naming this path; y, std or gamma not broadcasting
+    raises ValueError naming both shapes."""
+    with _generic_autograd():
+        try:
+            out = A(x)
+        except Exception as e:
+            raise RuntimeError(f"generic observation path: A raised {type(e).__name__} on an fp32 tensor of shape "
+                               f"{list(x.shape)} on {x.device}: {e}") from e
+        if not isinstance(out, Tensor):
+            raise TypeError(f"generic observation path: A returned {type(out).__name__}, not a tensor")
+        shape = tuple(out.shape)
+        ops = dict(A=A, shape=shape)
+        for name, v in (("y", y), ("std", std), ("gamma", gamma)):
+            t = torch.as_tensor(v).to(device=x.device, dtype=torch.float32)
+            try:
+                ok = torch.broadcast_shapes(tuple(t.shape), shape) == shape
+            except RuntimeError:
+                ok = False
+            if not ok:
+                raise ValueError(f"generic observation path: {name} of shape {tuple(t.shape)} does not broadcast to "
+                                 f"A(x) of shape {shape} for a trajectory of {list(x.shape)}")
+            ops[name] = t
+        std = ops.pop("std")
+        ops["std2"] = std * std
+    return ops
+
+
 def observed_windows(win_lo: int, win_hi: int, n_win_global: int, L: int, k: int, t_step) -> list:
     """Windows j in [win_lo, win_hi) whose part of the composed score meets an OBSERVED frame.  The likelihood's cotangent
     g = A^T((y - A x0)/var) (src/thor/score.py:53-56) is non-zero on observed frames only — frame f with f % t_step == 0
@@ -577,6 +650,9 @@ class _Runtime:
         self.cond = None
         self.points = None        # PointObservation: this rank's device plan (c2w_point_obs), see set_condition
         self.batch = None         # a batch of independent problems: its per-member operands, see set_condition
+        self.generic = None       # GenericObservation: every member's operands (generic_operands), see set_condition
+        self._x0 = self._grad = None  # the generic path's x0 and cotangent g, fp32 NCHW over the updated frames
+        self._grad_ready = False      # g is that of the current score evaluation
         self._engine_args = (C, 2 * k + 1, H, W, device)
         self._engine_windows = min(max_windows, self.n_windows)
         # an ensemble's convs are planned as a member's own run plans them (its window count per launch): tile width,
@@ -653,6 +729,8 @@ class _Runtime:
         """Global indices of this rank's windows whose OUTPUT carries a non-zero cotangent (see `observed_windows`)."""
         p = self.plan
         op = self.cond["op"]
+        if isinstance(op, GenericObservation):  # an arbitrary A may read any frame: every window
+            return list(range(p.win_lo, p.win_hi))
         if isinstance(op, CombinedObservation):
             obs = op.observed_frames(self.L, self.C)
         else:
@@ -719,6 +797,7 @@ class _Runtime:
         """eps <- composed window score of x at time t (src/thor/score.py:90-93 / :156-185).  With exact_grad the
         likelihood cotangent is pushed back through the same windows chunk by chunk: vjp <- J_eps^T g."""
         p = self.plan
+        self._grad_ready = False
         if self.members:  # every member's windows, chunked by the workspace: a launch may hold several members'
             self.engine.window_score_members(self.x, self.members, self.L, 0, self.n_windows, t, self.eps)
             return
@@ -762,6 +841,14 @@ class _Runtime:
         self.cond = cond
         self._sel = None
         self.points = None
+        self.generic = None
+        self._grad_ready = False
+        if cond is not None and isinstance(cond["op"], GenericObservation):
+            ops = self._generic_operands(cond)
+            self.generic = [ops] * max(1, self.members)  # an ensemble: every member on the same observation
+            if self.exact:
+                self.refresh_engine()  # the stashing workspace is sized by the selection
+            return
         # a std per observation (cond["obs_std"]): the coarse std^2 block next to y_dev, the point std in the plan
         obs_std = cond.get("obs_std") if cond is not None else None
         if cond is not None and isinstance(cond["op"], (PointObservation, CombinedObservation)):
@@ -789,6 +876,16 @@ class _Runtime:
         gamma / std^2 arrays on the host (batch_condition), for c2w_guided_step_batch."""
         if not self.members or len(conds) != self.members:
             raise ValueError(f"a batch conditioning needs one conditioning per member ({self.members}), got {len(conds)}")
+        self.generic, self._grad_ready = None, False
+        if isinstance(conds[0]["op"], GenericObservation):  # one family: every member's own A, y, std and gamma
+            ops = []
+            for m, c in enumerate(conds):
+                try:
+                    ops.append(self._generic_operands(c))
+                except (ValueError, RuntimeError, TypeError) as e:
+                    raise type(e)(f"sample_batch: member {m}: {e}") from e
+            self.cond, self._sel, self.points, self.generic = conds, None, None, ops
+            return
         b = batch_condition(conds, (self.L, self.C, self.H, self.W))
         self.cond, self._sel = conds, None
         f32 = lambda a: None if a is None else \
@@ -802,6 +899,38 @@ class _Runtime:
                           point_std2=host(b["point_std2"]), t_step=cg.t_step if cg else 1,
                           s_step=cg.s_step if cg else None)
 
+    def _generic_operands(self, cond: dict) -> dict:
+        """generic_operands of a GenericObservation conditioning, A evaluated once on an [L, C, H, W] fp32 tensor of the
+        compute device."""
+        with torch.cuda.device(self.device), torch.inference_mode(False):
+            probe = torch.zeros(self.L, self.C, self.H, self.W, dtype=torch.float32, device=self.device)
+            return generic_operands(cond["op"].A, cond["y"], cond["std"], cond["gamma"], probe)
+
+    def _generic_grad(self, mu: float, sigma: float) -> Tensor:
+        """The generic path's likelihood cotangent g = A^T((y - A x0)/var) of the updated frames, fp32 NCHW, once per
+        score evaluation: x0 by c2w_x0_nchw, then A and its VJP in torch on every member's [L, C, H, W] slice, gathered
+        member-major.  var = std^2 + gamma (sigma/mu)^2 with sigma/mu rounded to fp32, as the reference computes it from
+        fp32 schedule tensors.  Everything runs on the runtime's stream, without a host synchronisation."""
+        if self._grad_ready:
+            return self._grad
+        lo, n = self.own
+        with torch.cuda.device(self.device), _generic_autograd():
+            if self._x0 is None:  # outside inference mode: A's backward may save it
+                self._x0 = torch.empty(n, self.C, self.H, self.W, dtype=torch.float32, device=self.device)
+                self._grad = torch.empty_like(self._x0)
+            frame = self.H * self.W * self.C
+            _lib.check(self.lib.c2w_x0_nchw(self.x.data_ptr() + 4 * lo * frame, self.eps.data_ptr() + 4 * lo * frame,
+                                            mu, sigma, self._x0.data_ptr(), n, self.C, self.H * self.W, self.stream),
+                       "c2w_x0_nchw")
+            r2 = float((torch.tensor(sigma, dtype=torch.float32) / torch.tensor(mu, dtype=torch.float32)) ** 2)
+            for m, ops in enumerate(self.generic):
+                part = slice(m * self.L, (m + 1) * self.L) if self.members else slice(0, n)
+                ax, pullback = torch.func.vjp(ops["A"], self._x0[part])
+                (g,) = pullback((ops["y"] - ax) / (ops["std2"] + ops["gamma"] * r2))
+                self._grad[part].copy_(g)
+        self._grad_ready = True
+        return self._grad
+
     def _guide(self, mode: int, mu: float, sigma: float, mu_next: float, sigma_next: float, frames=None) -> None:
         p = self.plan
         g = _lib.Guide()
@@ -809,12 +938,19 @@ class _Runtime:
         s = self.s_tile
         pts = self.points if self.cond is not None else None
         bt = self.batch
-        if bt is not None:
+        gen = self.generic
+        if gen is not None and frames is not None:
+            raise NotImplementedError("the generic observation path updates every owned frame at once")
+        if gen is not None:
+            combined = per_obs = False
+        elif bt is not None:
             combined, per_obs = bt["kind"] == "combined", bt["per_obs"]
         else:
             combined = pts is not None and isinstance(self.cond["op"], CombinedObservation)
             per_obs = self.cond is not None and self.cond.get("obs_std") is not None  # g.std2 is not read
-        if bt is not None:  # a batch: every member's y block, std^2 and gamma come from the batch's arrays
+        if gen is not None:  # g is computed in torch (_generic_grad): y, std2, gamma, t_step and s_step are not read
+            g.y, g.t_step = None, 1
+        elif bt is not None:  # a batch: every member's y block, std^2 and gamma come from the batch's arrays
             g.y = self.y_dev.data_ptr() if self.y_dev is not None else None
             g.t_step = bt["t_step"]
             s = bt["s_step"] or s
@@ -851,13 +987,28 @@ class _Runtime:
                 g.halo = ph.handle
                 self._halo_pushed = True
         if mode == 1:
-            n_part = g.own_n * (pts["n_strips"] if pts is not None else self.H // s)
+            strips = -(-self.H // point_strip_rows(self.H, self.W)) if gen is not None else \
+                pts["n_strips"] if pts is not None else self.H // s
+            n_part = g.own_n * strips
             if self.partials is None or self.partials.numel() < n_part:
                 self.partials = torch.zeros(n_part, dtype=torch.float32, device=self.device)
             if self.eps_g is None:
                 self.eps_g = torch.zeros_like(self.x)
             g.eps_out, g.partials = self.eps_g.data_ptr(), self.partials.data_ptr()
             self._n_part = n_part
+        if gen is not None:
+            grad = self._generic_grad(mu, sigma)
+            with torch.cuda.device(self.device):
+                if mode == 2:  # the cotangent fed to the UNet VJP is g itself, in the state layout
+                    lo = g.own_lo * self.H * self.W * self.C
+                    _lib.check(self.lib.c2w_traj_pack(grad.data_ptr(), self.cot.data_ptr() + 4 * lo, g.own_n, self.C,
+                                                      self.H * self.W, self.stream), "c2w_traj_pack")
+                else:
+                    _lib.check(self.lib.c2w_guided_step_dense(ctypes.byref(g), grad.data_ptr(), self.stream),
+                               "c2w_guided_step_dense")
+            if mode == 0:  # x moved: the next g needs a new score evaluation
+                self._grad_ready = False
+            return
         with torch.cuda.device(self.device):
             if bt is not None:
                 obs = ctypes.byref(pts["obs"]) if pts is not None else None
@@ -1126,6 +1277,11 @@ class AbstractScoreFunction:
         if members and self.shard:
             raise NotImplementedError("ensemble sampling does not run on a time-sharded score function "
                                       "(enable_time_sharding); run one ensemble per rank instead")
+        if self.shard and self.likelihood is not None and \
+                isinstance(_operator_for(self.likelihood, L, C, H, W), GenericObservation):
+            raise NotImplementedError(f"the generic observation path (A = {self.likelihood['A']!r}, an operator the "
+                                      f"fused guidance kernels do not implement) does not run on a time-sharded score "
+                                      f"function (enable_time_sharding): A sees the whole trajectory")
         dev = self._compute_device(x)
         rank, world = (self.shard[0], self.shard[1]) if self.shard else (0, 1)
         key = (L, C, H, W, str(dev), rank, world, exact, members)
@@ -1152,14 +1308,9 @@ def condition_for(lk: dict, shape, members: int = 0) -> dict:
     CombinedObservation's split into its terms), gamma and std per variable, or a std per observation ("obs_std").
     members = M: an ensemble's, whose point plan repeats its frame slots per member."""
     L, C, H, W = (int(v) for v in shape)
-    if lk["op"] is None:
-        # geometry checks run in point_plan (set_condition) and, for the coarse term, below
-        if isinstance(lk["A"], (PointObservation, CombinedObservation)):
-            lk["op"] = lk["A"]
-        else:
-            lk["op"] = _recognise_operator(lk["A"], L, C, H, W, lk["y"].shape)
-        lk["gamma_c"] = _per_channel(lk["gamma"], C, "gamma")
-    op, y = lk["op"], lk["y"]
+    op, y = _operator_for(lk, L, C, H, W), lk["y"]
+    if isinstance(op, GenericObservation):  # y, std and gamma as given, checked against A(x) at runtime set-up
+        return dict(op=op, y=y, std=lk["std"], gamma=lk["gamma"])
     cond = dict(op=op, gamma=lk["gamma_c"])
     if members:  # the point plan repeats its frame slots per member
         cond["members"] = members
@@ -1175,6 +1326,17 @@ def condition_for(lk: dict, shape, members: int = 0) -> dict:
             y = coarse_grain_observation(op, y, L, C, H, W)
         cond.update(_single_std(op, lk["std"], y.shape, C))
     return dict(cond, y=y)
+
+
+def _operator_for(lk: dict, L: int, C: int, H: int, W: int):
+    """The operator record of a score function's `likelihood` (`_route_operator`), cached in lk with the per-variable
+    gamma of the fused operators."""
+    if lk["op"] is None:
+        # geometry checks run in point_plan (set_condition) and, for the coarse term, in condition_for
+        lk["op"] = _route_operator(lk["A"], L, C, H, W, lk["y"].shape)
+        if not isinstance(lk["op"], GenericObservation):
+            lk["gamma_c"] = _per_channel(lk["gamma"], C, "gamma")
+    return lk["op"]
 
 
 def _single_std(op, std, obs_shape, C: int) -> dict:

@@ -260,6 +260,19 @@ int c2w_guided_step_members(const c2w_guide* g, int32_t member_frames, const c2w
 int c2w_guided_step_batch(const c2w_guide* g, int32_t member_frames, const float* gamma, const float* std2,
                           const float* point_std2, const c2w_point_obs* obs, const float* coarse_std2,
                           const float* entry_std2, void* stream);
+/* Any differentiable observation operator A (the reference's condition_on with an arbitrary callable): the host
+ * evaluates A and its vector-Jacobian product on x0 and hands the dense likelihood cotangent in.
+ * c2w_x0_nchw: x0_out[f, c, pix] = (x[f, pix, c] - sigma * eps[f, pix, c]) / mu, fp32 NCHW [frames, C, hw] from the
+ * state layout, each operation rounded to fp32 as the reference's `(x - sigma * eps) / mu` (C = 1..8). */
+int c2w_x0_nchw(const float* x, const float* eps, float mu, float sigma, float* x0_out, int64_t frames, int32_t C,
+                int32_t hw, void* stream);
+/* The guidance step of c2w_guided_step with the cotangent g = A^T((y - A x0)/var) already computed: grad_nchw is fp32
+ * NCHW [own_n, C, H, W], g of local frame f at grad_nchw[((f - own_lo) * C + c) * H * W + pixel].  Modes 0 and 1, with
+ * or without vjp; mode 2 is refused (pack grad_nchw with c2w_traj_pack instead).  g->y, std2, gamma, t_step and s_step
+ * are not read; halo must be NULL.  CTA = a strip of max(1, min(H, C2W_POINT_STRIP_PIX / W)) rows of one frame: mode 1
+ * writes own_n * ceil(H / strip) partials in (frame, strip) order, so an ensemble's or a batch's members stored
+ * member-major have theirs in equal consecutive segments (c2w_reduce_partials_members). */
+int c2w_guided_step_dense(const c2w_guide* g, const float* grad_nchw, void* stream);
 /* sumsq[m] = the sum of partials [m * member_partials, (m + 1) * member_partials), m < n_members, each summed exactly as
  * c2w_reduce_partials sums that segment alone. */
 int c2w_reduce_partials_members(const float* partials, int32_t n_members, int32_t member_partials, double* sumsq,
