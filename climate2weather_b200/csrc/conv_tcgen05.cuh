@@ -5,9 +5,9 @@
 //   M = pixels (n, h, w flattened, NHWC activations, bf16),
 //   N = output channels, K = taps * Cin  (k index = (r*3 + s) * Cin + c).
 //
-// Feeding:   A is never materialised.  Generic path: for filter tap (r, s) the 128-pixel A tile (whole output rows)
-//            is a SHIFTED BOX of the NHWC input: one 4-D TMA load {64 ch, W, tile_h, tile_n} at
-//            (c0, s-1, h0+r-1, n0); out-of-bounds rows/columns are zero-filled by the TMA unit, which is exactly
+// Feeding:   A is never materialised.  Generic path: for filter tap (r, s) the 128-pixel A tile (whole output rows,
+//            or one 128-pixel segment of a row wider than 128) is a SHIFTED BOX of the NHWC input: one 4-D TMA load
+//            {64 ch, W or 128, tile_h, tile_n} at (c0, w0+s-1, h0+r-1, n0); out-of-bounds rows/columns are zero-filled by the TMA unit, which is exactly
 //            padding=1 / padding_mode=zeros (configs/sda_unet.yml:16).  Stride-2 convs use the same box with element
 //            strides {1, 2, 2, 1}.  Activation-reuse path (AR; stride-1 convs with 64/128-wide N tiles): the M tile is
 //            a 16 x 8 spatial block and ONE halo'd box [18 rows x 10 px][64 ch] per channel block serves all nine
@@ -117,6 +117,8 @@ struct ConvParams {
   // G mod Nw of member G div Nw, whose frames start at frame G + 2k (G div Nw); head / tail tests are member-local.
   // Last, in the struct's tail padding, so that the fields above keep their offsets.
   int member_win;
+  // Streamed 3x3 main loop: 128-pixel segments per output row (1: tiles of whole rows; Wo / 128 when Wo > 128)
+  int row_segs;
 };
 
 constexpr int kBlockM = 128;
@@ -541,9 +543,10 @@ conv_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
         const int nt = tile % p.num_n_tiles;
         const int mt = (tile / p.num_n_tiles) * CG + rank;
         int b1, b2, b3;
-        if (p.taps == 9) {
-          b1 = 0;
-          b2 = (mt % p.tiles_per_img) * p.tile_h * p.stride;
+        if (p.taps == 9) {  // row segments (Wo > 128): tile = 128-pixel segment tt % row_segs of row tt / row_segs
+          const int tt = mt % p.tiles_per_img;
+          b1 = (tt % p.row_segs) * kBlockM * p.stride;
+          b2 = (tt / p.row_segs) * p.tile_h * p.stride;
           b3 = (mt / p.tiles_per_img) * p.tile_n;
         } else {
           b1 = mt * kBlockM;
@@ -1237,15 +1240,18 @@ inline bool conv_launch_init(ConvLaunch* L, bool is_conv3x3, const __nv_bfloat16
   L->cg = variant < 0 ? conv_pick_cg(p.num_m_tiles) : ((variant & 1) ? 2 : 1);
   L->ar = 0;
   if (is_conv3x3) {
-    if (Wo > kBlockM || kBlockM % Wo != 0) return false;
-    int th = kBlockM / Wo;
+    // streamed M tile: whole output rows of 1..n images (Wo <= 128), or one 128-pixel segment of a row (Wo > 128)
+    const bool segs = Wo > kBlockM;
+    if (segs ? Wo % kBlockM != 0 : kBlockM % Wo != 0) return false;
+    int th = segs ? 1 : kBlockM / Wo;
     if (th > Ho) th = Ho;
     if (Ho % th != 0) return false;
-    const int tn = kBlockM / (Wo * th);
+    const int tn = segs ? 1 : kBlockM / (Wo * th);
     p.taps = 9;
     p.tile_h = th;
     p.tile_n = tn;
-    p.tiles_per_img = Ho / th;
+    p.row_segs = segs ? Wo / kBlockM : 1;
+    p.tiles_per_img = (Ho / th) * p.row_segs;
     // activation reuse: stride-1 convs with 64- or 128-wide N tiles per CTA pair on images that tile into 16 x 8 blocks
     static int ar_ok = -1;
     if (ar_ok < 0) {
@@ -1285,7 +1291,8 @@ inline bool conv_launch_init(ConvLaunch* L, bool is_conv3x3, const __nv_bfloat16
     } else {
       if (variant >= 0 && (variant & 4)) return false;  // AR was requested explicitly but does not apply
       const uint64_t dims[4] = {(uint64_t)cin, (uint64_t)W, (uint64_t)H, (uint64_t)n_img};
-      const uint32_t box[4] = {(uint32_t)kBlockK, (uint32_t)(Wo * stride), (uint32_t)(th * stride), (uint32_t)tn};
+      const uint32_t box[4] = {(uint32_t)kBlockK, (uint32_t)((Wo / p.row_segs) * stride), (uint32_t)(th * stride),
+                               (uint32_t)tn};
       const uint32_t est[4] = {1u, (uint32_t)stride, (uint32_t)stride, 1u};
       if (!make_tmap_bf16(&L->tmA, x, 4, dims, box, est)) return false;
     }

@@ -113,7 +113,6 @@ struct Plan {
   float* emb = nullptr;
   float* mods = nullptr;
   float* out32 = nullptr;
-  size_t attn_smem = 0;
 };
 
 inline int pad64(int c) { return (c + 63) / 64 * 64; }
@@ -318,6 +317,78 @@ int launch_attention_bwd_mma(const bf16* qkv, const bf16* go, bf16* gqkv, int n,
   return C2W_OK;
 }
 
+// Tiled attention (K4t / K8t) for the shapes whose K and V do not fit in shared memory: C a multiple of 64, <= 512.
+#define C2W_FLASH_DISPATCH(C, CALL)                                                                            \
+  switch (C) {                                                                                                 \
+    case 64: return CALL(64);                                                                                  \
+    case 128: return CALL(128);                                                                                \
+    case 192: return CALL(192);                                                                                \
+    case 256: return CALL(256);                                                                                \
+    case 320: return CALL(320);                                                                                \
+    case 384: return CALL(384);                                                                                \
+    case 448: return CALL(448);                                                                                \
+    case 512: return CALL(512);                                                                                \
+    default: return fail(C2W_ERR_INVALID, "attention: T=%d C=%d: the tiled kernels need C a multiple of 64, <= 512", \
+                         T, C);                                                                                \
+  }
+
+template <int C>
+int launch_attention_flash_c(const bf16* qkv, bf16* out, int n, int T, cudaStream_t st) {
+  static unsigned long long done = 0;
+  int rc = ensure_smem(attention_flash_kernel<C>, attention_flash_smem_bytes(C), &done);
+  if (rc) return rc;
+  const dim3 grid((T + kFlashRows - 1) / kFlashRows, C / attention_flash_co(C), n);
+  attention_flash_kernel<C><<<grid, 256, attention_flash_smem_bytes(C), st>>>(qkv, out, T,
+                                                                               1.0f / sqrtf(static_cast<float>(C)));
+  C2W_CUDA(cudaGetLastError());
+  return C2W_OK;
+}
+int launch_attention_flash(const bf16* qkv, bf16* out, int n, int T, int C, cudaStream_t st) {
+#define C2W_CALL(CC) launch_attention_flash_c<CC>(qkv, out, n, T, st)
+  C2W_FLASH_DISPATCH(C, C2W_CALL)
+#undef C2W_CALL
+}
+
+// scratch: fp32 [2][n][T] (log-sum-exp L and D = rowsum(P o gP) per query)
+template <int C>
+int launch_attention_bwd_flash_c(const bf16* qkv, const bf16* go, bf16* gqkv, float* scratch, int n, int T,
+                                 cudaStream_t st) {
+  static unsigned long long done_a = 0, done_b = 0, done_c = 0;
+  int rc = ensure_smem(attention_flash_bwd_q_kernel<C, false>, 0, &done_a);
+  if (!rc) rc = ensure_smem(attention_flash_bwd_q_kernel<C, true>, 0, &done_b);
+  if (!rc) rc = ensure_smem(attention_flash_bwd_kv_kernel<C>, 0, &done_c);
+  if (rc) return rc;
+  const float scale2 = 1.0f / sqrtf(static_cast<float>(C));
+  const int nb = (T + kFlashRows - 1) / kFlashRows, nc = C / attention_flash_co(C);
+  const size_t smq = attention_flash_bwd_q_smem_bytes(C), smkv = attention_flash_bwd_kv_smem_bytes(C);
+  attention_flash_bwd_q_kernel<C, false><<<dim3(nb, 1, n), 256, smq, st>>>(qkv, go, scratch, gqkv, T, n, scale2);
+  C2W_CUDA(cudaGetLastError());
+  attention_flash_bwd_q_kernel<C, true><<<dim3(nb, nc, n), 256, smq, st>>>(qkv, go, scratch, gqkv, T, n, scale2);
+  C2W_CUDA(cudaGetLastError());
+  attention_flash_bwd_kv_kernel<C><<<dim3(nb, nc, n), 256, smkv, st>>>(qkv, go, scratch, gqkv, T, n, scale2);
+  C2W_CUDA(cudaGetLastError());
+  return C2W_OK;
+}
+int launch_attention_bwd_flash(const bf16* qkv, const bf16* go, bf16* gqkv, float* scratch, int n, int T, int C,
+                               cudaStream_t st) {
+#define C2W_CALL(CC) launch_attention_bwd_flash_c<CC>(qkv, go, gqkv, scratch, n, T, st)
+  C2W_FLASH_DISPATCH(C, C2W_CALL)
+#undef C2W_CALL
+}
+
+// The backward runs tiled where the CUDA-core kernels' K, V and score rows do not fit in shared memory (T = 64 at
+// C = 128 / 256 / 512 keeps the tensor-core kernel).  Decided from (T, C) alone, so the plan sizes its scratch with it.
+bool attention_bwd_tiled(int T, int C) {
+  if (T == 64 && (C == 128 || C == 256 || C == 512)) return false;
+  const int QB = std::min(T, kAttnBwdRows);
+  return std::max(attention_bwd_scores_smem(T, C, QB), attention_bwd_grads_smem(T, C, QB)) >
+         static_cast<size_t>(kSmemLimit);
+}
+// fp32 scratch of one attention backward over n windows
+size_t attention_bwd_scratch_floats(int n, int T, int C) {
+  return attention_bwd_tiled(T, C) ? 2 * static_cast<size_t>(n) * T : 2 * static_cast<size_t>(n) * T * T;
+}
+
 int launch_attention_bwd(const bf16* qkv, const bf16* go, bf16* gqkv, float* scratch, int n, int T, int C,
                          cudaStream_t st) {
   C2W_REQUIRE(T % 8 == 0 && C % 8 == 0 && scratch, "attention backward: T %% 8 and C %% 8 must be 0 (T=%d C=%d)", T, C);
@@ -333,10 +404,9 @@ int launch_attention_bwd(const bf16* qkv, const bf16* go, bf16* gqkv, float* scr
       if (C == 128) return launch_attention_bwd_mma<128>(qkv, go, gqkv, n, st);
     }
   }
+  if (attention_bwd_tiled(T, C)) return launch_attention_bwd_flash(qkv, go, gqkv, scratch, n, T, C, st);
   const int QB = std::min(T, kAttnBwdRows);
   const size_t smem1 = attention_bwd_scores_smem(T, C, QB), smem2 = attention_bwd_grads_smem(T, C, QB);
-  C2W_REQUIRE(std::max(smem1, smem2) <= static_cast<size_t>(kSmemLimit),
-              "attention backward: T=%d C=%d needs %zu B of shared memory", T, C, std::max(smem1, smem2));
   static unsigned long long done1 = 0, done2 = 0;
   int rc = ensure_smem(attention_bwd_scores_kernel, smem1, &done1);
   if (rc) return rc;
@@ -390,6 +460,9 @@ int launch_attention(const bf16* qkv, bf16* out, int n, int T, int C, cudaStream
       if (C == 128) return launch_attention_mma<128>(qkv, out, n, st);
     }
   }
+  // K and V of a window and the scores of a 64-query block do not fit in shared memory: tiled kernel.  Decided from
+  // (T, C) alone, never from the window count, so that every chunking of a run computes the same bits.
+  if (attention_smem_bytes(T, C, 64) > static_cast<size_t>(kSmemLimit)) return launch_attention_flash(qkv, out, n, T, C, st);
   // Queries per CTA: the largest block that still gives every SM two CTAs' worth of work (K and V are re-read from L2
   // by every query block of a window, so bigger blocks move less data; smaller ones fill the machine).
   const int sms = c2w_num_sms();
@@ -541,8 +614,7 @@ int build_plan(c2w_handle* h, int n, bool vjp, bool per_t, void* base, size_t* b
     size_t sc = 0;
     for (int l = 0; l < nl; ++l)
       if (h->levels[l].attn) {
-        const size_t T = static_cast<size_t>(h->levels[l].H) * h->levels[l].W;
-        sc = std::max(sc, 2 * static_cast<size_t>(n) * T * T);
+        sc = std::max(sc, attention_bwd_scratch_floats(n, h->levels[l].H * h->levels[l].W, h->levels[l].C));
       }
     attn_scratch = B.take<float>(sc);
     gup = B.take<bf16>(up_elems);    // gradient w.r.t. the upsampled LayerNorm output of a tail
@@ -827,9 +899,6 @@ int build_plan(c2w_handle* h, int n, bool vjp, bool per_t, void* base, size_t* b
           op.T = T;
           op.C = L.C;
           P.ops.push_back(op);
-          P.attn_smem = std::max(P.attn_smem, attention_smem_bytes(op.T, op.C));
-          if (P.attn_smem > static_cast<size_t>(kSmemLimit))
-            return fail(C2W_ERR_INVALID, "attention at level %d (T=%d, C=%d) exceeds shared memory", l, op.T, op.C);
         }
         rc = add_conv(false, att_s, L.H, L.W, L.C, aw.proj, EPI_BIAS_RES, xs[l], false);
         if (rc) return rc;
@@ -1240,9 +1309,13 @@ int c2w_create(const c2w_config* cfg, c2w_handle** out) {
   for (int l = 0; l < cfg->n_levels; ++l) {
     C2W_REQUIRE(cfg->hidden_channels[l] % 64 == 0 && cfg->hidden_channels[l] <= 512,
                 "hidden_channels[%d]=%d: must be a multiple of 64 and <= 512", l, cfg->hidden_channels[l]);
-    C2W_REQUIRE(W >= 8 && W <= 128 && 128 % W == 0 && H >= 1, "level %d: width %d must be a power of two in [8,128]", l, W);
-    const int th = std::min(H, 128 / W);
-    C2W_REQUIRE(H % th == 0 && 128 % (W * th) == 0, "level %d: %dx%d does not tile into 128-pixel row blocks", l, H, W);
+    // the streamed K1 tile is a block of whole rows (a power-of-two width <= 128) or a 128-pixel row segment
+    const bool rows = W >= 8 && W <= 128 && 128 % W == 0 && H >= 1 && H % std::min(H, 128 / W) == 0 &&
+                      128 % (W * std::min(H, 128 / W)) == 0;
+    const bool segments = W % 128 == 0 && W > 128 && H >= 1;
+    C2W_REQUIRE(rows || segments,
+                "level %d: %dx%d: a level's width must be a power of two in [8,128] whose rows tile into 128-pixel "
+                "row blocks, or a multiple of 128", l, H, W);
     if (l + 1 < cfg->n_levels) {
       C2W_REQUIRE(H % 2 == 0 && W % 2 == 0, "level %d: %dx%d not divisible by the stride", l, H, W);
       H /= 2;

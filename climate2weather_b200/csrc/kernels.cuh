@@ -911,6 +911,405 @@ __global__ void __launch_bounds__(256) attention_bwd_mma_kernel(const bf16* __re
   attn_tile_times_slot<C, true>(dst + C, sG, s2, r0, cbase, lane);       // gk = scale2 gS^T q
 }
 
+// ------------------------------------------------------------------------------------------------ K4t / K8t
+// Tiled attention core for shapes whose K and V do not fit in shared memory (e.g. 256 tokens at 512 channels, the
+// shipped network's deepest level at 256 x 256), on the same warp MMAs (bf16 in, fp32 accumulate).  Blocks of 64
+// queries / 64 keys; a CTA of 8 warps owns one query block (forward, dQ) or one key block (dK, dV) and CO output
+// channels (CO = 128 when C % 128 == 0, else 64), so the output accumulators stay at 32 registers per thread; the
+// products over all C channels (scores, go v^T) are recomputed by each of the C / CO channel CTAs.
+//   forward: K and V stream through shared memory, fp32 online softmax (running max and sum per query row)
+//   backward (FlashAttention-2 style, no T x T scratch): K8t-a recomputes each query's log-sum-exp L and
+//   D = rowsum(P o gP) in one pass; K8t-b: gq = scale2 sum_keyblocks gS k; K8t-c: gk, gv summed over query blocks in a
+//   fixed order.  Every output element is written by one CTA: repeats are bit-identical.
+// Rows past T are zero-filled in shared memory and never stored; keys past T are masked out of every softmax.
+constexpr int kFlashRows = 64;
+__host__ __device__ constexpr int attention_flash_co(int C) { return C % 128 == 0 ? 128 : 64; }
+inline size_t attention_flash_smem_bytes(int C) {  // sQ, sK [64, C], sV [64, CO], P tile, alpha / l rows
+  return static_cast<size_t>(2) * kFlashRows * C * 2 + static_cast<size_t>(kFlashRows) * attention_flash_co(C) * 2 +
+         kFlashRows * 128 + 2 * kFlashRows * 4;
+}
+inline size_t attention_flash_bwd_q_smem_bytes(int C) {  // sQ, sgo, slot [64, C], chunk [64, CO], tile, L / D rows
+  return static_cast<size_t>(3) * kFlashRows * C * 2 + static_cast<size_t>(kFlashRows) * attention_flash_co(C) * 2 +
+         kFlashRows * 128 + 2 * kFlashRows * 4;
+}
+inline size_t attention_flash_bwd_kv_smem_bytes(int C) {  // sK, sV, slot [64, C], q chunk, P^T and gS^T tiles, L / D
+  return static_cast<size_t>(3) * kFlashRows * C * 2 + static_cast<size_t>(kFlashRows) * attention_flash_co(C) * 2 +
+         2 * kFlashRows * 128 + 2 * kFlashRows * 4;
+}
+// [64 rows][CH 16-B chunks] swizzled tile <- rows of `src` (row_stride elements apart); rows >= valid are zeroed
+template <int CH>
+__device__ __forceinline__ void flash_tile_load(uint32_t sdst, const bf16* src, int row_stride, int valid, int tid) {
+  for (int idx = tid; idx < kFlashRows * CH; idx += 256) {
+    const int r = idx / CH, cc = idx - r * CH;
+    const uint32_t dst = sdst + r * (CH * 16) + ((cc ^ (r & 7)) << 4);
+    if (r < valid) {
+      const bf16* g = src + static_cast<size_t>(r) * row_stride + cc * 8;
+      asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(g) : "memory");
+    } else {
+      asm volatile("st.shared.v4.b32 [%0], {%1, %1, %1, %1};" ::"r"(dst), "r"(0) : "memory");
+    }
+  }
+  asm volatile("cp.async.commit_group;" ::: "memory");
+}
+__device__ __forceinline__ void flash_wait_sync() {
+  asm volatile("cp.async.wait_group 0;" ::: "memory");
+  __syncthreads();
+}
+// [16 rows r0.. of a 64 x 64 fragment] -> bf16 tile (128 B rows, swizzled chunks)
+__device__ __forceinline__ void flash_store_tile(uint32_t sT, const float (&v)[8][4], int r0, int lane) {
+  const int g = lane >> 2, tq = lane & 3;
+  const int row0 = r0 + g, row1 = r0 + g + 8;
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    asm volatile("st.shared.b32 [%0], %1;" ::"r"(sT + row0 * 128 + ((j ^ (row0 & 7)) << 4) + tq * 4),
+                 "r"(pack_bf16x2(v[j][0], v[j][1])) : "memory");
+    asm volatile("st.shared.b32 [%0], %1;" ::"r"(sT + row1 * 128 + ((j ^ (row1 & 7)) << 4) + tq * 4),
+                 "r"(pack_bf16x2(v[j][2], v[j][3])) : "memory");
+  }
+}
+// acc[NT][4] += M[16 rows r0.. of a 64 x 64 bf16 tile] . X[64 rows][channels c0 .. c0 + 8 NT) (X: XP bytes per row)
+template <int NT>
+__device__ __forceinline__ void flash_tile_mma(float (&acc)[NT][4], uint32_t sM, uint32_t sX, int XP, int r0, int c0,
+                                               int lane) {
+  const int mat = lane >> 3, rr = lane & 7;
+  const int arow = r0 + rr + (mat & 1) * 8;
+#pragma unroll
+  for (int ks = 0; ks < 4; ++ks) {
+    uint32_t a[4];
+    ldmatrix_x4(a, sM + arow * 128 + (((2 * ks + (mat >> 1)) ^ (arow & 7)) << 4));
+    const int key = 16 * ks + rr + (mat & 1) * 8;
+#pragma unroll
+    for (int jp = 0; jp < NT / 2; ++jp) {
+      const int chunk = (c0 >> 3) + 2 * jp + (mat >> 1);
+      uint32_t b[4];
+      ldmatrix_x4_trans(b, sX + key * XP + ((chunk ^ (key & 7)) << 4));
+      mma_bf16_16816(acc[2 * jp], a, b[0], b[1]);
+      mma_bf16_16816(acc[2 * jp + 1], a, b[2], b[3]);
+    }
+  }
+}
+__device__ __forceinline__ float quad_max(float v) {
+  v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 1));
+  return fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 2));
+}
+__device__ __forceinline__ float quad_sum(float v) {
+  v += __shfl_xor_sync(0xffffffffu, v, 1);
+  return v + __shfl_xor_sync(0xffffffffu, v, 2);
+}
+
+// K4t, grid (query blocks, C / CO, windows): out = softmax(scale2 q k^T) v for CO channels of 64 queries.
+template <int C>
+__global__ void __launch_bounds__(256) attention_flash_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out,
+                                                              int T, float scale2) {
+  constexpr int CO = attention_flash_co(C), PQ = C * 2, PV = CO * 2, NT = CO / 16;
+  extern __shared__ __align__(128) uint8_t smraw[];
+  const uint32_t sQ = static_cast<uint32_t>(__cvta_generic_to_shared(smraw));
+  const uint32_t sK = sQ + kFlashRows * PQ, sV = sK + kFlashRows * PQ, sP = sV + kFlashRows * PV;
+  float* s_alpha = reinterpret_cast<float*>(smraw + 2 * kFlashRows * PQ + kFlashRows * PV + kFlashRows * 128);
+  float* s_l = s_alpha + kFlashRows;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, tq = lane & 3;
+  const int q0 = blockIdx.x * kFlashRows, co0 = blockIdx.y * CO;
+  const bf16* base = qkv + static_cast<size_t>(blockIdx.z) * T * 3 * C;
+  const int r0 = 16 * (warp & 3), cbase = (warp >> 2) * (CO / 2);
+  flash_tile_load<C / 8>(sQ, base + static_cast<size_t>(q0) * 3 * C, 3 * C, T - q0, tid);
+  float m0 = -INFINITY, m1 = -INFINITY, l0 = 0.f, l1 = 0.f;  // warps 0-3: running max / sum of rows r0 + g, + 8
+  float o[NT][4];
+#pragma unroll
+  for (int j = 0; j < NT; ++j)
+#pragma unroll
+    for (int e = 0; e < 4; ++e) o[j][e] = 0.f;
+  for (int k0 = 0; k0 < T; k0 += kFlashRows) {
+    __syncthreads();  // every warp is done with the previous K, V and P
+    flash_tile_load<C / 8>(sK, base + static_cast<size_t>(k0) * 3 * C + C, 3 * C, T - k0, tid);
+    flash_tile_load<CO / 8>(sV, base + static_cast<size_t>(k0) * 3 * C + 2 * C + co0, 3 * C, T - k0, tid);
+    flash_wait_sync();
+    if (warp < 4) {
+      float s[8][4];
+      attn_rows_dot_rows<C>(s, sQ, sK, r0, lane);
+      float x0 = -INFINITY, x1 = -INFINITY;
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        const bool ok0 = k0 + 8 * j + 2 * tq < T, ok1 = k0 + 8 * j + 2 * tq + 1 < T;
+        s[j][0] = ok0 ? s[j][0] * scale2 : -INFINITY;
+        s[j][1] = ok1 ? s[j][1] * scale2 : -INFINITY;
+        s[j][2] = ok0 ? s[j][2] * scale2 : -INFINITY;
+        s[j][3] = ok1 ? s[j][3] * scale2 : -INFINITY;
+        x0 = fmaxf(x0, fmaxf(s[j][0], s[j][1]));
+        x1 = fmaxf(x1, fmaxf(s[j][2], s[j][3]));
+      }
+      const float n0 = fmaxf(m0, quad_max(x0)), n1 = fmaxf(m1, quad_max(x1));
+      const float a0 = expf(m0 - n0), a1 = expf(m1 - n1);  // 0 on the first block (m = -inf)
+      float p0 = 0.f, p1 = 0.f;
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        s[j][0] = expf(s[j][0] - n0);
+        s[j][1] = expf(s[j][1] - n0);
+        s[j][2] = expf(s[j][2] - n1);
+        s[j][3] = expf(s[j][3] - n1);
+        p0 += s[j][0] + s[j][1];
+        p1 += s[j][2] + s[j][3];
+      }
+      l0 = l0 * a0 + quad_sum(p0);
+      l1 = l1 * a1 + quad_sum(p1);
+      m0 = n0;
+      m1 = n1;
+      flash_store_tile(sP, s, r0, lane);
+      if (tq == 0) {
+        s_alpha[r0 + g] = a0;
+        s_alpha[r0 + g + 8] = a1;
+      }
+    }
+    __syncthreads();
+    const float a0 = s_alpha[r0 + g], a1 = s_alpha[r0 + g + 8];
+#pragma unroll
+    for (int j = 0; j < NT; ++j) {
+      o[j][0] *= a0;
+      o[j][1] *= a0;
+      o[j][2] *= a1;
+      o[j][3] *= a1;
+    }
+    flash_tile_mma<NT>(o, sP, sV, PV, r0, cbase, lane);
+  }
+  if (warp < 4 && tq == 0) {
+    s_l[r0 + g] = l0;
+    s_l[r0 + g + 8] = l1;
+  }
+  __syncthreads();
+  const float i0 = 1.0f / s_l[r0 + g], i1 = 1.0f / s_l[r0 + g + 8];
+  const int row0 = q0 + r0 + g, row1 = row0 + 8;
+#pragma unroll
+  for (int j = 0; j < NT; ++j) {
+    const int col = co0 + cbase + 8 * j + 2 * tq;
+    const size_t w = static_cast<size_t>(blockIdx.z) * T;
+    if (row0 < T) *reinterpret_cast<uint32_t*>(out + (w + row0) * C + col) = pack_bf16x2(o[j][0] * i0, o[j][1] * i0);
+    if (row1 < T) *reinterpret_cast<uint32_t*>(out + (w + row1) * C + col) = pack_bf16x2(o[j][2] * i1, o[j][3] * i1);
+  }
+}
+
+// K8t-a (DQ = false), grid (query blocks, 1, windows): stats[0][w][t] = L = log-sum-exp of query t's scaled scores,
+// stats[1][w][t] = D = sum_s P gP.  K8t-b (DQ = true), grid (query blocks, C / CO, windows): gq for CO channels.
+template <int C, bool DQ>
+__global__ void __launch_bounds__(256) attention_flash_bwd_q_kernel(const bf16* __restrict__ qkv,
+                                                                    const bf16* __restrict__ go,
+                                                                    float* __restrict__ stats,
+                                                                    bf16* __restrict__ gqkv, int T, int n,
+                                                                    float scale2) {
+  constexpr int CO = attention_flash_co(C), PQ = C * 2, PC = CO * 2, NT = CO / 16;
+  extern __shared__ __align__(128) uint8_t smraw[];
+  const uint32_t sQ = static_cast<uint32_t>(__cvta_generic_to_shared(smraw));
+  const uint32_t sG = sQ + kFlashRows * PQ, sX = sG + kFlashRows * PQ, sKc = sX + kFlashRows * PQ;
+  const uint32_t sS = sKc + kFlashRows * PC;
+  float* s_L = reinterpret_cast<float*>(smraw + 3 * kFlashRows * PQ + kFlashRows * PC + kFlashRows * 128);
+  float* s_D = s_L + kFlashRows;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, tq = lane & 3;
+  const int q0 = blockIdx.x * kFlashRows, co0 = blockIdx.y * CO;
+  const size_t w = blockIdx.z;
+  const bf16* base = qkv + w * T * 3 * C;
+  const int r0 = 16 * (warp & 3), cbase = (warp >> 2) * (CO / 2);
+  flash_tile_load<C / 8>(sQ, base + static_cast<size_t>(q0) * 3 * C, 3 * C, T - q0, tid);
+  flash_tile_load<C / 8>(sG, go + (w * T + q0) * C, C, T - q0, tid);
+  if (DQ && tid < kFlashRows) {
+    const bool ok = q0 + tid < T;
+    s_L[tid] = ok ? stats[w * T + q0 + tid] : INFINITY;
+    s_D[tid] = ok ? stats[(n + w) * T + q0 + tid] : 0.f;
+  }
+  float m0 = -INFINITY, m1 = -INFINITY, l0 = 0.f, l1 = 0.f, d0 = 0.f, d1 = 0.f;  // K8t-a: online L and D
+  float dq[NT][4];
+#pragma unroll
+  for (int j = 0; j < NT; ++j)
+#pragma unroll
+    for (int e = 0; e < 4; ++e) dq[j][e] = 0.f;
+  for (int k0 = 0; k0 < T; k0 += kFlashRows) {
+    __syncthreads();
+    flash_tile_load<C / 8>(sX, base + static_cast<size_t>(k0) * 3 * C + C, 3 * C, T - k0, tid);  // k
+    if (DQ) flash_tile_load<CO / 8>(sKc, base + static_cast<size_t>(k0) * 3 * C + C + co0, 3 * C, T - k0, tid);
+    flash_wait_sync();
+    float p[8][4];
+    if (warp < 4) {
+      attn_rows_dot_rows<C>(p, sQ, sX, r0, lane);
+      if (DQ) {
+        const float L0 = s_L[r0 + g], L1 = s_L[r0 + g + 8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          const bool ok0 = k0 + 8 * j + 2 * tq < T, ok1 = k0 + 8 * j + 2 * tq + 1 < T;
+          p[j][0] = ok0 ? expf(p[j][0] * scale2 - L0) : 0.f;
+          p[j][1] = ok1 ? expf(p[j][1] * scale2 - L0) : 0.f;
+          p[j][2] = ok0 ? expf(p[j][2] * scale2 - L1) : 0.f;
+          p[j][3] = ok1 ? expf(p[j][3] * scale2 - L1) : 0.f;
+        }
+      } else {  // unnormalised exp(s - running max); D is rescaled with the sum
+        float x0 = -INFINITY, x1 = -INFINITY;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          const bool ok0 = k0 + 8 * j + 2 * tq < T, ok1 = k0 + 8 * j + 2 * tq + 1 < T;
+          p[j][0] = ok0 ? p[j][0] * scale2 : -INFINITY;
+          p[j][1] = ok1 ? p[j][1] * scale2 : -INFINITY;
+          p[j][2] = ok0 ? p[j][2] * scale2 : -INFINITY;
+          p[j][3] = ok1 ? p[j][3] * scale2 : -INFINITY;
+          x0 = fmaxf(x0, fmaxf(p[j][0], p[j][1]));
+          x1 = fmaxf(x1, fmaxf(p[j][2], p[j][3]));
+        }
+        const float n0 = fmaxf(m0, quad_max(x0)), n1 = fmaxf(m1, quad_max(x1));
+        const float a0 = expf(m0 - n0), a1 = expf(m1 - n1);
+        float s0 = 0.f, s1 = 0.f;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          p[j][0] = expf(p[j][0] - n0);
+          p[j][1] = expf(p[j][1] - n0);
+          p[j][2] = expf(p[j][2] - n1);
+          p[j][3] = expf(p[j][3] - n1);
+          s0 += p[j][0] + p[j][1];
+          s1 += p[j][2] + p[j][3];
+        }
+        l0 = l0 * a0 + quad_sum(s0);
+        l1 = l1 * a1 + quad_sum(s1);
+        d0 *= a0;
+        d1 *= a1;
+        m0 = n0;
+        m1 = n1;
+      }
+    }
+    __syncthreads();  // every warp is done with k
+    flash_tile_load<C / 8>(sX, base + static_cast<size_t>(k0) * 3 * C + 2 * C, 3 * C, T - k0, tid);  // v
+    flash_wait_sync();
+    if (warp < 4) {
+      float gp[8][4];
+      attn_rows_dot_rows<C>(gp, sG, sX, r0, lane);  // gP = go v^T
+      if (DQ) {
+        const float D0 = s_D[r0 + g], D1 = s_D[r0 + g + 8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          p[j][0] = scale2 * p[j][0] * (gp[j][0] - D0);
+          p[j][1] = scale2 * p[j][1] * (gp[j][1] - D0);
+          p[j][2] = scale2 * p[j][2] * (gp[j][2] - D1);
+          p[j][3] = scale2 * p[j][3] * (gp[j][3] - D1);
+        }
+        flash_store_tile(sS, p, r0, lane);
+      } else {
+        float e0 = 0.f, e1 = 0.f;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          e0 += p[j][0] * gp[j][0] + p[j][1] * gp[j][1];
+          e1 += p[j][2] * gp[j][2] + p[j][3] * gp[j][3];
+        }
+        d0 += quad_sum(e0);
+        d1 += quad_sum(e1);
+      }
+    }
+    if (DQ) {
+      __syncthreads();
+      flash_tile_mma<NT>(dq, sS, sKc, PC, r0, cbase, lane);  // gq += scale2 gS k
+    }
+  }
+  const int row0 = q0 + r0 + g, row1 = row0 + 8;
+  if (!DQ) {
+    if (warp < 4 && tq == 0) {
+      if (row0 < T) {
+        stats[w * T + row0] = m0 + logf(l0);
+        stats[(n + w) * T + row0] = d0 / l0;
+      }
+      if (row1 < T) {
+        stats[w * T + row1] = m1 + logf(l1);
+        stats[(n + w) * T + row1] = d1 / l1;
+      }
+    }
+    return;
+  }
+#pragma unroll
+  for (int j = 0; j < NT; ++j) {
+    const int col = co0 + cbase + 8 * j + 2 * tq;
+    if (row0 < T) *reinterpret_cast<uint32_t*>(gqkv + (w * T + row0) * 3 * C + col) = pack_bf16x2(dq[j][0], dq[j][1]);
+    if (row1 < T) *reinterpret_cast<uint32_t*>(gqkv + (w * T + row1) * 3 * C + col) = pack_bf16x2(dq[j][2], dq[j][3]);
+  }
+}
+
+// K8t-c, grid (key blocks, C / CO, windows): gk = scale2 gS^T q and gv = P^T go for CO channels of 64 keys, summed
+// over the query blocks in order.  P^T and gS^T are computed key-major (A = the key block's k / v rows).
+template <int C>
+__global__ void __launch_bounds__(256) attention_flash_bwd_kv_kernel(const bf16* __restrict__ qkv,
+                                                                     const bf16* __restrict__ go,
+                                                                     const float* __restrict__ stats,
+                                                                     bf16* __restrict__ gqkv, int T, int n,
+                                                                     float scale2) {
+  constexpr int CO = attention_flash_co(C), PQ = C * 2, PC = CO * 2, NT = CO / 16;
+  extern __shared__ __align__(128) uint8_t smraw[];
+  const uint32_t sK = static_cast<uint32_t>(__cvta_generic_to_shared(smraw));
+  const uint32_t sV = sK + kFlashRows * PQ, sX = sV + kFlashRows * PQ, sQc = sX + kFlashRows * PQ;
+  const uint32_t sP = sQc + kFlashRows * PC, sS = sP + kFlashRows * 128;
+  float* s_L = reinterpret_cast<float*>(smraw + 3 * kFlashRows * PQ + kFlashRows * PC + 2 * kFlashRows * 128);
+  float* s_D = s_L + kFlashRows;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, tq = lane & 3, g = lane >> 2;
+  const int k0 = blockIdx.x * kFlashRows, co0 = blockIdx.y * CO;
+  const size_t w = blockIdx.z;
+  const bf16* base = qkv + w * T * 3 * C;
+  const int r0 = 16 * (warp & 3), cbase = (warp >> 2) * (CO / 2);
+  flash_tile_load<C / 8>(sK, base + static_cast<size_t>(k0) * 3 * C + C, 3 * C, T - k0, tid);
+  flash_tile_load<C / 8>(sV, base + static_cast<size_t>(k0) * 3 * C + 2 * C, 3 * C, T - k0, tid);
+  float dk[NT][4], dv[NT][4];
+#pragma unroll
+  for (int j = 0; j < NT; ++j)
+#pragma unroll
+    for (int e = 0; e < 4; ++e) dk[j][e] = dv[j][e] = 0.f;
+  for (int q0 = 0; q0 < T; q0 += kFlashRows) {
+    __syncthreads();  // every warp is done with the previous go, q chunk and tiles
+    flash_tile_load<C / 8>(sX, base + static_cast<size_t>(q0) * 3 * C, 3 * C, T - q0, tid);  // q
+    flash_tile_load<CO / 8>(sQc, base + static_cast<size_t>(q0) * 3 * C + co0, 3 * C, T - q0, tid);
+    if (tid < kFlashRows) {
+      const bool ok = q0 + tid < T;
+      s_L[tid] = ok ? stats[w * T + q0 + tid] : INFINITY;
+      s_D[tid] = ok ? stats[(n + w) * T + q0 + tid] : 0.f;
+    }
+    flash_wait_sync();
+    float p[8][4];  // P^T[key r0 + g (+8)][query 8 j + 2 tq (+1)]
+    if (warp < 4) {
+      attn_rows_dot_rows<C>(p, sK, sX, r0, lane);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        const float La = s_L[8 * j + 2 * tq], Lb = s_L[8 * j + 2 * tq + 1];
+        p[j][0] = expf(p[j][0] * scale2 - La);
+        p[j][1] = expf(p[j][1] * scale2 - Lb);
+        p[j][2] = expf(p[j][2] * scale2 - La);
+        p[j][3] = expf(p[j][3] * scale2 - Lb);
+      }
+    }
+    __syncthreads();  // every warp is done with q
+    flash_tile_load<C / 8>(sX, go + (w * T + q0) * C, C, T - q0, tid);
+    flash_wait_sync();
+    if (warp < 4) {
+      float gp[8][4];
+      attn_rows_dot_rows<C>(gp, sV, sX, r0, lane);  // gP^T = v go^T
+      flash_store_tile(sP, p, r0, lane);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        const float Da = s_D[8 * j + 2 * tq], Db = s_D[8 * j + 2 * tq + 1];
+        gp[j][0] = scale2 * p[j][0] * (gp[j][0] - Da);
+        gp[j][1] = scale2 * p[j][1] * (gp[j][1] - Db);
+        gp[j][2] = scale2 * p[j][2] * (gp[j][2] - Da);
+        gp[j][3] = scale2 * p[j][3] * (gp[j][3] - Db);
+      }
+      flash_store_tile(sS, gp, r0, lane);
+    }
+    __syncthreads();
+    flash_tile_mma<NT>(dv, sP, sX, PQ, r0, co0 + cbase, lane);  // gv += P^T go
+    flash_tile_mma<NT>(dk, sS, sQc, PC, r0, cbase, lane);       // gk += scale2 gS^T q
+  }
+  const int row0 = k0 + r0 + g, row1 = row0 + 8;
+#pragma unroll
+  for (int j = 0; j < NT; ++j) {
+    const int col = co0 + cbase + 8 * j + 2 * tq;
+    bf16* o0 = gqkv + (w * T + row0) * 3 * C + col;
+    bf16* o1 = gqkv + (w * T + row1) * 3 * C + col;
+    if (row0 < T) {
+      *reinterpret_cast<uint32_t*>(o0 + C) = pack_bf16x2(dk[j][0], dk[j][1]);
+      *reinterpret_cast<uint32_t*>(o0 + 2 * C) = pack_bf16x2(dv[j][0], dv[j][1]);
+    }
+    if (row1 < T) {
+      *reinterpret_cast<uint32_t*>(o1 + C) = pack_bf16x2(dk[j][2], dk[j][3]);
+      *reinterpret_cast<uint32_t*>(o1 + 2 * C) = pack_bf16x2(dv[j][2], dv[j][3]);
+    }
+  }
+}
+
 // ------------------------------------------------------------------------------------------------ VJP kernels
 // Backward of the channel LayerNorm (model/nn.py:154,183; zuko LayerNorm, unbiased variance):
 //   g_v = inv * (g_y - mean_C(g_y) - y * sum_C(g_y y) / (C - 1)),   out = gres + g_v

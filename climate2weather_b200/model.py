@@ -287,6 +287,11 @@ class ScoreUNet(nn.Module):
     Arguments mirror model/score.py:46 and model/nn.py:108-121.  Supported: kernel_size=3, stride=2, spatial=2,
     SiLU activation, zero padding, forcing_dim=0 — i.e. configs/sda_unet.yml with train.py:164-173 — with any
     hidden_channels (multiples of 64, <= 512), hidden_blocks and attention_levels.
+
+    Geometry: every level l (H_l x W_l, halved from the patch per level) must have W_l >= 8 and either W_l a power
+    of two <= 128 whose rows tile into 128-pixel row blocks, or W_l a multiple of 128 (e.g. 128 x 256, 256 x 256,
+    512 x 512); H_l and W_l are even below the last level.  Other widths (96, 160, 192, ...) are refused when the
+    engine is created.
     """
 
     DEFAULT_MAX_WINDOWS = 16

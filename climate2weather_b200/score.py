@@ -243,7 +243,20 @@ def combined_strip_rows(H: int, W: int, s: int) -> int:
 def point_strip_rows(H: int, W: int) -> int:
     """Rows per CTA of the point-guidance kernel: the strip's pixel -> entry map fits C2W_POINT_STRIP_PIX ints of static
     shared memory (c2w_b200.h) — 16 rows, 8 KB at 128 x 128."""
+    if W > POINT_STRIP_PIX:
+        raise NotImplementedError(f"PointObservation: a row of {W} pixels exceeds the {POINT_STRIP_PIX} pixels the point "
+                                  "guidance kernel maps per strip")
     return max(1, min(H, POINT_STRIP_PIX // W))
+
+
+def guidance_tile(H: int, W: int) -> int:
+    """Tile side of the guidance and corrector kernels' per-CTA partial sums: divides H and W with at most 32 tiles per
+    row (16 at 128 x 128 and 256 x 256).  Patches with no such side (e.g. 16 x 1024) are refused before device work."""
+    for s in (16, 8, 32, 4, 64, 2, 128, 1):
+        if H % s == 0 and W % s == 0 and W // s <= 32:
+            return s
+    raise NotImplementedError(f"guided sampling on a {H} x {W} patch: no tile side s dividing H and W with W / s <= 32 "
+                              "(the guidance kernels' per-CTA partial sums)")
 
 
 POINT_STRIP_PIX = 2048  # C2W_POINT_STRIP_PIX
@@ -665,6 +678,7 @@ class _Runtime:
         self._engine_epoch = None
         self._sel = None          # exact_grad: cached selection of those windows (per conditioning)
         self._rest = None         # exact_grad: the other local windows (int32 device list)
+        self.s_tile = guidance_tile(H, W)  # refuses a patch the guidance kernels cannot tile, before device work
         self.refresh_engine()
         f32 = dict(dtype=torch.float32, device=device)
         self.x = torch.zeros(self.n_frames, H, W, C, **f32)
@@ -676,7 +690,6 @@ class _Runtime:
         self.sumsq = torch.zeros(max(1, self.members), dtype=torch.float64, device=device)  # one per member
         self.partials: Optional[Tensor] = None
         self.cond = None
-        self.s_tile = next(s for s in (16, 8, 32, 4, 64, 2, 128, 1) if H % s == 0 and W % s == 0 and W // s <= 32)
         self._peer_halo: Optional[PeerHalo] = None
         self._peer_halo_ok = True
         self._halo_pushed = False  # the last update kernel already stored the boundary frames into the neighbours' mailboxes

@@ -75,6 +75,10 @@ typedef struct c2w_guide {
 } c2w_guide;
 
 /* ---- lifecycle ------------------------------------------------------------------------------------------ */
+/* Geometry: every level l (H_l x W_l, halved from height x width per level) must have W_l >= 8 and either W_l a
+ * power of two <= 128 whose rows tile into 128-pixel row blocks, or W_l a multiple of 128; H_l and W_l are even below
+ * the last level.  c2w_create refuses any other geometry with a message naming the level, its H x W and this rule,
+ * before it looks for a device. */
 int c2w_create(const c2w_config* cfg, c2w_handle** out);
 void c2w_destroy(c2w_handle* h);
 const char* c2w_last_error(void);
@@ -343,7 +347,11 @@ int c2w_op_layernorm(const void* x_bf16, const float* mod, void* out_bf16, int64
                      int upsample, void* stream);
 int c2w_op_attention(const void* qkv_bf16, void* out_bf16, int n, int T, int C, void* stream);
 /* backward kernels of the VJP path: LayerNorm forward with its 1/std stash, LayerNorm backward (down: the forward
- * output was 2x nearest-upsampled, gy is [n, 2H, 2W, C]), attention-core backward (scratch: 2*n*T*T floats) */
+ * output was 2x nearest-upsampled, gy is [n, 2H, 2W, C]), attention-core backward (scratch: 2*n*T*T floats; the
+ * tiled kernels, which run where K and V of a window do not fit in shared memory, use the first 2*n*T of them).
+ * c2w_op_attention runs those tiled kernels for any T where K, V and the scores of 64 queries exceed shared memory,
+ * whatever n is.  Every shape a network plan admitted before keeps its kernel and bits; a direct call with few windows
+ * that used to fit with 16 or 32 queries per CTA (e.g. T = 128 at C = 384) now takes the tiled kernel. */
 int c2w_op_layernorm_inv(const void* x_bf16, const float* mod, void* out_bf16, float* inv, int64_t npix, int C,
                          void* stream);
 int c2w_op_layernorm_bwd(const void* gy_bf16, const void* y_bf16, const float* inv, const void* gres_bf16,
